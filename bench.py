@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            (N > 1: launched by torchrun, one rank/GPU)
   python bench.py --impl reference --gpus N --steps K --warmup W
+  python bench.py ... --dump-outputs DIR       (+ the last timed step's outputs as DIR/<name>.npy)
 
 One "step" = one full policy update on one synthetic batch of the named workload:
 value-net forward (NnVf.predict) -> GAE + standardise (compute_advantage, core.py:63-105) ->
@@ -60,7 +61,24 @@ def parse():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--nccl-only", action="store_true", help="sum over ranks with NCCL instead of the NVLink peer-memory exchange")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy "
+                         "(float32 / float64; the inputs are seeded, so two builds can be compared array by array)")
     return ap.parse_args()
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: one DIR/<name>.npy per array, integers widened to float64, at most DUMP_LIMIT_BYTES in all."""
+    arrays = {k: np.asarray(v, np.float32 if np.asarray(v).dtype == np.float32 else np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def workload_desc(wl, n_total):
@@ -475,6 +493,11 @@ def run_extra(args):
         return e0.elapsed_time(e1), int(lib.mrl_launch_count() - l0), res, evals[0] / steps
     sampler.start()
     ms, launches, res, n_eval = timed(step_resident, args.steps, max(args.warmup, 3))
+    if args.dump_outputs:
+        if ppo:
+            dump_outputs(args.dump_outputs, {"losses_before": res[0], "losses_after": res[1], "theta": net.get_params()})
+        else:
+            dump_outputs(args.dump_outputs, {"vf_losses": res, "vf_theta": vf.get_params()})
     pms, _, _, _ = timed(step_resident, args.steps, 1, profile=True)
     clocks = sampler.stop()
     kernels = kernel_table(lib, args.steps)
@@ -578,6 +601,8 @@ def main():
     world = int(os.environ.get("WORLD_SIZE", 1))
     local_rank = int(os.environ.get("LOCAL_RANK", 0))
     if args.impl == "reference":
+        if args.dump_outputs:
+            raise SystemExit("--dump-outputs: b200 arm only (the reference arm sizes its sample from a timing, so its inputs vary)")
         run_reference(args, wl, n_total, rank, world)
         return
 
@@ -707,6 +732,8 @@ def main():
     nv0 = nvlink_kib(local_rank) if (rank == 0 and world > 1) else None
     ms, launches, (stats, info) = timed(step_resident, args.steps, max(args.warmup, 3))
     nv1 = nvlink_kib(local_rank) if (rank == 0 and world > 1) else None
+    if args.dump_outputs and rank == 0:         # the parameters are replicated: rank 0's are everyone's
+        dump_outputs(args.dump_outputs, {"trpo_stats": stats, "trpo_info": list(info.values()), "theta": net.get_params()})
     nvlink = None
     if nv0 and nv1:
         nsteps = args.steps + max(args.warmup, 3)

@@ -138,12 +138,12 @@ def test_discount_and_filter_batch(golden):
     assert np.allclose(a.rs.mean, b.rs.mean, rtol=1e-13) and np.allclose(a.rs.var, b.rs.var, rtol=1e-12)
 
 
-def test_run_pg_cartpole_learns():
+def test_run_pg_cartpole_learns(tmp_path):
     """BASELINE config 1: CartPole-v0 TrpoAgent through run_pg.py's own flags; a functional check
     (mean episode reward rises), not a throughput number."""
     cmd = [sys.executable, os.path.join(ROOT, "run_pg.py"), "--env", "CartPole-v0", "--agent",
            "modular_rl.agentzoo.TrpoAgent", "--n_iter", "12", "--timesteps_per_batch", "2000", "--seed", "0",
-           "--cg_damping", "0.1", "--lam", "0.97", "--outfile", "/tmp/mrl_test_a.h5"]
+           "--cg_damping", "0.1", "--lam", "0.97", "--outfile", str(tmp_path / "a.h5")]
     out = subprocess.run(cmd, capture_output=True, text=True, timeout=900, cwd=ROOT)
     assert out.returncode == 0, out.stderr[-2000:]
     rews = [float(ln.split()[-1]) for ln in out.stdout.splitlines() if ln.startswith("EpRewMean")]
@@ -153,23 +153,24 @@ def test_run_pg_cartpole_learns():
     assert all(0 < k < 0.03 for k in kls), kls
 
 
-def test_coverage_smoke_pendulum():
+def test_coverage_smoke_pendulum(tmp_path):
     """coverage.sh:7 of the reference: one TRPO iteration on Pendulum with tiny settings."""
+    outfile = str(tmp_path / "b.h5")
     cmd = [sys.executable, os.path.join(ROOT, "run_pg.py"), "--snapshot_every=20", "--n_iter=1", "--cg_damping=0.1",
            "--timesteps_per_batch=5", "--lam=0.97", "--agent=modular_rl.agentzoo.TrpoAgent", "--max_kl=0.01",
-           "--env=Pendulum", "--gamma=0.98", "--hid_sizes=10,5", "--outfile", "/tmp/mrl_test_b.h5"]
+           "--env=Pendulum", "--gamma=0.98", "--hid_sizes=10,5", "--outfile", outfile]
     out = subprocess.run(cmd, capture_output=True, text=True, timeout=600, cwd=ROOT)
     assert out.returncode == 0, out.stderr[-2000:]
     assert "pol_surr_after" in out.stdout and "vf_EV_after" in out.stdout
     # --snapshot_every: the pickled agent lands next to the results (the reference stores the same bytes in
     # its hdf5 file, run_pg.py:141-142) and --load_snapshot resumes from it
-    snap = "/tmp/mrl_test_b.h5.dir/agent_snapshots/0001.pkl"
+    snap = outfile + ".dir/agent_snapshots/0001.pkl"
     assert os.path.exists(snap)
     from modular_rl_b200.misc_utils import load_agent_snapshot
     agent = load_agent_snapshot(snap)
     assert type(agent).__name__ == "TrpoAgent" and agent.policy.dims == [3, 10, 5, 1]
     # same --outfile: the snapshot is read before the previous run's results directory is cleared
-    out = subprocess.run(cmd + ["--load_snapshot", "/tmp/mrl_test_b.h5.dir"], capture_output=True, text=True,
+    out = subprocess.run(cmd + ["--load_snapshot", outfile + ".dir"], capture_output=True, text=True,
                          timeout=600, cwd=ROOT)
     assert out.returncode == 0, out.stderr[-2000:]
     assert "pol_surr_after" in out.stdout
@@ -274,14 +275,15 @@ def test_deterministic_agent_and_cem(kind):
         assert max(i["ymean"] for i in infos[1:]) > infos[0]["ymean"]
 
 
-def test_run_cem_cli():
+def test_run_cem_cli(tmp_path):
+    outfile = str(tmp_path / "cem.h5")
     cmd = [sys.executable, os.path.join(ROOT, "run_cem.py"), "--env=CartPole-v0",
            "--agent=modular_rl.agentzoo.DeterministicAgent", "--n_iter=2", "--batch_size=10", "--hid_sizes=8",
-           "--snapshot_every=2", "--outfile", "/tmp/mrl_test_cem.h5"]
+           "--snapshot_every=2", "--outfile", outfile]
     out = subprocess.run(cmd, capture_output=True, text=True, timeout=600, cwd=ROOT)
     assert out.returncode == 0, out.stderr[-2000:]
     assert "Iteration 1" in out.stdout and "ymean" in out.stdout
-    assert os.path.exists("/tmp/mrl_test_cem.h5.dir/agent_snapshots/0002.pkl")
+    assert os.path.exists(outfile + ".dir/agent_snapshots/0002.pkl")
 
 
 def test_multi_gpu_parity_two_ranks():
