@@ -2,6 +2,7 @@
 agentzoo.py API unchanged (TrpoAgent, PpoLbfgsAgent, the option tables and therefore the run_pg.py
 flags), built on device-resident networks instead of Keras models."""
 from . import _lib as L
+from . import parallel
 from .core import (Categorical, DiagGauss, NnVf, PG_OPTIONS, StochPolicyMLP, make_value_net)
 from .filters import ZFilter
 from .misc_utils import IDENTITY, comma_sep_ints, update_default_config
@@ -151,6 +152,8 @@ class PpoLbfgsAgent(AgentWithPolicy):
 
     def __init__(self, ob_space, ac_space, usercfg):
         cfg = update_default_config(self.options, usercfg)
+        if cfg["do_split"]:
+            parallel.reject_data_parallel("PpoLbfgsAgent with do_split=1")
         policy, self.baseline = make_mlps(ob_space, ac_space, cfg)
         obfilter, rewfilter = make_filters(cfg, ob_space)
         self.updater = PpoLbfgsUpdater(policy, cfg)
@@ -161,6 +164,7 @@ class PpoSgdAgent(AgentWithPolicy):
     options = MLP_OPTIONS + PG_OPTIONS + PpoSgdUpdater.options + FILTER_OPTIONS
 
     def __init__(self, ob_space, ac_space, usercfg):
+        parallel.reject_data_parallel("PpoSgdAgent")
         cfg = update_default_config(self.options, usercfg)
         policy, self.baseline = make_mlps(ob_space, ac_space, cfg)
         obfilter, rewfilter = make_filters(cfg, ob_space)

@@ -23,6 +23,7 @@ import scipy.optimize
 
 from . import _lib as L
 from . import distributions
+from . import parallel
 from .device import DeviceBatch, DeviceNet
 from .misc_utils import *  # noqa: F401,F403  (the reference star-imports misc_utils too)
 from .misc_utils import EzPickle, explained_variance, explained_variance_2d, update_default_config
@@ -45,15 +46,25 @@ def get_agent_cls(name):
 # Stats
 # ================================================================
 
-def add_episode_stats(stats, paths):
+def episode_arrays(paths):
+    """-> (total reward, length) of every path."""
     reward_key = "reward_raw" if "reward_raw" in paths[0] else "reward"
     episoderewards = np.array([path[reward_key].sum() for path in paths])
     pathlengths = np.array([pathlength(path) for path in paths])
+    return episoderewards, pathlengths
+
+
+def add_episode_stats(stats, paths):
+    add_episode_arrays(stats, *episode_arrays(paths))
+
+
+def add_episode_arrays(stats, episoderewards, pathlengths):
+    """add_episode_stats from the per-episode arrays (data-parallel training gathers these, not the paths)."""
     stats["EpisodeRewards"] = episoderewards
     stats["EpisodeLengths"] = pathlengths
     stats["NumEpBatch"] = len(episoderewards)
     stats["EpRewMean"] = episoderewards.mean()
-    stats["EpRewSEM"] = episoderewards.std() / np.sqrt(len(paths))
+    stats["EpRewSEM"] = episoderewards.std() / np.sqrt(len(episoderewards))
     stats["EpRewMax"] = episoderewards.max()
     stats["EpLenMean"] = pathlengths.mean()
     stats["EpLenMax"] = pathlengths.max()
@@ -115,8 +126,14 @@ _batch_cache = _BatchCache()
 
 
 def batch_for_paths(paths, timestep_limit=1.0):
-    """-> (DeviceBatch with observations + trajectory structure bound, offsets int64[n_paths+1])"""
-    return _batch_cache.get(paths, None if timestep_limit is None else (timestep_limit if timestep_limit else 1.0))
+    """-> (DeviceBatch with observations + trajectory structure bound, offsets int64[n_paths+1]).  For this rank's
+    paths of a data-parallel iteration the batch is told the timestep count of all ranks (the device sums divide
+    by it)."""
+    batch, offsets = _batch_cache.get(paths, None if timestep_limit is None else (timestep_limit if timestep_limit else 1.0))
+    n_total = parallel.global_timesteps(paths)
+    if n_total is not None:
+        batch.set_global_n(n_total)
+    return batch, offsets
 
 
 def _split(flat, offsets):
@@ -139,7 +156,8 @@ def compute_advantage(vf, paths, gamma, lam):
     else:                                                    # any Baseline with predict(path)
         base = concat([np.asarray(vf.predict(path)) for path in paths])
     reward = concat([np.asarray(path["reward"], np.float64) for path in paths])
-    ret, adv = batch.gae(reward, base, gamma, lam, standardize=True)
+    comm = parallel.context().comm if parallel.global_timesteps(paths) is not None else None
+    ret, adv = batch.gae(reward, base, gamma, lam, standardize=True, comm=comm)   # comm: moments of all ranks
     for path, r, b, a in zip(paths, _split(ret, offsets), _split(base, offsets), _split(adv, offsets)):
         path["return"] = r
         path["baseline"] = b
@@ -165,14 +183,24 @@ def run_policy_gradient_algorithm(env, agent, usercfg=None, callback=None):
     if cfg["parallel"]:
         raise NotImplementedError
     tstart = time.time()
-    seed_iter = itertools.count()
+    # data-parallel training (parallel.init_data_parallel ran): each rank collects its share of the trajectories,
+    # the filters and episode statistics are merged over ranks, the updates sum over ranks inside the library
+    dp = parallel.context() is not None
+    if dp:
+        parallel.attach_agent(agent)
+    seed_iter = parallel.seed_stream()           # itertools.count() in one process
     for _ in range(cfg["n_iter"]):
+        starts = parallel.begin_rollouts(agent) if dp else None
         paths = get_paths(env, agent, cfg, seed_iter)
+        episodes = parallel.sync_rollouts(agent, paths, starts) if dp else None
         compute_advantage(agent.baseline, paths, gamma=cfg["gamma"], lam=cfg["lam"])
         vf_stats = agent.baseline.fit(paths)
         pol_stats = agent.updater(paths)
         stats = OrderedDict()
-        add_episode_stats(stats, paths)
+        if dp:
+            add_episode_arrays(stats, episodes["rewards"], episodes["lengths"])
+        else:
+            add_episode_stats(stats, paths)
         add_prefixed_stats(stats, "vf", vf_stats)
         add_prefixed_stats(stats, "pol", pol_stats)
         stats["TimeElapsed"] = time.time() - tstart
@@ -189,9 +217,12 @@ VEC_ENVS = int(os.environ.get("MRL_VEC_ENVS", "0") or 0)
 def get_paths(env, agent, cfg, seed_iter):
     if cfg["parallel"]:
         raise NotImplementedError
+    n_timesteps = cfg["timesteps_per_batch"]
+    if parallel.context() is not None:           # this rank's share of the batch
+        n_timesteps = parallel.rank_quota(n_timesteps, parallel.context().world)
     if VEC_ENVS > 1:
-        return do_rollouts_vectorized(env, agent, cfg["timestep_limit"], cfg["timesteps_per_batch"], seed_iter, VEC_ENVS)
-    return do_rollouts_serial(env, agent, cfg["timestep_limit"], cfg["timesteps_per_batch"], seed_iter)
+        return do_rollouts_vectorized(env, agent, cfg["timestep_limit"], n_timesteps, seed_iter, VEC_ENVS)
+    return do_rollouts_serial(env, agent, cfg["timestep_limit"], n_timesteps, seed_iter)
 
 
 def _filter_block(filt, X):
@@ -597,12 +628,17 @@ class NnRegression(object):
         ypredold_ny = self.predict(x_nx)                     # leaves x bound in self._xbatch
         return self._fit_bound(self._xbatch, np.asarray(ytarg_ny), ypredold_ny)
 
-    def _fit_bound(self, batch, ytarg_ny, ypredold_ny):
+    def _fit_bound(self, batch, ytarg_ny, ypredold_ny, across_ranks=False):
+        """across_ranks: `batch` is one rank's shard of a data-parallel batch; the loss and gradient already sum
+        over ranks, the statistics are computed from the moments of all ranks."""
         nY = ytarg_ny.shape[1]
         target = ytarg_ny * self.mixfrac + ypredold_ny * (1 - self.mixfrac)
         batch.set_vf_target(target[:, 0])
         out = self.opt.update(batch)
         yprednew_ny = self.net.forward(batch)
+        if across_ranks:
+            out.update(parallel.regression_stats(ypredold_ny, yprednew_ny, ytarg_ny))
+            return out
         out["PredStdevBefore"] = ypredold_ny.std()
         out["PredStdevAfter"] = yprednew_ny.std()
         out["TargStdev"] = ytarg_ny.std()
@@ -637,7 +673,7 @@ class NnVf(Baseline):
         batch, _ = batch_for_paths(paths, self.timestep_limit)
         vtarg_n1 = concat([path["return"] for path in paths]).reshape(-1, 1)
         ypredold = self.reg.net.forward(batch)
-        return self.reg._fit_bound(batch, vtarg_n1, ypredold)
+        return self.reg._fit_bound(batch, vtarg_n1, ypredold, parallel.global_timesteps(paths) is not None)
 
 
 def make_value_net(ob_dim, hid_sizes, activation="tanh"):

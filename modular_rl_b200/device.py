@@ -9,6 +9,7 @@ from typing import Optional, Sequence
 import numpy as np
 
 from . import _lib as L
+from . import parallel
 
 _F = (np.dtype(np.float32), np.dtype(np.float64))
 
@@ -79,8 +80,16 @@ class Comm:
             self._h = C.c_void_p()
 
 
+def _snapshot_device(stored: int) -> int:
+    """Device a snapshot is rebuilt on: the loading rank's in data-parallel training, else the stored one."""
+    return parallel.current_device() if parallel.context() is not None else stored
+
+
 class DeviceBatch:
-    def __init__(self, ob_dim: int, with_time_feature: bool = True, device: int = 0):
+    def __init__(self, ob_dim: int, with_time_feature: bool = True, device: Optional[int] = None):
+        """device None: this process's device (parallel.current_device(), GPU 0 in a single-process run)."""
+        if device is None:
+            device = parallel.current_device()
         self._h = C.c_void_p()
         L.check(L.lib().mrl_batch_create(C.byref(self._h), device, int(ob_dim), int(with_time_feature)))
         self.ob_dim, self.device, self.with_time = int(ob_dim), device, bool(with_time_feature)
@@ -91,7 +100,7 @@ class DeviceBatch:
         return dict(ob_dim=self.ob_dim, with_time=self.with_time, device=self.device)
 
     def __setstate__(self, d):
-        self.__init__(d["ob_dim"], d["with_time"], d["device"])
+        self.__init__(d["ob_dim"], d["with_time"], _snapshot_device(d["device"]))
 
     def close(self):
         if getattr(self, "_h", None):
@@ -195,7 +204,9 @@ class DeviceBatch:
 
 
 class DeviceNet:
-    def __init__(self, dims: Sequence[int], head: int, activation: str = "tanh", device: int = 0):
+    def __init__(self, dims: Sequence[int], head: int, activation: str = "tanh", device: Optional[int] = None):
+        if device is None:
+            device = parallel.current_device()
         if activation not in L.ACTIVATIONS:
             raise ValueError(f"activation {activation!r} not supported (tanh, relu, sigmoid)")
         self.dims = [int(d) for d in dims]
@@ -215,7 +226,7 @@ class DeviceNet:
                     theta=self.get_params())
 
     def __setstate__(self, d):
-        self.__init__(d["dims"], d["head"], d["activation"], d["device"])
+        self.__init__(d["dims"], d["head"], d["activation"], _snapshot_device(d["device"]))
         self.set_params(d["theta"])
 
     def close(self):

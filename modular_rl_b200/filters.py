@@ -33,6 +33,8 @@ def zfilter_scan(X, state=None, demean=True, destd=True, clip=10.0, out_dtype=np
 class ZFilter(object):
     """y = (x-mean)/std using running estimates of mean,std (filters.py:17-40)."""
 
+    pushed = None       # RunningStat of the samples pushed since start_round() (data-parallel training), else None
+
     def __init__(self, shape, demean=True, destd=True, clip=10.0):
         self.demean = demean
         self.destd = destd
@@ -42,6 +44,8 @@ class ZFilter(object):
     def __call__(self, x, update=True):
         if update:
             self.rs.push(x)
+            if self.pushed is not None:
+                self.pushed.push(x)
         if self.demean:
             x = x - self.rs.mean
         if self.destd:
@@ -56,7 +60,15 @@ class ZFilter(object):
         shp = self.rs.shape
         Y, st = zfilter_scan(X.reshape(X.shape[0], -1), self.rs.state(), self.demean, self.destd, self.clip)
         self.rs.set_state(*st)
+        if self.pushed is not None:
+            _, st = zfilter_scan(X.reshape(X.shape[0], -1), self.pushed.state(), False, False, 0.0)
+            self.pushed.set_state(*st)
         return Y.reshape((X.shape[0],) + tuple(shp))
+
+    def start_round(self):
+        """Also record the samples pushed from now on in `pushed`, a state of their own: data-parallel training
+        merges every rank's samples of an iteration into one state (parallel.sync_rollouts)."""
+        self.pushed = RunningStat(self.rs.shape)
 
     def output_shape(self, input_space):
         return input_space.shape

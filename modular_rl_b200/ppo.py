@@ -16,6 +16,7 @@ import numpy as np
 import scipy.optimize
 
 from . import _lib as L
+from . import parallel
 from .core import EzFlat, concat
 from .device import DeviceBatch
 from .misc_utils import EzPickle, update_default_config, zipsame
@@ -63,6 +64,9 @@ class PpoLbfgsUpdater(EzFlat, EzPickle):
         train_stop = int(0.75 * N) if cfg["do_split"] else N
         tr, te = slice(0, train_stop), slice(train_stop, None)
         train = self._bind(self._train, ob_no[tr], action_na[tr], advantage_n[tr], prob_np[tr])
+        n_total = parallel.global_timesteps(paths)
+        if n_total is not None and not cfg["do_split"]:
+            train.set_global_n(n_total)          # this rank's shard of the batch of all ranks
         kl_cutoff = cfg["kl_target"] * 2.0
 
         thprev = self.get_params_flat().astype(np.float64)

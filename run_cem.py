@@ -15,6 +15,7 @@ import sys
 import numpy as np
 
 import modular_rl as mrl
+from modular_rl_b200 import parallel
 from modular_rl_b200.envs import make
 
 
@@ -70,6 +71,7 @@ class IterationLog(object):
 
 
 def main(argv=None):
+    parallel.reject_data_parallel("run_cem.py")
     args, agent_cls = parse_cli(sys.argv[1:] if argv is None else argv)
     env = make(args.env)
     # a snapshot may live in the results directory of the previous run: read it before that directory is cleared

@@ -4,6 +4,12 @@
 run_pg.py:79-102), with the policy update executed by the B200 library.
 
   python run_pg.py --env CartPole-v0 --agent modular_rl.agentzoo.TrpoAgent --n_iter 20 --timesteps_per_batch 5000
+
+Under torchrun (WORLD_SIZE > 1) it trains data-parallel, one process per GPU: every rank collects its share of
+--timesteps_per_batch and each update runs over the trajectories of all ranks.  Only rank 0 prints and writes
+results and snapshots.
+
+  torchrun --nproc-per-node 8 run_pg.py --env Pendulum-v0 --agent modular_rl.agentzoo.TrpoAgent --vec_envs 16 ...
 """
 import argparse
 import os
@@ -14,6 +20,7 @@ import sys
 import numpy as np
 
 from modular_rl import *  # noqa: F401,F403
+from modular_rl_b200 import parallel
 from modular_rl_b200.envs import make
 
 try:
@@ -33,14 +40,20 @@ def main():
                         help="environments stepped in lockstep with one batched device forward per step "
                              "(0: serial rollouts as the reference); not an agent option")
     args, _ = parser.parse_known_args([arg for arg in sys.argv[1:] if arg not in ('-h', '--help')])
+    dp = parallel.init_data_parallel() if parallel.launched_data_parallel() else None
+    root = parallel.is_root()
+    if not root:
+        sys.stdout = open(os.devnull, "w")          # the updaters' and the loop's lines come from rank 0 only
     env = make(args.env)
     env_spec = env.spec
     # read the snapshot before the results directory of a previous run (which may hold it) is cleared
     snapshot_agent = load_agent_snapshot(args.load_snapshot) if args.load_snapshot else None
+    parallel.barrier()                               # every rank has read it before rank 0 clears the directory
     mondir = args.outfile + ".dir"
-    if os.path.exists(mondir):
-        shutil.rmtree(mondir)
-    os.makedirs(mondir)
+    if root:
+        if os.path.exists(mondir):
+            shutil.rmtree(mondir)
+        os.makedirs(mondir)
     agent_ctor = get_agent_cls(args.agent)
     update_argument_parser(parser, agent_ctor.options)
     args = parser.parse_args()
@@ -58,7 +71,7 @@ def main():
         assert isinstance(agent, agent_ctor), "snapshot holds a %s" % type(agent).__name__
     else:
         agent = agent_ctor(env.observation_space, env.action_space, cfg)
-    if args.use_hdf:
+    if args.use_hdf and root:
         hdf, diagnostics = prepare_h5_file(args)
 
     counter = [0]
@@ -81,11 +94,13 @@ def main():
         if args.plot:
             animate_rollout(env, agent, min(500, args.timestep_limit))
 
-    run_policy_gradient_algorithm(env, agent, callback=callback, usercfg=cfg)
+    run_policy_gradient_algorithm(env, agent, callback=callback if root else None, usercfg=cfg)
 
-    if args.use_hdf:
+    if args.use_hdf and root:
         hdf['env_id'] = env_spec.id
     env.close()
+    if dp is not None:
+        parallel.shutdown_data_parallel()
 
 
 if __name__ == "__main__":
