@@ -685,8 +685,7 @@ extern "C" int mrl_net_create(mrl_net** out, int device, int n_layers, const int
   R(n->p32, P * 4); R(n->x32, P * 4); R(n->fullstep, P * 8);
   R(n->cgstate, sizeof(CgState)); R(n->scal, 32 * 8); R(n->cgscratch, CG_SCRATCH_DOUBLES * 8);
   {
-    const char* off = getenv("MRL_FVP_TC");
-    n->tc_fvp = fvp_tc_supported(n->g) && !(off && off[0] == '0');
+    n->tc_fvp = fvp_tc_supported(n->g);
     if (n->tc_fvp) {
       R(n->WC, fvp_tc_image_floats(n->g, 0) * 4);
       R(n->VC, fvp_tc_image_floats(n->g, 1) * 4);
@@ -926,10 +925,10 @@ static int pass_backward(mrl_net* n, mrl_batch* b, int mode, const double* coef_
     x.trace = n->trace.as<long long>();
     x.N = b->N; x.n_tiles = b->n_tiles; x.slab_tiles = pl.slab_tiles; x.n_slabs = pl.n_slabs;
     CKP(PK_MIDB_FVP, launch_fvp_tc(g, x, st), 1);
-  } else if (chain_bwd_shape(g, mode) != 0) CKP(mode == MRL_MODE_FVP ? PK_MIDB_FVP : PK_MIDB_GRAD, launch_chain_backward(g, a, pl.n_slabs, st), 1);
+  } else if (mode == MRL_MODE_GRAD && chain_bwd_shape(g) != 0) CKP(PK_MIDB_GRAD, launch_chain_backward(g, a, pl.n_slabs, st), 1);
   else CKP(mode == MRL_MODE_FVP ? PK_MIDB_FVP : PK_MIDB_GRAD, launch_mid_backward(g, a, pl.n_slabs, st), 1);
   CKP(PK_L1G, launch_l1_grad_tc(g, b->XG.as<float>(), (b->xdim + 127) / 128, n->DG.as<float>(), n->part1.as<float>(),
-                                pl.slab_tiles, b->n_tiles, pl.n_slabs, st, 0), 1);
+                                pl.slab_tiles, b->n_tiles, pl.n_slabs, st), 1);
   const int world = world_of(n);
   // terms that are not sums over timesteps are divided by `world` so that the sum over ranks restores them
   const double vls = (mode == MRL_MODE_FVP) ? 2.0 / world : 0.0;
@@ -938,21 +937,14 @@ static int pass_backward(mrl_net* n, mrl_batch* b, int mode, const double* coef_
   // over ranks itself (comm.h); otherwise out64 holds this rank's share and NCCL sums it
   P2pPush push;
   P2pGather gather;
-  const bool fused = p2p && !getenv("MRL_P2P_SPLIT");   // MRL_P2P_SPLIT=1: separate receiving kernel (A/B comparisons)
   if (p2p) {
     RET(mrl_comm_p2p_begin(n->comm, g.P, &push));
-    if (fused) RET(mrl_comm_p2p_pending(n->comm, &gather));
+    RET(mrl_comm_p2p_pending(n->comm, &gather));
   }
   CKP(PK_REDUCE, launch_reduce_partials(g, n->part1.as<float>(), n->partm.as<float>(), pl.n_slabs, 1.0 / (double)b->Nglobal,
                              l2c2 != 0.0 ? n->theta.as<float>() : nullptr, l2c2 / world,
-                             mode == MRL_MODE_FVP ? v_dev : nullptr, vls, (world > 1 && !fused) ? nullptr : out32,
-                             (p2p && !fused) ? nullptr : out64, p2p ? &push : nullptr, fused ? &gather : nullptr, st), 1);
-  if (p2p && !fused) {
-    prof_mark(PK_REDUCE, st, true);
-    RET(mrl_comm_p2p_finish(n->comm, g.P, out64, out32, st));
-    prof_mark(PK_REDUCE, st, false);
-    g_launches += 1;
-  }
+                             mode == MRL_MODE_FVP ? v_dev : nullptr, vls, (world > 1 && !p2p) ? nullptr : out32,
+                             out64, p2p ? &push : nullptr, p2p ? &gather : nullptr, st), 1);
   if (world > 1 && !p2p) {
     RET(mrl_comm_allreduce_f64(n->comm, out64, g.P, st));
     if (out32) {

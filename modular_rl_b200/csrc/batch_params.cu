@@ -143,7 +143,6 @@ __global__ void __launch_bounds__(RED_PX * RED_SY) reduce_partials_kernel(
   }
   if (push.world == 0) return;
   const unsigned int ticket = p2p_push_done(push);
-  if (ga.world == 0) return;            // the caller's next kernel is the receiving side (mrl_comm_p2p_finish)
   // exchange phase: the last RED_GATHER_CTAS CTAs to finish phase 1 stay, everybody else leaves
   const int total = (int)gridDim.x, stay = total < RED_GATHER_CTAS ? total : RED_GATHER_CTAS;
   const int j = (int)ticket - (total - stay);
@@ -348,9 +347,10 @@ cudaError_t launch_reduce_partials(const NetGeom& g, const float* part1, const f
   no_gather.world = 0;
   const int n_chunks = (g.P + RED_PX - 1) / RED_PX;
   int grid = n_chunks;
-  if (push && gather && gather->world != push->world) return cudaErrorInvalidValue;
+  // the kernel that pushes this rank's share also gathers the sum over ranks
+  if ((push == nullptr) != (gather == nullptr) || (push && gather->world != push->world)) return cudaErrorInvalidValue;
   reduce_partials_kernel<<<grid, dim3(RED_PX, RED_SY), 0, st>>>(g, part1, partm, n_slabs, scale, theta, l2c2, vflat, vls, out32,
-                                                             out64, push ? *push : no_push, (push && gather) ? *gather : no_gather);
+                                                             out64, push ? *push : no_push, gather ? *gather : no_gather);
   return cudaGetLastError();
 }
 

@@ -35,7 +35,7 @@ size_t l1tc_dg_floats(const NetGeom& g, long long n_tiles);
 cudaError_t launch_pack_xg(const void* src, int dtype, long long ld, int ncols, long long N, float* XG, int xg_ftiles,
                            long long n_tiles, cudaStream_t st);
 cudaError_t launch_l1_grad_tc(const NetGeom& g, const float* XG, int xg_ftiles, const float* DG, float* part1,
-                              int slab_tiles, int n_tiles, int n_slabs, cudaStream_t st, int dg_mn_major = 0);
+                              int slab_tiles, int n_tiles, int n_slabs, cudaStream_t st);
 
 // ---- mlp_mid.cu
 struct MidFwdArgs {
@@ -66,7 +66,7 @@ size_t mid_backward_smem(const NetGeom& g, int mode);
 cudaError_t launch_mid_forward(const NetGeom& g, const MidFwdArgs& a, int n_slabs, cudaStream_t st);
 cudaError_t launch_mid_backward(const NetGeom& g, const MidBwdArgs& a, int n_slabs, cudaStream_t st);
 
-// ---- mlp_chain.cu  (register-resident per-warp chain for the Fisher-vector product)
+// ---- mlp_chain.cu  (register-resident per-warp chains for the forward and gradient passes)
 #define CH_WARPS 12          // backward chain: 12 warps x 16 timesteps = 3 cache tiles per pass
 #define CH_NE 3             // weight-gradient entries per warp
 #define CH_NTJ 4            // n-tiles (8 columns each) per entry
@@ -82,8 +82,8 @@ struct ChainEntry {
   int nmax;    // valid output features from the first n-tile (d[l] - 8 nt0)
 };
 struct ChainJobs { ChainEntry e[CH_WARPS][CH_NE]; };
-int chain_bwd_shape(const NetGeom& g, int mode);   // 0: not covered by an instantiated chain shape
-cudaError_t launch_chain_backward(const NetGeom& g, const MidBwdArgs& a, int n_slabs, cudaStream_t st);
+int chain_bwd_shape(const NetGeom& g);   // 0: not covered by an instantiated chain shape
+cudaError_t launch_chain_backward(const NetGeom& g, const MidBwdArgs& a, int n_slabs, cudaStream_t st);   // gradient mode
 int chain_fwd_shape(const NetGeom& g);
 cudaError_t launch_chain_forward(const NetGeom& g, const MidFwdArgs& a, int n_slabs, cudaStream_t st);
 

@@ -1,14 +1,15 @@
-// Layers >= 2 of the MLP as register-resident per-warp chains: forward (losses, activation cache),
-// gradient and Fisher-vector product (trpo.py:37-63; ppo.py:35-49; core.py:613-617).
+// Layers >= 2 of the MLP as register-resident per-warp chains: forward (losses, activation cache) and
+// gradient (trpo.py:37-43,60-63; ppo.py:35-49; core.py:613-617).  The Fisher-vector product runs in
+// mlp_fvp_tc.cu.
 //
-// Backward kernel (gradient / Fvp): one CTA of 12 warps owns a slab of <= 1024 timesteps and walks it in
+// Backward kernel (gradient): one CTA of 12 warps owns a slab of <= 1024 timesteps and walks it in
 // chain tiles of 192 timesteps (3 cache tiles).
 //
-//   chain phase  Each warp owns 16 timesteps and carries them through the whole R-forward (Pearlmutter)
-//                and reverse sweep WITHOUT block barriers: the m16n8 accumulator fragment of one layer is
+//   chain phase  Each warp owns 16 timesteps and carries them from the head gradient through the whole
+//                reverse sweep WITHOUT block barriers: the m16n8 accumulator fragment of one layer is
 //                the A fragment of the next (k-slot t <-> feature 2t, slot t+4 <-> feature 2t+1, so no
 //                shuffle is needed), weights are read from shared memory in an 8x8-block layout that is
-//                bank-conflict free for both W (R-forward) and W^T (delta) fragment reads, cached
+//                bank-conflict free for both W (forward) and W^T (delta) fragment reads, cached
 //                activations come straight from HBM/L2 in fragment order (a thread's two fragment rows are
 //                adjacent timesteps: 64-bit accesses).  Every product is 3xTF32 (mma_tf32.cuh).  delta_l
 //                (l >= 2) is left in shared memory as fp32 rows, delta_1 goes to HBM as the pre-split
@@ -30,15 +31,6 @@
 #define CH_T (16 * CH_WARPS)        // timesteps per chain tile
 #define CH_LDE (CH_T + 8)           // floats between consecutive delta rows in shared memory (= 8 mod 32: the
                                     // 64-bit fragment reads of the grad phase are bank-conflict free)
-#ifndef MRL_CACHED_EARLY
-#define MRL_CACHED_EARLY 0   // request h2 / h3 / head rows before the layer-2 loop (1) or after it (0)
-#endif
-#ifndef MRL_H1_LATE
-#define MRL_H1_LATE 0
-#endif
-#ifndef MRL_PF_DIST
-#define MRL_PF_DIST 2
-#endif
 #define FW_WARPS 8                  // forward chain kernel: 256 threads, 2 CTAs per SM
 #define FW_THREADS (32 * FW_WARPS)
 
@@ -59,7 +51,7 @@ struct ChainShape {
     return s;
   }
   __host__ __device__ static constexpr int erows() { return eoff(L_ + 1); }
-  __host__ __device__ static constexpr int vboff(int l) {  // tangent bias of layer l (l >= 1)
+  __host__ __device__ static constexpr int vboff(int l) {  // bias of layer l (l >= 1) in the forward kernel
     int s = 0;
     for (int k = 1; k < l; ++k) s += 8 * nt(k);
     return s;
@@ -71,9 +63,9 @@ struct ChainShape {
     for (int k = 2; k <= L_; ++k) s += ((8 * nt(k - 1) + 15) / 16) * nt(k);
     return s;
   }
-  __host__ __device__ static constexpr size_t smem_floats(bool fvp) {
-    return (size_t)(fvp ? 2 : 1) * wfloats() + (fvp ? vbfloats() : 0) + 16 * nt(L_) + CH_WARPS * 8 * (N1_ + nt(L_)) +
-           (size_t)gblocks() * 128 + (size_t)erows() * CH_LDE;
+  __host__ __device__ static constexpr size_t smem_floats() {   // backward kernel
+    return (size_t)wfloats() + 16 * nt(L_) + CH_WARPS * 8 * (N1_ + nt(L_)) + (size_t)gblocks() * 128 +
+           (size_t)erows() * CH_LDE;
   }
 };
 
@@ -182,23 +174,6 @@ __device__ __forceinline__ void to_frags(const float (&d)[NT][4], uint32_t (&hi)
   for (int n = 0; n < NT; ++n) to_frag(d[n], hi[n], lo[n]);
 }
 
-// Rh = act'(h) * (acc + vb) for a hidden layer -> fragments of the next GEMM
-template <int ACT, int NT>
-__device__ __forceinline__ void epi_rhidden(const float (&acc)[NT][4], const float (&h)[NT][4],
-                                            const float* __restrict__ vbl, uint32_t (&hi)[NT][4],
-                                            uint32_t (&lo)[NT][4], int lane) {
-  const int t = lane & 3;
-#pragma unroll
-  for (int n = 0; n < NT; ++n) {
-    const float2 b = *reinterpret_cast<const float2*>(vbl + 8 * n + 2 * t);
-    float v[4];
-    v[0] = dact_from_h<ACT>(h[n][0]) * (acc[n][0] + b.x);
-    v[1] = dact_from_h<ACT>(h[n][1]) * (acc[n][1] + b.y);
-    v[2] = dact_from_h<ACT>(h[n][2]) * (acc[n][2] + b.x);
-    v[3] = dact_from_h<ACT>(h[n][3]) * (acc[n][3] + b.y);
-    to_frag(v, hi[n], lo[n]);
-  }
-}
 // delta_{l-1} = acc * act'(h_{l-1})
 template <int ACT, int NT>
 __device__ __forceinline__ void epi_delta(const float (&acc)[NT][4], const float (&h)[NT][4], float (&d)[NT][4]) {
@@ -206,46 +181,6 @@ __device__ __forceinline__ void epi_delta(const float (&acc)[NT][4], const float
   for (int n = 0; n < NT; ++n)
 #pragma unroll
     for (int i = 0; i < 4; ++i) d[n][i] = acc[n][i] * dact_from_h<ACT>(h[n][i]);
-}
-
-// Fisher metric at the head (SURVEY A.3): delta_L from Rz_L = acc + vb_L; rows >= N contribute nothing.
-template <int NT>
-__device__ __forceinline__ void head_metric(const float (&acc)[NT][4], const float* __restrict__ vbl,
-                                            const float* __restrict__ ivar, const float (&p)[NT][4], bool cat,
-                                            bool valid0, bool valid1, float (&d)[NT][4], int lane) {
-  const int t = lane & 3;
-  float rz[NT][4];
-  float s0 = 0.f, s1 = 0.f;
-#pragma unroll
-  for (int n = 0; n < NT; ++n) {
-    const float2 b = *reinterpret_cast<const float2*>(vbl + 8 * n + 2 * t);
-    rz[n][0] = acc[n][0] + b.x; rz[n][1] = acc[n][1] + b.y;
-    rz[n][2] = acc[n][2] + b.x; rz[n][3] = acc[n][3] + b.y;
-    if (cat) {
-      s0 += p[n][0] * rz[n][0] + p[n][1] * rz[n][1];
-      s1 += p[n][2] * rz[n][2] + p[n][3] * rz[n][3];
-    }
-  }
-  if (cat) {   // the four lanes of a quad hold one row: p . Rz over all columns
-    s0 += __shfl_xor_sync(0xffffffffu, s0, 1); s0 += __shfl_xor_sync(0xffffffffu, s0, 2);
-    s1 += __shfl_xor_sync(0xffffffffu, s1, 1); s1 += __shfl_xor_sync(0xffffffffu, s1, 2);
-  }
-#pragma unroll
-  for (int n = 0; n < NT; ++n) {
-    float v[4];
-    if (cat) {                       // M = diag(p) - p p^T
-      v[0] = p[n][0] * (rz[n][0] - s0); v[1] = p[n][1] * (rz[n][1] - s0);
-      v[2] = p[n][2] * (rz[n][2] - s1); v[3] = p[n][3] * (rz[n][3] - s1);
-    } else {                         // M = diag(1/sigma^2) on the mean block
-      const float2 iv = *reinterpret_cast<const float2*>(ivar + 8 * n + 2 * t);
-      v[0] = rz[n][0] * iv.x; v[1] = rz[n][1] * iv.y;
-      v[2] = rz[n][2] * iv.x; v[3] = rz[n][3] * iv.y;
-    }
-    if (!valid0) { v[0] = 0.f; v[1] = 0.f; }
-    if (!valid1) { v[2] = 0.f; v[3] = 0.f; }
-#pragma unroll
-    for (int i = 0; i < 4; ++i) d[n][i] = v[i];
-  }
 }
 
 // dL/dz_L of the surrogate / penalised surrogate / squared error at the head (trpo.py:43, ppo.py:47-49,
@@ -357,70 +292,6 @@ __device__ __forceinline__ void head_grad(int head, const float (&ho)[NT][4], co
   }
 }
 
-// R-forward of layer 2: A = Rh1 = act'(h1) * (x.V1 + vb1) and A = h1, streamed from HBM per k-step
-template <int ACT, int N1, int N2>
-__device__ __forceinline__ void rfwd_layer2(float (&acc)[N2][4], const float* __restrict__ zp,
-                                            const float* __restrict__ hp, int d1, bool ok,
-                                            const float* __restrict__ vb1, const float* __restrict__ W,
-                                            const float* __restrict__ V, int lane) {
-  const int t = lane & 3;
-  constexpr int D = MRL_PF_DIST;          // k-steps requested ahead of use (register prefetch)
-  float zq[D + 1][4], hq[D + 1][4];       // [0] = current k-step
-#pragma unroll
-  for (int i = 0; i < D; ++i) {
-    ldfrag(zq[i], zp, 8 * i + 2 * t, d1, ok && i < N1);
-    ldfrag(hq[i], hp, 8 * i + 2 * t, d1, ok && i < N1);
-  }
-#pragma unroll 1
-  for (int ks = 0; ks < N1; ++ks) {
-    ldfrag(zq[D], zp, 8 * (ks + D) + 2 * t, d1, ok && ks + D < N1);
-    ldfrag(hq[D], hp, 8 * (ks + D) + 2 * t, d1, ok && ks + D < N1);
-    const float2 b = *reinterpret_cast<const float2*>(vb1 + 8 * ks + 2 * t);
-    float r[4];
-    r[0] = dact_from_h<ACT>(hq[0][0]) * (zq[0][0] + b.x);
-    r[1] = dact_from_h<ACT>(hq[0][1]) * (zq[0][1] + b.y);
-    r[2] = dact_from_h<ACT>(hq[0][2]) * (zq[0][2] + b.x);
-    r[3] = dact_from_h<ACT>(hq[0][3]) * (zq[0][3] + b.y);
-    uint32_t ah[4], al[4];
-    to_frag(r, ah, al);
-    kstep<N2, false>(acc, ah, al, W, ks, 0, N2, lane);
-    to_frag(hq[0], ah, al);
-    kstep<N2, false>(acc, ah, al, V, ks, 0, N2, lane);
-#pragma unroll
-    for (int i = 0; i < D; ++i)
-#pragma unroll
-      for (int c = 0; c < 4; ++c) { zq[i][c] = zq[i + 1][c]; hq[i][c] = hq[i + 1][c]; }
-  }
-}
-// R-forward of layer l >= 3: A = Rh_{l-1} (fragments) with W_l, and A = h_{l-1} with V_l
-template <int NI, int NO>
-__device__ __forceinline__ void rfwd_layer(float (&acc)[NO][4], const uint32_t (&rhi)[NI][4],
-                                           const uint32_t (&rlo)[NI][4], const float (&hin)[NI][4],
-                                           const float* __restrict__ W, const float* __restrict__ V, int lane) {
-  if constexpr (NO <= 4) {   // narrow layer: the two terms go to separate accumulators (longer dependency distance)
-    float acc2[NO][4];
-    zero_acc(acc2);
-#pragma unroll
-    for (int ks = 0; ks < NI; ++ks) {
-      kstep<NO, false>(acc, rhi[ks], rlo[ks], W, ks, 0, NO, lane);
-      uint32_t ah[4], al[4];
-      to_frag(hin[ks], ah, al);
-      kstep<NO, false>(acc2, ah, al, V, ks, 0, NO, lane);
-    }
-#pragma unroll
-    for (int n = 0; n < NO; ++n)
-#pragma unroll
-      for (int i = 0; i < 4; ++i) acc[n][i] += acc2[n][i];
-  } else {
-#pragma unroll
-    for (int ks = 0; ks < NI; ++ks) {
-      kstep<NO, false>(acc, rhi[ks], rlo[ks], W, ks, 0, NO, lane);
-      uint32_t ah[4], al[4];
-      to_frag(hin[ks], ah, al);
-      kstep<NO, false>(acc, ah, al, V, ks, 0, NO, lane);
-    }
-  }
-}
 // delta_{l-1} pre-activation = delta_l . W_l^T for in-blocks nb .. nb+NI-1
 template <int NI, int NO>
 __device__ __forceinline__ void delta_layer(float (&acc)[NI][4], const uint32_t (&dhi)[NO][4],
@@ -453,17 +324,11 @@ __device__ __forceinline__ void delta1_block(const uint32_t (&dhi)[NO][4], const
                                              int lane) {
   const int g = lane >> 2, t = lane & 3;
   float h1[NH][4];
-#if !MRL_H1_LATE
 #pragma unroll
   for (int n = 0; n < NH; ++n) ldfrag(h1[n], hp, 8 * (nb + n) + 2 * t, d1, ok);
-#endif
   float acc[NH][4];
   zero_acc(acc);
   delta_layer<NH, NO>(acc, dhi, dlo, W2, nb, lane);
-#if MRL_H1_LATE
-#pragma unroll
-  for (int n = 0; n < NH; ++n) ldfrag(h1[n], hp, 8 * (nb + n) + 2 * t, d1, ok);
-#endif
 #pragma unroll
   for (int n = 0; n < NH; ++n) {
     float v[4];
@@ -555,20 +420,17 @@ __device__ __forceinline__ void grad_entry(float* __restrict__ Gs, const float* 
     *reinterpret_cast<float4*>(Gs + (q * 32 + lane) * 4) = make_float4(G[q][0], G[q][1], G[q][2], G[q][3]);
 }
 
-template <class S, int ACT, int MODE>
+template <class S, int ACT>
 __global__ void __launch_bounds__(CH_THREADS, 1) chain_bwd_kernel(NetGeom g, MidBwdArgs a, ChainJobs jobs, int n_slabs) {
   constexpr int L = S::L;
-  constexpr int N1 = S::nt(1), N2 = S::nt(2), N3 = S::nt(3), N4 = S::nt(4);
+  constexpr int N1 = S::nt(1), N2 = S::nt(2), N3 = S::nt(3);
   constexpr int NL = S::nt(L);
-  constexpr bool FVP = MODE == MRL_MODE_FVP;
   extern __shared__ __align__(16) float smem[];
   float* Ws = smem;
-  float* Vs = Ws + S::wfloats();                       // tangent weights (Fvp only)
-  float* vb = Vs + (FVP ? S::wfloats() : 0);           // tangent biases (Fvp only)
-  float* ivar = vb + (FVP ? S::vbfloats() : 0);
+  float* ivar = Ws + S::wfloats();
   float* sig = ivar + 8 * NL;
   float* gb1s = sig + 8 * NL;                          // [warp][8 N1] layer-1 bias partials
-  float* glss = gb1s + CH_WARPS * 8 * N1;              // [warp][8 NL] logstd partials (gradient mode)
+  float* glss = gb1s + CH_WARPS * 8 * N1;              // [warp][8 NL] logstd partials
   float* Gs = glss + CH_WARPS * 8 * NL;                // weight-gradient accumulator blocks of all entries
   float* E = Gs + S::gblocks() * 128;                  // delta rows [row][CH_LDE]
   __shared__ uint64_t e_full, e_free;   // delta rows of the current chain tile: all stored / all consumed
@@ -582,7 +444,7 @@ __global__ void __launch_bounds__(CH_THREADS, 1) chain_bwd_kernel(NetGeom g, Mid
   }
   uint32_t tile_no = 0;                 // chain tiles processed by this CTA (barrier phase = tile_no & 1)
 
-  // ---- weights of theta (W) and of the tangent (V) into the 8x8-block layout, tangent biases, sigma, 1/sigma^2
+  // ---- weights into the 8x8-block layout, sigma, 1/sigma^2
 #pragma unroll
   for (int l = 2; l <= L; ++l) {
     const int kin = 8 * S::nt(l - 1), nout = 8 * S::nt(l);
@@ -593,13 +455,7 @@ __global__ void __launch_bounds__(CH_THREADS, 1) chain_bwd_kernel(NetGeom g, Mid
       const bool ok = i < g.d[l - 1] && j < g.d[l];
       const int dst = ((i >> 3) * S::nt(l) + (j >> 3)) * 64 + blk_row(j & 7) * 8 + (i & 7);
       dw[dst] = ok ? src[i * g.ldw[l] + j] : 0.f;
-      if (FVP) Vs[S::woff(l) + dst] = ok ? a.imgv[g.off_W[l] + i * g.ldw[l] + j] : 0.f;
     }
-  }
-  if (FVP) {
-#pragma unroll
-    for (int l = 1; l <= L; ++l)
-      for (int f = tid; f < 8 * S::nt(l); f += CH_THREADS) vb[S::vboff(l) + f] = f < g.d[l] ? a.imgv[g.off_b[l] + f] : 0.f;
   }
   for (int f = tid; f < 8 * NL; f += CH_THREADS) {
     const float ls = (gauss && f < g.d[L]) ? a.img[g.off_pm_logstd + f] : 0.f;
@@ -607,12 +463,12 @@ __global__ void __launch_bounds__(CH_THREADS, 1) chain_bwd_kernel(NetGeom g, Mid
     ivar[f] = (gauss && f < g.d[L]) ? expf(-2.f * ls) : 0.f;
   }
   float cs = 1.f, ck = 0.f;
-  if (!FVP && a.coef) { cs = (float)a.coef[0]; ck = (float)a.coef[1]; }
+  if (a.coef) { cs = (float)a.coef[0]; ck = (float)a.coef[1]; }
 
   for (int slab = blockIdx.x; slab < n_slabs; slab += gridDim.x) {   // persistent: weights stay in shared memory
   const int t0 = slab * a.slab_tiles, t1 = min(t0 + a.slab_tiles, a.n_tiles);
   for (int i = tid; i < S::gblocks() * 128; i += CH_THREADS) Gs[i] = 0.f;
-  float gls[NL][2];   // logstd gradient partials of this thread's columns (gradient mode, DiagGauss)
+  float gls[NL][2];   // logstd gradient partials of this thread's columns (DiagGauss)
 #pragma unroll
   for (int n = 0; n < NL; ++n) { gls[n][0] = 0.f; gls[n][1] = 0.f; }
   for (int i = tid; i < CH_WARPS * 8 * N1; i += CH_THREADS) gb1s[i] = 0.f;
@@ -635,55 +491,26 @@ __global__ void __launch_bounds__(CH_THREADS, 1) chain_bwd_kernel(NetGeom g, Mid
         const char* pc = reinterpret_cast<const char*>(a.cache + (size_t)(ct0 + CH_TILES) * g.act_rows * MRL_LDT) + (size_t)warp * cchunk;
         const unsigned cn = warp == CH_WARPS - 1 ? cbytes - (CH_WARPS - 1) * cchunk : cchunk;
         asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(pc), "r"(cn) : "memory");
-        const float* side = FVP ? a.Zt : a.aux;                    // Fvp: x.V1 ; gradient: adv / actions / old probs
-        const int srows = FVP ? g.d[1] : g.naux;
-        const unsigned zbytes = (unsigned)(nt2 * srows * MRL_LDT * 4);
+        const unsigned zbytes = (unsigned)(nt2 * g.naux * MRL_LDT * 4);   // side inputs: adv / actions / old probs
         const unsigned zchunk = (zbytes / CH_WARPS) & ~15u;
-        const char* pz = reinterpret_cast<const char*>(side + (size_t)(ct0 + CH_TILES) * srows * MRL_LDT) + (size_t)warp * zchunk;
+        const char* pz = reinterpret_cast<const char*>(a.aux + (size_t)(ct0 + CH_TILES) * g.naux * MRL_LDT) + (size_t)warp * zchunk;
         const unsigned zn = warp == CH_WARPS - 1 ? zbytes - (CH_WARPS - 1) * zchunk : zchunk;
         asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(pz), "r"(zn) : "memory");
       }
       float h2[N2][4];
       float h3[L == 4 ? N3 : 1][4];
-      float ph[NL][4];   // cached head output: probabilities (Fvp, Categorical) / mean | probs | value (gradient)
-      auto load_cached = [&]() {
+      float ph[NL][4];   // cached head output: mean | probs | value
 #pragma unroll
-        for (int n = 0; n < N2; ++n) ldfrag(h2[n], cb + g.off_act[2] * MRL_LDT, 8 * n + 2 * t, g.d[2], ok);
-        if constexpr (L == 4) {
+      for (int n = 0; n < N2; ++n) ldfrag(h2[n], cb + g.off_act[2] * MRL_LDT, 8 * n + 2 * t, g.d[2], ok);
+      if constexpr (L == 4) {
 #pragma unroll
-          for (int n = 0; n < N3; ++n) ldfrag(h3[n], cb + g.off_act[3] * MRL_LDT, 8 * n + 2 * t, g.d[3], ok);
-        }
-#pragma unroll
-        for (int n = 0; n < NL; ++n) ldfrag(ph[n], cb + g.off_act[L] * MRL_LDT, 8 * n + 2 * t, g.d[L], ok && (cat || !FVP));
-      };
-      if (MRL_CACHED_EARLY || !FVP) load_cached();
-      float dL[NL][4];   // delta_L (accumulator order)
-      if constexpr (FVP) {
-        // ---- R-forward (Pearlmutter) and the Fisher metric
-        const float* zb = a.Zt + (size_t)ctile * g.d[1] * MRL_LDT + rr;
-        float acc2[N2][4];
-        zero_acc(acc2);
-        rfwd_layer2<ACT, N1, N2>(acc2, zb, cb, g.d[1], ok, vb + S::vboff(1), Ws + S::woff(2), Vs + S::woff(2), lane);
-        if (!MRL_CACHED_EARLY) load_cached();
-        uint32_t r2h[N2][4], r2l[N2][4];
-        epi_rhidden<ACT, N2>(acc2, h2, vb + S::vboff(2), r2h, r2l, lane);
-        float acc3[N3][4];
-        zero_acc(acc3);
-        rfwd_layer<N2, N3>(acc3, r2h, r2l, h2, Ws + S::woff(3), Vs + S::woff(3), lane);
-        if constexpr (L == 3) {
-          head_metric<N3>(acc3, vb + S::vboff(3), ivar, ph, cat, valid0, valid1, dL, lane);
-        } else {
-          uint32_t r3h[N3][4], r3l[N3][4];
-          epi_rhidden<ACT, N3>(acc3, h3, vb + S::vboff(3), r3h, r3l, lane);
-          float acc4[NL][4];
-          zero_acc(acc4);
-          rfwd_layer<N3, NL>(acc4, r3h, r3l, h3, Ws + S::woff(4), Vs + S::woff(4), lane);
-          head_metric<NL>(acc4, vb + S::vboff(4), ivar, ph, cat, valid0, valid1, dL, lane);
-        }
-      } else {
-        const float* auxb = a.aux + (size_t)ctile * g.naux * MRL_LDT + rr;
-        head_grad<NL>(g.head, ph, auxb, g.d[L], sig, ivar, cs, ck, a.reverse_kl, valid0, valid1, ok, gls, dL, lane);
+        for (int n = 0; n < N3; ++n) ldfrag(h3[n], cb + g.off_act[3] * MRL_LDT, 8 * n + 2 * t, g.d[3], ok);
       }
+#pragma unroll
+      for (int n = 0; n < NL; ++n) ldfrag(ph[n], cb + g.off_act[L] * MRL_LDT, 8 * n + 2 * t, g.d[L], ok);
+      float dL[NL][4];   // delta_L (accumulator order)
+      const float* auxb = a.aux + (size_t)ctile * g.naux * MRL_LDT + rr;
+      head_grad<NL>(g.head, ph, auxb, g.d[L], sig, ivar, cs, ck, a.reverse_kl, valid0, valid1, ok, gls, dL, lane);
       // ---- reverse sweep
       bar_wait(&e_free, (tile_no & 1) ^ 1);   // the previous tile's grad phase has read its delta rows (passes at once for tile 0)
       store_E<NL>(E + (size_t)S::eoff(L) * CH_LDE, dL, warp, lane);
@@ -794,7 +621,7 @@ __global__ void __launch_bounds__(CH_THREADS, 1) chain_bwd_kernel(NetGeom g, Mid
     for (int w = 0; w < CH_WARPS; ++w) s += gb1s[w * 8 * N1 + f];   // fixed order -> deterministic
     part[g.off_b[1] + f] = s;
   }
-  if (!FVP && gauss) {   // logstd gradient: this thread's column sums -> across rows (shuffles) -> across warps (fixed order)
+  if (gauss) {   // logstd gradient: this thread's column sums -> across rows (shuffles) -> across warps (fixed order)
 #pragma unroll
     for (int n = 0; n < NL; ++n)
 #pragma unroll
@@ -813,7 +640,7 @@ __global__ void __launch_bounds__(CH_THREADS, 1) chain_bwd_kernel(NetGeom g, Mid
       part[g.off_pm_logstd + j] = sum;
     }
   } else {
-    for (int j = tid; j < g.d[L]; j += CH_THREADS) part[g.off_pm_logstd + j] = 0.f;   // fvp[logstd] is set by the reduce
+    for (int j = tid; j < g.d[L]; j += CH_THREADS) part[g.off_pm_logstd + j] = 0.f;
   }
   __syncthreads();   // gb1s / glss are reused by the next slab
   }
@@ -867,9 +694,8 @@ static bool build_jobs(const NetGeom& g, ChainJobs* jobs) {
 }
 
 template <class S>
-static bool shape_fits(const NetGeom& g, int mode) {
+static bool shape_fits(const NetGeom& g) {
   if (g.L != S::L || g.act != MRL_ACT_TANH) return false;
-  if (mode == MRL_MODE_FVP && g.head != MRL_HEAD_GAUSS && g.head != MRL_HEAD_CAT) return false;
   for (int l = 1; l <= S::L; ++l)
     if ((g.d[l] + 7) / 8 > S::nt(l)) return false;
   // the padded layer-1 width must cover every n-group of the layer-1 gradient operand but one
@@ -878,17 +704,17 @@ static bool shape_fits(const NetGeom& g, int mode) {
   return build_jobs<S>(g, &jobs);
 }
 
-template <class S, int MODE>
+template <class S>
 static cudaError_t launch_shape(const NetGeom& g, const MidBwdArgs& a, int n_slabs, cudaStream_t st) {
   ChainJobs jobs;
   if (!build_jobs<S>(g, &jobs)) return cudaErrorInvalidConfiguration;
-  const size_t sm = S::smem_floats(MODE == MRL_MODE_FVP) * 4;
+  const size_t sm = S::smem_floats() * 4;
   {
-    cudaError_t e = mrl_func_smem((const void*)chain_bwd_kernel<S, MRL_ACT_TANH, MODE>, sm);
+    cudaError_t e = mrl_func_smem((const void*)chain_bwd_kernel<S, MRL_ACT_TANH>, sm);
     if (e != cudaSuccess) return e;
   }
   const int sms = mrl_sm_count();
-  chain_bwd_kernel<S, MRL_ACT_TANH, MODE><<<n_slabs < sms ? n_slabs : sms, CH_THREADS, sm, st>>>(g, a, jobs, n_slabs);
+  chain_bwd_kernel<S, MRL_ACT_TANH><<<n_slabs < sms ? n_slabs : sms, CH_THREADS, sm, st>>>(g, a, jobs, n_slabs);
   return cudaGetLastError();
 }
 
@@ -897,24 +723,21 @@ typedef ChainShape<3, 8, 8, 3, 0> ShapeB;     // 64-64 hidden, <= 24 outputs (18
 typedef ChainShape<4, 13, 7, 4, 3> ShapeC;    // 100-50-25 hidden, <= 24 outputs (Humanoid policy and value nets)
 
 // 0 = not supported (use the job-list kernel of mlp_mid.cu), else the shape id
-int chain_bwd_shape(const NetGeom& g, int mode) {
-  if (shape_fits<ShapeA>(g, mode)) return 1;
-  if (shape_fits<ShapeB>(g, mode)) return 2;
-  if (shape_fits<ShapeC>(g, mode)) return 3;
+int chain_bwd_shape(const NetGeom& g) {
+  if (shape_fits<ShapeA>(g)) return 1;
+  if (shape_fits<ShapeB>(g)) return 2;
+  if (shape_fits<ShapeC>(g)) return 3;
   return 0;
 }
 
-template <int MODE>
-static cudaError_t launch_mode(const NetGeom& g, const MidBwdArgs& a, int n_slabs, cudaStream_t st) {
-  switch (chain_bwd_shape(g, MODE)) {
-    case 1: return launch_shape<ShapeA, MODE>(g, a, n_slabs, st);
-    case 2: return launch_shape<ShapeB, MODE>(g, a, n_slabs, st);
-    case 3: return launch_shape<ShapeC, MODE>(g, a, n_slabs, st);
+cudaError_t launch_chain_backward(const NetGeom& g, const MidBwdArgs& a, int n_slabs, cudaStream_t st) {
+  if (a.mode != MRL_MODE_GRAD) return cudaErrorInvalidValue;   // the chain computes gradients only
+  switch (chain_bwd_shape(g)) {
+    case 1: return launch_shape<ShapeA>(g, a, n_slabs, st);
+    case 2: return launch_shape<ShapeB>(g, a, n_slabs, st);
+    case 3: return launch_shape<ShapeC>(g, a, n_slabs, st);
     default: return cudaErrorInvalidConfiguration;
   }
-}
-cudaError_t launch_chain_backward(const NetGeom& g, const MidBwdArgs& a, int n_slabs, cudaStream_t st) {
-  return a.mode == MRL_MODE_FVP ? launch_mode<MRL_MODE_FVP>(g, a, n_slabs, st) : launch_mode<MRL_MODE_GRAD>(g, a, n_slabs, st);
 }
 
 // ====================================================================================================

@@ -1,7 +1,7 @@
 // Fisher-vector product of layers >= 2 on the 5th-generation tensor cores (tcgen05 + TMEM), split-precision 3xTF32:
 // R-forward (Pearlmutter), Fisher metric at the head, reverse sweep, hidden-layer weight / bias gradient partials and
-// the delta_1 operand of the layer-1 gradient GEMM (trpo.py:45-58; SURVEY A.3).  Replaces the warp-level mma.sync chain
-// (mlp_chain.cu, chain_bwd_kernel<FVP>) for the Fvp, which was issue-bound on the legacy tensor path.
+// the delta_1 operand of the layer-1 gradient GEMM (trpo.py:45-58; SURVEY A.3).  On tcgen05 because a warp-level
+// mma.sync chain (as in mlp_chain.cu) was issue-bound on the legacy tensor path for the Fvp.
 //
 // One CTA (16 warps) walks 128-timestep tiles (M = 128 = the TMEM lanes) of its slab.  Every GEMM of the chain runs in
 // TS mode: the A operand (activations of the 128 timesteps) is written into tensor memory by the epilogue warps that
@@ -25,7 +25,7 @@
 // slab in TMEM.  A row of ones in each (k) tile yields the bias gradients.  Several layers share one 128-row tile when
 // their rows fit (Humanoid: h_2 and h_3 against [delta_3 | delta_4]).
 //
-// Warp roles (512 threads): 0 producer of the weight ring (+ L2 prefetch of the next tile's activations), 1 chain MMA
+// Warp roles (512 threads): 0 producer of the weight ring, 1 chain MMA
 // issuer (+ TMEM allocation), 2 (k) MMA issuer, 3 idle, 4-7 / 8-11 epilogue groups 0 / 1 (TMEM lane quarter = warp % 4),
 // 12-15 converters.  All hand-overs are mbarriers with a spin watchdog: a protocol bug traps, it never hangs the GPU.
 #include "common.cuh"
@@ -120,9 +120,6 @@ __device__ __forceinline__ void tmem_ld8(uint32_t taddr, uint32_t (&r)[8]) {
 // launch gives every thread 128 registers (512 threads = the whole register file); the control warps and the
 // converters hand most of theirs back, the epilogue warps - which keep prefetched activations in registers to hide
 // the L2 latency - take them.
-#ifndef FT_ROT
-#define FT_ROT 1          // rotate the (k) operand stores against bank conflicts (see the delta epilogue)
-#endif
 #define FT_REGS_CTRL 32
 #define FT_REGS_CONV 72
 #define FT_REGS_EPI 88
@@ -152,7 +149,7 @@ struct FtArgs {
   const float* logstd;  // theta image logstd block (DiagGauss) or nullptr
   const float* Zt;      // x . V_1, tile-major [tile][d1][LDT]
   const float* cache;   // activations of theta, tile-major [tile][act_rows][LDT]
-  float* DG;            // delta_1 operand of the layer-1 gradient GEMM, MN-major: [t/8][hi | lo][n/4][8 t][4 n]
+  float* DG;            // delta_1 operand of the layer-1 gradient GEMM, K-major: [t/8][hi | lo][khalf][n/8][8 n][4 t]
   float* partm;         // [n_slabs][pmid]
   float* dbg;           // debug dump of the first tile (nullptr: off)
   long long* trace;     // pipeline trace of CTA 0 (nullptr: off)
@@ -238,9 +235,11 @@ __global__ void __launch_bounds__(FT_THREADS, 1) fvp_tc_kernel(NetGeom g, FtPlan
   if (warp < 4) {
   ft_reg_dec<FT_REGS_CTRL>();
   if (warp == 0) {
-    // ================================================================ producer: both weight rings + L2 prefetch
+    // ================================================================ producer: both weight rings
     // The two rings drain at unrelated rates (R phase of tile i + 1 next to the delta phase of tile i), so the one
     // producer thread never blocks on either: it probes both and refills whichever has a free stage.
+    // No L2 prefetch of the next tile's activations: it competes with the demand loads (1 M Humanoid timesteps: none
+    // 1.04 ms, one bulk prefetch per tile 1.07, 16 KB pieces 1.22).
     if (lane == 0) {
       long long total_tiles = 0;
       for (int slab = blockIdx.x; slab < a.n_slabs; slab += gridDim.x)
@@ -251,38 +250,6 @@ __global__ void __launch_bounds__(FT_THREADS, 1) fvp_tc_kernel(NetGeom g, FtPlan
       long long r_left = total_tiles * r_per, d_left = total_tiles * d_per;
       uint32_t rc = 0, dc = 0;                       // stages issued so far
       int rst = 0, rkg = 0, dst_ = 0, dkg = 0;       // position inside the tile
-      // optional L2 prefetch of the next tile's activations and x.V_1 (off: it competes with the demand loads, see FT_PF)
-      int pf_slab = blockIdx.x, pf_mt = blockIdx.x * a.slab_mt;
-      auto prefetch_piece = [&](const float* p, size_t bytes) {
-        for (size_t o = 0; o < bytes; o += 16384) {
-          const uint32_t nb = (uint32_t)(bytes - o < 16384 ? bytes - o : 16384);
-          asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(reinterpret_cast<const char*>(p) + o), "r"(nb) : "memory");
-        }
-      };
-      auto prefetch_next = [&]() {
-        int mt = pf_mt + 1, slab = pf_slab;
-        if (mt >= min(slab * a.slab_mt + a.slab_mt, a.n_mtiles)) { slab += gridDim.x; mt = slab * a.slab_mt; }
-        pf_slab = slab; pf_mt = mt;
-        if (slab >= a.n_slabs) return;
-        const int t0 = 2 * mt, nt = min(2, a.n_tiles - t0);
-        if (nt <= 0) return;
-#ifndef FT_AHEAD2
-#define FT_AHEAD2 0
-#endif
-#ifndef FT_PF
-#define FT_PF 0       // measured at 1 M Humanoid timesteps: no L2 prefetch 1.04 ms, one bulk prefetch per tile 1.07, 16 KB pieces 1.22
-#endif
-#if FT_PF == 2
-        prefetch_piece(a.cache + (size_t)t0 * tile_c, (size_t)nt * tile_c * 4);
-        prefetch_piece(a.Zt + (size_t)t0 * tile_z, (size_t)nt * tile_z * 4);
-#elif FT_PF == 1
-        asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(a.cache + (size_t)t0 * tile_c),
-                     "r"((uint32_t)(nt * tile_c * 4)) : "memory");
-        asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(a.Zt + (size_t)t0 * tile_z),
-                     "r"((uint32_t)(nt * tile_z * 4)) : "memory");
-#endif
-        (void)prefetch_piece;
-      };
       while (r_left > 0 || d_left > 0) {
         bool progressed = false;
         if (r_left > 0) {
@@ -295,7 +262,6 @@ __global__ void __launch_bounds__(FT_THREADS, 1) fvp_tc_kernel(NetGeom g, FtPlan
             mbar_expect_tx(&rw_full[ws], 2u * nk * kgf * 4u);
             bulk_g2s(dst, a.WC + st.w_off + (size_t)rkg * kgf, nk * kgf * 4u, &rw_full[ws]);
             bulk_g2s(dst + 2 * kgf, a.VC + st.v_off + (size_t)rkg * kgf, nk * kgf * 4u, &rw_full[ws]);
-            if (rst == 0 && rkg == 0) prefetch_next();
             ++rc; --r_left; progressed = true;
             rkg += 2;
             if (rkg >= st.kgs) { rkg = 0; if (++rst == nR) rst = 0; }
@@ -561,11 +527,7 @@ __global__ void __launch_bounds__(FT_THREADS, 1) fvp_tc_kernel(NetGeom g, FtPlan
           const int ul = r + 1, kgs = P.rs[r].kgs;
           const float* hrow = cb + (size_t)g.off_act[ul] * MRL_LDT;
           const float* vbl = vb_s + P.vboff[ul];
-#if FT_AHEAD2
-          float hc[8], zc[8], hn[8], zn[8], hf[8], zf[8];     // current, next and next-but-one k-group of this group
-#else
-          float hc[8], zc[8], hn[8], zn[8];
-#endif
+          float hc[8], zc[8], hn[8], zn[8];                   // current and next k-group of this group
           auto request = [&](int kg, float (&hb)[8], float (&zz)[8]) {
             const float* ph = hrow + (size_t)(8 * kg) * MRL_LDT;
 #pragma unroll
@@ -579,9 +541,6 @@ __global__ void __launch_bounds__(FT_THREADS, 1) fvp_tc_kernel(NetGeom g, FtPlan
           int kg = (e - (int)(u & 1)) & 1;            // this group's first k-group of the stage
           u += kgs;
           if (kg < kgs) request(kg, hc, zc);
-#if FT_AHEAD2
-          if (kg + 2 < kgs) request(kg + 2, hn, zn);
-#endif
           uint32_t src_acc = 0;
           if (tr_on) FT_TR(3, (1 << 24) | (r << 8));
           if (r > 0) {
@@ -592,11 +551,7 @@ __global__ void __launch_bounds__(FT_THREADS, 1) fvp_tc_kernel(NetGeom g, FtPlan
           if (tr_on) FT_TR(3, (2 << 24) | (r << 8));
           for (; kg < kgs; kg += 2, ++ue) {
             const uint32_t freeq = mbar_try(&ra_empty[e], (ue & 1) ^ 1);
-#if FT_AHEAD2
-            if (kg + 4 < kgs) request(kg + 4, hf, zf);
-#else
             if (kg + 2 < kgs) request(kg + 2, hn, zn);
-#endif
             float val[8];
             const float4 vb0 = *reinterpret_cast<const float4*>(vbl + 8 * kg), vb1 = *reinterpret_cast<const float4*>(vbl + 8 * kg + 4);
             const float vbk[8] = {vb0.x, vb0.y, vb0.z, vb0.w, vb1.x, vb1.y, vb1.z, vb1.w};
@@ -631,13 +586,8 @@ __global__ void __launch_bounds__(FT_THREADS, 1) fvp_tc_kernel(NetGeom g, FtPlan
             __syncwarp();
             if (lane == 0) mbar_arrive(&ra_full[e]);
             if (tr_on) FT_TR(3, (5 << 24) | (r << 8) | kg);
-#if FT_AHEAD2
-#pragma unroll
-            for (int i = 0; i < 8; ++i) { hc[i] = hn[i]; zc[i] = zn[i]; hn[i] = hf[i]; zn[i] = zf[i]; }
-#else
 #pragma unroll
             for (int i = 0; i < 8; ++i) { hc[i] = hn[i]; zc[i] = zn[i]; }
-#endif
           }
         }
         ++tcount;
@@ -652,9 +602,7 @@ __global__ void __launch_bounds__(FT_THREADS, 1) fvp_tc_kernel(NetGeom g, FtPlan
       const int e = (warp - 12) >> 2;
       const uint32_t ring = tlane + P.dring_col + 16 * e;
       float* gb1w = gb1s + (warp - 12) * 128;
-#if FT_ROT
-      const int rot = (m >> 2) & 7;
-#endif
+      const int rot = (m >> 2) & 7;   // (k) operand stores are rotated against bank conflicts (see below)
       const bool cat = g.head == MRL_HEAD_CAT;
       const int nu = a.nu;
       uint32_t u = 0, ue = 0, tcount = 0;
@@ -758,9 +706,8 @@ __global__ void __launch_bounds__(FT_THREADS, 1) fvp_tc_kernel(NetGeom g, FtPlan
                   // the same block as the K-major B operand of the (k) GEMM: [n][timestep].  In the no-swizzle core-matrix
                   // order the 32 timesteps of a warp at one n hit 4 banks (8-way conflict), so the eight values are
                   // rotated per lane quad and one store instruction hits 32 banks.  The rotation costs 96 select
-                  // instructions per k-group, but the plain order (FT_ROT=0) measured SLOWER: 1.095 vs 1.046 ms
+                  // instructions per k-group, but the plain order measured SLOWER: 1.095 vs 1.046 ms
                   float* kp = kb + (size_t)kg * 1024;
-#if FT_ROT
                   ft_rot8(hi, rot);
                   ft_rot8(lo, rot);
 #pragma unroll
@@ -769,13 +716,6 @@ __global__ void __launch_bounds__(FT_THREADS, 1) fvp_tc_kernel(NetGeom g, FtPlan
                     kp[nn] = __uint_as_float(hi[i]);
                     kp[nn + lo_off] = __uint_as_float(lo[i]);
                   }
-#else
-#pragma unroll
-                  for (int i = 0; i < 8; ++i) {
-                    kp[4 * i] = __uint_as_float(hi[i]);
-                    kp[4 * i + lo_off] = __uint_as_float(lo[i]);
-                  }
-#endif
                 }
                 asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
                 tc_fence_before();

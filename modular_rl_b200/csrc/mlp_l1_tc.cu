@@ -25,7 +25,6 @@
 // HBM), warps 6..13 = converters (TC_CGROUPS groups of four, one TMEM lane quarter per warp; stage uses alternate between the groups).  The forward kernel double-
 // buffers its accumulator so the epilogue of tile i overlaps the MMAs of tile i+1.  Persistent grid.
 // The pipeline was tuned with a clock64 trace of every hand-over (-DMRL_TRACE, tools/micro/l1_trace.py).
-#include <cstdlib>
 #include "common.cuh"
 #include "kernels.h"
 #include "tc_common.cuh"
@@ -263,7 +262,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) l1_grad_tc_kernel(const float* 
                                                                    int xg_ftiles, int nu, int d0, int n1p,
                                                                    int slab_tiles, int n_tiles, int n_slabs,
                                                                    int acc_stride, int tmem_cols, int nss, int nts,
-                                                                   int dg_mn, int cgroups) {
+                                                                   int cgroups) {
   extern __shared__ __align__(1024) unsigned char smem_raw[];
   // two rings: nss shared-memory stages (raw A blocks + B) cover the HBM latency; nts tensor-memory slots hold
   // the converted A operand (hi, lo) of the stages the MMA thread is working on - tensor memory is mostly taken
@@ -316,13 +315,10 @@ __global__ void __launch_bounds__(TC_THREADS, 1) l1_grad_tc_kernel(const float* 
       }
     }
   } else if (warp == 1) {   // MMA issuer: the whole warp walks the loop, one elected lane issues
-    // delta_1 as the B operand comes in one of two layouts (both nu x 8 timesteps per stage, hi block then lo block):
-    //   K-major  [khalf][ngroup nu/8][8 n][4 t]   (mlp_chain.cu / mlp_mid.cu writers: LBO = the K halves, SBO = 8-row groups)
-    //   MN-major [n/4][8 t][4 n]                   (mlp_fvp_tc.cu: a timestep thread stores 4 features = 16 bytes at once;
-    //                                               core matrix = 8 k x 16 bytes along N, SBO = stride between N chunks)
-    const uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(nu >> 3) << 17) | ((TC_M >> 4) << 24) |
-                           (dg_mn ? (1u << 16) : 0u);
-    const uint32_t lboB = dg_mn ? nu * 32 : nu * 4 * 4;
+    // delta_1, the B operand, is K-major: nu x 8 timesteps per stage, hi block then lo block, each
+    // [khalf][ngroup nu/8][8 n][4 t] (LBO = the K halves, SBO = 8-row groups)
+    const uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(nu >> 3) << 17) | ((TC_M >> 4) << 24);
+    const uint32_t lboB = nu * 4 * 4;
     const uint32_t desc_hi = (uint32_t)(umma_desc(0, 0, 128) >> 32);
     const uint32_t dB0 = umma_desc_lo(smem_u32(stages) + offB, lboB);
     int s = 0, a = 0, aph = 0;
@@ -487,22 +483,21 @@ cudaError_t launch_l1_forward_tc(const NetGeom& g, const float* XA, int xa_kgrou
   // behind the accumulators, 512 columns in all).  Measured at 1M x 376 -> 100: one converter group, 5 stages of
   // 3 k-groups 0.447 ms (2: 0.47, 4: 0.42-0.44, 5: 0.44); two groups, 4 stages of 4: 0.437; two groups, 4 x 3: 0.470;
   // two groups, 8 x 2: 0.535.
-  static const int kps_env = getenv("MRL_L1_KPS") ? atoi(getenv("MRL_L1_KPS")) : 0;          // experiment knobs
-  static const int cg_env = getenv("MRL_L1_CGROUPS") ? atoi(getenv("MRL_L1_CGROUPS")) : 0;
   int kps = 0, nstages = 0, cgroups = 1;
   for (int pass = 0; pass < 2; ++pass) {
     // first choice: 4 k-groups per stage converted by two groups (needs an even ring of >= 4 stages, see TC_CGROUPS);
     // otherwise 3 per stage and one group
-    kps = kps_env > 0 ? kps_env : (pass == 0 ? 4 : 3);
+    kps = pass == 0 ? 4 : 3;
     const size_t sb = (size_t)kps * (TC_M * 8 * 4 + 2 * (size_t)nu * 8 * 4);
     nstages = (int)((227 * 1024 - 512) / sb);
     const int tmem_room = (512 - n_acc * acc_cols) / (kps * 16);
     if (nstages > tmem_room) nstages = tmem_room;
     if (nstages > TC_STAGES) nstages = TC_STAGES;
     cgroups = (pass == 0 && nstages >= 4) ? 2 : 1;
-    if (cg_env > 0) cgroups = (cg_env >= 2 && nstages >= 2) ? 2 : 1;
-    if (cgroups == 2) nstages &= ~1;
-    if (cgroups == 2 || cg_env > 0 || kps_env > 0) break;
+    if (cgroups == 2) {
+      nstages &= ~1;
+      break;
+    }
   }
   if (nstages < 2) return cudaErrorInvalidConfiguration;
   const size_t stage_bytes = (size_t)kps * (TC_M * 8 * 4 + 2 * (size_t)nu * 8 * 4);
@@ -560,7 +555,7 @@ static bool l1g_plan(const NetGeom& g, int* acc_stride, int* nts, int* nss, int*
 }
 
 cudaError_t launch_l1_grad_tc(const NetGeom& g, const float* XG, int xg_ftiles, const float* DG, float* part1,
-                              int slab_tiles, int n_tiles, int n_slabs, cudaStream_t st, int dg_mn_major) {
+                              int slab_tiles, int n_tiles, int n_slabs, cudaStream_t st) {
   const int nu = l1tc_nu(g);
   const int ftiles = (g.d[0] + TC_M - 1) / TC_M;
   int acc_stride, nts, nss, tmem_cols;
@@ -570,14 +565,12 @@ cudaError_t launch_l1_grad_tc(const NetGeom& g, const float* XG, int xg_ftiles, 
     cudaError_t e = mrl_func_smem((const void*)l1_grad_tc_kernel, smem);
     if (e != cudaSuccess) return e;
   }
-  static const int cg_env = getenv("MRL_L1_CGROUPS") ? atoi(getenv("MRL_L1_CGROUPS")) : 0;   // experiment knob
-  int cgroups = (nts >= 2 && nss >= 4) ? 2 : 1;   // two converter groups need even rings (see TC_CGROUPS)
-  if (cg_env > 0) cgroups = (cg_env >= 2 && nts >= 2 && nss >= 2) ? 2 : 1;
+  const int cgroups = (nts >= 2 && nss >= 4) ? 2 : 1;   // two converter groups need even rings (see TC_CGROUPS)
   if (cgroups == 2) { nts &= ~1; nss &= ~1; }
   const int sms = mrl_sm_count();
   const int grid = n_slabs < sms ? n_slabs : sms;
   l1_grad_tc_kernel<<<grid, TC_THREADS, smem, st>>>(XG, DG, part1, ftiles, xg_ftiles, nu, g.d[0], g.n1p, slab_tiles,
-                                                    n_tiles, n_slabs, acc_stride, tmem_cols, nss, nts, dg_mn_major, cgroups);
+                                                    n_tiles, n_slabs, acc_stride, tmem_cols, nss, nts, cgroups);
   return cudaGetLastError();
 }
 

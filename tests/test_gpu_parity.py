@@ -360,8 +360,9 @@ def test_ppo_lossgrad_golden(dev, golden, tag, ptag):
 @pytest.mark.parametrize("name,N", [("hopper", 160_001), ("humanoid", 20_000), ("cat128", 9_999),
                                     ("hopper", 7), ("humanoid", 65), ("cartpole", 129)])
 def test_chain_kernels_many_slabs(dev, name, N):
-    """The chain kernels (mlp_chain.cu) on batches that need several slabs per CTA (persistent loop, last slab and
-    last chain tile partial, N not a multiple of 64): losses, gradient and Fvp against the oracle."""
+    """The chain kernels on batches that need several slabs per CTA (persistent loop, last slab and last chain tile
+    partial, N not a multiple of 64): losses and gradient (mlp_chain.cu) and Fvp (the tcgen05 chain, mlp_fvp_tc.cu)
+    against the oracle."""
     from modular_rl_b200 import synth
     _, _, pm, *_ = _oracle()
     dims, head, _ = SHAPES[name]
