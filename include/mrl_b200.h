@@ -189,6 +189,40 @@ int mrl_net_adam_reset(mrl_net* net, void* stream);
 int mrl_population_forward(int device, int n_layers, const int* dims, int activation, const float* thetas,
                            long long ld_theta, const float* obs, int n_members, float* out, int loc, void* stream);
 
+/* ---------------------------------------------------------------- device-resident rollouts (core.py:182-221)
+ * The rollout loop of the two built-in environments (modular_rl_b200/envs.py) on the device: one launch runs one ROUND,
+ * n_envs environments from reset until every episode has ended or reached timestep_limit, in the lockstep order of
+ * core.rollouts_vectorized: per step the observation ZFilter over the live environments in index order, the policy
+ * forward on the net's parameters in place, the action draw, the float64 dynamics of envs.py and the reward ZFilter
+ * statistics.  Resets and action noise come from Philox4x32-10 keyed by `seed` (DESIGN.md "Device rollouts").
+ *   mrl_rollout_create: env MRL_ENV_CARTPOLE or MRL_ENV_PENDULUM; 1 <= n_envs <= mrl_rollout_max_envs().
+ *   mrl_rollout_run: `policy` must live on the handle's device, take the environment's observation and end in its
+ *     action head (CartPole: Categorical with 2 outputs; Pendulum: DiagGauss with d = 1).  A NULL filter cfg or
+ *     enabled == 0 is the identity.  ob_state = {n, M[ob_dim], S[ob_dim]} and rew_state = {n, M, S} (host) are read and
+ *     replaced by the states after the round; *_pushed (may be NULL) receive the statistics of this round's samples
+ *     alone.  want_states != 0 also records the raw environment state of every step.  Synchronises `stream`;
+ *     *n_timesteps = timesteps collected.
+ *   mrl_rollout_read: the last round, path-major (episode i = environment i): lengths int32[n_envs],
+ *     terminated uint8[n_envs], observation f64 [n x ob_dim] (filtered), action int32 [n] (Categorical) or
+ *     f32 [n x d] (DiagGauss), prob f32 [n x 2] (probabilities or [mean, std]), raw reward f64 [n],
+ *     states f64 [n x state_dim] (CartPole 4, Pendulum 2: (theta, theta_dot)).  Any pointer may be NULL. */
+#define MRL_ENV_CARTPOLE 0
+#define MRL_ENV_PENDULUM 1
+typedef struct mrl_rollout mrl_rollout;
+typedef struct {
+  int enabled, demean, destd;
+  double clip;   /* 0: no clipping */
+} mrl_zfilter_cfg;
+int mrl_rollout_max_envs(void);
+int mrl_rollout_create(mrl_rollout** out, int device, int env, int n_envs, int timestep_limit);
+int mrl_rollout_destroy(mrl_rollout* r);
+int mrl_rollout_run(mrl_rollout* r, mrl_net* policy, unsigned long long seed, int stochastic,
+                    const mrl_zfilter_cfg* ob_cfg, double* ob_state, double* ob_pushed,
+                    const mrl_zfilter_cfg* rew_cfg, double* rew_state, double* rew_pushed,
+                    int want_states, long long* n_timesteps, void* stream);
+int mrl_rollout_read(mrl_rollout* r, int* lengths, unsigned char* terminated, double* obs, void* act, float* prob,
+                     double* reward, double* states);
+
 #ifdef __cplusplus
 }
 #endif

@@ -15,6 +15,7 @@ HOST, DEVICE = 0, 1
 F32, F64, I32, I64 = 0, 1, 2, 3
 GAUSS, CATEGORICAL, VALUE = 0, 1, 2
 ACTIVATIONS = {"tanh": 0, "relu": 1, "sigmoid": 2}
+DEVICE_ENVS = {"cartpole": 0, "pendulum": 1}      # MRL_ENV_CARTPOLE, MRL_ENV_PENDULUM
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("MRL_LIB") or os.path.join(_HERE, "libmrl_b200.so")   # MRL_LIB: kernel experiments only
@@ -26,6 +27,10 @@ _DT = {np.dtype(np.float32): F32, np.dtype(np.float64): F64, np.dtype(np.int32):
 class TrpoCfg(C.Structure):
     _fields_ = [("cg_damping", C.c_double), ("max_kl", C.c_double), ("residual_tol", C.c_double),
                 ("accept_ratio", C.c_double), ("cg_iters", C.c_int), ("max_backtracks", C.c_int)]
+
+
+class ZFilterCfg(C.Structure):
+    _fields_ = [("enabled", C.c_int), ("demean", C.c_int), ("destd", C.c_int), ("clip", C.c_double)]
 
 
 _lib = None
@@ -84,6 +89,12 @@ _SIGS = {
     "mrl_comm_p2p_export": (_I, [_P, _LL, _P]),
     "mrl_comm_p2p_connect": (_I, [_P, _P]),
     "mrl_comm_p2p_enable": (_I, [_P, _I]),
+    "mrl_rollout_max_envs": (_I, []),
+    "mrl_rollout_create": (_I, [C.POINTER(_P), _I, _I, _I, _I]),
+    "mrl_rollout_destroy": (_I, [_P]),
+    "mrl_rollout_run": (_I, [_P, _P, C.c_ulonglong, _I, C.POINTER(ZFilterCfg), _P, _P, C.POINTER(ZFilterCfg), _P, _P,
+                             _I, C.POINTER(_LL), _P]),
+    "mrl_rollout_read": (_I, [_P, _P, _P, _P, _P, _P, _P, _P]),
 }
 
 

@@ -24,7 +24,7 @@ import scipy.optimize
 from . import _lib as L
 from . import distributions
 from . import parallel
-from .device import DeviceBatch, DeviceNet
+from .device import DeviceBatch, DeviceNet, DeviceRollouts
 from .misc_utils import *  # noqa: F401,F403  (the reference star-imports misc_utils too)
 from .misc_utils import EzPickle, explained_variance, explained_variance_2d, update_default_config
 
@@ -212,6 +212,10 @@ def run_policy_gradient_algorithm(env, agent, usercfg=None, callback=None):
 # 0 / 1 = the reference's serial rollouts.  Not an agent option - the reference's option tables stay unchanged -
 # but a process setting: MRL_VEC_ENVS in the environment or run_pg.py --vec_envs.
 VEC_ENVS = int(os.environ.get("MRL_VEC_ENVS", "0") or 0)
+# Environments per device-resident rollout round (0: host rollouts): the whole round of a built-in environment runs in
+# one kernel launch (do_rollouts_device).  Resets and action noise come from the device's Philox stream, not numpy's,
+# so the numbers differ from a host run with the same seed.  MRL_DEVICE_ENVS or run_pg.py --device_envs.
+DEVICE_ENVS = int(os.environ.get("MRL_DEVICE_ENVS", "0") or 0)
 
 
 def get_paths(env, agent, cfg, seed_iter):
@@ -220,6 +224,11 @@ def get_paths(env, agent, cfg, seed_iter):
     n_timesteps = cfg["timesteps_per_batch"]
     if parallel.context() is not None:           # this rank's share of the batch
         n_timesteps = parallel.rank_quota(n_timesteps, parallel.context().world)
+    if DEVICE_ENVS > 0:
+        if VEC_ENVS > 0:
+            raise ValueError("device rollouts (DEVICE_ENVS = %d) and host lockstep rollouts (VEC_ENVS = %d) are both set; "
+                             "choose one" % (DEVICE_ENVS, VEC_ENVS))
+        return do_rollouts_device(env, agent, cfg["timestep_limit"], n_timesteps, seed_iter, DEVICE_ENVS)
     if VEC_ENVS > 1:
         return do_rollouts_vectorized(env, agent, cfg["timestep_limit"], n_timesteps, seed_iter, VEC_ENVS)
     return do_rollouts_serial(env, agent, cfg["timestep_limit"], n_timesteps, seed_iter)
@@ -286,6 +295,84 @@ def do_rollouts_vectorized(env, agent, timestep_limit, n_timesteps, seed_iter, n
         for path in rollouts_vectorized(envs, agent, timestep_limit):
             paths.append(path)
             timesteps_sofar += pathlength(path)
+        if timesteps_sofar > n_timesteps:
+            break
+    return paths
+
+
+def _device_filter(filt, what):
+    """ZFilter -> the filter; IDENTITY -> None; anything else has no device implementation."""
+    from .filters import ZFilter
+    if filt is IDENTITY:
+        return None
+    if isinstance(filt, ZFilter):
+        return filt
+    raise TypeError("device rollouts support a ZFilter or IDENTITY as the %s, not %r" % (what, filt))
+
+
+def check_device_rollouts(env, agent):
+    """Raise, before anything runs, for what do_rollouts_device cannot run: an environment without a device
+    implementation, filters other than ZFilter / IDENTITY, a policy without a DeviceNet.  -> the env's device kind."""
+    from . import envs
+    kind = envs.device_kind(env)
+    _device_filter(agent.obfilter, "observation filter")
+    _device_filter(agent.rewfilter, "reward filter")
+    if not isinstance(getattr(agent.policy, "net", None), DeviceNet):
+        raise TypeError("device rollouts need a policy with a DeviceNet (StochPolicyMLP); %s has none"
+                        % type(agent.policy).__name__)
+    return kind
+
+
+_device_rollouts = {}        # (kind, n_envs, timestep_limit, device) -> DeviceRollouts: buffers kept across iterations
+
+
+def _filter_arg(filt):
+    return None if filt is None else (filt.rs.state(), filt.demean, filt.destd, filt.clip)
+
+
+def _advance_filter(filt, state, pushed):
+    """The filter takes the state after the round; a data-parallel iteration also merges the round's own samples into
+    `pushed` (parallel.sync_rollouts exchanges that)."""
+    filt.rs.set_state(*state)
+    if filt.pushed is not None:
+        filt.pushed.set_state(*parallel.merge_filter_states(filt.pushed.state(), [pushed]))
+
+
+def device_paths(out, categorical):
+    """Path dicts with the keys and dtypes of rollouts_vectorized from the compacted arrays of DeviceRollouts.run."""
+    offsets = np.concatenate([[0], np.cumsum(out["lengths"], dtype=np.int64)])
+    act = out["action"].astype(np.int64) if categorical else out["action"]
+    paths = []
+    for i in range(len(out["lengths"])):
+        a, b = offsets[i], offsets[i + 1]
+        paths.append({"observation": out["observation"][a:b], "action": act[a:b], "prob": out["prob"][a:b],
+                      "reward": out["reward"][a:b], "terminated": bool(out["terminated"][i])})
+    return paths
+
+
+def do_rollouts_device(env, agent, timestep_limit, n_timesteps, seed_iter, n_envs):
+    """do_rollouts_vectorized with each round of n_envs environments run on the device in one kernel launch: one
+    next(seed_iter) per round (the Philox key of its resets and action draws), rounds until more than n_timesteps are
+    collected (strict, core.py:219)."""
+    kind = check_device_rollouts(env, agent)
+    net = agent.policy.net
+    key = (kind, int(n_envs), int(timestep_limit), net.device)
+    if key not in _device_rollouts:
+        _device_rollouts[key] = DeviceRollouts(env, n_envs, timestep_limit, device=net.device)
+    ro = _device_rollouts[key]
+    obf = _device_filter(agent.obfilter, "observation filter")
+    rwf = _device_filter(agent.rewfilter, "reward filter")
+    stochastic = getattr(agent, "stochastic", True)
+    paths = []
+    timesteps_sofar = 0
+    while True:
+        out = ro.run(net, next(seed_iter), stochastic, _filter_arg(obf), _filter_arg(rwf))
+        if obf is not None:
+            _advance_filter(obf, out["ob_state"], out["ob_pushed"])
+        if rwf is not None:
+            _advance_filter(rwf, out["rew_state"], out["rew_pushed"])
+        paths += device_paths(out, ro.categorical)
+        timesteps_sofar += len(out["reward"])
         if timesteps_sofar > n_timesteps:
             break
     return paths

@@ -45,10 +45,10 @@ static int fail(const char* fmt, ...) {
   } while (0)
 
 // ---- optional per-kernel-class timing with CUDA events on the launching stream (bench.py's roofline)
-enum { PK_L1F = 0, PK_MIDF, PK_MIDB_GRAD, PK_MIDB_FVP, PK_L1G, PK_REDUCE, PK_CG, PK_GAE, PK_PACK, PK_COUNT };
+enum { PK_L1F = 0, PK_MIDF, PK_MIDB_GRAD, PK_MIDB_FVP, PK_L1G, PK_REDUCE, PK_CG, PK_GAE, PK_PACK, PK_ROLLOUT, PK_COUNT };
 static const char* kPkNames[PK_COUNT] = {"l1_forward", "mid_forward", "mid_backward_grad", "mid_backward_fvp",
                                          "l1_grad",    "reduce",      "cg_vector",         "gae",
-                                         "pack_params"};
+                                         "pack_params", "rollout"};
 struct Prof {
   bool on = false;
   std::vector<cudaEvent_t> pool;
@@ -1265,5 +1265,170 @@ extern "C" int mrl_net_get_trpo_vectors(mrl_net* n, double* stepdir, double* ful
     scalars[0] = n->h_cg->shs; scalars[1] = n->h_cg->lm; scalars[2] = n->h_cg->expected_rate;
     scalars[3] = n->h_cg->rdotr;
   }
+  return 0;
+}
+
+// ======================================================================== device-resident rollouts (rollout.cu)
+struct mrl_rollout {
+  int device = 0, env = 0, N = 0, T = 0, d0 = 0, sd = 0, dout = 0, head = 0;
+  DevBuf s_obs, s_state, s_prob, s_act, s_rew, lengths, term, headbuf, body, filt;
+  double* h_head = nullptr;      // pinned: header, then lengths int32[N], terminated int32[N]
+  double* h_filt = nullptr;      // pinned: incoming filter states
+  char* h_body = nullptr;        // pinned: compacted rows of the last round
+  size_t h_body_cap = 0;
+  long long total = 0;
+  int with_states = 0;
+};
+static int ro_head_doubles(int d0) { return 9 + 4 * d0; }
+
+extern "C" int mrl_rollout_max_envs(void) { return RO_MAX_ENVS; }
+
+extern "C" int mrl_rollout_destroy(mrl_rollout* r) {
+  if (!r) return 0;
+  cudaSetDevice(r->device);
+  DevBuf* bufs[] = {&r->s_obs, &r->s_state, &r->s_prob, &r->s_act, &r->s_rew, &r->lengths, &r->term, &r->headbuf,
+                    &r->body, &r->filt};
+  for (DevBuf* d : bufs) d->release();
+  if (r->h_head) cudaFreeHost(r->h_head);
+  if (r->h_filt) cudaFreeHost(r->h_filt);
+  if (r->h_body) cudaFreeHost(r->h_body);
+  delete r;
+  return 0;
+}
+
+extern "C" int mrl_rollout_create(mrl_rollout** out, int device, int env, int n_envs, int timestep_limit) {
+  if (!out) return fail("mrl_rollout_create: null output");
+  int d0, sd, dout;
+  const int head = rollout_env_dims(env, &d0, &sd, &dout);
+  if (head < 0) return fail("mrl_rollout_create: unknown env %d (MRL_ENV_CARTPOLE or MRL_ENV_PENDULUM)", env);
+  if (n_envs < 1 || n_envs > RO_MAX_ENVS)
+    return fail("mrl_rollout_create: n_envs = %d; the rollout kernel runs 1..%d environments per round", n_envs, RO_MAX_ENVS);
+  if (timestep_limit < 1) return fail("mrl_rollout_create: timestep_limit must be >= 1");
+  CK(cudaSetDevice(device));
+  mrl_rollout* r = new mrl_rollout();
+  r->device = device; r->env = env; r->N = n_envs; r->T = timestep_limit;
+  r->d0 = d0; r->sd = sd; r->dout = dout; r->head = head;
+  const size_t rows = (size_t)n_envs * timestep_limit;
+  const RolloutLayout lay = rollout_layout((long long)rows, d0, sd, 2, head == MRL_HEAD_CAT ? 1 : dout, 1);
+  cudaError_t e = cudaSuccess;
+  auto R = [&](DevBuf& b, size_t bytes) { if (e == cudaSuccess) e = b.reserve(bytes); };
+  R(r->s_obs, rows * d0 * 8); R(r->s_state, rows * sd * 8); R(r->s_prob, rows * 2 * 4);
+  R(r->s_act, rows * dout * 4); R(r->s_rew, rows * 8); R(r->lengths, (size_t)n_envs * 4); R(r->term, (size_t)n_envs * 4);
+  R(r->headbuf, (size_t)ro_head_doubles(d0) * 8); R(r->body, lay.end); R(r->filt, (size_t)(4 + 2 * d0) * 8);
+  const size_t hb = (size_t)ro_head_doubles(d0) * 8 + (size_t)n_envs * 8;
+  if (e == cudaSuccess) e = cudaMallocHost(&r->h_head, hb);
+  if (e == cudaSuccess) e = cudaMallocHost(&r->h_filt, (size_t)(4 + 2 * d0) * 8);
+  if (e != cudaSuccess) {
+    mrl_rollout_destroy(r);
+    return fail("mrl_rollout_create: %s", cudaGetErrorString(e));
+  }
+  *out = r;
+  return 0;
+}
+
+extern "C" int mrl_rollout_run(mrl_rollout* r, mrl_net* policy, unsigned long long seed, int stochastic,
+                               const mrl_zfilter_cfg* ob_cfg, double* ob_state, double* ob_pushed,
+                               const mrl_zfilter_cfg* rew_cfg, double* rew_state, double* rew_pushed,
+                               int want_states, long long* n_timesteps, void* stream) {
+  if (!r || !policy || !n_timesteps) return fail("mrl_rollout_run: bad arguments");
+  const bool ob_on = ob_cfg && ob_cfg->enabled, rew_on = rew_cfg && rew_cfg->enabled;
+  if ((ob_on && !ob_state) || (rew_on && !rew_state)) return fail("mrl_rollout_run: an enabled filter needs its state");
+  const NetGeom& g = policy->g;
+  const char* env_name = r->env == MRL_ENV_CARTPOLE ? "CartPole" : "Pendulum";
+  if (policy->device != r->device)
+    return fail("mrl_rollout_run: the policy lives on device %d, the rollouts on device %d", policy->device, r->device);
+  if (g.d[0] != r->d0)
+    return fail("mrl_rollout_run: %s observations have %d entries, the policy takes %d", env_name, r->d0, g.d[0]);
+  if (g.head != r->head || g.d[g.L] != r->dout)
+    return fail("mrl_rollout_run: %s needs a %s head with %d outputs (the policy has a %s head with %d)", env_name,
+                r->head == MRL_HEAD_CAT ? "Categorical" : "DiagGauss", r->dout,
+                g.head == MRL_HEAD_CAT ? "Categorical" : (g.head == MRL_HEAD_GAUSS ? "DiagGauss" : "value"), g.d[g.L]);
+  CK(cudaSetDevice(r->device));
+  cudaStream_t st = (cudaStream_t)stream;
+  const int d0 = r->d0;
+
+  RolloutArgs a = {};
+  a.N = r->N; a.T = r->T;
+  int n_ctas, threads;
+  rollout_shape(r->N, &n_ctas, &a.per_cta, &threads);
+  a.L = g.L;
+  int wmax = 1;
+  for (int l = 0; l <= g.L; ++l) {
+    a.d[l] = g.d[l];
+    if (l > 0 && l < g.L && g.d[l] > wmax) wmax = g.d[l];
+  }
+  a.P = g.P;
+  a.ldh = wmax + 1;                               // odd stride: the rows of one warp fall into distinct banks
+  a.rows_chunk = 8192 / a.ldh < 128 ? 8192 / a.ldh : 128;   // 64 KB of activations
+  a.w_floats = (size_t)g.P * 4 <= 128 * 1024 ? g.P : 0;
+  a.theta = policy->theta.as<float>();
+  a.seed = seed;
+  a.stochastic = stochastic != 0;
+  a.ob_on = ob_on; a.rew_on = rew_on;
+  a.ob_demean = ob_on && ob_cfg->demean; a.ob_destd = ob_on && ob_cfg->destd; a.ob_clip = ob_on ? ob_cfg->clip : 0.0;
+  double* hf = r->h_filt;
+  for (int i = 0; i < 4 + 2 * d0; ++i) hf[i] = 0.0;
+  if (ob_on) for (int i = 0; i < 1 + 2 * d0; ++i) hf[i] = ob_state[i];
+  if (rew_on) for (int i = 0; i < 3; ++i) hf[1 + 2 * d0 + i] = rew_state[i];
+  CK(cudaMemcpyAsync(r->filt.p, hf, (size_t)(4 + 2 * d0) * 8, cudaMemcpyHostToDevice, st));
+  a.filt_in = r->filt.as<double>();
+  a.s_obs = r->s_obs.as<double>(); a.s_state = want_states ? r->s_state.as<double>() : nullptr;
+  a.s_prob = r->s_prob.as<float>(); a.s_act = r->s_act.p; a.s_rew = r->s_rew.as<double>();
+  a.lengths = r->lengths.as<int>(); a.term = r->term.as<int>();
+  a.head = r->headbuf.as<double>(); a.body = r->body.as<char>();
+  const size_t smem = rollout_smem_bytes(a, d0, r->dout);
+  int dev_smem = 0;
+  CK(cudaDeviceGetAttribute(&dev_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, r->device));
+  if (smem + 16384 > (size_t)dev_smem)
+    return fail("mrl_rollout_run: the rollout kernel needs %zu B of shared memory per CTA, device offers %d", smem, dev_smem);
+  CKP(PK_ROLLOUT, launch_rollout(a, r->env, g.act, n_ctas, threads, smem, st), 1);
+
+  // header + lengths + terminated, then the collected rows only
+  const int nh = ro_head_doubles(d0);
+  int* h_len = (int*)(r->h_head + nh);
+  CK(cudaMemcpyAsync(r->h_head, r->headbuf.p, (size_t)nh * 8, cudaMemcpyDeviceToHost, st));
+  CK(cudaMemcpyAsync(h_len, r->lengths.p, (size_t)r->N * 4, cudaMemcpyDeviceToHost, st));
+  CK(cudaMemcpyAsync(h_len + r->N, r->term.p, (size_t)r->N * 4, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  const double* h = r->h_head;
+  r->total = (long long)h[0];
+  r->with_states = want_states != 0;
+  const RolloutLayout lay = rollout_layout(r->total, d0, r->sd, 2, r->head == MRL_HEAD_CAT ? 1 : r->dout,
+                                           r->with_states);
+  if (lay.end > r->h_body_cap) {
+    if (r->h_body) cudaFreeHost(r->h_body);
+    r->h_body = nullptr;
+    r->h_body_cap = 0;
+    CK(cudaMallocHost(&r->h_body, lay.end + lay.end / 4 + 256));
+    r->h_body_cap = lay.end + lay.end / 4 + 256;
+  }
+  if (lay.end) CK(cudaMemcpyAsync(r->h_body, r->body.p, lay.end, cudaMemcpyDeviceToHost, st));
+  CK(cudaStreamSynchronize(st));
+  if (ob_on) {
+    for (int i = 0; i < 1 + 2 * d0; ++i) ob_state[i] = h[1 + i];
+    if (ob_pushed) for (int i = 0; i < 1 + 2 * d0; ++i) ob_pushed[i] = h[2 + 2 * d0 + i];
+  }
+  if (rew_on) {
+    for (int i = 0; i < 3; ++i) rew_state[i] = h[3 + 4 * d0 + i];
+    if (rew_pushed) for (int i = 0; i < 3; ++i) rew_pushed[i] = h[6 + 4 * d0 + i];
+  }
+  *n_timesteps = r->total;
+  return 0;
+}
+
+extern "C" int mrl_rollout_read(mrl_rollout* r, int* lengths, unsigned char* terminated, double* obs, void* act,
+                                float* prob, double* reward, double* states) {
+  if (!r) return fail("mrl_rollout_read: null handle");
+  if (states && !r->with_states) return fail("mrl_rollout_read: the last round did not record states (want_states = 0)");
+  const int* h_len = (const int*)(r->h_head + ro_head_doubles(r->d0));
+  if (lengths) memcpy(lengths, h_len, (size_t)r->N * 4);
+  if (terminated) for (int i = 0; i < r->N; ++i) terminated[i] = (unsigned char)h_len[r->N + i];
+  const long long n = r->total;
+  const RolloutLayout lay = rollout_layout(n, r->d0, r->sd, 2, r->head == MRL_HEAD_CAT ? 1 : r->dout, r->with_states);
+  if (obs) memcpy(obs, r->h_body + lay.obs, (size_t)n * r->d0 * 8);
+  if (reward) memcpy(reward, r->h_body + lay.rew, (size_t)n * 8);
+  if (states) memcpy(states, r->h_body + lay.state, (size_t)n * r->sd * 8);
+  if (prob) memcpy(prob, r->h_body + lay.prob, (size_t)n * 2 * 4);
+  if (act) memcpy(act, r->h_body + lay.act, (size_t)n * (r->head == MRL_HEAD_CAT ? 1 : r->dout) * 4);
   return 0;
 }

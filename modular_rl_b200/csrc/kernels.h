@@ -143,3 +143,43 @@ cudaError_t launch_zfilter_scan(const void* x, int x_f64, long long N, int d, do
                                 int demean, int destd, double clip, void* y, int y_f64, double* scratch,
                                 cudaStream_t st);
 long long zfilter_scratch_doubles(long long N, int d);
+
+// ---- rollout.cu  (device-resident rollouts of the built-in environments, one cluster launch per round)
+#define RO_MAX_CTAS 8          // CTAs of the round's cluster (the portable cluster size)
+#define RO_MAX_THREADS 512     // environments (threads) per CTA
+#define RO_MIN_PER_CTA 32      // fewer environments per CTA than this: use fewer CTAs
+#define RO_MAX_ENVS (RO_MAX_CTAS * RO_MAX_THREADS)
+struct RolloutArgs {
+  int N, T, per_cta;           // environments, timestep limit, environments per CTA
+  int L, d[MRL_MAX_LAYERS + 1], P;
+  int w_floats;                // theta floats staged in shared memory (0: read through L2)
+  int rows_chunk, ldh;         // forward: rows per chunk, activation row stride (floats)
+  const float* theta;          // the policy's flat parameters (reference order), read in place
+  unsigned long long seed;
+  int stochastic;
+  int ob_on, ob_demean, ob_destd, rew_on;
+  double ob_clip;
+  const double* filt_in;       // (n, M[d0], S[d0]) of the observation filter, then (n, M, S) of the reward filter
+  // [T][N] staging rows
+  double* s_obs; double* s_state /* nullptr: not recorded */; float* s_prob; void* s_act; double* s_rew;
+  int* lengths; int* term;
+  double* head;                // total, observation state, its round part, reward state, its round part
+  char* body;                  // compacted path-major rows (rollout_layout)
+};
+// Byte offsets of the compacted arrays for n timesteps: f64 sections first, so that every section stays aligned
+struct RolloutLayout { size_t obs, rew, state, prob, act, end; };
+__host__ __device__ inline RolloutLayout rollout_layout(long long n, int d0, int sd, int pd, int ad, int with_states) {
+  RolloutLayout o;
+  size_t p = 0;
+  o.obs = p;   p += (size_t)n * d0 * 8;
+  o.rew = p;   p += (size_t)n * 8;
+  o.state = p; p += with_states ? (size_t)n * sd * 8 : 0;
+  o.prob = p;  p += (size_t)n * pd * 4;
+  o.act = p;   p += (size_t)n * ad * 4;     // int32 (Categorical) or float32 [d] (DiagGauss)
+  o.end = p;
+  return o;
+}
+int rollout_env_dims(int env, int* d0, int* sd, int* dout);   // -> head, -1 for an unknown env
+void rollout_shape(int N, int* n_ctas, int* per_cta, int* threads);
+size_t rollout_smem_bytes(const RolloutArgs& a, int d0, int dout);
+cudaError_t launch_rollout(const RolloutArgs& a, int env, int act, int n_ctas, int threads, size_t smem, cudaStream_t st);

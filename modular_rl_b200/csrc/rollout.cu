@@ -1,0 +1,480 @@
+// Device-resident rollouts of the two built-in environments (envs.py: CartPole-v0, Pendulum-v0).
+//
+// One launch runs one ROUND: N environments from reset until every episode has ended or reached the timestep limit,
+// in the lockstep order of core.rollouts_vectorized (core.py:182-221 run per environment).  Per step t, over the
+// environments still live, in index order:
+//   observation ZFilter (filters.py:30-38): sample j is normalised with Welford statistics that include the incoming
+//     state and every live sample of this step with a smaller index, itself included;
+//   policy forward (FP32) on the float32 cast of the filtered observation, reading the net's flat theta;
+//   action: Categorical inverse-CDF sample / DiagGauss mean + std * z, or maxprob when not stochastic;
+//   dynamics in float64 with the equations and evaluation order of envs.py;
+//   reward ZFilter: the raw rewards of the step advance its statistics (only they matter, SURVEY A.5).
+//
+// Layout: ONE thread-block cluster (<= RO_MAX_CTAS CTAs) per round; CTA c owns environments [c * per_cta, ...), one
+// environment per thread.  The ZFilter prefix crosses every environment at every step: each CTA scans its own
+// environments (Kogge-Stone Chan merges inside a warp, then the warp totals in order), publishes its total in its
+// shared memory, and after the cluster barrier every CTA folds the totals of the lower-ranked CTAs from distributed
+// shared memory in rank order.  One cluster barrier per step; the slots are double-buffered by step parity so that a
+// slot is never rewritten before every CTA has read it.  The merge tree depends on N only (not on timing), so a round
+// is deterministic.  The reward statistics of step t travel with the exchange of step t + 1.
+//
+// Forward: the live environments of a CTA are compacted (their rank in the scan) and pushed through the MLP in chunks
+// of rows; thread o computes output unit o % dout of row o / dout with an in-order FP32 FMA chain, activations of
+// the chunk in shared memory, theta staged in shared memory when it fits (4-64-64-2 is 18 KB), else read through L2.
+//
+// Random numbers: Philox4x32-10 keyed by the round seed, counter (environment, step, purpose, block), so no draw
+// depends on the thread / CTA mapping.  DESIGN.md "Device rollouts" gives the mapping to uniforms and normals.
+//
+// After the round the rows, staged as [step][environment], are compacted into path-major order (offsets from a scan of
+// the episode lengths) in the same launch, so the host copies only the collected timesteps.
+#include "common.cuh"
+#include "kernels.h"
+#include "../../include/mrl_b200.h"
+
+#include <cooperative_groups.h>
+namespace cgr = cooperative_groups;
+
+#define RO_KMAX 5   // observation features + the reward, scanned together
+
+// ---------------------------------------------------------------------------------------------------- Philox4x32-10
+__device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint32_t k0, uint32_t k1) {
+#pragma unroll
+  for (int i = 0; i < 10; ++i) {
+    if (i) { k0 += 0x9E3779B9u; k1 += 0xBB67AE85u; }
+    const uint32_t lo0 = 0xD2511F53u * c.x, hi0 = __umulhi(0xD2511F53u, c.x);
+    const uint32_t lo1 = 0xCD9E8D57u * c.z, hi1 = __umulhi(0xCD9E8D57u, c.z);
+    c = make_uint4(hi1 ^ c.y ^ k0, lo1, hi0 ^ c.w ^ k1, lo0);
+  }
+  return c;
+}
+// 53-bit uniform in [0, 1) from two words: the high word gives the top 32 bits, the high 21 bits of the low word the rest
+__device__ __forceinline__ double u53(uint32_t hi, uint32_t lo) {
+  return (double)(((unsigned long long)hi << 21) | (lo >> 11)) * 0x1p-53;
+}
+enum { RO_PURPOSE_RESET = 0, RO_PURPOSE_ACTION = 1 };
+
+// ---------------------------------------------------------------------------------------------------- Welford
+struct Wf { double n, m, s; };
+__device__ __forceinline__ Wf wf_merge(const Wf& a, const Wf& b) {   // Chan merge, `a` holds the earlier samples
+  if (b.n == 0.0) return a;
+  if (a.n == 0.0) return b;
+  Wf o;
+  o.n = a.n + b.n;
+  const double d = b.m - a.m;
+  o.m = a.m + d * (b.n / o.n);
+  o.s = a.s + b.s + d * d * (a.n * b.n / o.n);
+  return o;
+}
+__device__ __forceinline__ Wf wf_shfl_up(const Wf& w, int o) {
+  Wf r;
+  r.n = __shfl_up_sync(0xffffffffu, w.n, o);
+  r.m = __shfl_up_sync(0xffffffffu, w.m, o);
+  r.s = __shfl_up_sync(0xffffffffu, w.s, o);
+  return r;
+}
+
+// Inclusive scan of K Welford triples over the CTA's threads in index order; `tot` receives the CTA totals.
+template <int K>
+__device__ __forceinline__ void block_scan(Wf (&w)[K], Wf (*wtot)[RO_KMAX], Wf* tot) {
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+#pragma unroll
+    for (int k = 0; k < K; ++k) {
+      const Wf u = wf_shfl_up(w[k], o);
+      if (lane >= o) w[k] = wf_merge(u, w[k]);
+    }
+  }
+  __syncthreads();                       // the previous readers of wtot are done
+  if (lane == 31)
+#pragma unroll
+    for (int k = 0; k < K; ++k) wtot[warp][k] = w[k];
+  __syncthreads();
+  if (threadIdx.x < K) {                 // exclusive prefix of the warp totals, in warp order
+    const int k = threadIdx.x;
+    Wf acc = {0.0, 0.0, 0.0};
+    for (int i = 0; i < nw; ++i) {
+      const Wf t = wtot[i][k];
+      wtot[i][k] = acc;
+      acc = wf_merge(acc, t);
+    }
+    tot[k] = acc;
+  }
+  __syncthreads();
+#pragma unroll
+  for (int k = 0; k < K; ++k) w[k] = wf_merge(wtot[warp][k], w[k]);
+}
+
+// ---------------------------------------------------------------------------------------------------- environments
+template <int ENV> struct EnvT;
+template <> struct EnvT<MRL_ENV_CARTPOLE> {
+  static constexpr int D0 = 4, SD = 4, DOUT = 2, PD = 2, HEAD = MRL_HEAD_CAT;   // prob row: 2 probabilities
+  __device__ static void reset(double* s, int e, uint32_t k0, uint32_t k1) {   // uniform(-0.05, 0.05, size=4)
+    const uint4 a = philox4x32_10(make_uint4((uint32_t)e, 0u, RO_PURPOSE_RESET, 0u), k0, k1);
+    const uint4 b = philox4x32_10(make_uint4((uint32_t)e, 0u, RO_PURPOSE_RESET, 1u), k0, k1);
+    const double u[4] = {u53(a.x, a.y), u53(a.z, a.w), u53(b.x, b.y), u53(b.z, b.w)};
+#pragma unroll
+    for (int i = 0; i < 4; ++i) s[i] = -0.05 + (0.05 - -0.05) * u[i];
+  }
+  __device__ static void obs(const double* s, double* x) {
+#pragma unroll
+    for (int i = 0; i < 4; ++i) x[i] = s[i];
+  }
+  // envs.py CartPoleEnv.step; reward 1.0 on every step, the terminating one included
+  __device__ static bool step(double* s, int action, float, double* reward) {
+    const double gravity = 9.8, masscart = 1.0, masspole = 0.1, length = 0.5, force_mag = 10.0, tau = 0.02;
+    const double theta_threshold = 12 * 2 * M_PI / 360, x_threshold = 2.4;
+    const double x = s[0], x_dot = s[1], th = s[2], th_dot = s[3];
+    const double force = action == 1 ? force_mag : -force_mag;
+    const double total_mass = masspole + masscart;
+    const double pml = masspole * length;
+    const double c = cos(th), sn = sin(th);
+    const double temp = (force + pml * th_dot * th_dot * sn) / total_mass;
+    const double thacc = (gravity * sn - c * temp) / (length * (4.0 / 3.0 - masspole * c * c / total_mass));
+    const double xacc = temp - pml * thacc * c / total_mass;
+    s[0] = x + tau * x_dot;
+    s[1] = x_dot + tau * xacc;
+    s[2] = th + tau * th_dot;
+    s[3] = th_dot + tau * thacc;
+    *reward = 1.0;
+    return s[0] < -x_threshold || s[0] > x_threshold || s[2] < -theta_threshold || s[2] > theta_threshold;
+  }
+};
+__device__ __forceinline__ double py_mod(double a, double b) {   // Python's float %: the sign of the divisor
+  double r = fmod(a, b);
+  if (r != 0.0) {
+    if ((b < 0.0) != (r < 0.0)) r += b;
+  } else {
+    r = copysign(0.0, b);
+  }
+  return r;
+}
+template <> struct EnvT<MRL_ENV_PENDULUM> {
+  static constexpr int D0 = 3, SD = 2, DOUT = 1, PD = 2, HEAD = MRL_HEAD_GAUSS;  // prob row: mean, std
+  __device__ static void reset(double* s, int e, uint32_t k0, uint32_t k1) {   // uniform([-pi, -1], [pi, 1])
+    const uint4 a = philox4x32_10(make_uint4((uint32_t)e, 0u, RO_PURPOSE_RESET, 0u), k0, k1);
+    s[0] = -M_PI + (M_PI - -M_PI) * u53(a.x, a.y);
+    s[1] = -1.0 + (1.0 - -1.0) * u53(a.z, a.w);
+  }
+  __device__ static void obs(const double* s, double* x) {
+    x[0] = cos(s[0]);
+    x[1] = sin(s[0]);
+    x[2] = s[1];
+  }
+  // envs.py PendulumEnv.step: u clipped for the dynamics and the cost only; the new angle uses the unclipped velocity
+  __device__ static bool step(double* s, int, float action, double* reward) {
+    const double max_speed = 8.0, max_torque = 2.0, dt = 0.05, g = 10.0, m = 1.0, l = 1.0;
+    const double th = s[0], thdot = s[1];
+    const double u = fmin(fmax((double)action, -max_torque), max_torque);
+    const double angle = py_mod(th + M_PI, 2 * M_PI) - M_PI;
+    const double cost = angle * angle + .1 * thdot * thdot + .001 * (u * u);
+    double newthdot = thdot + (-3 * g / (2 * l) * sin(th + M_PI) + 3. / (m * l * l) * u) * dt;
+    const double newth = th + newthdot * dt;
+    newthdot = fmin(fmax(newthdot, -max_speed), max_speed);
+    s[0] = newth;
+    s[1] = newthdot;
+    *reward = -cost;
+    return false;
+  }
+};
+
+// ---------------------------------------------------------------------------------------------------- policy forward
+// rows [0, nrows) of xin [nrows][d0] -> out [nrows][dout]: raw head output (softmax logits / Gauss mean)
+template <int ACT>
+__device__ void mlp_rows(const RolloutArgs& a, const float* W, const float* xin, int nrows, float* h, float* out) {
+  for (int c0 = 0; c0 < nrows; c0 += a.rows_chunk) {
+    const int nr = min(a.rows_chunk, nrows - c0);
+    const float* src = xin + (size_t)c0 * a.d[0];
+    int lds = a.d[0], cur = 0;
+    const float* th = W;
+    for (int l = 1; l <= a.L; ++l) {
+      const int din = a.d[l - 1], dout = a.d[l];
+      const float* Wl = th;                        // [din][dout], C order (the reference's flat order)
+      const float* bl = th + (size_t)din * dout;
+      const bool last = l == a.L;
+      float* dst = last ? out + (size_t)c0 * dout : h + (size_t)cur * a.rows_chunk * a.ldh;
+      const int ldd = last ? dout : a.ldh;
+      for (int o = threadIdx.x; o < nr * dout; o += blockDim.x) {
+        const int r = o / dout, j = o - r * dout;
+        const float* hr = src + (size_t)r * lds;
+        float acc = 0.f;
+        for (int k = 0; k < din; ++k) acc = fmaf(hr[k], Wl[(size_t)k * dout + j], acc);
+        acc += bl[j];
+        dst[(size_t)r * ldd + j] = last ? acc : act_fn<ACT>(acc);
+      }
+      __syncthreads();
+      src = dst;
+      lds = ldd;
+      cur ^= 1;
+      th += (size_t)din * dout + dout;
+    }
+  }
+}
+
+// ---------------------------------------------------------------------------------------------------- the round
+template <int ENV, int ACT>
+__global__ void __launch_bounds__(RO_MAX_THREADS, 1) rollout_kernel(const RolloutArgs a) {
+  using E = EnvT<ENV>;
+  constexpr int D0 = E::D0, SD = E::SD, DOUT = E::DOUT, PD = E::PD, K = D0 + 1;   // K - 1: the reward
+  cgr::cluster_group cluster = cgr::this_cluster();
+  const int rank = (int)cluster.block_rank(), nc = (int)cluster.num_blocks();
+
+  __shared__ Wf slot[2][RO_KMAX];          // this CTA's totals of the step (read by every CTA of the cluster)
+  __shared__ Wf wtot[RO_MAX_THREADS / 32][RO_KMAX];
+  __shared__ Wf ctatot[RO_KMAX];
+  __shared__ Wf pre[RO_KMAX];              // filter state + totals of the lower-ranked CTAs (this step)
+  __shared__ Wf run[RO_KMAX];              // running filter states: observation features, reward
+  __shared__ Wf pushed[RO_KMAX];           // statistics of this round's samples alone
+  __shared__ double live_total;
+  __shared__ long long lslot, lbase, ltotal;
+  __shared__ long long wlen[RO_MAX_THREADS / 32];
+  extern __shared__ __align__(16) float dsm[];
+  float* Ws = dsm;                                            // theta (a.w_floats; 0 when read through L2)
+  float* H = Ws + a.w_floats;                                 // [2][rows_chunk][ldh]
+  float* XIN = H + 2 * (size_t)a.rows_chunk * a.ldh;          // [per_cta][D0]
+  float* OUT = XIN + (size_t)a.per_cta * D0;                  // [per_cta][DOUT]
+
+  for (int i = threadIdx.x; i < a.w_floats; i += blockDim.x) Ws[i] = a.theta[i];
+  const float* W = a.w_floats ? Ws : a.theta;
+  if (threadIdx.x < K) {
+    const int k = threadIdx.x;
+    const double* f = a.filt_in;
+    run[k] = k < D0 ? Wf{f[0], f[1 + k], f[1 + D0 + k]} : Wf{f[1 + 2 * D0], f[2 + 2 * D0], f[3 + 2 * D0]};
+    pushed[k] = Wf{0.0, 0.0, 0.0};
+  }
+
+  const uint32_t k0 = (uint32_t)a.seed, k1 = (uint32_t)(a.seed >> 32);
+  const int le = threadIdx.x, e = rank * a.per_cta + le;
+  const bool mine = le < a.per_cta && e < a.N;
+  double s[SD];
+  if (mine) E::reset(s, e, k0, k1);
+  else
+#pragma unroll
+    for (int i = 0; i < SD; ++i) s[i] = 0.0;
+  bool live = mine, term = false, rlive = false;
+  double rew = 0.0;
+  int len = 0;
+  float logstd_exp[DOUT];
+#pragma unroll
+  for (int j = 0; j < DOUT; ++j) logstd_exp[j] = E::HEAD == MRL_HEAD_GAUSS ? expf(a.theta[a.P - DOUT + j]) : 0.f;
+
+  for (int t = 0;; ++t) {
+    const bool now = live && t < a.T;
+    double x[D0];
+    E::obs(s, x);
+    Wf w[K];
+#pragma unroll
+    for (int k = 0; k < D0; ++k) w[k] = now ? Wf{1.0, x[k], 0.0} : Wf{0.0, 0.0, 0.0};
+    w[D0] = rlive ? Wf{1.0, rew, 0.0} : Wf{0.0, 0.0, 0.0};   // the rewards of step t - 1
+    block_scan<K>(w, wtot, ctatot);
+    if (threadIdx.x < K) slot[t & 1][threadIdx.x] = ctatot[threadIdx.x];
+    cluster.sync();
+    if (threadIdx.x < K) {
+      const int k = threadIdx.x;
+      Wf tot = {0.0, 0.0, 0.0}, excl = {0.0, 0.0, 0.0};
+      for (int r = 0; r < nc; ++r) {
+        const Wf v = *cluster.map_shared_rank(&slot[t & 1][k], r);
+        if (r < rank) excl = wf_merge(excl, v);
+        tot = wf_merge(tot, v);
+      }
+      const bool on = k < D0 ? a.ob_on : a.rew_on;
+      pre[k] = wf_merge(run[k], excl);
+      if (on) {
+        run[k] = wf_merge(run[k], tot);
+        pushed[k] = wf_merge(pushed[k], tot);
+      }
+      if (k == 0) live_total = tot.n;
+    }
+    __syncthreads();
+    if (live_total == 0.0) break;          // every episode has ended (or t == T): uniform over the cluster
+    rlive = false;
+    const int row = (int)w[0].n - 1;       // rank of this environment among the CTA's live ones
+    const int nlive = (int)ctatot[0].n;
+    const size_t st_row = (size_t)t * a.N + e;
+    if (now) {
+#pragma unroll
+      for (int k = 0; k < D0; ++k) {
+        double y = x[k];
+        if (a.ob_on) {
+          const Wf f = wf_merge(pre[k], w[k]);
+          if (a.ob_demean) y = y - f.m;
+          if (a.ob_destd) {
+            const double var = f.n > 1.0 ? f.s / (f.n - 1.0) : f.m * f.m;   // running_stat.py:26-27
+            y = y / (sqrt(var) + 1e-8);
+          }
+          if (a.ob_clip != 0.0) y = fmin(fmax(y, -a.ob_clip), a.ob_clip);
+        }
+        a.s_obs[st_row * D0 + k] = y;
+        XIN[row * D0 + k] = (float)y;
+      }
+      if (a.s_state)
+#pragma unroll
+        for (int i = 0; i < SD; ++i) a.s_state[st_row * SD + i] = s[i];
+    }
+    __syncthreads();
+    mlp_rows<ACT>(a, W, XIN, nlive, H, OUT);
+    if (now) {
+      const uint4 rnd = philox4x32_10(make_uint4((uint32_t)e, (uint32_t)t, RO_PURPOSE_ACTION, 0u), k0, k1);
+      const double u0 = u53(rnd.x, rnd.y), u1 = u53(rnd.z, rnd.w);
+      int ai = 0;
+      float af = 0.f;
+      float* prob = a.s_prob + st_row * PD;
+      if (E::HEAD == MRL_HEAD_CAT) {
+        float z[DOUT], p[DOUT], mx = -INFINITY, sum = 0.f;
+#pragma unroll
+        for (int j = 0; j < DOUT; ++j) { z[j] = OUT[row * DOUT + j]; mx = fmaxf(mx, z[j]); }
+#pragma unroll
+        for (int j = 0; j < DOUT; ++j) { p[j] = expf(z[j] - mx); sum += p[j]; }
+#pragma unroll
+        for (int j = 0; j < DOUT; ++j) { p[j] = p[j] / sum; prob[j] = p[j]; }
+        if (a.stochastic) {                // argmax(cumsum(p) > u): float32 cumsum, compared in float64
+          float c = 0.f;
+          bool found = false;
+#pragma unroll
+          for (int j = 0; j < DOUT; ++j) {
+            c += p[j];
+            if (!found && (double)c > u0) { ai = j; found = true; }
+          }
+        } else {                           // argmax, first maximum
+          float best = p[0];
+#pragma unroll
+          for (int j = 1; j < DOUT; ++j) if (p[j] > best) { best = p[j]; ai = j; }
+        }
+        ((int*)a.s_act)[st_row] = ai;
+      } else {
+        const float mean = OUT[row * DOUT], sd = logstd_exp[0];
+        prob[0] = mean;
+        prob[1] = sd;
+        if (a.stochastic) {                // randn().astype(float32) * std + mean, in float32
+          const float z = (float)(sqrt(-2.0 * log(1.0 - u0)) * cos(2.0 * M_PI * u1));
+          af = __fadd_rn(__fmul_rn(z, sd), mean);
+        } else {
+          af = mean;
+        }
+        ((float*)a.s_act)[st_row] = af;
+      }
+      const bool done = E::step(s, ai, af, &rew);
+      a.s_rew[st_row] = rew;
+      rlive = true;
+      ++len;
+      if (done) { term = true; live = false; }
+    }
+  }
+
+  // ---- compaction: path-major rows at offsets from an exclusive scan of the lengths (CTA rank order, then index)
+  if (mine) { a.lengths[e] = len; a.term[e] = term ? 1 : 0; }
+  long long incl = len;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    const long long u = __shfl_up_sync(0xffffffffu, incl, o);
+    if (lane >= o) incl += u;
+  }
+  if (lane == 31) wlen[warp] = incl;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    long long acc = 0;
+    for (int i = 0; i < (int)(blockDim.x >> 5); ++i) { const long long v = wlen[i]; wlen[i] = acc; acc += v; }
+    lslot = acc;
+  }
+  cluster.sync();
+  if (threadIdx.x == 0) {
+    long long base = 0, tot = 0;
+    for (int r = 0; r < nc; ++r) {
+      const long long v = *cluster.map_shared_rank(&lslot, r);
+      if (r < rank) base += v;
+      tot += v;
+    }
+    lbase = base;
+    ltotal = tot;
+  }
+  __syncthreads();
+  const long long off = lbase + wlen[warp] + incl - len, total = ltotal;
+  const RolloutLayout lay = rollout_layout(total, D0, SD, PD, E::HEAD == MRL_HEAD_CAT ? 1 : DOUT, a.s_state != nullptr);
+  double* b_obs = (double*)(a.body + lay.obs);
+  double* b_rew = (double*)(a.body + lay.rew);
+  double* b_st = (double*)(a.body + lay.state);
+  float* b_prob = (float*)(a.body + lay.prob);
+  for (int tt = 0; tt < len; ++tt) {
+    const size_t src = (size_t)tt * a.N + e, dst = (size_t)(off + tt);
+#pragma unroll
+    for (int k = 0; k < D0; ++k) b_obs[dst * D0 + k] = a.s_obs[src * D0 + k];
+    b_rew[dst] = a.s_rew[src];
+    if (a.s_state)
+#pragma unroll
+      for (int i = 0; i < SD; ++i) b_st[dst * SD + i] = a.s_state[src * SD + i];
+#pragma unroll
+    for (int j = 0; j < PD; ++j) b_prob[dst * PD + j] = a.s_prob[src * PD + j];
+    if (E::HEAD == MRL_HEAD_CAT) ((int*)(a.body + lay.act))[dst] = ((const int*)a.s_act)[src];
+    else
+#pragma unroll
+      for (int j = 0; j < DOUT; ++j) ((float*)(a.body + lay.act))[dst * DOUT + j] = ((const float*)a.s_act)[src * DOUT + j];
+  }
+  if (rank == 0 && threadIdx.x == 0) {   // header: total, observation state, its pushed part, reward state, pushed
+    double* h = a.head;
+    h[0] = (double)total;
+    h[1] = run[0].n;
+    h[2 + 2 * D0] = pushed[0].n;
+    for (int k = 0; k < D0; ++k) {
+      h[2 + k] = run[k].m; h[2 + D0 + k] = run[k].s;
+      h[3 + 2 * D0 + k] = pushed[k].m; h[3 + 3 * D0 + k] = pushed[k].s;
+    }
+    double* r = h + 3 + 4 * D0;
+    r[0] = run[D0].n; r[1] = run[D0].m; r[2] = run[D0].s;
+    r[3] = pushed[D0].n; r[4] = pushed[D0].m; r[5] = pushed[D0].s;
+  }
+  cluster.sync();                        // no CTA leaves while another may still read its slots
+}
+
+// ---------------------------------------------------------------------------------------------------- launcher
+int rollout_env_dims(int env, int* d0, int* sd, int* dout) {
+  if (env == MRL_ENV_CARTPOLE) { *d0 = EnvT<MRL_ENV_CARTPOLE>::D0; *sd = EnvT<MRL_ENV_CARTPOLE>::SD; *dout = EnvT<MRL_ENV_CARTPOLE>::DOUT; return MRL_HEAD_CAT; }
+  if (env == MRL_ENV_PENDULUM) { *d0 = EnvT<MRL_ENV_PENDULUM>::D0; *sd = EnvT<MRL_ENV_PENDULUM>::SD; *dout = EnvT<MRL_ENV_PENDULUM>::DOUT; return MRL_HEAD_GAUSS; }
+  return -1;
+}
+
+void rollout_shape(int N, int* n_ctas, int* per_cta, int* threads) {
+  int nc = (N + RO_MIN_PER_CTA - 1) / RO_MIN_PER_CTA;
+  nc = nc < 1 ? 1 : (nc > RO_MAX_CTAS ? RO_MAX_CTAS : nc);
+  const int pc = (N + nc - 1) / nc;
+  int th = round_up(pc, 32);
+  *n_ctas = nc;
+  *per_cta = pc;
+  *threads = th < 128 ? 128 : th;
+}
+
+size_t rollout_smem_bytes(const RolloutArgs& a, int d0, int dout) {
+  return ((size_t)a.w_floats + 2 * (size_t)a.rows_chunk * a.ldh + (size_t)a.per_cta * (d0 + dout)) * 4;
+}
+
+template <int ENV, int ACT>
+static cudaError_t launch_t(const RolloutArgs& a, int n_ctas, int threads, size_t smem, cudaStream_t st) {
+  const void* f = (const void*)rollout_kernel<ENV, ACT>;
+  cudaError_t e = mrl_func_smem(f, smem);
+  if (e != cudaSuccess) return e;
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3(n_ctas);
+  cfg.blockDim = dim3(threads);
+  cfg.dynamicSmemBytes = smem;
+  cfg.stream = st;
+  cudaLaunchAttribute at[1];
+  at[0].id = cudaLaunchAttributeClusterDimension;
+  at[0].val.clusterDim.x = n_ctas;
+  at[0].val.clusterDim.y = 1;
+  at[0].val.clusterDim.z = 1;
+  cfg.attrs = at;
+  cfg.numAttrs = 1;
+  return cudaLaunchKernelEx(&cfg, rollout_kernel<ENV, ACT>, a);
+}
+
+cudaError_t launch_rollout(const RolloutArgs& a, int env, int act, int n_ctas, int threads, size_t smem, cudaStream_t st) {
+#define RO_ACTS(ENV)                                                          \
+  switch (act) {                                                              \
+    case MRL_ACT_TANH: return launch_t<ENV, MRL_ACT_TANH>(a, n_ctas, threads, smem, st); \
+    case MRL_ACT_RELU: return launch_t<ENV, MRL_ACT_RELU>(a, n_ctas, threads, smem, st); \
+    default: return launch_t<ENV, MRL_ACT_SIGMOID>(a, n_ctas, threads, smem, st);        \
+  }
+  if (env == MRL_ENV_CARTPOLE) { RO_ACTS(MRL_ENV_CARTPOLE) }
+  RO_ACTS(MRL_ENV_PENDULUM)
+#undef RO_ACTS
+}

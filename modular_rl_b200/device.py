@@ -327,6 +327,83 @@ class DeviceNet:
         return sd, fs, dict(shs=sc[0], lm=sc[1], expected_improve_rate=sc[2], cg_rdotr=sc[3])
 
 
+class DeviceRollouts:
+    """mrl_rollout_*: rounds of n_envs lockstep rollouts of a built-in environment, each round one kernel launch on
+    the device (the policy forward, the action draws, the dynamics and both ZFilters included).  `env`: a built-in
+    environment's id ("CartPole-v0", "Pendulum-v0") or instance."""
+
+    def __init__(self, env, n_envs: int, timestep_limit: int, device: Optional[int] = None):
+        from .envs import device_kind
+        kind = device_kind(env)
+        if device is None:
+            device = parallel.current_device()
+        self._h = C.c_void_p()
+        L.check(L.lib().mrl_rollout_create(C.byref(self._h), device, L.DEVICE_ENVS[kind], int(n_envs), int(timestep_limit)))
+        self.kind, self.n_envs, self.timestep_limit, self.device = kind, int(n_envs), int(timestep_limit), device
+        self.ob_dim, self.state_dim = (4, 4) if kind == "cartpole" else (3, 2)
+        self.categorical = kind == "cartpole"
+        self.act_dim = 1
+
+    @staticmethod
+    def max_envs() -> int:
+        return int(L.lib().mrl_rollout_max_envs())
+
+    def close(self):
+        if getattr(self, "_h", None):
+            L.lib().mrl_rollout_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    @staticmethod
+    def _filter_in(filt, size):
+        """filt: None (identity) or (state (n, M, S), demean, destd, clip) -> (cfg, state in/out, pushed out)."""
+        if filt is None:
+            return None, None, None
+        (n, M, S), demean, destd, clip = filt
+        state = np.concatenate([[float(n)], np.asarray(M, np.float64).ravel(), np.asarray(S, np.float64).ravel()])
+        assert state.size == 1 + 2 * size, (state.size, size)
+        cfg = L.ZFilterCfg(1, int(bool(demean)), int(bool(destd)), float(clip or 0.0))
+        return cfg, state, np.zeros_like(state)
+
+    @staticmethod
+    def _state_out(state, size):
+        return None if state is None else (float(state[0]), state[1:1 + size].copy(), state[1 + size:].copy())
+
+    def run(self, net: DeviceNet, seed: int, stochastic: bool = True, obfilter=None, rewfilter=None,
+            want_states: bool = False, stream=None) -> dict:
+        """One round.  obfilter / rewfilter: None (identity) or ((n, M, S), demean, destd, clip).  Returns the
+        compacted path-major arrays (lengths, terminated, observation, action, prob, reward[, states]) and the filter
+        states after the round plus those of this round's samples alone (ob_state, ob_pushed, rew_state, rew_pushed;
+        None for an identity filter)."""
+        d = self.ob_dim
+        ocfg, ost, opu = self._filter_in(obfilter, d)
+        rcfg, rst, rpu = self._filter_in(rewfilter, 1)
+        n = C.c_longlong()
+        L.check(L.lib().mrl_rollout_run(self._h, net._h, int(seed) & 0xFFFFFFFFFFFFFFFF, int(bool(stochastic)),
+                                        C.byref(ocfg) if ocfg else None, L.ptr(ost), L.ptr(opu),
+                                        C.byref(rcfg) if rcfg else None, L.ptr(rst), L.ptr(rpu),
+                                        int(bool(want_states)), C.byref(n), stream))
+        T = int(n.value)
+        out = dict(lengths=np.empty(self.n_envs, np.int32), terminated=np.empty(self.n_envs, np.uint8),
+                   observation=np.empty((T, d), np.float64),
+                   action=np.empty(T, np.int32) if self.categorical else np.empty((T, self.act_dim), np.float32),
+                   prob=np.empty((T, 2 * self.act_dim if not self.categorical else 2), np.float32),
+                   reward=np.empty(T, np.float64))
+        states = np.empty((T, self.state_dim), np.float64) if want_states else None
+        L.check(L.lib().mrl_rollout_read(self._h, L.ptr(out["lengths"]), L.ptr(out["terminated"]), L.ptr(out["observation"]),
+                                         L.ptr(out["action"]), L.ptr(out["prob"]), L.ptr(out["reward"]), L.ptr(states)))
+        if want_states:
+            out["states"] = states
+        out["ob_state"], out["ob_pushed"] = self._state_out(ost, d), self._state_out(opu, d)
+        out["rew_state"], out["rew_pushed"] = self._state_out(rst, 1), self._state_out(rpu, 1)
+        return out
+
+
 def population_forward(dims: Sequence[int], activation: str, thetas, obs, device: int = 0) -> np.ndarray:
     """mrl_population_forward: out[m] = MLP_{thetas[m]}(obs[m]) for all members in one launch (linear last layer).
     thetas [M, P] holds Dense kernels and biases in the reference's flat order (no logstd block)."""

@@ -17,6 +17,7 @@ class _Spec(object):
 
 
 class CartPoleEnv(object):
+    device_kind = "cartpole"        # rollout.cu implements these dynamics (core.do_rollouts_device)
     gravity, masscart, masspole, length, force_mag, tau = 9.8, 1.0, 0.1, 0.5, 10.0, 0.02
     theta_threshold = 12 * 2 * math.pi / 360
     x_threshold = 2.4
@@ -57,6 +58,7 @@ class CartPoleEnv(object):
 
 
 class PendulumEnv(object):
+    device_kind = "pendulum"
     max_speed, max_torque, dt, g, m, l = 8.0, 2.0, 0.05, 10.0, 1.0, 1.0
 
     def __init__(self):
@@ -105,3 +107,15 @@ def make(name):
     except ImportError:
         raise KeyError("unknown environment %r (built in: %s; gym is not installed)" % (name, sorted(_REGISTRY)))
     return gym_make(name)
+
+
+def device_kind(env):
+    """The device implementation of a built-in environment (an instance or an id): 'cartpole' or 'pendulum'.
+    Raises ValueError for any other environment."""
+    cls = _REGISTRY.get(env) if isinstance(env, str) else type(env)
+    kind = getattr(cls, "device_kind", None)
+    if kind is None:
+        name = env if isinstance(env, str) else getattr(getattr(env, "spec", None), "id", type(env).__name__)
+        raise ValueError("environment %s has no device implementation; device rollouts run the built-in environments "
+                         "only: %s" % (name, ", ".join(sorted(_REGISTRY))))
+    return kind

@@ -39,7 +39,15 @@ def main():
     parser.add_argument("--vec_envs", type=int, default=0,
                         help="environments stepped in lockstep with one batched device forward per step "
                              "(0: serial rollouts as the reference); not an agent option")
+    parser.add_argument("--device_envs", type=int, default=0,
+                        help="environments per rollout round run on the GPU in one kernel launch (built-in CartPole "
+                             "and Pendulum only; 0: host rollouts); resets and action noise come from the device's "
+                             "Philox stream, so results differ from a host run with the same --seed")
     args, _ = parser.parse_known_args([arg for arg in sys.argv[1:] if arg not in ('-h', '--help')])
+    if args.device_envs and args.vec_envs:
+        parser.error("--device_envs and --vec_envs select different rollout paths; give one")
+    if args.device_envs < 0:
+        parser.error("--device_envs must be >= 0")
     dp = parallel.init_data_parallel() if parallel.launched_data_parallel() else None
     root = parallel.is_root()
     if not root:
@@ -60,9 +68,11 @@ def main():
     if args.timestep_limit == 0:
         args.timestep_limit = env_spec.max_episode_steps
     cfg = args.__dict__
+    from modular_rl_b200 import core as _core
     if args.vec_envs > 1:
-        from modular_rl_b200 import core as _core
         _core.VEC_ENVS = args.vec_envs
+    if args.device_envs:
+        _core.DEVICE_ENVS = args.device_envs
     np.random.seed(args.seed)
     if args.load_snapshot:
         # the reference declares the flag (misc_utils.py:102) without reading it; here it resumes from a
@@ -71,6 +81,8 @@ def main():
         assert isinstance(agent, agent_ctor), "snapshot holds a %s" % type(agent).__name__
     else:
         agent = agent_ctor(env.observation_space, env.action_space, cfg)
+    if args.device_envs:
+        _core.check_device_rollouts(env, agent)     # an unsupported env / filter / policy fails before any rollout
     if args.use_hdf and root:
         hdf, diagnostics = prepare_h5_file(args)
 
