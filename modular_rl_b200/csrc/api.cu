@@ -631,10 +631,9 @@ extern "C" int mrl_zfilter_scan(const void* x, int x_dtype, long long N, int d, 
 struct mrl_net {
   int device = 0;
   NetGeom g;
-  DevBuf trace;
   DevBuf adam_m, adam_v, sgd_acc;   // PpoSgd: Adam moments (float32) and the running sum of the minibatch losses
   long long adam_t = 0;
-  DevBuf WC, VC, dbg;      // tcgen05 Fisher-vector chain: weight images of theta / of the tangent, debug dump
+  DevBuf WC, VC;           // tcgen05 Fisher-vector chain: weight images of theta / of the tangent
   bool tc_fvp = false;
   DevBuf DG, WBt, WBv, theta, theta_prev, theta_trial, img, imgv, vflat, Z1, cache, part1, partm, loss_part, out32,
       out64, g32, cg_b, cg_x, cg_r, cg_p, p32, x32, fullstep, cgstate, cgscratch, scal, headout, stage;
@@ -689,8 +688,6 @@ extern "C" int mrl_net_create(mrl_net** out, int device, int n_layers, const int
     if (n->tc_fvp) {
       R(n->WC, fvp_tc_image_floats(n->g, 0) * 4);
       R(n->VC, fvp_tc_image_floats(n->g, 1) * 4);
-      if (getenv("MRL_FVP_TC_DEBUG")) R(n->dbg, (size_t)8 * 128 * 128 * 4);
-      if (getenv("MRL_FVP_TC_TRACE")) { R(n->trace, (size_t)8 * 4096 * 2 * 8); if (e == cudaSuccess) e = cudaMemset(n->trace.p, 0, (size_t)8 * 4096 * 2 * 8); }
     }
   }
   if (e == cudaSuccess) e = cudaMallocHost(&n->h_scal, 32 * 8);
@@ -708,7 +705,7 @@ extern "C" int mrl_net_create(mrl_net** out, int device, int n_layers, const int
 extern "C" int mrl_net_destroy(mrl_net* n) {
   if (!n) return 0;
   cudaSetDevice(n->device);
-  DevBuf* bufs[] = {&n->adam_m, &n->adam_v, &n->sgd_acc, &n->trace, &n->WC, &n->VC, &n->dbg, &n->DG, &n->WBt, &n->WBv, &n->theta, &n->theta_prev, &n->theta_trial, &n->img, &n->imgv, &n->vflat,
+  DevBuf* bufs[] = {&n->adam_m, &n->adam_v, &n->sgd_acc, &n->WC, &n->VC, &n->DG, &n->WBt, &n->WBv, &n->theta, &n->theta_prev, &n->theta_trial, &n->img, &n->imgv, &n->vflat,
                     &n->Z1, &n->cache, &n->part1, &n->partm, &n->loss_part, &n->out32, &n->out64, &n->g32,
                     &n->cg_b, &n->cg_x, &n->cg_r, &n->cg_p, &n->p32, &n->x32, &n->fullstep, &n->cgstate, &n->cgscratch, &n->scal,
                     &n->headout, &n->stage};
@@ -921,8 +918,6 @@ static int pass_backward(mrl_net* n, mrl_batch* b, int mode, const double* coef_
     FvpTcArgs x;
     x.WC = n->WC.as<float>(); x.VC = n->VC.as<float>(); x.vflat = v_dev; x.img = n->img.as<float>();
     x.Zt = n->Z1.as<float>(); x.cache = n->cache.as<float>(); x.DG = n->DG.as<float>(); x.partm = n->partm.as<float>();
-    x.dbg = n->dbg.as<float>();
-    x.trace = n->trace.as<long long>();
     x.N = b->N; x.n_tiles = b->n_tiles; x.slab_tiles = pl.slab_tiles; x.n_slabs = pl.n_slabs;
     CKP(PK_MIDB_FVP, launch_fvp_tc(g, x, st), 1);
   } else if (mode == MRL_MODE_GRAD && chain_bwd_shape(g) != 0) CKP(PK_MIDB_GRAD, launch_chain_backward(g, a, pl.n_slabs, st), 1);
@@ -1233,24 +1228,6 @@ extern "C" int mrl_net_trpo_step(mrl_net* n, mrl_batch* b, const mrl_trpo_cfg* c
     info[4] = skipped ? 0 : cg_run + 1;   // Fvp evaluations the reference would make; launches after an early break are no-ops
     info[5] = loss_passes;
   }
-  return 0;
-}
-
-// debug: stage outputs of the first 128-timestep tile of the last tcgen05 Fvp (MRL_FVP_TC_DEBUG=1): [8][128][128] floats
-extern "C" int mrl_debug_fvp_tc_read(mrl_net* n, float* out) {
-  if (!n || !n->dbg.p || !out) return fail("mrl_debug_fvp_tc_read: debug dump not enabled");
-  CK(cudaSetDevice(n->device));
-  CK(cudaDeviceSynchronize());
-  CK(cudaMemcpy(out, n->dbg.p, (size_t)8 * 128 * 128 * 4, cudaMemcpyDeviceToHost));
-  return 0;
-}
-
-extern "C" int mrl_debug_fvp_tc_trace(mrl_net* n, long long* out) {
-  if (!n || !n->trace.p || !out) return fail("mrl_debug_fvp_tc_trace: trace not enabled (MRL_FVP_TC_TRACE=1)");
-  CK(cudaSetDevice(n->device));
-  CK(cudaDeviceSynchronize());
-  CK(cudaMemcpy(out, n->trace.p, (size_t)8 * 4096 * 2 * 8, cudaMemcpyDeviceToHost));
-  CK(cudaMemset(n->trace.p, 0, (size_t)8 * 4096 * 2 * 8));
   return 0;
 }
 

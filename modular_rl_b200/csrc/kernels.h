@@ -97,8 +97,6 @@ struct FvpTcArgs {
   const float* cache;   // activation cache of theta
   float* DG;            // out: delta_1 operand of the layer-1 gradient GEMM
   float* partm;         // out: [n_slabs][pmid]
-  float* dbg;           // debug dump of the first 128-timestep tile or nullptr
-  long long* trace;     // pipeline trace of CTA 0 or nullptr
   long long N;
   int n_tiles, slab_tiles /* even */, n_slabs;
 };

@@ -127,21 +127,6 @@ template <int N> __device__ __forceinline__ void ft_reg_dec() { asm volatile("se
 template <int N> __device__ __forceinline__ void ft_reg_inc() { asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(N)); }
 static_assert(4 * 32 * FT_REGS_CTRL + 4 * 32 * FT_REGS_CONV + 16 * 32 * FT_REGS_EPI <= FT_THREADS * 80, "register pool of the launch (80 registers per thread)");
 
-// Pipeline trace of CTA 0 (experiments: MRL_FVP_TC_TRACE=1, tools/micro/fvp_trace.py): per role, (clock64, code) pairs
-#define FT_TRN 4096
-#ifndef FT_TRACE
-#define FT_TR(role, code) do { (void)trn; } while (0)
-#else
-#define FT_TR(role, code)                                                                        \
-  do {                                                                                           \
-    if (a.trace && blockIdx.x == 0 && trn < FT_TRN) {                                            \
-      a.trace[((size_t)(role) * FT_TRN + trn) * 2] = clock64();                                  \
-      a.trace[((size_t)(role) * FT_TRN + trn) * 2 + 1] = (long long)(code);                      \
-      ++trn;                                                                                     \
-    }                                                                                            \
-  } while (0)
-#endif
-
 struct FtArgs {
   const float* WC;      // chain weight images of theta
   const float* VC;      // tangent weight images
@@ -151,8 +136,6 @@ struct FtArgs {
   const float* cache;   // activations of theta, tile-major [tile][act_rows][LDT]
   float* DG;            // delta_1 operand of the layer-1 gradient GEMM, K-major: [t/8][hi | lo][khalf][n/8][8 n][4 t]
   float* partm;         // [n_slabs][pmid]
-  float* dbg;           // debug dump of the first tile (nullptr: off)
-  long long* trace;     // pipeline trace of CTA 0 (nullptr: off)
   long long N;
   int n_tiles, n_mtiles, slab_mt, n_slabs, nu;
 };
@@ -288,7 +271,6 @@ __global__ void __launch_bounds__(FT_THREADS, 1) fvp_tc_kernel(NetGeom g, FtPlan
     const uint32_t desc_hi = (uint32_t)(umma_desc(0, 0, 128) >> 32);
     const uint32_t ring_u32 = smem_u32(rring);
     uint32_t wc = 0, u = 0, tcount = 0;
-    int trn = 0;
     for (int slab = blockIdx.x; slab < a.n_slabs; slab += gridDim.x) {
       const int mt0 = slab * a.slab_mt, mt1 = min(mt0 + a.slab_mt, a.n_mtiles);
       for (int mt = mt0; mt < mt1; ++mt) {
@@ -308,10 +290,8 @@ __global__ void __launch_bounds__(FT_THREADS, 1) fvp_tc_kernel(NetGeom g, FtPlan
           const uint32_t bw = umma_desc_lo(ring_u32 + (uint32_t)ws * (uint32_t)P.rstage_floats * 4u, lbo);
           for (int c = 0; c < nk; ++c, ++u) {
             const int e = u & 1;
-            if (lane == 0) FT_TR(0, (1 << 24) | (r << 8) | (kg0 + c));
             mbar_wait_sleep(&ra_full[e], (u >> 1) & 1);
             tc_fence_after();
-            if (lane == 0) FT_TR(0, (2 << 24) | (r << 8) | (kg0 + c));
             if (elect_one()) {
               const uint32_t bW = bw + ((c * kgb) >> 4), bV = bw + ((2 * kgb + c * kgb) >> 4);
               const uint32_t tr = tmem_base + P.rring_col + 32 * e, th = tr + 16;   // [Rh hi 8 | Rh lo 8 | h hi 8 | h lo 8]
@@ -337,7 +317,6 @@ __global__ void __launch_bounds__(FT_THREADS, 1) fvp_tc_kernel(NetGeom g, FtPlan
     const uint32_t desc_hi = (uint32_t)(umma_desc(0, 0, 128) >> 32);
     const uint32_t ring_u32 = smem_u32(dring);
     uint32_t wc = 0, u = 0;
-    int trn = 0;
     for (int slab = blockIdx.x; slab < a.n_slabs; slab += gridDim.x) {
       const int mt0 = slab * a.slab_mt, mt1 = min(mt0 + a.slab_mt, a.n_mtiles);
       for (int mt = mt0; mt < mt1; ++mt) {
@@ -353,10 +332,8 @@ __global__ void __launch_bounds__(FT_THREADS, 1) fvp_tc_kernel(NetGeom g, FtPlan
           const uint32_t bw = umma_desc_lo(ring_u32 + (uint32_t)ws * (uint32_t)P.dstage_floats * 4u, lbo);
           for (int c = 0; c < nk; ++c, ++u) {
             const int e = u & 1;
-            if (lane == 0) FT_TR(1, (1 << 24) | (k << 8) | (kg0 + c));
             mbar_wait_sleep(&da_full[e], (u >> 1) & 1);
             tc_fence_after();
-            if (lane == 0) FT_TR(1, (2 << 24) | (k << 8) | (kg0 + c));
             if (elect_one()) {
               const uint32_t bW = bw + ((c * kgb) >> 4);
               const uint32_t td = tmem_base + P.dring_col + 16 * e;                  // [delta hi 8 | delta lo 8]
@@ -378,7 +355,6 @@ __global__ void __launch_bounds__(FT_THREADS, 1) fvp_tc_kernel(NetGeom g, FtPlan
     const uint32_t desc_hi = (uint32_t)(umma_desc(0, 0, 4096) >> 32);   // SBO = 32 k-chunks x 128 B between n-groups
     const uint32_t kbuf_u32 = smem_u32(kbuf);
     uint32_t kc = 0, tcount = 0, scount = 0;
-    int trn = 0;
     for (int slab = blockIdx.x; slab < a.n_slabs; slab += gridDim.x, ++scount) {
       const int mt0 = slab * a.slab_mt, mt1 = min(mt0 + a.slab_mt, a.n_mtiles);
       mbar_wait_sleep(gacc_empty, (scount & 1) ^ 1);      // the previous slab's accumulators have been flushed
@@ -391,12 +367,10 @@ __global__ void __launch_bounds__(FT_THREADS, 1) fvp_tc_kernel(NetGeom g, FtPlan
           const uint32_t bbase = umma_desc_lo(kbuf_u32 + (uint32_t)P.pass_buf[p] * 4u, 128);   // LBO = 128 B: adjacent k-chunks
           const uint32_t lo_off = ((uint32_t)Np_ * 512u) >> 4;                                  // lo half of the buffer
           mbar_wait_sleep(&d_full[p], tcount & 1);          // this tile's delta blocks of the pass are in shared memory
-          if (lane == 0) FT_TR(2, (1 << 24) | (p << 8));
           for (int ks = 0; ks < 16; ++ks, ++kc) {
             const int sl = kc % FT_KSLOTS;
             mbar_wait_sleep(&kconv[sl], (kc / FT_KSLOTS) & 1);
             tc_fence_after();
-            if (lane == 0) FT_TR(2, (2 << 24) | (p << 8) | ks);
             if (elect_one()) {
               const uint32_t ta = tmem_base + P.kslot_col + 16 * sl;     // [h^T hi 8 | lo 8]
               const uint32_t db = bbase + ((uint32_t)ks * 256u >> 4);
@@ -420,13 +394,11 @@ __global__ void __launch_bounds__(FT_THREADS, 1) fvp_tc_kernel(NetGeom g, FtPlan
     const int q = warp & 3, m = q * 32 + lane;
     const uint32_t tlane = tmem_base + ((uint32_t)(q * 32) << 16);
     uint32_t kc = 0, scount = 0;
-    int trn = 0;
     for (int slab = blockIdx.x; slab < a.n_slabs; slab += gridDim.x, ++scount) {
       const int mt0 = slab * a.slab_mt, mt1 = min(mt0 + a.slab_mt, a.n_mtiles);
       for (int mt = mt0; mt < mt1; ++mt) {
         for (int p = 0; p < P.n_pass; ++p) {
           const int crow = P.row_cache[p][m];
-          if (warp == 20 && lane == 0) FT_TR(5, (1 << 24) | (p << 8));
           // the 16 k-steps (8 timesteps each) of the tile in groups of two; group g + 1 is requested before group g is
           // converted, so the L2 latency is covered by the conversion of two k-steps
           float4 xa[2][2], xb[2][2];
@@ -473,7 +445,6 @@ __global__ void __launch_bounds__(FT_THREADS, 1) fvp_tc_kernel(NetGeom g, FtPlan
             if (g2 + 2 < 8) request(g2 + 2, xa);
             convert(xb);
           }
-          if (warp == 20 && lane == 0) FT_TR(5, (2 << 24) | (p << 8));
         }
       }
       // ---- slab flush: accumulator rows -> fp32 slab partial (weights of layers >= 2, their biases from the ones row)
@@ -515,8 +486,6 @@ __global__ void __launch_bounds__(FT_THREADS, 1) fvp_tc_kernel(NetGeom g, FtPlan
       const int e = (warp - 4) >> 2;
       const uint32_t ring = tlane + P.rring_col + 32 * e;
       uint32_t u = 0, ue = 0, tcount = 0;
-      int trn = 0;
-      const bool tr_on = warp == 4 && lane == 0;
       for (int slab = blockIdx.x; slab < a.n_slabs; slab += gridDim.x) {
       const int mt0 = slab * a.slab_mt, mt1 = min(mt0 + a.slab_mt, a.n_mtiles);
       for (int mt = mt0; mt < mt1; ++mt) {
@@ -542,13 +511,11 @@ __global__ void __launch_bounds__(FT_THREADS, 1) fvp_tc_kernel(NetGeom g, FtPlan
           u += kgs;
           if (kg < kgs) request(kg, hc, zc);
           uint32_t src_acc = 0;
-          if (tr_on) FT_TR(3, (1 << 24) | (r << 8));
           if (r > 0) {
             mbar_wait_sleep(&racc_full[r - 1], tcount & 1);
             tc_fence_after();
             src_acc = tlane + P.rs[r - 1].acc_col;
           }
-          if (tr_on) FT_TR(3, (2 << 24) | (r << 8));
           for (; kg < kgs; kg += 2, ++ue) {
             const uint32_t freeq = mbar_try(&ra_empty[e], (ue & 1) ^ 1);
             if (kg + 2 < kgs) request(kg + 2, hn, zn);
@@ -564,17 +531,11 @@ __global__ void __launch_bounds__(FT_THREADS, 1) fvp_tc_kernel(NetGeom g, FtPlan
 #pragma unroll
               for (int i = 0; i < 8; ++i) val[i] = dact_from_h<ACT>(hc[i]) * (__uint_as_float(v[i]) + vbk[i]);
             }
-            if (a.dbg && mt == 0) {
-#pragma unroll
-              for (int i = 0; i < 8; ++i) a.dbg[((size_t)r * 128 + m) * 128 + 8 * kg + i] = val[i];
-            }
             uint32_t hi[8], lo[8];
 #pragma unroll
             for (int i = 0; i < 8; ++i) ft_split(val[i], hi[i], lo[i]);
-            if (tr_on) FT_TR(3, (3 << 24) | (r << 8) | kg);
             if (!freeq) mbar_wait_sleep(&ra_empty[e], (ue & 1) ^ 1);
             tc_fence_after();
-            if (tr_on) FT_TR(3, (4 << 24) | (r << 8) | kg);
             tmem_st8(ring, hi);
             tmem_st8(ring + 8, lo);
 #pragma unroll
@@ -585,7 +546,6 @@ __global__ void __launch_bounds__(FT_THREADS, 1) fvp_tc_kernel(NetGeom g, FtPlan
             tc_fence_before();
             __syncwarp();
             if (lane == 0) mbar_arrive(&ra_full[e]);
-            if (tr_on) FT_TR(3, (5 << 24) | (r << 8) | kg);
 #pragma unroll
             for (int i = 0; i < 8; ++i) { hc[i] = hn[i]; zc[i] = zn[i]; }
           }
@@ -606,8 +566,6 @@ __global__ void __launch_bounds__(FT_THREADS, 1) fvp_tc_kernel(NetGeom g, FtPlan
       const bool cat = g.head == MRL_HEAD_CAT;
       const int nu = a.nu;
       uint32_t u = 0, ue = 0, tcount = 0;
-      int trn = 0;
-      const bool tr_on = warp == 12 && lane == 0;
       for (int slab = blockIdx.x; slab < a.n_slabs; slab += gridDim.x) {
         const int mt0 = slab * a.slab_mt, mt1 = min(mt0 + a.slab_mt, a.n_mtiles);
         for (int mt = mt0; mt < mt1; ++mt, ++tcount) {
@@ -643,7 +601,6 @@ __global__ void __launch_bounds__(FT_THREADS, 1) fvp_tc_kernel(NetGeom g, FtPlan
               u += kgs;
               if (kg < kgs) request(kg, hc);
               uint32_t src_acc;
-              if (tr_on) FT_TR(4, (1 << 24) | (l << 8) | c);
               if (c == 0) {
                 if (is_head) {
                   mbar_wait_sleep(&racc_full[nR - 1], tcount & 1);
@@ -657,7 +614,6 @@ __global__ void __launch_bounds__(FT_THREADS, 1) fvp_tc_kernel(NetGeom g, FtPlan
               } else {
                 src_acc = tlane + (is_head ? P.rs[nR - 1].acc_col : P.ds[k - c - 1].acc_col);
               }
-              if (tr_on) FT_TR(4, (2 << 24) | (l << 8) | c);
               float sdot = 0.f;     // Categorical: p . Rz over the whole row
               if (is_head && cat) {
                 for (int c0 = 0; c0 < P.Np[L]; c0 += 8) {
@@ -689,17 +645,11 @@ __global__ void __launch_bounds__(FT_THREADS, 1) fvp_tc_kernel(NetGeom g, FtPlan
                   } else o = acc * dact_from_h<ACT>(hc[i]);                            // padding columns: zero accumulator
                   val[i] = o;
                 }
-                if (a.dbg && mt == 0 && c == 0) {
-#pragma unroll
-                  for (int i = 0; i < 8; ++i) a.dbg[((size_t)(nR + L - l) * 128 + m) * 128 + 8 * kg + i] = val[i];
-                }
                 uint32_t hi[8], lo[8];
 #pragma unroll
                 for (int i = 0; i < 8; ++i) ft_split(val[i], hi[i], lo[i]);
-                if (tr_on) FT_TR(4, (3 << 24) | (l << 8) | kg);
                 if (!freeq) mbar_wait_sleep(&da_empty[e], (ue & 1) ^ 1);
                 tc_fence_after();
-                if (tr_on) FT_TR(4, (4 << 24) | (l << 8) | kg);
                 tmem_st8(ring, hi);
                 tmem_st8(ring + 8, lo);
                 if (c == 0) {
@@ -721,7 +671,6 @@ __global__ void __launch_bounds__(FT_THREADS, 1) fvp_tc_kernel(NetGeom g, FtPlan
                 tc_fence_before();
                 __syncwarp();
                 if (lane == 0) mbar_arrive(&da_full[e]);
-                if (tr_on) FT_TR(4, (5 << 24) | (l << 8) | kg);
 #pragma unroll
                 for (int i = 0; i < 8; ++i) hc[i] = hn[i];
               }
@@ -752,10 +701,8 @@ __global__ void __launch_bounds__(FT_THREADS, 1) fvp_tc_kernel(NetGeom g, FtPlan
                 };
                 int j0 = 8 * e;
                 if (j0 < st.N) request1(st.col0 + j0, h1c);
-                if (tr_on) FT_TR(4, (6 << 24) | c);
                 mbar_wait_sleep(&dacc_full[k], tcount & 1);
                 tc_fence_after();
-                if (tr_on) FT_TR(4, (7 << 24) | c);
                 const uint32_t facc = tlane + st.acc_col;
                 // quad base: timesteps 4 (T / 4) .. + 3 of feature n: + (n / 8) * 32 + (n % 8) * 4
                 float* dgq = a.DG + (size_t)(T >> 3) * (2 * nu * 8) + ((T >> 2) & 1) * (nu * 4);
@@ -767,10 +714,6 @@ __global__ void __launch_bounds__(FT_THREADS, 1) fvp_tc_kernel(NetGeom g, FtPlan
                   float val[8];
 #pragma unroll
                   for (int i = 0; i < 8; ++i) val[i] = __uint_as_float(v[i]) * dact_from_h<ACT>(h1c[i]);   // padding columns are zero
-                  if (a.dbg && mt == 0) {
-#pragma unroll
-                    for (int i = 0; i < 8; ++i) a.dbg[((size_t)(nR + L - 1) * 128 + m) * 128 + c0 + i] = val[i];
-                  }
 #pragma unroll
                   for (int hq = 0; hq < 2; ++hq) {
                     float tq[4] = {val[4 * hq], val[4 * hq + 1], val[4 * hq + 2], val[4 * hq + 3]};
@@ -811,7 +754,6 @@ __global__ void __launch_bounds__(FT_THREADS, 1) fvp_tc_kernel(NetGeom g, FtPlan
                   for (int i = 0; i < 8; ++i) h1c[i] = h1n[i];
                 }
                 tc_fence_before();
-                if (tr_on) FT_TR(4, (8 << 24) | c);
               }
             }
           }
@@ -1035,7 +977,7 @@ cudaError_t launch_fvp_tc(const NetGeom& g, const FvpTcArgs& x, cudaStream_t st)
   FtArgs a;
   a.WC = x.WC; a.VC = x.VC; a.vflat = x.vflat;
   a.logstd = g.head == MRL_HEAD_GAUSS ? x.img + g.off_pm_logstd : nullptr;
-  a.Zt = x.Zt; a.cache = x.cache; a.DG = x.DG; a.partm = x.partm; a.dbg = x.dbg; a.trace = x.trace;
+  a.Zt = x.Zt; a.cache = x.cache; a.DG = x.DG; a.partm = x.partm;
   a.N = x.N;
   a.n_tiles = x.n_tiles;
   a.n_mtiles = (x.n_tiles + 1) / 2;

@@ -1,10 +1,11 @@
 """CPU-side checks of the drop-in boundary: the shared library builds (nvcc cross-compiles
-without a GPU), loads, and exports every symbol include/mrl_b200.h declares; argument errors are
+without a GPU), loads, and exports exactly the mrl_* symbols include/mrl_b200.h declares; argument errors are
 reported through return codes + mrl_last_error (no exception crosses the ABI); and nothing under
 modular_rl_b200/ imports the oracle.  No compute call is made here."""
 import ctypes as C
 import os
 import re
+import subprocess
 
 import pytest
 
@@ -34,6 +35,13 @@ def test_every_declared_symbol_is_exported_and_bound(lib):
         assert hasattr(lib, n), f"{n} declared in mrl_b200.h but not exported"
     assert set(names) == set(_lib.exported_symbols()), set(names) ^ set(_lib.exported_symbols())
     assert lib.mrl_version() >= 100
+
+
+def test_library_exports_only_declared_symbols(lib):
+    from modular_rl_b200 import _lib
+    out = subprocess.run(["nm", "-D", "--defined-only", _lib.LIB_PATH], check=True, capture_output=True, text=True).stdout
+    exported = sorted({f[-1] for f in (line.split() for line in out.splitlines()) if f and f[-1].startswith("mrl_")})
+    assert exported == _declared(), set(exported) ^ set(_declared())
 
 
 def test_argument_errors_are_return_codes(lib):

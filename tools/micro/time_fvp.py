@@ -26,6 +26,6 @@ nk = lib.mrl_profile_kinds()
 ms = (C.c_double * nk)(); cnt = (C.c_longlong * nk)()
 lib.mrl_profile_read(ms, cnt)
 lib.mrl_profile_kind_name.restype = C.c_char_p
-print("N=%d dbg=%s stages=%s |" % (N, os.environ.get("MRL_L1_DEBUG"), os.environ.get("MRL_L1_STAGES")),
+print("N=%d |" % N,
       "  ".join("%s %.4f" % (lib.mrl_profile_kind_name(k).decode(), ms[k] / cnt[k]) for k in range(nk) if cnt[k]),
       "| |fvp| %.6e" % float(np.linalg.norm(f)))
