@@ -55,7 +55,7 @@ struct MidBwdArgs {
   const float* aux;
   const float* cache;
   const double* coef;  // device: {c_surr, c_kl} (gradient mode)
-  float* DG;           // out: delta_1 as the tcgen05 B operand [tg][hi|lo][khalf][ngroup][8][4] 
+  float* DG;           // out: delta_1 as the tcgen05 B operand, raw fp32 [tg][khalf][ngroup][8][4]
   int nu;              // padded layer-1 width of DG
   float* partm;        // out: [n_slabs][pmid]
   long long N;
@@ -95,7 +95,7 @@ struct FvpTcArgs {
   const float* img;     // theta image (logstd block)
   const float* Zt;      // x . V_1, tile-major
   const float* cache;   // activation cache of theta
-  float* DG;            // out: delta_1 operand of the layer-1 gradient GEMM
+  float* DG;            // out: delta_1 operand of the layer-1 gradient GEMM, raw fp32 [tg][khalf][ngroup][8][4]
   float* partm;         // out: [n_slabs][pmid]
   long long N;
   int n_tiles, slab_tiles /* even */, n_slabs;

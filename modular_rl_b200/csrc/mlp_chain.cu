@@ -315,8 +315,8 @@ __device__ __forceinline__ void delta_layer(float (&acc)[NI][4], const uint32_t 
   }
 }
 
-// delta_1 for in-blocks nb .. nb+NH-1: bias partial sums + the split-precision tcgen05 operand DG
-// [tg = t/8][hi|lo][khalf][ngroup nu/8][8 n][4 timesteps]  (mlp_l1_tc.cu)
+// delta_1 for in-blocks nb .. nb+NH-1: bias partial sums + the tcgen05 operand DG as raw fp32
+// [tg = t/8][khalf][ngroup nu/8][8 n][4 timesteps]  (mlp_l1_tc.cu splits it into (hi, lo))
 template <int ACT, int NH, int nb, int N1, int NO>
 __device__ __forceinline__ void delta1_block(const uint32_t (&dhi)[NO][4], const uint32_t (&dlo)[NO][4],
                                              const float* __restrict__ W2, const float* __restrict__ hp,
@@ -348,16 +348,11 @@ __device__ __forceinline__ void delta1_block(const uint32_t (&dhi)[NO][4], const
     }
     if (ok && 8 * (nb + n) < nu) {
       // dg -> the warp's first timestep group.  This thread's timesteps 2g, 2g+1 are adjacent inside a group of 4:
-      // one 64-bit store per feature and precision part.
-      float* p0 = dg + (size_t)(g >> 2) * (2 * nu * 8) + ((g >> 1) & 1) * (nu * 4) + (nb + n) * 32 + (2 * t) * 4 + 2 * (g & 1);
+      // one 64-bit store per feature.
+      float* p0 = dg + (size_t)(g >> 2) * (nu * 8) + ((g >> 1) & 1) * (nu * 4) + (nb + n) * 32 + (2 * t) * 4 + 2 * (g & 1);
 #pragma unroll
-      for (int b = 0; b < 2; ++b) {   // features 2t, 2t+1 of the n-tile
-        uint32_t h0, l0, h1_, l1_;
-        split_tf32(v[b], h0, l0);
-        split_tf32(v[b + 2], h1_, l1_);
-        *reinterpret_cast<float2*>(p0 + b * 4) = make_float2(__uint_as_float(h0), __uint_as_float(h1_));
-        *reinterpret_cast<float2*>(p0 + b * 4 + nu * 8) = make_float2(__uint_as_float(l0), __uint_as_float(l1_));
-      }
+      for (int b = 0; b < 2; ++b)   // features 2t, 2t+1 of the n-tile
+        *reinterpret_cast<float2*>(p0 + b * 4) = make_float2(v[b], v[b + 2]);
     }
   }
 }
@@ -539,7 +534,7 @@ __global__ void __launch_bounds__(CH_THREADS, 1) chain_bwd_kernel(NetGeom g, Mid
         to_frags<N2>(d2, d2h, d2l);
       }
       warp_arrive(&e_full, lane);           // this warp's delta rows are complete; delta_1 below needs nobody else
-      float* dg = a.DG + (size_t)(ct0 * 8 + 2 * warp) * (2 * a.nu * 8);
+      float* dg = a.DG + (size_t)(ct0 * 8 + 2 * warp) * (a.nu * 8);
       constexpr int NA = (N1 + 1) / 2, NB = N1 - NA;
       delta1_block<ACT, NA, 0, N1, N2>(d2h, d2l, Ws + S::woff(2), cb, g.d[1], ok, gb1s + warp * 8 * N1, dg, a.nu, lane);
       if constexpr (NB > 0)
@@ -547,7 +542,7 @@ __global__ void __launch_bounds__(CH_THREADS, 1) chain_bwd_kernel(NetGeom g, Mid
       if (ok && a.nu > 8 * N1) {   // the one operand n-group beyond the chain's padded width is zeros
         float* dgz = dg + 8 * N1 * 4 + lane;
 #pragma unroll
-        for (int k = 0; k < 8; ++k) dgz[(size_t)k * (a.nu * 4)] = 0.f;   // [tg 2][hi|lo 2][khalf 2] x 32 floats
+        for (int k = 0; k < 4; ++k) dgz[(size_t)k * (a.nu * 4)] = 0.f;   // [tg 2][khalf 2] x 32 floats
       }
     }
     bar_wait(&e_full, tile_no & 1);

@@ -134,7 +134,7 @@ struct FtArgs {
   const float* logstd;  // theta image logstd block (DiagGauss) or nullptr
   const float* Zt;      // x . V_1, tile-major [tile][d1][LDT]
   const float* cache;   // activations of theta, tile-major [tile][act_rows][LDT]
-  float* DG;            // delta_1 operand of the layer-1 gradient GEMM, K-major: [t/8][hi | lo][khalf][n/8][8 n][4 t]
+  float* DG;            // delta_1 operand of the layer-1 gradient GEMM, K-major raw fp32: [t/8][khalf][n/8][8 n][4 t]
   float* partm;         // [n_slabs][pmid]
   long long N;
   int n_tiles, n_mtiles, slab_mt, n_slabs, nu;
@@ -688,9 +688,9 @@ __global__ void __launch_bounds__(FT_THREADS, 1) fvp_tc_kernel(NetGeom g, FtPlan
               }
               if (l == 2) {
                 // ---- final, chunk c: delta_1 = d_1' * act'(h_1) -> DG (K-major tcgen05 B operand of the layer-1 gradient
-                // GEMM: [t/8][hi|lo][khalf][n/8][8 n][4 t]) + bias partial sums.  The two groups take alternate 8-column
-                // blocks; a 4 x 4 transpose inside each lane quad turns (4 features of my timestep) into (my feature at
-                // the quad's 4 timesteps) = one 16-byte store.
+                // GEMM as raw fp32: [t/8][khalf][n/8][8 n][4 t]; l1_grad_tc_kernel splits it into (hi, lo)) + bias partial
+                // sums.  The two groups take alternate 8-column blocks; a 4 x 4 transpose inside each lane quad turns
+                // (4 features of my timestep) into (my feature at the quad's 4 timesteps) = one 16-byte store.
                 const FtDStage st = P.ds[k];
                 const float* h1row = cb + (size_t)g.off_act[1] * MRL_LDT;
                 float h1c[8], h1n[8];
@@ -705,7 +705,7 @@ __global__ void __launch_bounds__(FT_THREADS, 1) fvp_tc_kernel(NetGeom g, FtPlan
                 tc_fence_after();
                 const uint32_t facc = tlane + st.acc_col;
                 // quad base: timesteps 4 (T / 4) .. + 3 of feature n: + (n / 8) * 32 + (n % 8) * 4
-                float* dgq = a.DG + (size_t)(T >> 3) * (2 * nu * 8) + ((T >> 2) & 1) * (nu * 4);
+                float* dgq = a.DG + (size_t)(T >> 3) * (nu * 8) + ((T >> 2) & 1) * (nu * 4);
                 for (; j0 < st.N; j0 += 16) {
                   const int c0 = st.col0 + j0;
                   if (j0 + 16 < st.N) request1(c0 + 16, h1n);
@@ -718,14 +718,10 @@ __global__ void __launch_bounds__(FT_THREADS, 1) fvp_tc_kernel(NetGeom g, FtPlan
                   for (int hq = 0; hq < 2; ++hq) {
                     float tq[4] = {val[4 * hq], val[4 * hq + 1], val[4 * hq + 2], val[4 * hq + 3]};
                     ft_quad_transpose(tq, lane);
-                    uint32_t hi[4], lo[4];
-#pragma unroll
-                    for (int i = 0; i < 4; ++i) ft_split(tq[i], hi[i], lo[i]);
                     if (ok) {
                       const int n = c0 + 4 * hq + (lane & 3);
                       float* p = dgq + (n >> 3) * 32 + (n & 7) * 4;
-                      *reinterpret_cast<uint4*>(p) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
-                      *reinterpret_cast<uint4*>(p + nu * 8) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
+                      *reinterpret_cast<float4*>(p) = make_float4(tq[0], tq[1], tq[2], tq[3]);
                     }
                   }
                   // column sums over the warp's 32 timesteps: 8 -> 4 -> 2 -> 1 values per lane, then the quad

@@ -14,7 +14,8 @@
 //
 // A (the observations) is fed to the tensor core from TENSOR MEMORY (TS-mode tcgen05.mma): four converter
 // warps read each landed raw block from shared memory, split it into (hi, lo) in registers and write both with
-// tcgen05.st into a ring of TMEM slots; B (weights / delta_1: small, pre-split hi | lo) stays in shared memory.
+// tcgen05.st into a ring of TMEM slots; B (weights: small, pre-split hi | lo; delta_1: raw, split in place by the
+// same converter warps) stays in shared memory.
 // With both operands in shared memory (round 1b/1c-early) the three MMAs of a k-group read 22.5 KB of it and the
 // copies + converter another 23 KB: shared-memory bandwidth (128 B/cycle), not the tensor pipe, set the pace.
 //   stage (forward):  [A raw fp32: 3 k-groups x 4 KB][B: 3 x (hi | lo) x [khalf 2][ngroup NU/8][8][4]]
@@ -237,7 +238,8 @@ __global__ void __launch_bounds__(TC_THREADS, 1) l1_forward_tc_kernel(const floa
 // part1[slab][f][n] = sum_{t in slab} X[t][f] * delta1[t][n]  on the tensor cores:
 // D[128 features x NU] += A[128 x 8 timesteps] . B[NU x 8 timesteps]^T, K = timesteps.
 //   XG: [tg = t/8][ftile][khalf][fgroup 16][8 features][4 timesteps]  raw fp32 (split by the converter warps)
-//   DG: [tg][hi|lo][khalf][ngroup NU/8][8][4 timesteps]       (written by mid_backward_kernel)
+//   DG: [tg][khalf][ngroup NU/8][8][4 timesteps]  raw fp32 delta_1 (written by the reverse sweep: fvp_tc_kernel,
+//       chain_bwd_kernel or mid_backward_kernel; split into (hi, lo) in shared memory by the converter warps)
 // One CTA accumulates a whole slab (<= 1024 timesteps) for all feature tiles in TMEM (ftiles x
 // acc_cols columns), then the epilogue warps store the fp32 partial that reduce_partials_kernel sums
 // in fp64.  Same warp roles and stage ring as the forward kernel.
@@ -260,8 +262,10 @@ __global__ void __launch_bounds__(TC_THREADS, 1) l1_grad_tc_kernel(const float* 
   uint64_t* tempty = tfull + 1;
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(tempty + 1);
   unsigned char* stages = smem_raw + 512;
-  // a stage = one group of 8 timesteps: [A raw fp32: ftiles x 4 KB][B = delta_1 (hi | lo)]; HBM order = stage order
-  const uint32_t blkA = TC_M * 8 * 4, bytesB = 2 * nu * 8 * 4;
+  // a stage = one group of 8 timesteps: [A raw fp32: ftiles x 4 KB][B = delta_1 (hi | lo)]; HBM order = stage order.
+  // DG holds delta_1 as raw fp32 (half the bytes of a pre-split copy): it lands in the hi block, the converter group
+  // of the stage splits it in place and writes lo behind it
+  const uint32_t blkA = TC_M * 8 * 4, bytesD = nu * 8 * 4, bytesB = 2 * bytesD;
   const uint32_t offB = ftiles * blkA;
   const uint32_t stage_bytes = offB + bytesB;
   const uint32_t a_col0 = ftiles * acc_stride;              // TMEM: accumulators, then the A ring [slot][ftile][hi 8 | lo 8]
@@ -292,9 +296,9 @@ __global__ void __launch_bounds__(TC_THREADS, 1) l1_grad_tc_kernel(const float* 
         for (int tg = t0 * 8; tg < t1 * 8; ++tg) {
           mbar_wait_guard(&sempty[s], ph ^ 1);
           unsigned char* st = stages + (size_t)s * stage_bytes;
-          mbar_expect_tx(&full[s], offB + bytesB);
+          mbar_expect_tx(&full[s], offB + bytesD);
           bulk_g2s(st, XG + (size_t)tg * xg_ftiles * (TC_M * 8), offB, &full[s]);
-          bulk_g2s(st + offB, DG + (size_t)tg * (2 * nu * 8), bytesB, &full[s]);
+          bulk_g2s(st + offB, DG + (size_t)tg * (nu * 8), bytesD, &full[s]);
           if (++s == nss) { s = 0; ph ^= 1; }
         }
       }
@@ -313,7 +317,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) l1_grad_tc_kernel(const float* 
       mbar_wait_guard(&tempty[0], (scount & 1) ^ 1);
       tc_fence_after();
       for (int tg = t0 * 8; tg < t1 * 8; ++tg) {
-        mbar_wait_guard(&conv[a], aph);   // raised after the converters saw full[s]: covers A (tensor memory) and B
+        mbar_wait_guard(&conv[a], aph);   // raised after the converters saw full[s]: covers A (tensor memory) and B (split)
         tc_fence_after();
         if (elect_one()) {
           const uint32_t db = dB0 + s * (stage_bytes >> 4);
@@ -333,7 +337,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) l1_grad_tc_kernel(const float* 
         if (++a == nts) { a = 0; aph ^= 1; }
       }
     }
-  } else if (warp >= 6) {   // converters: raw A rows -> tensor memory (hi, lo)
+  } else if (warp >= 6) {   // converters: raw A rows -> tensor memory (hi, lo); raw delta_1 -> (hi | lo) in place
     const int quarter = warp & 3;
     const int m = quarter * 32 + lane;
     const int cgroup = (warp - 6) >> 2;
@@ -360,6 +364,22 @@ __global__ void __launch_bounds__(TC_THREADS, 1) l1_grad_tc_kernel(const float* 
           tmem_st8(ta, hi);
           tmem_st8(ta + 8, lo);
           ta += 16;
+        }
+        {   // delta_1 (B) in shared memory, while the tensor-memory stores drain: raw -> hi in place, lo one block behind
+          float4* pb = reinterpret_cast<float4*>(stages + (size_t)s * stage_bytes + offB);
+          for (int i = m; i < 2 * nu; i += TC_M) {
+            const float4 x = pb[i];
+            uint32_t hi[4], lo[4];
+            const float xs[4] = {x.x, x.y, x.z, x.w};
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {
+              hi[k] = (__float_as_uint(xs[k]) + 0x1000u) & 0xffffe000u;
+              lo[k] = __float_as_uint(xs[k] - __uint_as_float(hi[k])) + 0x1000u;
+            }
+            pb[i] = make_float4(__uint_as_float(hi[0]), __uint_as_float(hi[1]), __uint_as_float(hi[2]), __uint_as_float(hi[3]));
+            pb[i + 2 * nu] = make_float4(__uint_as_float(lo[0]), __uint_as_float(lo[1]), __uint_as_float(lo[2]), __uint_as_float(lo[3]));
+          }
+          fence_proxy_async();   // generic-proxy writes, read by tcgen05.mma through the async proxy
         }
         asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
         tc_fence_before();
@@ -511,7 +531,7 @@ cudaError_t launch_pack_xa(const void* src, int dtype, long long ld, int ncols, 
   return cudaGetLastError();
 }
 size_t l1tc_xg_floats(int xg_ftiles, long long n_tiles) { return (size_t)n_tiles * 8 * xg_ftiles * TC_M * 8; }
-size_t l1tc_dg_floats(const NetGeom& g, long long n_tiles) { return (size_t)n_tiles * 8 * 2 * l1tc_nu(g) * 8; }
+size_t l1tc_dg_floats(const NetGeom& g, long long n_tiles) { return (size_t)n_tiles * 8 * l1tc_nu(g) * 8; }
 
 cudaError_t launch_pack_xg(const void* src, int dtype, long long ld, int ncols, long long N, float* XG, int xg_ftiles,
                            long long n_tiles, cudaStream_t st) {

@@ -555,19 +555,14 @@ __global__ void __launch_bounds__(MRL_BWD_THREADS, 1) mid_backward_kernel(NetGeo
       const float* D1 = E;  // off_act[1] == 0
       const int n1 = g.d[1];
       for (int job = ln.warp; job < ((n1 + 7) >> 3); job += NW) bias_job(job, ln, D1, n1, G + g.off_b[1]);
-      if (a.DG) {   // split-precision tensor-core operand: 4 consecutive timesteps of one column per thread
+      if (a.DG) {   // tensor-core operand (raw fp32, split by l1_grad_tc_kernel): 4 consecutive timesteps of one column per thread
         const int nu = a.nu;
         for (int i = tid; i < 16 * nu; i += MRL_BWD_THREADS) {
           const int tq = i / nu, n = i % nu;       // timesteps 4*tq .. +3 of this tile
           float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
           if (n < n1) v = *reinterpret_cast<const float4*>(D1 + n * MRL_LDT + 4 * tq);
-          uint32_t hx, hy, hz, hw, lx, ly, lz, lw;   // integer split (see split_tf32); UMMA reads the top 19 bits
-          split_tf32(v.x, hx, lx); split_tf32(v.y, hy, ly); split_tf32(v.z, hz, lz); split_tf32(v.w, hw, lw);
-          const float4 h = make_float4(__uint_as_float(hx), __uint_as_float(hy), __uint_as_float(hz), __uint_as_float(hw));
-          const float4 l = make_float4(__uint_as_float(lx), __uint_as_float(ly), __uint_as_float(lz), __uint_as_float(lw));
-          float* base = a.DG + ((size_t)tile * 8 + (tq >> 1)) * (2 * nu * 8) + (tq & 1) * (nu * 4) + (n >> 3) * 32 + (n & 7) * 4;
-          *reinterpret_cast<float4*>(base) = h;
-          *reinterpret_cast<float4*>(base + nu * 8) = l;
+          float* base = a.DG + ((size_t)tile * 8 + (tq >> 1)) * (nu * 8) + (tq & 1) * (nu * 4) + (n >> 3) * 32 + (n & 7) * 4;
+          *reinterpret_cast<float4*>(base) = v;
         }
       }
     }
