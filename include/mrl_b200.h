@@ -205,7 +205,18 @@ int mrl_population_forward(int device, int n_layers, const int* dims, int activa
  *   mrl_rollout_read: the last round, path-major (episode i = environment i): lengths int32[n_envs],
  *     terminated uint8[n_envs], observation f64 [n x ob_dim] (filtered), action int32 [n] (Categorical) or
  *     f32 [n x d] (DiagGauss), prob f32 [n x 2] (probabilities or [mean, std]), raw reward f64 [n],
- *     states f64 [n x state_dim] (CartPole 4, Pendulum 2: (theta, theta_dot)).  Any pointer may be NULL. */
+ *     states f64 [n x state_dim] (CartPole 4, Pendulum 2: (theta, theta_dot)).  Any pointer may be NULL.  After a
+ *     round without rows (mrl_rollout_run_population, want_rows = 0) only lengths and terminated may be non-NULL.
+ *   mrl_rollout_run_population: one round in which environment m acts deterministically with its own theta_m (the
+ *     cross-entropy method's population, cem.py:43-44,88-91).  n_members <= the handle's n_envs environments run;
+ *     thetas [n_members x ld_theta] float32 where `theta_loc` says (MRL_HOST: one copy into a device buffer the handle
+ *     keeps; MRL_DEVICE: read in place), each row the Dense kernels and biases of n_layers layers of widths dims[0..]
+ *     (1..256) in the reference's flat order, no logstd block, ld_theta >= that count.  The action is taken from the
+ *     raw last-layer output: its argmax, first maximum (CartPole), or the output itself (Pendulum).
+ *     returns[n_members] (host, float64) = the sum of each episode's raw rewards in step order.  Filters as
+ *     mrl_rollout_run.  want_rows != 0 records the rows for mrl_rollout_read, the prob row then holding the raw
+ *     outputs (CartPole: the two logits; Pendulum: [mean, 1]); want_states (needs want_rows) the raw states.
+ *     Synchronises `stream`; *n_timesteps = timesteps collected. */
 #define MRL_ENV_CARTPOLE 0
 #define MRL_ENV_PENDULUM 1
 typedef struct mrl_rollout mrl_rollout;
@@ -220,6 +231,13 @@ int mrl_rollout_run(mrl_rollout* r, mrl_net* policy, unsigned long long seed, in
                     const mrl_zfilter_cfg* ob_cfg, double* ob_state, double* ob_pushed,
                     const mrl_zfilter_cfg* rew_cfg, double* rew_state, double* rew_pushed,
                     int want_states, long long* n_timesteps, void* stream);
+int mrl_rollout_run_population(mrl_rollout* r, int n_layers, const int* dims, int activation,
+                               const float* thetas, long long ld_theta, int theta_loc, int n_members,
+                               unsigned long long seed,
+                               const mrl_zfilter_cfg* ob_cfg, double* ob_state, double* ob_pushed,
+                               const mrl_zfilter_cfg* rew_cfg, double* rew_state, double* rew_pushed,
+                               double* returns, int want_rows, int want_states,
+                               long long* n_timesteps, void* stream);
 int mrl_rollout_read(mrl_rollout* r, int* lengths, unsigned char* terminated, double* obs, void* act, float* prob,
                      double* reward, double* states);
 

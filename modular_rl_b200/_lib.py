@@ -94,6 +94,9 @@ _SIGS = {
     "mrl_rollout_destroy": (_I, [_P]),
     "mrl_rollout_run": (_I, [_P, _P, C.c_ulonglong, _I, C.POINTER(ZFilterCfg), _P, _P, C.POINTER(ZFilterCfg), _P, _P,
                              _I, C.POINTER(_LL), _P]),
+    "mrl_rollout_run_population": (_I, [_P, _I, C.POINTER(_I), _I, _P, _LL, _I, _I, C.c_ulonglong,
+                                        C.POINTER(ZFilterCfg), _P, _P, C.POINTER(ZFilterCfg), _P, _P,
+                                        _P, _I, _I, C.POINTER(_LL), _P]),
     "mrl_rollout_read": (_I, [_P, _P, _P, _P, _P, _P, _P, _P]),
 }
 

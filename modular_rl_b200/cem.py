@@ -3,8 +3,11 @@ modular_rl/cem.py API (cem, CEM_OPTIONS, run_cem_algorithm), SURVEY section 8f r
 
 Every population member is scored by one rollout with its theta loaded into the device-resident net
 (`agent.set_from_flat`), so the per-step `act` is the same device forward the policy-gradient agents use.
-The search arithmetic itself is a few numpy lines on the host, as in the reference."""
+The search arithmetic itself is a few numpy lines on the host, as in the reference.  With DEVICE_ENVS on, a
+generation of a built-in environment is scored by one device rollout round instead (evaluate_population_device)."""
 from __future__ import print_function
+
+import itertools
 
 import numpy as np
 
@@ -51,6 +54,36 @@ def evaluate_population(env, agent, ths, timestep_limit):
         _filter_block(agent.rewfilter, np.asarray(rews, np.float64))
         live = still
     return total
+
+
+# Score each generation of a built-in environment with one device rollout round (evaluate_population_device) instead
+# of host rollouts.  Not a CEM option - the reference's option table stays unchanged - but a process setting:
+# run_cem.py --device_envs.
+DEVICE_ENVS = False
+
+
+def evaluate_population_device(env, agent, ths, timestep_limit, seed):
+    """evaluate_population with the whole population run on the device in ONE kernel launch: environment m of the
+    round acts with ths[m] (the argmax of the raw outputs / the raw output), its score is the float64 sum of its raw
+    rewards in step order, and the agent's filters take the states after the round.  `seed` keys the Philox stream of
+    the round's resets, so start states come from the device and not from numpy's generator (which this call never
+    touches).  Raises before any device call for an environment, filter or policy the device cannot run."""
+    from .core import _advance_filter, _device_filter, _device_rollouts, _filter_arg, check_device_rollouts
+    from .device import DeviceRollouts
+    kind = check_device_rollouts(env, agent)
+    pol = agent.policy
+    ths = np.asarray(ths, np.float32)
+    key = (kind, int(ths.shape[0]), int(timestep_limit), pol.net.device)
+    if key not in _device_rollouts:
+        _device_rollouts[key] = DeviceRollouts(env, ths.shape[0], timestep_limit, device=pol.net.device)
+    obf = _device_filter(agent.obfilter, "observation filter")
+    rwf = _device_filter(agent.rewfilter, "reward filter")
+    out = _device_rollouts[key].run_population(pol.dims, pol.activation, ths, seed, _filter_arg(obf), _filter_arg(rwf))
+    if obf is not None:
+        _advance_filter(obf, out["ob_state"], out["ob_pushed"])
+    if rwf is not None:
+        _advance_filter(rwf, out["rew_state"], out["rew_pushed"])
+    return out["returns"]
 
 
 class _GaussianSearch(object):
@@ -117,15 +150,26 @@ def run_cem_algorithm(env, agent, usercfg=None, callback=None):
     """cem.py:63-98.  `parallel=1`: the reference forks a process pool around a CPU Theano function (every worker with
     its own copy of the agent and its filters); a forked child cannot share this process's CUDA context, so here
     parallel=1 scores the whole population in lockstep with one population-batched device forward per environment step
-    (`evaluate_population`).  parallel=0 scores one candidate after another as cem.py:43 does."""
+    (`evaluate_population`).  parallel=0 scores one candidate after another as cem.py:43 does.
+
+    DEVICE_ENVS on (CartPole / Pendulum only): each generation is scored by one device rollout round
+    (`evaluate_population_device`), its Philox seed a counter started from cfg["seed"], one value per generation.
+    The host paths draw the environments' resets from numpy's global generator; the device path does not touch it,
+    so the search's own randn calls are its only numpy draws.  Start states, scores and therefore later generations
+    differ from a host run with the same seed (as with run_pg.py --device_envs); equal seeds give identical device
+    runs."""
     cfg = update_default_config(CEM_OPTIONS, usercfg)
     if cfg["std_decay_time"] < 0:
         cfg["std_decay_time"] = cfg["n_iter"] / 2
     if usercfg:
         cfg.update(usercfg)
     print("cem config", {k: cfg[k] for (k, _, _, _) in CEM_OPTIONS})
+    if cfg["parallel"] and DEVICE_ENVS:
+        raise ValueError("parallel=1 (host population path) and DEVICE_ENVS select different scoring paths; choose one")
     if cfg["parallel"]:
         print("parallel=1: population-batched evaluation (one device forward per step for all candidates)")
+    if DEVICE_ENVS:
+        print("device_envs: one device rollout round per generation")
     timestep_limit = cfg["timestep_limit"]
 
     def objective(th):
@@ -134,6 +178,9 @@ def run_cem_algorithm(env, agent, usercfg=None, callback=None):
         return path["reward"].sum()
     if cfg["parallel"]:
         objective.population = lambda ths: evaluate_population(env, agent, ths, timestep_limit)
+    if DEVICE_ENVS:
+        seeds = itertools.count(int(cfg.get("seed", 0)))
+        objective.population = lambda ths: evaluate_population_device(env, agent, ths, timestep_limit, next(seeds))
 
     th_mean = agent.get_flat()
     for info in cem(objective, th_mean, cfg["batch_size"], cfg["n_iter"], cfg["elite_frac"],

@@ -1248,13 +1248,14 @@ extern "C" int mrl_net_get_trpo_vectors(mrl_net* n, double* stepdir, double* ful
 // ======================================================================== device-resident rollouts (rollout.cu)
 struct mrl_rollout {
   int device = 0, env = 0, N = 0, T = 0, d0 = 0, sd = 0, dout = 0, head = 0;
-  DevBuf s_obs, s_state, s_prob, s_act, s_rew, lengths, term, headbuf, body, filt;
+  DevBuf s_obs, s_state, s_prob, s_act, s_rew, lengths, term, headbuf, body, filt, returns, thetas;
   double* h_head = nullptr;      // pinned: header, then lengths int32[N], terminated int32[N]
   double* h_filt = nullptr;      // pinned: incoming filter states
   char* h_body = nullptr;        // pinned: compacted rows of the last round
   size_t h_body_cap = 0;
   long long total = 0;
-  int with_states = 0;
+  int n_round = 0;               // environments of the last round (a population round may run fewer than N)
+  int with_states = 0, with_rows = 1;
 };
 static int ro_head_doubles(int d0) { return 9 + 4 * d0; }
 
@@ -1264,7 +1265,7 @@ extern "C" int mrl_rollout_destroy(mrl_rollout* r) {
   if (!r) return 0;
   cudaSetDevice(r->device);
   DevBuf* bufs[] = {&r->s_obs, &r->s_state, &r->s_prob, &r->s_act, &r->s_rew, &r->lengths, &r->term, &r->headbuf,
-                    &r->body, &r->filt};
+                    &r->body, &r->filt, &r->returns, &r->thetas};
   for (DevBuf* d : bufs) d->release();
   if (r->h_head) cudaFreeHost(r->h_head);
   if (r->h_filt) cudaFreeHost(r->h_filt);
@@ -1283,7 +1284,7 @@ extern "C" int mrl_rollout_create(mrl_rollout** out, int device, int env, int n_
   if (timestep_limit < 1) return fail("mrl_rollout_create: timestep_limit must be >= 1");
   CK(cudaSetDevice(device));
   mrl_rollout* r = new mrl_rollout();
-  r->device = device; r->env = env; r->N = n_envs; r->T = timestep_limit;
+  r->device = device; r->env = env; r->N = n_envs; r->T = timestep_limit; r->n_round = n_envs;
   r->d0 = d0; r->sd = sd; r->dout = dout; r->head = head;
   const size_t rows = (size_t)n_envs * timestep_limit;
   const RolloutLayout lay = rollout_layout((long long)rows, d0, sd, 2, head == MRL_HEAD_CAT ? 1 : dout, 1);
@@ -1292,6 +1293,7 @@ extern "C" int mrl_rollout_create(mrl_rollout** out, int device, int env, int n_
   R(r->s_obs, rows * d0 * 8); R(r->s_state, rows * sd * 8); R(r->s_prob, rows * 2 * 4);
   R(r->s_act, rows * dout * 4); R(r->s_rew, rows * 8); R(r->lengths, (size_t)n_envs * 4); R(r->term, (size_t)n_envs * 4);
   R(r->headbuf, (size_t)ro_head_doubles(d0) * 8); R(r->body, lay.end); R(r->filt, (size_t)(4 + 2 * d0) * 8);
+  R(r->returns, (size_t)n_envs * 8);
   const size_t hb = (size_t)ro_head_doubles(d0) * 8 + (size_t)n_envs * 8;
   if (e == cudaSuccess) e = cudaMallocHost(&r->h_head, hb);
   if (e == cudaSuccess) e = cudaMallocHost(&r->h_filt, (size_t)(4 + 2 * d0) * 8);
@@ -1303,84 +1305,75 @@ extern "C" int mrl_rollout_create(mrl_rollout** out, int device, int env, int n_
   return 0;
 }
 
-extern "C" int mrl_rollout_run(mrl_rollout* r, mrl_net* policy, unsigned long long seed, int stochastic,
-                               const mrl_zfilter_cfg* ob_cfg, double* ob_state, double* ob_pushed,
-                               const mrl_zfilter_cfg* rew_cfg, double* rew_state, double* rew_pushed,
-                               int want_states, long long* n_timesteps, void* stream) {
-  if (!r || !policy || !n_timesteps) return fail("mrl_rollout_run: bad arguments");
-  const bool ob_on = ob_cfg && ob_cfg->enabled, rew_on = rew_cfg && rew_cfg->enabled;
-  if ((ob_on && !ob_state) || (rew_on && !rew_state)) return fail("mrl_rollout_run: an enabled filter needs its state");
-  const NetGeom& g = policy->g;
-  const char* env_name = r->env == MRL_ENV_CARTPOLE ? "CartPole" : "Pendulum";
-  if (policy->device != r->device)
-    return fail("mrl_rollout_run: the policy lives on device %d, the rollouts on device %d", policy->device, r->device);
-  if (g.d[0] != r->d0)
-    return fail("mrl_rollout_run: %s observations have %d entries, the policy takes %d", env_name, r->d0, g.d[0]);
-  if (g.head != r->head || g.d[g.L] != r->dout)
-    return fail("mrl_rollout_run: %s needs a %s head with %d outputs (the policy has a %s head with %d)", env_name,
-                r->head == MRL_HEAD_CAT ? "Categorical" : "DiagGauss", r->dout,
-                g.head == MRL_HEAD_CAT ? "Categorical" : (g.head == MRL_HEAD_GAUSS ? "DiagGauss" : "value"), g.d[g.L]);
-  CK(cudaSetDevice(r->device));
-  cudaStream_t st = (cudaStream_t)stream;
-  const int d0 = r->d0;
-
-  RolloutArgs a = {};
-  a.N = r->N; a.T = r->T;
-  int n_ctas, threads;
-  rollout_shape(r->N, &n_ctas, &a.per_cta, &threads);
-  a.L = g.L;
+// The net's geometry in the round's arguments: layer widths and the activation rows of the forward in shared memory.
+static void ro_net_args(RolloutArgs& a, int L, const int* d) {
+  a.L = L;
   int wmax = 1;
-  for (int l = 0; l <= g.L; ++l) {
-    a.d[l] = g.d[l];
-    if (l > 0 && l < g.L && g.d[l] > wmax) wmax = g.d[l];
+  for (int l = 0; l <= L; ++l) {
+    a.d[l] = d[l];
+    if (l > 0 && l < L && d[l] > wmax) wmax = d[l];
   }
-  a.P = g.P;
   a.ldh = wmax + 1;                               // odd stride: the rows of one warp fall into distinct banks
   a.rows_chunk = 8192 / a.ldh < 128 ? 8192 / a.ldh : 128;   // 64 KB of activations
-  a.w_floats = (size_t)g.P * 4 <= 128 * 1024 ? g.P : 0;
-  a.theta = policy->theta.as<float>();
-  a.seed = seed;
-  a.stochastic = stochastic != 0;
+}
+
+// Filters in, one launch, and the copies back of a round (mrl_rollout_run, mrl_rollout_run_population).  `a` holds
+// the round's shape, net and parameters; `returns` (population rounds) receives the scores on the host.
+static int ro_round(mrl_rollout* r, RolloutArgs& a, int act, bool pop, const char* who,
+                    const mrl_zfilter_cfg* ob_cfg, double* ob_state, double* ob_pushed,
+                    const mrl_zfilter_cfg* rew_cfg, double* rew_state, double* rew_pushed,
+                    double* returns, int want_rows, int want_states, long long* n_timesteps, cudaStream_t st) {
+  const bool ob_on = ob_cfg && ob_cfg->enabled, rew_on = rew_cfg && rew_cfg->enabled;
+  const int d0 = r->d0;
+  int n_ctas, threads;
+  rollout_shape(a.N, &n_ctas, &a.per_cta, &threads);
   a.ob_on = ob_on; a.rew_on = rew_on;
   a.ob_demean = ob_on && ob_cfg->demean; a.ob_destd = ob_on && ob_cfg->destd; a.ob_clip = ob_on ? ob_cfg->clip : 0.0;
-  double* hf = r->h_filt;
-  for (int i = 0; i < 4 + 2 * d0; ++i) hf[i] = 0.0;
-  if (ob_on) for (int i = 0; i < 1 + 2 * d0; ++i) hf[i] = ob_state[i];
-  if (rew_on) for (int i = 0; i < 3; ++i) hf[1 + 2 * d0 + i] = rew_state[i];
-  CK(cudaMemcpyAsync(r->filt.p, hf, (size_t)(4 + 2 * d0) * 8, cudaMemcpyHostToDevice, st));
+  a.want_rows = want_rows != 0;
   a.filt_in = r->filt.as<double>();
   a.s_obs = r->s_obs.as<double>(); a.s_state = want_states ? r->s_state.as<double>() : nullptr;
   a.s_prob = r->s_prob.as<float>(); a.s_act = r->s_act.p; a.s_rew = r->s_rew.as<double>();
   a.lengths = r->lengths.as<int>(); a.term = r->term.as<int>();
   a.head = r->headbuf.as<double>(); a.body = r->body.as<char>();
-  const size_t smem = rollout_smem_bytes(a, d0, r->dout);
+  a.returns = r->returns.as<double>();
+  const size_t smem = rollout_smem_bytes(a, d0, r->dout, pop);
   int dev_smem = 0;
   CK(cudaDeviceGetAttribute(&dev_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, r->device));
   if (smem + 16384 > (size_t)dev_smem)
-    return fail("mrl_rollout_run: the rollout kernel needs %zu B of shared memory per CTA, device offers %d", smem, dev_smem);
-  CKP(PK_ROLLOUT, launch_rollout(a, r->env, g.act, n_ctas, threads, smem, st), 1);
+    return fail("%s: the rollout kernel needs %zu B of shared memory per CTA, device offers %d", who, smem, dev_smem);
+  double* hf = r->h_filt;
+  for (int i = 0; i < 4 + 2 * d0; ++i) hf[i] = 0.0;
+  if (ob_on) for (int i = 0; i < 1 + 2 * d0; ++i) hf[i] = ob_state[i];
+  if (rew_on) for (int i = 0; i < 3; ++i) hf[1 + 2 * d0 + i] = rew_state[i];
+  CK(cudaMemcpyAsync(r->filt.p, hf, (size_t)(4 + 2 * d0) * 8, cudaMemcpyHostToDevice, st));
+  CKP(PK_ROLLOUT, launch_rollout(a, r->env, act, pop, n_ctas, threads, smem, st), 1);
 
-  // header + lengths + terminated, then the collected rows only
+  // header + lengths + terminated (+ scores), then the collected rows only
   const int nh = ro_head_doubles(d0);
   int* h_len = (int*)(r->h_head + nh);
   CK(cudaMemcpyAsync(r->h_head, r->headbuf.p, (size_t)nh * 8, cudaMemcpyDeviceToHost, st));
-  CK(cudaMemcpyAsync(h_len, r->lengths.p, (size_t)r->N * 4, cudaMemcpyDeviceToHost, st));
-  CK(cudaMemcpyAsync(h_len + r->N, r->term.p, (size_t)r->N * 4, cudaMemcpyDeviceToHost, st));
+  CK(cudaMemcpyAsync(h_len, r->lengths.p, (size_t)a.N * 4, cudaMemcpyDeviceToHost, st));
+  CK(cudaMemcpyAsync(h_len + a.N, r->term.p, (size_t)a.N * 4, cudaMemcpyDeviceToHost, st));
+  if (returns) CK(cudaMemcpyAsync(returns, r->returns.p, (size_t)a.N * 8, cudaMemcpyDeviceToHost, st));
   CK(cudaStreamSynchronize(st));
   const double* h = r->h_head;
   r->total = (long long)h[0];
-  r->with_states = want_states != 0;
-  const RolloutLayout lay = rollout_layout(r->total, d0, r->sd, 2, r->head == MRL_HEAD_CAT ? 1 : r->dout,
-                                           r->with_states);
-  if (lay.end > r->h_body_cap) {
-    if (r->h_body) cudaFreeHost(r->h_body);
-    r->h_body = nullptr;
-    r->h_body_cap = 0;
-    CK(cudaMallocHost(&r->h_body, lay.end + lay.end / 4 + 256));
-    r->h_body_cap = lay.end + lay.end / 4 + 256;
+  r->n_round = a.N;
+  r->with_rows = want_rows != 0;
+  r->with_states = want_rows && want_states;
+  if (r->with_rows) {
+    const RolloutLayout lay = rollout_layout(r->total, d0, r->sd, 2, r->head == MRL_HEAD_CAT ? 1 : r->dout,
+                                             r->with_states);
+    if (lay.end > r->h_body_cap) {
+      if (r->h_body) cudaFreeHost(r->h_body);
+      r->h_body = nullptr;
+      r->h_body_cap = 0;
+      CK(cudaMallocHost(&r->h_body, lay.end + lay.end / 4 + 256));
+      r->h_body_cap = lay.end + lay.end / 4 + 256;
+    }
+    if (lay.end) CK(cudaMemcpyAsync(r->h_body, r->body.p, lay.end, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
   }
-  if (lay.end) CK(cudaMemcpyAsync(r->h_body, r->body.p, lay.end, cudaMemcpyDeviceToHost, st));
-  CK(cudaStreamSynchronize(st));
   if (ob_on) {
     for (int i = 0; i < 1 + 2 * d0; ++i) ob_state[i] = h[1 + i];
     if (ob_pushed) for (int i = 0; i < 1 + 2 * d0; ++i) ob_pushed[i] = h[2 + 2 * d0 + i];
@@ -1393,13 +1386,106 @@ extern "C" int mrl_rollout_run(mrl_rollout* r, mrl_net* policy, unsigned long lo
   return 0;
 }
 
+static const char* ro_env_name(const mrl_rollout* r) { return r->env == MRL_ENV_CARTPOLE ? "CartPole" : "Pendulum"; }
+
+extern "C" int mrl_rollout_run(mrl_rollout* r, mrl_net* policy, unsigned long long seed, int stochastic,
+                               const mrl_zfilter_cfg* ob_cfg, double* ob_state, double* ob_pushed,
+                               const mrl_zfilter_cfg* rew_cfg, double* rew_state, double* rew_pushed,
+                               int want_states, long long* n_timesteps, void* stream) {
+  if (!r || !policy || !n_timesteps) return fail("mrl_rollout_run: bad arguments");
+  const bool ob_on = ob_cfg && ob_cfg->enabled, rew_on = rew_cfg && rew_cfg->enabled;
+  if ((ob_on && !ob_state) || (rew_on && !rew_state)) return fail("mrl_rollout_run: an enabled filter needs its state");
+  const NetGeom& g = policy->g;
+  const char* env_name = ro_env_name(r);
+  if (policy->device != r->device)
+    return fail("mrl_rollout_run: the policy lives on device %d, the rollouts on device %d", policy->device, r->device);
+  if (g.d[0] != r->d0)
+    return fail("mrl_rollout_run: %s observations have %d entries, the policy takes %d", env_name, r->d0, g.d[0]);
+  if (g.head != r->head || g.d[g.L] != r->dout)
+    return fail("mrl_rollout_run: %s needs a %s head with %d outputs (the policy has a %s head with %d)", env_name,
+                r->head == MRL_HEAD_CAT ? "Categorical" : "DiagGauss", r->dout,
+                g.head == MRL_HEAD_CAT ? "Categorical" : (g.head == MRL_HEAD_GAUSS ? "DiagGauss" : "value"), g.d[g.L]);
+  CK(cudaSetDevice(r->device));
+  RolloutArgs a = {};
+  a.N = r->N; a.T = r->T;
+  ro_net_args(a, g.L, g.d);
+  a.P = g.P;
+  a.w_floats = (size_t)g.P * 4 <= 128 * 1024 ? g.P : 0;
+  a.theta = policy->theta.as<float>();
+  a.seed = seed;
+  a.stochastic = stochastic != 0;
+  return ro_round(r, a, g.act, false, "mrl_rollout_run", ob_cfg, ob_state, ob_pushed, rew_cfg, rew_state, rew_pushed,
+                  nullptr, 1, want_states, n_timesteps, (cudaStream_t)stream);
+}
+
+extern "C" int mrl_rollout_run_population(mrl_rollout* r, int n_layers, const int* dims, int activation,
+                                          const float* thetas, long long ld_theta, int theta_loc, int n_members,
+                                          unsigned long long seed,
+                                          const mrl_zfilter_cfg* ob_cfg, double* ob_state, double* ob_pushed,
+                                          const mrl_zfilter_cfg* rew_cfg, double* rew_state, double* rew_pushed,
+                                          double* returns, int want_rows, int want_states, long long* n_timesteps,
+                                          void* stream) {
+  const char* who = "mrl_rollout_run_population";
+  if (!r || !dims || !thetas || !returns || !n_timesteps) return fail("%s: bad arguments", who);
+  const bool ob_on = ob_cfg && ob_cfg->enabled, rew_on = rew_cfg && rew_cfg->enabled;
+  if ((ob_on && !ob_state) || (rew_on && !rew_state)) return fail("%s: an enabled filter needs its state", who);
+  if (want_states && !want_rows) return fail("%s: want_states = 1 needs want_rows = 1", who);
+  if (n_layers < 1 || n_layers > MRL_MAX_LAYERS)
+    return fail("%s: n_layers = %d; the rollout kernel runs 1..%d layers", who, n_layers, MRL_MAX_LAYERS);
+  const char* env_name = ro_env_name(r);
+  if (dims[0] != r->d0) return fail("%s: %s observations have %d entries, dims[0] = %d", who, env_name, r->d0, dims[0]);
+  if (dims[n_layers] != r->dout)
+    return fail("%s: %s actions take %d outputs, dims[%d] = %d", who, env_name, r->dout, n_layers, dims[n_layers]);
+  long long P = 0;
+  for (int l = 1; l <= n_layers; ++l) {
+    if (dims[l] < 1 || dims[l] > 256) return fail("%s: dims[%d] = %d; widths must be in 1..256", who, l, dims[l]);
+    P += (long long)dims[l - 1] * dims[l] + dims[l];
+  }
+  if (activation != MRL_ACT_TANH && activation != MRL_ACT_RELU && activation != MRL_ACT_SIGMOID)
+    return fail("%s: unknown activation %d (0 tanh, 1 relu, 2 sigmoid)", who, activation);
+  if (ld_theta < P) return fail("%s: ld_theta = %lld is smaller than the %lld Dense parameters", who, ld_theta, P);
+  if (n_members < 1 || n_members > r->N)
+    return fail("%s: n_members = %d; the handle runs 1..%d environments", who, n_members, r->N);
+  if (theta_loc != MRL_HOST && theta_loc != MRL_DEVICE) return fail("%s: theta_loc = %d (MRL_HOST or MRL_DEVICE)", who, theta_loc);
+  CK(cudaSetDevice(r->device));
+  cudaStream_t st = (cudaStream_t)stream;
+  const float* th = thetas;
+  if (theta_loc == MRL_HOST) {
+    const size_t bytes = (size_t)n_members * (size_t)ld_theta * 4;
+    CK(r->thetas.reserve(bytes));
+    CK(cudaMemcpyAsync(r->thetas.p, thetas, bytes, cudaMemcpyHostToDevice, st));
+    th = r->thetas.as<float>();
+  } else {
+    cudaPointerAttributes pa;
+    if (cudaPointerGetAttributes(&pa, thetas) != cudaSuccess) {
+      cudaGetLastError();
+      pa.type = cudaMemoryTypeUnregistered;
+    }
+    if ((pa.type != cudaMemoryTypeDevice && pa.type != cudaMemoryTypeManaged) || pa.device != r->device)
+      return fail("%s: theta_loc = MRL_DEVICE but thetas is not device memory of device %d", who, r->device);
+  }
+  RolloutArgs a = {};
+  a.N = n_members; a.T = r->T;
+  ro_net_args(a, n_layers, dims);
+  a.P = (int)P;
+  a.w_floats = 0;                                 // each environment reads its own theta through L2
+  a.theta = th;
+  a.ld_theta = ld_theta;
+  a.seed = seed;
+  return ro_round(r, a, activation, true, who, ob_cfg, ob_state, ob_pushed, rew_cfg, rew_state, rew_pushed,
+                  returns, want_rows, want_states, n_timesteps, st);
+}
+
 extern "C" int mrl_rollout_read(mrl_rollout* r, int* lengths, unsigned char* terminated, double* obs, void* act,
                                 float* prob, double* reward, double* states) {
   if (!r) return fail("mrl_rollout_read: null handle");
+  if (!r->with_rows && (obs || act || prob || reward || states))
+    return fail("mrl_rollout_read: the last round did not record rows (want_rows = 0); only lengths and terminated");
   if (states && !r->with_states) return fail("mrl_rollout_read: the last round did not record states (want_states = 0)");
+  const int N = r->n_round;
   const int* h_len = (const int*)(r->h_head + ro_head_doubles(r->d0));
-  if (lengths) memcpy(lengths, h_len, (size_t)r->N * 4);
-  if (terminated) for (int i = 0; i < r->N; ++i) terminated[i] = (unsigned char)h_len[r->N + i];
+  if (lengths) memcpy(lengths, h_len, (size_t)N * 4);
+  if (terminated) for (int i = 0; i < N; ++i) terminated[i] = (unsigned char)h_len[N + i];
   const long long n = r->total;
   const RolloutLayout lay = rollout_layout(n, r->d0, r->sd, 2, r->head == MRL_HEAD_CAT ? 1 : r->dout, r->with_states);
   if (obs) memcpy(obs, r->h_body + lay.obs, (size_t)n * r->d0 * 8);

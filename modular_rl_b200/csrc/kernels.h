@@ -163,6 +163,10 @@ struct RolloutArgs {
   int* lengths; int* term;
   double* head;                // total, observation state, its round part, reward state, its round part
   char* body;                  // compacted path-major rows (rollout_layout)
+  // population rounds (rollout_kernel<ENV, ACT, true>): environment e acts with theta + e * ld_theta
+  long long ld_theta;
+  double* returns;             // [N] the sum of each episode's raw rewards, in step order
+  int want_rows;               // 0: no staging rows, no compaction (lengths, terminated, returns and the header only)
 };
 // Byte offsets of the compacted arrays for n timesteps: f64 sections first, so that every section stays aligned
 struct RolloutLayout { size_t obs, rew, state, prob, act, end; };
@@ -179,5 +183,6 @@ __host__ __device__ inline RolloutLayout rollout_layout(long long n, int d0, int
 }
 int rollout_env_dims(int env, int* d0, int* sd, int* dout);   // -> head, -1 for an unknown env
 void rollout_shape(int N, int* n_ctas, int* per_cta, int* threads);
-size_t rollout_smem_bytes(const RolloutArgs& a, int d0, int dout);
-cudaError_t launch_rollout(const RolloutArgs& a, int env, int act, int n_ctas, int threads, size_t smem, cudaStream_t st);
+size_t rollout_smem_bytes(const RolloutArgs& a, int d0, int dout, bool pop);
+cudaError_t launch_rollout(const RolloutArgs& a, int env, int act, bool pop, int n_ctas, int threads, size_t smem,
+                           cudaStream_t st);

@@ -179,9 +179,11 @@ template <> struct EnvT<MRL_ENV_PENDULUM> {
 };
 
 // ---------------------------------------------------------------------------------------------------- policy forward
-// rows [0, nrows) of xin [nrows][d0] -> out [nrows][dout]: raw head output (softmax logits / Gauss mean)
-template <int ACT>
-__device__ void mlp_rows(const RolloutArgs& a, const float* W, const float* xin, int nrows, float* h, float* out) {
+// rows [0, nrows) of xin [nrows][d0] -> out [nrows][dout]: raw head output (softmax logits / Gauss mean).
+// POP: row r uses the theta of environment rowe[r], W + rowe[r] * a.ld_theta.
+template <int ACT, bool POP>
+__device__ void mlp_rows(const RolloutArgs& a, const float* W, const float* xin, int nrows, float* h, float* out,
+                         const int* rowe) {
   for (int c0 = 0; c0 < nrows; c0 += a.rows_chunk) {
     const int nr = min(a.rows_chunk, nrows - c0);
     const float* src = xin + (size_t)c0 * a.d[0];
@@ -197,9 +199,16 @@ __device__ void mlp_rows(const RolloutArgs& a, const float* W, const float* xin,
       for (int o = threadIdx.x; o < nr * dout; o += blockDim.x) {
         const int r = o / dout, j = o - r * dout;
         const float* hr = src + (size_t)r * lds;
+        const float* Wr = Wl;
+        const float* br = bl;
+        if constexpr (POP) {
+          const size_t m = (size_t)rowe[c0 + r] * a.ld_theta;
+          Wr += m;
+          br += m;
+        }
         float acc = 0.f;
-        for (int k = 0; k < din; ++k) acc = fmaf(hr[k], Wl[(size_t)k * dout + j], acc);
-        acc += bl[j];
+        for (int k = 0; k < din; ++k) acc = fmaf(hr[k], Wr[(size_t)k * dout + j], acc);
+        acc += br[j];
         dst[(size_t)r * ldd + j] = last ? acc : act_fn<ACT>(acc);
       }
       __syncthreads();
@@ -212,7 +221,11 @@ __device__ void mlp_rows(const RolloutArgs& a, const float* W, const float* xin,
 }
 
 // ---------------------------------------------------------------------------------------------------- the round
-template <int ENV, int ACT>
+// POP (population round, the cross-entropy method): environment e acts deterministically with its own Dense theta
+// (a.theta + e * a.ld_theta, no logstd block, read through L2), on the argmax of the raw outputs (CartPole) or the
+// raw output (Pendulum); a.returns[e] = the float64 sum of its raw rewards in step order; without a.want_rows no
+// staging rows are written and nothing is compacted.
+template <int ENV, int ACT, bool POP>
 __global__ void __launch_bounds__(RO_MAX_THREADS, 1) rollout_kernel(const RolloutArgs a) {
   using E = EnvT<ENV>;
   constexpr int D0 = E::D0, SD = E::SD, DOUT = E::DOUT, PD = E::PD, K = D0 + 1;   // K - 1: the reward
@@ -233,6 +246,8 @@ __global__ void __launch_bounds__(RO_MAX_THREADS, 1) rollout_kernel(const Rollou
   float* H = Ws + a.w_floats;                                 // [2][rows_chunk][ldh]
   float* XIN = H + 2 * (size_t)a.rows_chunk * a.ldh;          // [per_cta][D0]
   float* OUT = XIN + (size_t)a.per_cta * D0;                  // [per_cta][DOUT]
+  int* ROWE = (int*)(OUT + (size_t)a.per_cta * DOUT);         // POP: [per_cta] live row -> environment
+  const bool rows = !POP || a.want_rows;
 
   for (int i = threadIdx.x; i < a.w_floats; i += blockDim.x) Ws[i] = a.theta[i];
   const float* W = a.w_floats ? Ws : a.theta;
@@ -254,9 +269,10 @@ __global__ void __launch_bounds__(RO_MAX_THREADS, 1) rollout_kernel(const Rollou
   bool live = mine, term = false, rlive = false;
   double rew = 0.0;
   int len = 0;
+  double ret = 0.0;
   float logstd_exp[DOUT];
 #pragma unroll
-  for (int j = 0; j < DOUT; ++j) logstd_exp[j] = E::HEAD == MRL_HEAD_GAUSS ? expf(a.theta[a.P - DOUT + j]) : 0.f;
+  for (int j = 0; j < DOUT; ++j) logstd_exp[j] = E::HEAD == MRL_HEAD_GAUSS && !POP ? expf(a.theta[a.P - DOUT + j]) : 0.f;
 
   for (int t = 0;; ++t) {
     const bool now = live && t < a.T;
@@ -304,22 +320,44 @@ __global__ void __launch_bounds__(RO_MAX_THREADS, 1) rollout_kernel(const Rollou
           }
           if (a.ob_clip != 0.0) y = fmin(fmax(y, -a.ob_clip), a.ob_clip);
         }
-        a.s_obs[st_row * D0 + k] = y;
+        if (rows) a.s_obs[st_row * D0 + k] = y;
         XIN[row * D0 + k] = (float)y;
       }
       if (a.s_state)
 #pragma unroll
         for (int i = 0; i < SD; ++i) a.s_state[st_row * SD + i] = s[i];
+      if constexpr (POP) ROWE[row] = e;
     }
     __syncthreads();
-    mlp_rows<ACT>(a, W, XIN, nlive, H, OUT);
+    mlp_rows<ACT, POP>(a, W, XIN, nlive, H, OUT, ROWE);
     if (now) {
       const uint4 rnd = philox4x32_10(make_uint4((uint32_t)e, (uint32_t)t, RO_PURPOSE_ACTION, 0u), k0, k1);
       const double u0 = u53(rnd.x, rnd.y), u1 = u53(rnd.z, rnd.w);
       int ai = 0;
       float af = 0.f;
       float* prob = a.s_prob + st_row * PD;
-      if (E::HEAD == MRL_HEAD_CAT) {
+      if constexpr (POP) {                 // the raw outputs: argmax (first maximum) / the output itself
+        if (E::HEAD == MRL_HEAD_CAT) {     // numpy's argmax: the first NaN wins, else the first maximum
+          float best = OUT[row * DOUT];
+#pragma unroll
+          for (int j = 1; j < DOUT; ++j) {
+            const float v = OUT[row * DOUT + j];
+            if (!isnan(best) && (v > best || isnan(v))) { best = v; ai = j; }
+          }
+          if (rows) {
+#pragma unroll
+            for (int j = 0; j < DOUT; ++j) prob[j] = OUT[row * DOUT + j];
+            ((int*)a.s_act)[st_row] = ai;
+          }
+        } else {
+          af = OUT[row * DOUT];
+          if (rows) {
+            prob[0] = af;
+            prob[1] = 1.f;
+            ((float*)a.s_act)[st_row] = af;
+          }
+        }
+      } else if (E::HEAD == MRL_HEAD_CAT) {
         float z[DOUT], p[DOUT], mx = -INFINITY, sum = 0.f;
 #pragma unroll
         for (int j = 0; j < DOUT; ++j) { z[j] = OUT[row * DOUT + j]; mx = fmaxf(mx, z[j]); }
@@ -354,7 +392,8 @@ __global__ void __launch_bounds__(RO_MAX_THREADS, 1) rollout_kernel(const Rollou
         ((float*)a.s_act)[st_row] = af;
       }
       const bool done = E::step(s, ai, af, &rew);
-      a.s_rew[st_row] = rew;
+      if (rows) a.s_rew[st_row] = rew;
+      if constexpr (POP) ret += rew;
       rlive = true;
       ++len;
       if (done) { term = true; live = false; }
@@ -363,6 +402,7 @@ __global__ void __launch_bounds__(RO_MAX_THREADS, 1) rollout_kernel(const Rollou
 
   // ---- compaction: path-major rows at offsets from an exclusive scan of the lengths (CTA rank order, then index)
   if (mine) { a.lengths[e] = len; a.term[e] = term ? 1 : 0; }
+  if (POP && mine) a.returns[e] = ret;
   long long incl = len;
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
 #pragma unroll
@@ -395,7 +435,7 @@ __global__ void __launch_bounds__(RO_MAX_THREADS, 1) rollout_kernel(const Rollou
   double* b_rew = (double*)(a.body + lay.rew);
   double* b_st = (double*)(a.body + lay.state);
   float* b_prob = (float*)(a.body + lay.prob);
-  for (int tt = 0; tt < len; ++tt) {
+  for (int tt = 0; tt < (rows ? len : 0); ++tt) {
     const size_t src = (size_t)tt * a.N + e, dst = (size_t)(off + tt);
 #pragma unroll
     for (int k = 0; k < D0; ++k) b_obs[dst * D0 + k] = a.s_obs[src * D0 + k];
@@ -443,13 +483,13 @@ void rollout_shape(int N, int* n_ctas, int* per_cta, int* threads) {
   *threads = th < 128 ? 128 : th;
 }
 
-size_t rollout_smem_bytes(const RolloutArgs& a, int d0, int dout) {
-  return ((size_t)a.w_floats + 2 * (size_t)a.rows_chunk * a.ldh + (size_t)a.per_cta * (d0 + dout)) * 4;
+size_t rollout_smem_bytes(const RolloutArgs& a, int d0, int dout, bool pop) {
+  return ((size_t)a.w_floats + 2 * (size_t)a.rows_chunk * a.ldh + (size_t)a.per_cta * (d0 + dout + (pop ? 1 : 0))) * 4;
 }
 
-template <int ENV, int ACT>
+template <int ENV, int ACT, bool POP>
 static cudaError_t launch_t(const RolloutArgs& a, int n_ctas, int threads, size_t smem, cudaStream_t st) {
-  const void* f = (const void*)rollout_kernel<ENV, ACT>;
+  const void* f = (const void*)rollout_kernel<ENV, ACT, POP>;
   cudaError_t e = mrl_func_smem(f, smem);
   if (e != cudaSuccess) return e;
   cudaLaunchConfig_t cfg = {};
@@ -464,17 +504,24 @@ static cudaError_t launch_t(const RolloutArgs& a, int n_ctas, int threads, size_
   at[0].val.clusterDim.z = 1;
   cfg.attrs = at;
   cfg.numAttrs = 1;
-  return cudaLaunchKernelEx(&cfg, rollout_kernel<ENV, ACT>, a);
+  return cudaLaunchKernelEx(&cfg, rollout_kernel<ENV, ACT, POP>, a);
 }
 
-cudaError_t launch_rollout(const RolloutArgs& a, int env, int act, int n_ctas, int threads, size_t smem, cudaStream_t st) {
+template <bool POP>
+static cudaError_t launch_pop(const RolloutArgs& a, int env, int act, int n_ctas, int threads, size_t smem, cudaStream_t st) {
 #define RO_ACTS(ENV)                                                          \
   switch (act) {                                                              \
-    case MRL_ACT_TANH: return launch_t<ENV, MRL_ACT_TANH>(a, n_ctas, threads, smem, st); \
-    case MRL_ACT_RELU: return launch_t<ENV, MRL_ACT_RELU>(a, n_ctas, threads, smem, st); \
-    default: return launch_t<ENV, MRL_ACT_SIGMOID>(a, n_ctas, threads, smem, st);        \
+    case MRL_ACT_TANH: return launch_t<ENV, MRL_ACT_TANH, POP>(a, n_ctas, threads, smem, st); \
+    case MRL_ACT_RELU: return launch_t<ENV, MRL_ACT_RELU, POP>(a, n_ctas, threads, smem, st); \
+    default: return launch_t<ENV, MRL_ACT_SIGMOID, POP>(a, n_ctas, threads, smem, st);        \
   }
   if (env == MRL_ENV_CARTPOLE) { RO_ACTS(MRL_ENV_CARTPOLE) }
   RO_ACTS(MRL_ENV_PENDULUM)
 #undef RO_ACTS
+}
+
+cudaError_t launch_rollout(const RolloutArgs& a, int env, int act, bool pop, int n_ctas, int threads, size_t smem,
+                           cudaStream_t st) {
+  return pop ? launch_pop<true>(a, env, act, n_ctas, threads, smem, st)
+             : launch_pop<false>(a, env, act, n_ctas, threads, smem, st);
 }

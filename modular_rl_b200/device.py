@@ -388,15 +388,53 @@ class DeviceRollouts:
                                         C.byref(ocfg) if ocfg else None, L.ptr(ost), L.ptr(opu),
                                         C.byref(rcfg) if rcfg else None, L.ptr(rst), L.ptr(rpu),
                                         int(bool(want_states)), C.byref(n), stream))
-        T = int(n.value)
-        out = dict(lengths=np.empty(self.n_envs, np.int32), terminated=np.empty(self.n_envs, np.uint8),
-                   observation=np.empty((T, d), np.float64),
-                   action=np.empty(T, np.int32) if self.categorical else np.empty((T, self.act_dim), np.float32),
-                   prob=np.empty((T, 2 * self.act_dim if not self.categorical else 2), np.float32),
-                   reward=np.empty(T, np.float64))
+        return self._read(self.n_envs, int(n.value), True, want_states, ost, opu, rst, rpu)
+
+    def run_population(self, dims: Sequence[int], activation: str, thetas, seed: int, obfilter=None, rewfilter=None,
+                       want_rows: bool = False, want_states: bool = False, stream=None) -> dict:
+        """One round in which environment m acts deterministically with its own parameters thetas[m] (the
+        cross-entropy method's population).  thetas: [M, ld] float32, numpy (host) or a torch CUDA tensor (read in
+        place); each row holds the Dense kernels and biases of the net `dims` in the reference's flat order (no logstd
+        block), ld >= their count, M <= n_envs.  Filters as `run`.  Returns `returns` (float64 [M], the sum of each
+        episode's raw rewards), lengths, terminated, the four filter states, and with want_rows the row arrays of `run`
+        (prob: CartPole's two raw outputs, Pendulum's [mean, 1])."""
+        dims = [int(x) for x in dims]
+        if _is_torch_cuda(thetas):
+            import torch
+            keep = thetas.to(torch.float32).contiguous()
+            th_ptr, loc = C.c_void_p(keep.data_ptr()), L.DEVICE
+        else:
+            keep = np.ascontiguousarray(thetas, np.float32)
+            th_ptr, loc = L.ptr(keep), L.HOST
+        if keep.ndim != 2:
+            raise ValueError("thetas must be [members, ld_theta], got shape %s" % (tuple(keep.shape),))
+        M, ld = int(keep.shape[0]), int(keep.shape[1])
+        ocfg, ost, opu = self._filter_in(obfilter, self.ob_dim)
+        rcfg, rst, rpu = self._filter_in(rewfilter, 1)
+        returns = np.empty(M, np.float64)
+        n = C.c_longlong()
+        arr = (C.c_int * len(dims))(*dims)
+        L.check(L.lib().mrl_rollout_run_population(
+            self._h, len(dims) - 1, arr, L.ACTIVATIONS[activation], th_ptr, ld, loc, M,
+            int(seed) & 0xFFFFFFFFFFFFFFFF, C.byref(ocfg) if ocfg else None, L.ptr(ost), L.ptr(opu),
+            C.byref(rcfg) if rcfg else None, L.ptr(rst), L.ptr(rpu), L.ptr(returns), int(bool(want_rows)),
+            int(bool(want_states)), C.byref(n), stream))
+        out = self._read(M, int(n.value), want_rows, want_states, ost, opu, rst, rpu)
+        out["returns"] = returns
+        return out
+
+    def _read(self, n_envs, T, want_rows, want_states, ost, opu, rst, rpu) -> dict:
+        d = self.ob_dim
+        out = dict(lengths=np.empty(n_envs, np.int32), terminated=np.empty(n_envs, np.uint8))
+        if want_rows:
+            out.update(observation=np.empty((T, d), np.float64),
+                       action=np.empty(T, np.int32) if self.categorical else np.empty((T, self.act_dim), np.float32),
+                       prob=np.empty((T, 2 * self.act_dim if not self.categorical else 2), np.float32),
+                       reward=np.empty(T, np.float64))
         states = np.empty((T, self.state_dim), np.float64) if want_states else None
-        L.check(L.lib().mrl_rollout_read(self._h, L.ptr(out["lengths"]), L.ptr(out["terminated"]), L.ptr(out["observation"]),
-                                         L.ptr(out["action"]), L.ptr(out["prob"]), L.ptr(out["reward"]), L.ptr(states)))
+        L.check(L.lib().mrl_rollout_read(self._h, L.ptr(out["lengths"]), L.ptr(out["terminated"]),
+                                         L.ptr(out.get("observation")), L.ptr(out.get("action")),
+                                         L.ptr(out.get("prob")), L.ptr(out.get("reward")), L.ptr(states)))
         if want_states:
             out["states"] = states
         out["ob_state"], out["ob_pushed"] = self._state_out(ost, d), self._state_out(opu, d)

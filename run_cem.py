@@ -2,7 +2,7 @@
 """Cross-entropy-method driver with the reference's run_cem.py command line (GENERAL_OPTIONS, --env, --agent, --plot,
 the agent's own options, CEM_OPTIONS - run_cem.py:13-30).  Candidates are scored through the device-resident
 deterministic policy; with --parallel 1 the whole population is scored in lockstep by one population-batched forward
-per environment step.
+per environment step; with --device_envs (CartPole and Pendulum) each generation is one device rollout round.
 
   python run_cem.py --env CartPole-v0 --agent modular_rl.agentzoo.DeterministicAgent --n_iter 10 --batch_size 40
 """
@@ -34,11 +34,28 @@ def parse_cli(argv):
     ap.add_argument("--env", required=True)
     ap.add_argument("--agent", required=True)
     ap.add_argument("--plot", action="store_true")
+    ap.add_argument("--device_envs", action="store_true",
+                    help="score each generation in one GPU rollout round, one environment per candidate (built-in "
+                         "CartPole and Pendulum only); resets come from the device's Philox stream, so results differ "
+                         "from a host run with the same --seed")
     first, _ = ap.parse_known_args([a for a in argv if a not in ("-h", "--help")])
     agent_cls = mrl.get_agent_cls(first.agent)
     mrl.update_argument_parser(ap, agent_cls.options)
     mrl.update_argument_parser(ap, mrl.CEM_OPTIONS)
-    return ap.parse_args(argv), agent_cls
+    args = ap.parse_args(argv)
+    if args.device_envs:
+        from modular_rl_b200.device import DeviceRollouts
+        from modular_rl_b200.envs import device_kind
+        if args.parallel:
+            ap.error("--device_envs and --parallel 1 select different population paths; give one")
+        if args.batch_size > DeviceRollouts.max_envs():
+            ap.error("--device_envs runs a generation in one round of at most %d environments; --batch_size is %d"
+                     % (DeviceRollouts.max_envs(), args.batch_size))
+        try:
+            device_kind(args.env)
+        except ValueError as e:
+            ap.error(str(e))
+    return args, agent_cls
 
 
 class IterationLog(object):
@@ -84,6 +101,10 @@ def main(argv=None):
     np.random.seed(args.seed)
     cfg = vars(args)
     agent = restored if restored is not None else agent_cls(env.observation_space, env.action_space, cfg)
+    if args.device_envs:
+        from modular_rl_b200 import cem, core
+        core.check_device_rollouts(env, agent)     # an unsupported filter / policy fails before any rollout
+        cem.DEVICE_ENVS = True
     hdf, diagnostics = mrl.prepare_h5_file(args) if args.use_hdf else (None, None)
     mrl.run_cem_algorithm(env, agent, callback=IterationLog(args, env, agent, results_dir, hdf, diagnostics), usercfg=cfg)
     if hdf is not None:
