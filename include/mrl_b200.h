@@ -190,41 +190,58 @@ int mrl_population_forward(int device, int n_layers, const int* dims, int activa
                            long long ld_theta, const float* obs, int n_members, float* out, int loc, void* stream);
 
 /* ---------------------------------------------------------------- device-resident rollouts (core.py:182-221)
- * The rollout loop of the two built-in environments (modular_rl_b200/envs.py) on the device: one launch runs one ROUND,
+ * The rollout loop of the built-in environments (modular_rl_b200/envs.py) on the device: one launch runs one ROUND,
  * n_envs environments from reset until every episode has ended or reached timestep_limit, in the lockstep order of
  * core.rollouts_vectorized: per step the observation ZFilter over the live environments in index order, the policy
  * forward on the net's parameters in place, the action draw, the float64 dynamics of envs.py and the reward ZFilter
  * statistics.  Resets and action noise come from Philox4x32-10 keyed by `seed` (DESIGN.md "Device rollouts").
- *   mrl_rollout_create: env MRL_ENV_CARTPOLE or MRL_ENV_PENDULUM; 1 <= n_envs <= mrl_rollout_max_envs().
+ *   Environments (observation entries, action head, prob row width, state layout):
+ *     MRL_ENV_CARTPOLE                 CartPole-v0               4, Categorical 2, 2, (x, x_dot, theta, theta_dot)
+ *     MRL_ENV_PENDULUM                 Pendulum-v0               3, DiagGauss d = 1, 2, (theta, theta_dot)
+ *     MRL_ENV_ACROBOT                  Acrobot-v1                6, Categorical 3, 3, (theta1, theta2, dtheta1, dtheta2)
+ *     MRL_ENV_MOUNTAIN_CAR             MountainCar-v0            2, Categorical 3, 3, (position, velocity)
+ *     MRL_ENV_MOUNTAIN_CAR_CONTINUOUS  MountainCarContinuous-v0  2, DiagGauss d = 1, 2, (position, velocity)
+ *     The prob row holds K probabilities for a Categorical head with K outputs and [mean, std] (2d) for DiagGauss.
+ *   mrl_rollout_env_info: the shapes of `env` above (host code, no device needed): observation entries, state
+ *     entries, head (MRL_CATEGORICAL / MRL_GAUSS) and the policy's outputs.  Fails for an unknown env.
+ *   mrl_rollout_create: one of the environments above; 1 <= n_envs <= mrl_rollout_max_envs().  Allocates the staging
+ *     rows of a round, n_envs x timestep_limit rows of (observation, state, prob, action, reward), and a compacted
+ *     output buffer of as many rows.  At 4096 environments that is about 0.2 GB each for Acrobot (500 steps, 104 B a
+ *     row) and for MountainCarContinuous (999 steps, 52 B a row), computed from the row sizes.
  *   mrl_rollout_run: `policy` must live on the handle's device, take the environment's observation and end in its
- *     action head (CartPole: Categorical with 2 outputs; Pendulum: DiagGauss with d = 1).  A NULL filter cfg or
+ *     action head (the table above).  A NULL filter cfg or
  *     enabled == 0 is the identity.  ob_state = {n, M[ob_dim], S[ob_dim]} and rew_state = {n, M, S} (host) are read and
  *     replaced by the states after the round; *_pushed (may be NULL) receive the statistics of this round's samples
  *     alone.  want_states != 0 also records the raw environment state of every step.  Synchronises `stream`;
  *     *n_timesteps = timesteps collected.
  *   mrl_rollout_read: the last round, path-major (episode i = environment i): lengths int32[n_envs],
  *     terminated uint8[n_envs], observation f64 [n x ob_dim] (filtered), action int32 [n] (Categorical) or
- *     f32 [n x d] (DiagGauss), prob f32 [n x 2] (probabilities or [mean, std]), raw reward f64 [n],
- *     states f64 [n x state_dim] (CartPole 4, Pendulum 2: (theta, theta_dot)).  Any pointer may be NULL.  After a
+ *     f32 [n x d] (DiagGauss), prob f32 [n x prob width] (probabilities or [mean, std]), raw reward f64 [n],
+ *     states f64 [n x state_dim] (the state layouts above).  Any pointer may be NULL.  After a
  *     round without rows (mrl_rollout_run_population, want_rows = 0) only lengths and terminated may be non-NULL.
  *   mrl_rollout_run_population: one round in which environment m acts deterministically with its own theta_m (the
  *     cross-entropy method's population, cem.py:43-44,88-91).  n_members <= the handle's n_envs environments run;
  *     thetas [n_members x ld_theta] float32 where `theta_loc` says (MRL_HOST: one copy into a device buffer the handle
  *     keeps; MRL_DEVICE: read in place), each row the Dense kernels and biases of n_layers layers of widths dims[0..]
  *     (1..256) in the reference's flat order, no logstd block, ld_theta >= that count.  The action is taken from the
- *     raw last-layer output: its argmax, first maximum (CartPole), or the output itself (Pendulum).
+ *     raw last-layer output: for a Categorical head its argmax (first maximum; a NaN output wins as in numpy), for
+ *     DiagGauss the output itself, which the dynamics clip (MountainCarContinuous penalises the unclipped value).
  *     returns[n_members] (host, float64) = the sum of each episode's raw rewards in step order.  Filters as
  *     mrl_rollout_run.  want_rows != 0 records the rows for mrl_rollout_read, the prob row then holding the raw
- *     outputs (CartPole: the two logits; Pendulum: [mean, 1]); want_states (needs want_rows) the raw states.
+ *     outputs (Categorical: the K logits; DiagGauss: [mean, 1]); want_states (needs want_rows) the raw states.
  *     Synchronises `stream`; *n_timesteps = timesteps collected. */
 #define MRL_ENV_CARTPOLE 0
 #define MRL_ENV_PENDULUM 1
+#define MRL_ENV_ACROBOT 2
+#define MRL_ENV_MOUNTAIN_CAR 3
+#define MRL_ENV_MOUNTAIN_CAR_CONTINUOUS 4
 typedef struct mrl_rollout mrl_rollout;
 typedef struct {
   int enabled, demean, destd;
   double clip;   /* 0: no clipping */
 } mrl_zfilter_cfg;
 int mrl_rollout_max_envs(void);
+int mrl_rollout_env_info(int env, int* ob_dim, int* state_dim, int* head, int* n_out);
 int mrl_rollout_create(mrl_rollout** out, int device, int env, int n_envs, int timestep_limit);
 int mrl_rollout_destroy(mrl_rollout* r);
 int mrl_rollout_run(mrl_rollout* r, mrl_net* policy, unsigned long long seed, int stochastic,

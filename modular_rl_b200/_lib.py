@@ -15,7 +15,9 @@ HOST, DEVICE = 0, 1
 F32, F64, I32, I64 = 0, 1, 2, 3
 GAUSS, CATEGORICAL, VALUE = 0, 1, 2
 ACTIVATIONS = {"tanh": 0, "relu": 1, "sigmoid": 2}
-DEVICE_ENVS = {"cartpole": 0, "pendulum": 1}      # MRL_ENV_CARTPOLE, MRL_ENV_PENDULUM
+# envs.py device_kind -> MRL_ENV_CARTPOLE, MRL_ENV_PENDULUM, MRL_ENV_ACROBOT, MRL_ENV_MOUNTAIN_CAR,
+# MRL_ENV_MOUNTAIN_CAR_CONTINUOUS
+DEVICE_ENVS = {"cartpole": 0, "pendulum": 1, "acrobot": 2, "mountaincar": 3, "mountaincar_continuous": 4}
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("MRL_LIB") or os.path.join(_HERE, "libmrl_b200.so")   # MRL_LIB: kernel experiments only
@@ -90,6 +92,7 @@ _SIGS = {
     "mrl_comm_p2p_connect": (_I, [_P, _P]),
     "mrl_comm_p2p_enable": (_I, [_P, _I]),
     "mrl_rollout_max_envs": (_I, []),
+    "mrl_rollout_env_info": (_I, [_I, C.POINTER(_I), C.POINTER(_I), C.POINTER(_I), C.POINTER(_I)]),
     "mrl_rollout_create": (_I, [C.POINTER(_P), _I, _I, _I, _I]),
     "mrl_rollout_destroy": (_I, [_P]),
     "mrl_rollout_run": (_I, [_P, _P, C.c_ulonglong, _I, C.POINTER(ZFilterCfg), _P, _P, C.POINTER(ZFilterCfg), _P, _P,

@@ -152,7 +152,7 @@ def run_cem_algorithm(env, agent, usercfg=None, callback=None):
     parallel=1 scores the whole population in lockstep with one population-batched device forward per environment step
     (`evaluate_population`).  parallel=0 scores one candidate after another as cem.py:43 does.
 
-    DEVICE_ENVS on (CartPole / Pendulum only): each generation is scored by one device rollout round
+    DEVICE_ENVS on (the built-in environments of envs.py only): each generation is scored by one device rollout round
     (`evaluate_population_device`), its Philox seed a counter started from cfg["seed"], one value per generation.
     The host paths draw the environments' resets from numpy's global generator; the device path does not touch it,
     so the search's own randn calls are its only numpy draws.  Start states, scores and therefore later generations

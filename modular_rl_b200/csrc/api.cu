@@ -1247,7 +1247,7 @@ extern "C" int mrl_net_get_trpo_vectors(mrl_net* n, double* stepdir, double* ful
 
 // ======================================================================== device-resident rollouts (rollout.cu)
 struct mrl_rollout {
-  int device = 0, env = 0, N = 0, T = 0, d0 = 0, sd = 0, dout = 0, head = 0;
+  int device = 0, env = 0, N = 0, T = 0, d0 = 0, sd = 0, dout = 0, pd = 0, head = 0;   // pd: prob row width
   DevBuf s_obs, s_state, s_prob, s_act, s_rew, lengths, term, headbuf, body, filt, returns, thetas;
   double* h_head = nullptr;      // pinned: header, then lengths int32[N], terminated int32[N]
   double* h_filt = nullptr;      // pinned: incoming filter states
@@ -1258,8 +1258,22 @@ struct mrl_rollout {
   int with_states = 0, with_rows = 1;
 };
 static int ro_head_doubles(int d0) { return 9 + 4 * d0; }
+static int ro_act_width(const mrl_rollout* r) { return r->head == MRL_HEAD_CAT ? 1 : r->dout; }
+static const char* ro_env_names = "MRL_ENV_CARTPOLE, MRL_ENV_PENDULUM, MRL_ENV_ACROBOT, MRL_ENV_MOUNTAIN_CAR or "
+                                  "MRL_ENV_MOUNTAIN_CAR_CONTINUOUS";
 
 extern "C" int mrl_rollout_max_envs(void) { return RO_MAX_ENVS; }
+
+extern "C" int mrl_rollout_env_info(int env, int* ob_dim, int* state_dim, int* head, int* n_out) {
+  int d0, sd, dout, pd;
+  const int h = rollout_env_dims(env, &d0, &sd, &dout, &pd);
+  if (h < 0) return fail("mrl_rollout_env_info: unknown env %d (%s)", env, ro_env_names);
+  if (ob_dim) *ob_dim = d0;
+  if (state_dim) *state_dim = sd;
+  if (head) *head = h;
+  if (n_out) *n_out = dout;
+  return 0;
+}
 
 extern "C" int mrl_rollout_destroy(mrl_rollout* r) {
   if (!r) return 0;
@@ -1276,22 +1290,22 @@ extern "C" int mrl_rollout_destroy(mrl_rollout* r) {
 
 extern "C" int mrl_rollout_create(mrl_rollout** out, int device, int env, int n_envs, int timestep_limit) {
   if (!out) return fail("mrl_rollout_create: null output");
-  int d0, sd, dout;
-  const int head = rollout_env_dims(env, &d0, &sd, &dout);
-  if (head < 0) return fail("mrl_rollout_create: unknown env %d (MRL_ENV_CARTPOLE or MRL_ENV_PENDULUM)", env);
+  int d0, sd, dout, pd;
+  const int head = rollout_env_dims(env, &d0, &sd, &dout, &pd);
+  if (head < 0) return fail("mrl_rollout_create: unknown env %d (%s)", env, ro_env_names);
   if (n_envs < 1 || n_envs > RO_MAX_ENVS)
     return fail("mrl_rollout_create: n_envs = %d; the rollout kernel runs 1..%d environments per round", n_envs, RO_MAX_ENVS);
   if (timestep_limit < 1) return fail("mrl_rollout_create: timestep_limit must be >= 1");
   CK(cudaSetDevice(device));
   mrl_rollout* r = new mrl_rollout();
   r->device = device; r->env = env; r->N = n_envs; r->T = timestep_limit; r->n_round = n_envs;
-  r->d0 = d0; r->sd = sd; r->dout = dout; r->head = head;
+  r->d0 = d0; r->sd = sd; r->dout = dout; r->pd = pd; r->head = head;
   const size_t rows = (size_t)n_envs * timestep_limit;
-  const RolloutLayout lay = rollout_layout((long long)rows, d0, sd, 2, head == MRL_HEAD_CAT ? 1 : dout, 1);
+  const RolloutLayout lay = rollout_layout((long long)rows, d0, sd, pd, ro_act_width(r), 1);
   cudaError_t e = cudaSuccess;
   auto R = [&](DevBuf& b, size_t bytes) { if (e == cudaSuccess) e = b.reserve(bytes); };
-  R(r->s_obs, rows * d0 * 8); R(r->s_state, rows * sd * 8); R(r->s_prob, rows * 2 * 4);
-  R(r->s_act, rows * dout * 4); R(r->s_rew, rows * 8); R(r->lengths, (size_t)n_envs * 4); R(r->term, (size_t)n_envs * 4);
+  R(r->s_obs, rows * d0 * 8); R(r->s_state, rows * sd * 8); R(r->s_prob, rows * pd * 4);
+  R(r->s_act, rows * ro_act_width(r) * 4); R(r->s_rew, rows * 8); R(r->lengths, (size_t)n_envs * 4); R(r->term, (size_t)n_envs * 4);
   R(r->headbuf, (size_t)ro_head_doubles(d0) * 8); R(r->body, lay.end); R(r->filt, (size_t)(4 + 2 * d0) * 8);
   R(r->returns, (size_t)n_envs * 8);
   const size_t hb = (size_t)ro_head_doubles(d0) * 8 + (size_t)n_envs * 8;
@@ -1362,8 +1376,7 @@ static int ro_round(mrl_rollout* r, RolloutArgs& a, int act, bool pop, const cha
   r->with_rows = want_rows != 0;
   r->with_states = want_rows && want_states;
   if (r->with_rows) {
-    const RolloutLayout lay = rollout_layout(r->total, d0, r->sd, 2, r->head == MRL_HEAD_CAT ? 1 : r->dout,
-                                             r->with_states);
+    const RolloutLayout lay = rollout_layout(r->total, d0, r->sd, r->pd, ro_act_width(r), r->with_states);
     if (lay.end > r->h_body_cap) {
       if (r->h_body) cudaFreeHost(r->h_body);
       r->h_body = nullptr;
@@ -1386,7 +1399,15 @@ static int ro_round(mrl_rollout* r, RolloutArgs& a, int act, bool pop, const cha
   return 0;
 }
 
-static const char* ro_env_name(const mrl_rollout* r) { return r->env == MRL_ENV_CARTPOLE ? "CartPole" : "Pendulum"; }
+static const char* ro_env_name(const mrl_rollout* r) {
+  switch (r->env) {
+    case MRL_ENV_CARTPOLE: return "CartPole";
+    case MRL_ENV_PENDULUM: return "Pendulum";
+    case MRL_ENV_ACROBOT: return "Acrobot";
+    case MRL_ENV_MOUNTAIN_CAR: return "MountainCar";
+    default: return "MountainCarContinuous";
+  }
+}
 
 extern "C" int mrl_rollout_run(mrl_rollout* r, mrl_net* policy, unsigned long long seed, int stochastic,
                                const mrl_zfilter_cfg* ob_cfg, double* ob_state, double* ob_pushed,
@@ -1487,11 +1508,11 @@ extern "C" int mrl_rollout_read(mrl_rollout* r, int* lengths, unsigned char* ter
   if (lengths) memcpy(lengths, h_len, (size_t)N * 4);
   if (terminated) for (int i = 0; i < N; ++i) terminated[i] = (unsigned char)h_len[N + i];
   const long long n = r->total;
-  const RolloutLayout lay = rollout_layout(n, r->d0, r->sd, 2, r->head == MRL_HEAD_CAT ? 1 : r->dout, r->with_states);
+  const RolloutLayout lay = rollout_layout(n, r->d0, r->sd, r->pd, ro_act_width(r), r->with_states);
   if (obs) memcpy(obs, r->h_body + lay.obs, (size_t)n * r->d0 * 8);
   if (reward) memcpy(reward, r->h_body + lay.rew, (size_t)n * 8);
   if (states) memcpy(states, r->h_body + lay.state, (size_t)n * r->sd * 8);
-  if (prob) memcpy(prob, r->h_body + lay.prob, (size_t)n * 2 * 4);
-  if (act) memcpy(act, r->h_body + lay.act, (size_t)n * (r->head == MRL_HEAD_CAT ? 1 : r->dout) * 4);
+  if (prob) memcpy(prob, r->h_body + lay.prob, (size_t)n * r->pd * 4);
+  if (act) memcpy(act, r->h_body + lay.act, (size_t)n * ro_act_width(r) * 4);
   return 0;
 }

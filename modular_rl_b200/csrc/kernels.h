@@ -181,7 +181,8 @@ __host__ __device__ inline RolloutLayout rollout_layout(long long n, int d0, int
   o.end = p;
   return o;
 }
-int rollout_env_dims(int env, int* d0, int* sd, int* dout);   // -> head, -1 for an unknown env
+// observation entries, state entries, policy outputs, prob row width -> head, -1 for an unknown env
+int rollout_env_dims(int env, int* d0, int* sd, int* dout, int* pd);
 void rollout_shape(int N, int* n_ctas, int* per_cta, int* threads);
 size_t rollout_smem_bytes(const RolloutArgs& a, int d0, int dout, bool pop);
 cudaError_t launch_rollout(const RolloutArgs& a, int env, int act, bool pop, int n_ctas, int threads, size_t smem,

@@ -1,4 +1,5 @@
-// Device-resident rollouts of the two built-in environments (envs.py: CartPole-v0, Pendulum-v0).
+// Device-resident rollouts of the built-in environments (envs.py: CartPole-v0, Pendulum-v0, Acrobot-v1,
+// MountainCar-v0, MountainCarContinuous-v0).
 //
 // One launch runs one ROUND: N environments from reset until every episode has ended or reached the timestep limit,
 // in the lockstep order of core.rollouts_vectorized (core.py:182-221 run per environment).  Per step t, over the
@@ -34,7 +35,7 @@
 #include <cooperative_groups.h>
 namespace cgr = cooperative_groups;
 
-#define RO_KMAX 5   // observation features + the reward, scanned together
+#define RO_KMAX 7   // observation features + the reward, scanned together (Acrobot: 6 + 1)
 
 // ---------------------------------------------------------------------------------------------------- Philox4x32-10
 __device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint32_t k0, uint32_t k1) {
@@ -178,6 +179,119 @@ template <> struct EnvT<MRL_ENV_PENDULUM> {
   }
 };
 
+// The dynamics below are written with __dmul_rn for every product so that no product is contracted with a sum into an
+// FMA: each operation rounds as the float64 arithmetic of envs.py does, and only cos / sin may differ in the last bits.
+__device__ __forceinline__ double mul(double a, double b) { return __dmul_rn(a, b); }
+
+template <> struct EnvT<MRL_ENV_ACROBOT> {
+  static constexpr int D0 = 6, SD = 4, DOUT = 3, PD = 3, HEAD = MRL_HEAD_CAT;   // prob row: 3 probabilities
+  __device__ static void reset(double* s, int e, uint32_t k0, uint32_t k1) {   // uniform(-0.1, 0.1, size=4)
+    const uint4 a = philox4x32_10(make_uint4((uint32_t)e, 0u, RO_PURPOSE_RESET, 0u), k0, k1);
+    const uint4 b = philox4x32_10(make_uint4((uint32_t)e, 0u, RO_PURPOSE_RESET, 1u), k0, k1);
+    const double u[4] = {u53(a.x, a.y), u53(a.z, a.w), u53(b.x, b.y), u53(b.z, b.w)};
+#pragma unroll
+    for (int i = 0; i < 4; ++i) s[i] = -0.1 + mul(0.1 - -0.1, u[i]);
+  }
+  __device__ static void obs(const double* s, double* x) {
+    x[0] = cos(s[0]);
+    x[1] = sin(s[0]);
+    x[2] = cos(s[1]);
+    x[3] = sin(s[1]);
+    x[4] = s[2];
+    x[5] = s[3];
+  }
+  // envs.py AcrobotEnv._dsdt: y = (theta1, theta2, dtheta1, dtheta2), torque a -> k = d/dt of y
+  __device__ static void dsdt(const double* y, double a, double* k) {
+    const double m1 = 1.0, m2 = 1.0, l1 = 1.0, lc1 = 0.5, lc2 = 0.5, I1 = 1.0, I2 = 1.0, g = 9.8;
+    const double th1 = y[0], th2 = y[1], dth1 = y[2], dth2 = y[3];
+    double s2, c2;
+    sincos(th2, &s2, &c2);                         // one argument reduction: keeps the kernel at 128 registers, no spills
+    const double d1 = mul(m1, mul(lc1, lc1)) + mul(m2, mul(l1, l1) + mul(lc2, lc2) + mul(mul(mul(2.0, l1), lc2), c2)) + I1 + I2;
+    const double d2 = mul(m2, mul(lc2, lc2) + mul(mul(l1, lc2), c2)) + I2;
+    const double phi2 = mul(mul(mul(m2, lc2), g), cos(th1 + th2 - M_PI / 2.0));
+    const double phi1 = mul(mul(mul(mul(-m2, l1), lc2), mul(dth2, dth2)), s2)
+                        - mul(mul(mul(mul(mul(mul(2.0, m2), l1), lc2), dth2), dth1), s2)
+                        + mul(mul(mul(m1, lc1) + mul(m2, l1), g), cos(th1 - M_PI / 2.0)) + phi2;
+    const double dd2 = (a + mul(d2 / d1, phi1) - mul(mul(mul(mul(m2, l1), lc2), mul(dth1, dth1)), s2) - phi2)
+                       / (mul(m2, mul(lc2, lc2)) + I2 - mul(d2, d2) / d1);
+    k[0] = dth1;
+    k[1] = dth2;
+    k[2] = -(mul(d2, dd2) + phi1) / d1;
+    k[3] = dd2;
+  }
+  // envs.py AcrobotEnv.step: one RK4 step of the torque-augmented state (the torque's derivative is 0, so it stays a
+  // constant), the sum (k1 + 2 k2) + 2 k3 + k4 accumulated stage by stage in that order, then wrap, bound, terminal
+  __device__ static bool step(double* s, int action, float, double* reward) {
+    const double dt = 0.2, dt2 = dt / 2.0, max_vel_1 = 4 * M_PI, max_vel_2 = 9 * M_PI;
+    const double a = action == 0 ? -1.0 : (action == 1 ? 0.0 : 1.0);
+    double k[4], y[4], acc[4];
+    dsdt(s, a, k);
+#pragma unroll
+    for (int i = 0; i < 4; ++i) { acc[i] = k[i]; y[i] = s[i] + mul(dt2, k[i]); }
+    dsdt(y, a, k);
+#pragma unroll
+    for (int i = 0; i < 4; ++i) { acc[i] = acc[i] + mul(2.0, k[i]); y[i] = s[i] + mul(dt2, k[i]); }
+    dsdt(y, a, k);
+#pragma unroll
+    for (int i = 0; i < 4; ++i) { acc[i] = acc[i] + mul(2.0, k[i]); y[i] = s[i] + mul(dt, k[i]); }
+    dsdt(y, a, k);
+#pragma unroll
+    for (int i = 0; i < 4; ++i) y[i] = s[i] + mul(dt / 6.0, acc[i] + k[i]);
+#pragma unroll
+    for (int i = 0; i < 2; ++i) {                  // wrap into [-pi, pi] with envs.py's loops (not fmod)
+      double x = y[i];
+      const double diff = M_PI - -M_PI;
+      while (x > M_PI) x = x - diff;
+      while (x < -M_PI) x = x + diff;
+      s[i] = x;
+    }
+    s[2] = fmin(fmax(y[2], -max_vel_1), max_vel_1);
+    s[3] = fmin(fmax(y[3], -max_vel_2), max_vel_2);
+    const bool terminal = -cos(s[0]) - cos(s[1] + s[0]) > 1.0;
+    *reward = terminal ? 0.0 : -1.0;
+    return terminal;
+  }
+};
+
+// envs.py MountainCarEnv._move: velocity += dv and the clips, the left wall, the goal test; state (position, velocity)
+__device__ __forceinline__ bool mountain_car_move(double* s, double dv, double goal) {
+  const double min_position = -1.2, max_position = 0.6, max_speed = 0.07;
+  const double velocity = fmin(fmax(s[1] + dv, -max_speed), max_speed);
+  const double position = fmin(fmax(s[0] + velocity, min_position), max_position);
+  s[0] = position;
+  s[1] = position == min_position && velocity < 0.0 ? 0.0 : velocity;
+  return position >= goal && s[1] >= 0.0;
+}
+__device__ __forceinline__ void mountain_car_reset(double* s, int e, uint32_t k0, uint32_t k1) {   // [uniform(-0.6, -0.4), 0]
+  const uint4 a = philox4x32_10(make_uint4((uint32_t)e, 0u, RO_PURPOSE_RESET, 0u), k0, k1);
+  s[0] = -0.6 + mul(-0.4 - -0.6, u53(a.x, a.y));
+  s[1] = 0.0;
+}
+template <> struct EnvT<MRL_ENV_MOUNTAIN_CAR> {
+  static constexpr int D0 = 2, SD = 2, DOUT = 3, PD = 3, HEAD = MRL_HEAD_CAT;   // prob row: 3 probabilities
+  __device__ static void reset(double* s, int e, uint32_t k0, uint32_t k1) { mountain_car_reset(s, e, k0, k1); }
+  __device__ static void obs(const double* s, double* x) { x[0] = s[0]; x[1] = s[1]; }
+  // envs.py MountainCarEnv.step; reward -1 on every step, the terminating one included
+  __device__ static bool step(double* s, int action, float, double* reward) {
+    const double dv = mul((double)(action - 1), 0.001) + mul(cos(mul(3.0, s[0])), -0.0025);
+    *reward = -1.0;
+    return mountain_car_move(s, dv, 0.5);
+  }
+};
+template <> struct EnvT<MRL_ENV_MOUNTAIN_CAR_CONTINUOUS> {
+  static constexpr int D0 = 2, SD = 2, DOUT = 1, PD = 2, HEAD = MRL_HEAD_GAUSS;  // prob row: mean, std
+  __device__ static void reset(double* s, int e, uint32_t k0, uint32_t k1) { mountain_car_reset(s, e, k0, k1); }
+  __device__ static void obs(const double* s, double* x) { x[0] = s[0]; x[1] = s[1]; }
+  // envs.py MountainCarContinuousEnv.step: the force is the clipped action, the penalty takes the unclipped one
+  __device__ static bool step(double* s, int, float action, double* reward) {
+    const double a = (double)action;
+    const double force = fmin(fmax(a, -1.0), 1.0);
+    const bool done = mountain_car_move(s, mul(force, 0.0015) - mul(0.0025, cos(mul(3.0, s[0]))), 0.45);
+    *reward = (done ? 100.0 : 0.0) - mul(0.1, mul(a, a));
+    return done;
+  }
+};
+
 // ---------------------------------------------------------------------------------------------------- policy forward
 // rows [0, nrows) of xin [nrows][d0] -> out [nrows][dout]: raw head output (softmax logits / Gauss mean).
 // POP: row r uses the theta of environment rowe[r], W + rowe[r] * a.ld_theta.
@@ -222,13 +336,15 @@ __device__ void mlp_rows(const RolloutArgs& a, const float* W, const float* xin,
 
 // ---------------------------------------------------------------------------------------------------- the round
 // POP (population round, the cross-entropy method): environment e acts deterministically with its own Dense theta
-// (a.theta + e * a.ld_theta, no logstd block, read through L2), on the argmax of the raw outputs (CartPole) or the
-// raw output (Pendulum); a.returns[e] = the float64 sum of its raw rewards in step order; without a.want_rows no
+// (a.theta + e * a.ld_theta, no logstd block, read through L2), on the argmax of the raw outputs (Categorical heads)
+// or the raw output (DiagGauss heads); a.returns[e] = the float64 sum of its raw rewards in step order; without a.want_rows no
 // staging rows are written and nothing is compacted.
 template <int ENV, int ACT, bool POP>
 __global__ void __launch_bounds__(RO_MAX_THREADS, 1) rollout_kernel(const RolloutArgs a) {
   using E = EnvT<ENV>;
   constexpr int D0 = E::D0, SD = E::SD, DOUT = E::DOUT, PD = E::PD, K = D0 + 1;   // K - 1: the reward
+  static_assert(K <= RO_KMAX, "RO_KMAX must cover the observation features and the reward");
+  static_assert(PD == (E::HEAD == MRL_HEAD_CAT ? DOUT : 2 * DOUT), "prob row: K probabilities / mean and std");
   cgr::cluster_group cluster = cgr::this_cluster();
   const int rank = (int)cluster.block_rank(), nc = (int)cluster.num_blocks();
 
@@ -276,11 +392,13 @@ __global__ void __launch_bounds__(RO_MAX_THREADS, 1) rollout_kernel(const Rollou
 
   for (int t = 0;; ++t) {
     const bool now = live && t < a.T;
-    double x[D0];
-    E::obs(s, x);
     Wf w[K];
+    {
+      double x[D0];
+      E::obs(s, x);
 #pragma unroll
-    for (int k = 0; k < D0; ++k) w[k] = now ? Wf{1.0, x[k], 0.0} : Wf{0.0, 0.0, 0.0};
+      for (int k = 0; k < D0; ++k) w[k] = now ? Wf{1.0, x[k], 0.0} : Wf{0.0, 0.0, 0.0};
+    }
     w[D0] = rlive ? Wf{1.0, rew, 0.0} : Wf{0.0, 0.0, 0.0};   // the rewards of step t - 1
     block_scan<K>(w, wtot, ctatot);
     if (threadIdx.x < K) slot[t & 1][threadIdx.x] = ctatot[threadIdx.x];
@@ -308,6 +426,8 @@ __global__ void __launch_bounds__(RO_MAX_THREADS, 1) rollout_kernel(const Rollou
     const int nlive = (int)ctatot[0].n;
     const size_t st_row = (size_t)t * a.N + e;
     if (now) {
+      double x[D0];
+      E::obs(s, x);                        // recomputed, not kept live across the scan (Acrobot's 6 entries spill)
 #pragma unroll
       for (int k = 0; k < D0; ++k) {
         double y = x[k];
@@ -467,10 +587,21 @@ __global__ void __launch_bounds__(RO_MAX_THREADS, 1) rollout_kernel(const Rollou
 }
 
 // ---------------------------------------------------------------------------------------------------- launcher
-int rollout_env_dims(int env, int* d0, int* sd, int* dout) {
-  if (env == MRL_ENV_CARTPOLE) { *d0 = EnvT<MRL_ENV_CARTPOLE>::D0; *sd = EnvT<MRL_ENV_CARTPOLE>::SD; *dout = EnvT<MRL_ENV_CARTPOLE>::DOUT; return MRL_HEAD_CAT; }
-  if (env == MRL_ENV_PENDULUM) { *d0 = EnvT<MRL_ENV_PENDULUM>::D0; *sd = EnvT<MRL_ENV_PENDULUM>::SD; *dout = EnvT<MRL_ENV_PENDULUM>::DOUT; return MRL_HEAD_GAUSS; }
-  return -1;
+template <int ENV>
+static int env_dims(int* d0, int* sd, int* dout, int* pd) {
+  using E = EnvT<ENV>;
+  *d0 = E::D0; *sd = E::SD; *dout = E::DOUT; *pd = E::PD;
+  return E::HEAD;
+}
+int rollout_env_dims(int env, int* d0, int* sd, int* dout, int* pd) {
+  switch (env) {
+    case MRL_ENV_CARTPOLE: return env_dims<MRL_ENV_CARTPOLE>(d0, sd, dout, pd);
+    case MRL_ENV_PENDULUM: return env_dims<MRL_ENV_PENDULUM>(d0, sd, dout, pd);
+    case MRL_ENV_ACROBOT: return env_dims<MRL_ENV_ACROBOT>(d0, sd, dout, pd);
+    case MRL_ENV_MOUNTAIN_CAR: return env_dims<MRL_ENV_MOUNTAIN_CAR>(d0, sd, dout, pd);
+    case MRL_ENV_MOUNTAIN_CAR_CONTINUOUS: return env_dims<MRL_ENV_MOUNTAIN_CAR_CONTINUOUS>(d0, sd, dout, pd);
+    default: return -1;
+  }
 }
 
 void rollout_shape(int N, int* n_ctas, int* per_cta, int* threads) {
@@ -515,8 +646,13 @@ static cudaError_t launch_pop(const RolloutArgs& a, int env, int act, int n_ctas
     case MRL_ACT_RELU: return launch_t<ENV, MRL_ACT_RELU, POP>(a, n_ctas, threads, smem, st); \
     default: return launch_t<ENV, MRL_ACT_SIGMOID, POP>(a, n_ctas, threads, smem, st);        \
   }
-  if (env == MRL_ENV_CARTPOLE) { RO_ACTS(MRL_ENV_CARTPOLE) }
-  RO_ACTS(MRL_ENV_PENDULUM)
+  switch (env) {   // mrl_rollout_create accepts only these
+    case MRL_ENV_CARTPOLE: RO_ACTS(MRL_ENV_CARTPOLE)
+    case MRL_ENV_ACROBOT: RO_ACTS(MRL_ENV_ACROBOT)
+    case MRL_ENV_MOUNTAIN_CAR: RO_ACTS(MRL_ENV_MOUNTAIN_CAR)
+    case MRL_ENV_MOUNTAIN_CAR_CONTINUOUS: RO_ACTS(MRL_ENV_MOUNTAIN_CAR_CONTINUOUS)
+    default: RO_ACTS(MRL_ENV_PENDULUM)
+  }
 #undef RO_ACTS
 }
 

@@ -327,10 +327,22 @@ class DeviceNet:
         return sd, fs, dict(shs=sc[0], lm=sc[1], expected_improve_rate=sc[2], cg_rdotr=sc[3])
 
 
+def rollout_env_info(kind: str) -> dict:
+    """mrl_rollout_env_info for an envs.py device kind: ob_dim, state_dim, categorical, n_out (the policy's outputs:
+    K classes or the DiagGauss dimension d), act_dim (1 for Categorical, else d) and prob_dim (K, or 2d for
+    [mean, std])."""
+    ob, st, head, n_out = C.c_int(), C.c_int(), C.c_int(), C.c_int()
+    L.check(L.lib().mrl_rollout_env_info(L.DEVICE_ENVS[kind], C.byref(ob), C.byref(st), C.byref(head), C.byref(n_out)))
+    cat = head.value == L.CATEGORICAL
+    return dict(ob_dim=ob.value, state_dim=st.value, categorical=cat, n_out=n_out.value,
+                act_dim=1 if cat else n_out.value, prob_dim=n_out.value if cat else 2 * n_out.value)
+
+
 class DeviceRollouts:
     """mrl_rollout_*: rounds of n_envs lockstep rollouts of a built-in environment, each round one kernel launch on
     the device (the policy forward, the action draws, the dynamics and both ZFilters included).  `env`: a built-in
-    environment's id ("CartPole-v0", "Pendulum-v0") or instance."""
+    environment's id ("CartPole-v0", "Pendulum-v0", "Acrobot-v1", "MountainCar-v0", "MountainCarContinuous-v0") or
+    instance."""
 
     def __init__(self, env, n_envs: int, timestep_limit: int, device: Optional[int] = None):
         from .envs import device_kind
@@ -340,9 +352,9 @@ class DeviceRollouts:
         self._h = C.c_void_p()
         L.check(L.lib().mrl_rollout_create(C.byref(self._h), device, L.DEVICE_ENVS[kind], int(n_envs), int(timestep_limit)))
         self.kind, self.n_envs, self.timestep_limit, self.device = kind, int(n_envs), int(timestep_limit), device
-        self.ob_dim, self.state_dim = (4, 4) if kind == "cartpole" else (3, 2)
-        self.categorical = kind == "cartpole"
-        self.act_dim = 1
+        info = rollout_env_info(kind)
+        self.ob_dim, self.state_dim, self.categorical = info["ob_dim"], info["state_dim"], info["categorical"]
+        self.act_dim, self.prob_dim = info["act_dim"], info["prob_dim"]
 
     @staticmethod
     def max_envs() -> int:
@@ -377,9 +389,11 @@ class DeviceRollouts:
     def run(self, net: DeviceNet, seed: int, stochastic: bool = True, obfilter=None, rewfilter=None,
             want_states: bool = False, stream=None) -> dict:
         """One round.  obfilter / rewfilter: None (identity) or ((n, M, S), demean, destd, clip).  Returns the
-        compacted path-major arrays (lengths, terminated, observation, action, prob, reward[, states]) and the filter
-        states after the round plus those of this round's samples alone (ob_state, ob_pushed, rew_state, rew_pushed;
-        None for an identity filter)."""
+        compacted path-major arrays and the filter states after the round plus those of this round's samples alone
+        (ob_state, ob_pushed, rew_state, rew_pushed; None for an identity filter).  The arrays: lengths int32 and
+        terminated uint8 per environment; per timestep observation float64 [T, ob_dim] (filtered), action (int32 [T]
+        for a Categorical head, float32 [T, d] for DiagGauss), prob float32 [T, prob_dim] (the K probabilities, or
+        [mean, std]), reward float64 [T] (raw) and with want_states the raw states float64 [T, state_dim]."""
         d = self.ob_dim
         ocfg, ost, opu = self._filter_in(obfilter, d)
         rcfg, rst, rpu = self._filter_in(rewfilter, 1)
@@ -397,7 +411,8 @@ class DeviceRollouts:
         place); each row holds the Dense kernels and biases of the net `dims` in the reference's flat order (no logstd
         block), ld >= their count, M <= n_envs.  Filters as `run`.  Returns `returns` (float64 [M], the sum of each
         episode's raw rewards), lengths, terminated, the four filter states, and with want_rows the row arrays of `run`
-        (prob: CartPole's two raw outputs, Pendulum's [mean, 1])."""
+        (prob: the K raw outputs of a Categorical head, [mean, 1] for DiagGauss).  Members act on the argmax of their
+        raw outputs (first maximum) or on the raw output itself, which the environment clips."""
         dims = [int(x) for x in dims]
         if _is_torch_cuda(thetas):
             import torch
@@ -429,7 +444,7 @@ class DeviceRollouts:
         if want_rows:
             out.update(observation=np.empty((T, d), np.float64),
                        action=np.empty(T, np.int32) if self.categorical else np.empty((T, self.act_dim), np.float32),
-                       prob=np.empty((T, 2 * self.act_dim if not self.categorical else 2), np.float32),
+                       prob=np.empty((T, self.prob_dim), np.float32),
                        reward=np.empty(T, np.float64))
         states = np.empty((T, self.state_dim), np.float64) if want_states else None
         L.check(L.lib().mrl_rollout_read(self._h, L.ptr(out["lengths"]), L.ptr(out["terminated"]),

@@ -1,7 +1,9 @@
-"""Two classic-control environments with the old gym API (reset() -> ob, step(a) -> ob, rew, done,
+"""The classic-control environments with the old gym API (reset() -> ob, step(a) -> ob, rew, done,
 info) so that BASELINE config 1 (CartPole-v0 TrpoAgent via run_pg.py) and the reference's coverage
-smoke (Pendulum, coverage.sh:7) run without gym, which is not installed here.  Dynamics follow the
-published classic-control equations (Barto-Sutton-Anderson cart-pole; torque-limited pendulum)."""
+smoke (run_cem.py on Acrobot, run_pg.py on Pendulum, coverage.sh:6-7) run without gym, which is not installed here.
+Dynamics follow the published classic-control equations (Barto-Sutton-Anderson cart-pole; torque-limited pendulum;
+Sutton-Barto acrobot; Moore's mountain car, discrete and continuous).  Every one of them also runs on the device
+(rollout.cu), which replays the float64 arithmetic of these classes."""
 import math
 
 import numpy as np
@@ -94,8 +96,170 @@ class PendulumEnv(object):
         pass
 
 
+class AcrobotEnv(object):
+    """Acrobot-v1, the "book" dynamics of Sutton & Barto: two links hanging from a fixed pivot, torque on the joint
+    between them.  Limit 500 steps.  Constants dt = 0.2, m1 = m2 = l1 = 1, lc1 = lc2 = 0.5, I1 = I2 = 1, g = 9.8;
+    velocity bounds 4 pi and 9 pi; torques [-1, 0, +1] indexed by the action.
+
+    State (theta1, theta2, dtheta1, dtheta2), reset uniform(-0.1, 0.1, size=4).  Observation [cos theta1, sin theta1,
+    cos theta2, sin theta2, dtheta1, dtheta2].  A step takes one classical RK4 step over [0, dt] of the state augmented
+    with the torque (k1..k4, y0 + dt / 6 * (k1 + 2 k2 + 2 k3 + k4)), wraps both angles into [-pi, pi] with `while`
+    loops, clips both velocities to their bounds, and ends the episode when -cos theta1 - cos(theta2 + theta1) > 1;
+    reward -1 on every other step, 0 on the terminal one.  The derivative (_dsdt):
+        d1 = m1 lc1^2 + m2 (l1^2 + lc2^2 + 2 l1 lc2 cos theta2) + I1 + I2
+        d2 = m2 (lc2^2 + l1 lc2 cos theta2) + I2
+        phi2 = m2 lc2 g cos(theta1 + theta2 - pi/2)
+        phi1 = -m2 l1 lc2 dtheta2^2 sin theta2 - 2 m2 l1 lc2 dtheta2 dtheta1 sin theta2
+               + (m1 lc1 + m2 l1) g cos(theta1 - pi/2) + phi2
+        ddtheta2 = (a + d2 / d1 phi1 - m2 l1 lc2 dtheta1^2 sin theta2 - phi2) / (m2 lc2^2 + I2 - d2^2 / d1)
+        ddtheta1 = -(d2 ddtheta2 + phi1) / d1
+    The device rollouts (rollout.cu) replay this code operation by operation, so its evaluation order is the spec."""
+    device_kind = "acrobot"
+    dt = 0.2
+    m1, m2, l1, lc1, lc2, I1, I2, g = 1.0, 1.0, 1.0, 0.5, 0.5, 1.0, 1.0, 9.8
+    MAX_VEL_1, MAX_VEL_2 = 4 * math.pi, 9 * math.pi
+    AVAIL_TORQUE = (-1.0, 0.0, 1.0)
+
+    def __init__(self):
+        high = np.array([1.0, 1.0, 1.0, 1.0, self.MAX_VEL_1, self.MAX_VEL_2])
+        self.observation_space = Box(-high, high)
+        self.action_space = Discrete(3)
+        self.spec = _Spec("Acrobot-v1", 500)
+        self.state = None
+
+    def _ob(self):
+        s = self.state
+        return np.array([math.cos(s[0]), math.sin(s[0]), math.cos(s[1]), math.sin(s[1]), s[2], s[3]])
+
+    def reset(self):
+        self.state = np.random.uniform(-0.1, 0.1, size=(4,))
+        return self._ob()
+
+    def _dsdt(self, y):
+        """d/dt of the augmented state y = (theta1, theta2, dtheta1, dtheta2, a)."""
+        m1, m2, l1, lc1, lc2, I1, I2, g = self.m1, self.m2, self.l1, self.lc1, self.lc2, self.I1, self.I2, self.g
+        theta1, theta2, dtheta1, dtheta2, a = y
+        d1 = m1 * (lc1 * lc1) + m2 * (l1 * l1 + lc2 * lc2 + 2 * l1 * lc2 * math.cos(theta2)) + I1 + I2
+        d2 = m2 * (lc2 * lc2 + l1 * lc2 * math.cos(theta2)) + I2
+        phi2 = m2 * lc2 * g * math.cos(theta1 + theta2 - math.pi / 2.0)
+        phi1 = (-m2 * l1 * lc2 * (dtheta2 * dtheta2) * math.sin(theta2)
+                - 2 * m2 * l1 * lc2 * dtheta2 * dtheta1 * math.sin(theta2)
+                + (m1 * lc1 + m2 * l1) * g * math.cos(theta1 - math.pi / 2.0) + phi2)
+        ddtheta2 = ((a + d2 / d1 * phi1 - m2 * l1 * lc2 * (dtheta1 * dtheta1) * math.sin(theta2) - phi2)
+                    / (m2 * (lc2 * lc2) + I2 - d2 * d2 / d1))
+        ddtheta1 = -(d2 * ddtheta2 + phi1) / d1
+        return (dtheta1, dtheta2, ddtheta1, ddtheta2, 0.0)
+
+    def _rk4(self, y0):
+        dt = self.dt
+        dt2 = dt / 2.0
+        k1 = self._dsdt(y0)
+        k2 = self._dsdt([y + dt2 * k for y, k in zip(y0, k1)])
+        k3 = self._dsdt([y + dt2 * k for y, k in zip(y0, k2)])
+        k4 = self._dsdt([y + dt * k for y, k in zip(y0, k3)])
+        return [y + dt / 6.0 * (a + 2 * b + 2 * c + d) for y, a, b, c, d in zip(y0, k1, k2, k3, k4)]
+
+    @staticmethod
+    def _wrap(x, m, M):
+        diff = M - m
+        while x > M:
+            x = x - diff
+        while x < m:
+            x = x + diff
+        return x
+
+    def step(self, action):
+        s = [float(v) for v in self.state]
+        ns = self._rk4(s + [self.AVAIL_TORQUE[int(action)]])
+        th1 = self._wrap(ns[0], -math.pi, math.pi)
+        th2 = self._wrap(ns[1], -math.pi, math.pi)
+        dth1 = min(max(ns[2], -self.MAX_VEL_1), self.MAX_VEL_1)
+        dth2 = min(max(ns[3], -self.MAX_VEL_2), self.MAX_VEL_2)
+        self.state = np.array([th1, th2, dth1, dth2])
+        terminal = bool(-math.cos(th1) - math.cos(th2 + th1) > 1.0)
+        return self._ob(), (0.0 if terminal else -1.0), terminal, {}
+
+    def render(self):
+        pass
+
+    def close(self):
+        pass
+
+
+class MountainCarEnv(object):
+    """MountainCar-v0: an underpowered car in a valley must reach the hill top at position 0.5.  Limit 200 steps,
+    Discrete(3) actions (push left, none, right).  State and observation (position, velocity), a Box from
+    [-1.2, -0.07] to [0.6, 0.07]; reset [uniform(-0.6, -0.4), 0].  A step:
+        velocity += (a - 1) * 0.001 + cos(3 position) * (-0.0025), clipped to [-0.07, 0.07]
+        position += velocity, clipped to [-1.2, 0.6]
+        velocity = 0 if position == -1.2 and velocity < 0 (the left wall)
+        done = position >= 0.5 and velocity >= 0; reward -1 on every step.
+    The device rollouts (rollout.cu) replay this code operation by operation, so its evaluation order is the spec."""
+    device_kind = "mountaincar"
+    min_position, max_position, max_speed, goal_position = -1.2, 0.6, 0.07, 0.5
+    force, gravity = 0.001, 0.0025
+
+    def __init__(self):
+        self.observation_space = Box(np.array([self.min_position, -self.max_speed]),
+                                     np.array([self.max_position, self.max_speed]))
+        self.action_space = Discrete(3)
+        self.spec = _Spec("MountainCar-v0", 200)
+        self.state = None
+
+    def reset(self):
+        self.state = np.array([np.random.uniform(-0.6, -0.4), 0.0])
+        return np.array(self.state)
+
+    def _move(self, position, velocity, dv, goal):
+        """The shared tail of both MountainCars: velocity += dv, the clips, the left wall, the goal test."""
+        velocity = min(max(velocity + dv, -self.max_speed), self.max_speed)
+        position = min(max(position + velocity, self.min_position), self.max_position)
+        if position == self.min_position and velocity < 0:
+            velocity = 0.0
+        self.state = np.array([position, velocity])
+        return bool(position >= goal and velocity >= 0)
+
+    def step(self, action):
+        position, velocity = float(self.state[0]), float(self.state[1])
+        dv = (int(action) - 1) * self.force + math.cos(3 * position) * (-self.gravity)
+        done = self._move(position, velocity, dv, self.goal_position)
+        return np.array(self.state), -1.0, done, {}
+
+    def render(self):
+        pass
+
+    def close(self):
+        pass
+
+
+class MountainCarContinuousEnv(MountainCarEnv):
+    """MountainCarContinuous-v0: MountainCar with a force a in Box([-1], [1]).  Limit 999 steps, goal position 0.45;
+    reset, observation, clips and the left wall as MountainCar.  A step:
+        force = clip(a[0], -1, 1); velocity += force * 0.0015 - 0.0025 cos(3 position)
+        done = position >= 0.45 and velocity >= 0
+        reward = (100 if done else 0) - 0.1 * a[0]^2, with the UNCLIPPED action.
+    The device rollouts (rollout.cu) replay this code operation by operation, so its evaluation order is the spec."""
+    device_kind = "mountaincar_continuous"
+    goal_position, power = 0.45, 0.0015
+
+    def __init__(self):
+        super(MountainCarContinuousEnv, self).__init__()
+        self.action_space = Box(np.array([-1.0]), np.array([1.0]))
+        self.spec = _Spec("MountainCarContinuous-v0", 999)
+
+    def step(self, action):
+        position, velocity = float(self.state[0]), float(self.state[1])
+        a = float(np.asarray(action).reshape(-1)[0])
+        force = min(max(a, -1.0), 1.0)
+        done = self._move(position, velocity, force * self.power - 0.0025 * math.cos(3 * position), self.goal_position)
+        reward = (100.0 if done else 0.0) - 0.1 * (a * a)
+        return np.array(self.state), reward, done, {}
+
+
 _REGISTRY = {"CartPole-v0": CartPoleEnv, "CartPole": CartPoleEnv, "Pendulum-v0": PendulumEnv,
-             "Pendulum": PendulumEnv}
+             "Pendulum": PendulumEnv, "Acrobot-v1": AcrobotEnv, "Acrobot": AcrobotEnv,
+             "MountainCar-v0": MountainCarEnv, "MountainCar": MountainCarEnv,
+             "MountainCarContinuous-v0": MountainCarContinuousEnv, "MountainCarContinuous": MountainCarContinuousEnv}
 
 
 def make(name):
@@ -110,8 +274,8 @@ def make(name):
 
 
 def device_kind(env):
-    """The device implementation of a built-in environment (an instance or an id): 'cartpole' or 'pendulum'.
-    Raises ValueError for any other environment."""
+    """The device implementation of a built-in environment (an instance or an id): 'cartpole', 'pendulum',
+    'acrobot', 'mountaincar' or 'mountaincar_continuous'.  Raises ValueError for any other environment."""
     cls = _REGISTRY.get(env) if isinstance(env, str) else type(env)
     kind = getattr(cls, "device_kind", None)
     if kind is None:

@@ -2,7 +2,7 @@
 """Cross-entropy-method driver with the reference's run_cem.py command line (GENERAL_OPTIONS, --env, --agent, --plot,
 the agent's own options, CEM_OPTIONS - run_cem.py:13-30).  Candidates are scored through the device-resident
 deterministic policy; with --parallel 1 the whole population is scored in lockstep by one population-batched forward
-per environment step; with --device_envs (CartPole and Pendulum) each generation is one device rollout round.
+per environment step; with --device_envs (the built-in environments) each generation is one device rollout round.
 
   python run_cem.py --env CartPole-v0 --agent modular_rl.agentzoo.DeterministicAgent --n_iter 10 --batch_size 40
 """
@@ -36,7 +36,7 @@ def parse_cli(argv):
     ap.add_argument("--plot", action="store_true")
     ap.add_argument("--device_envs", action="store_true",
                     help="score each generation in one GPU rollout round, one environment per candidate (built-in "
-                         "CartPole and Pendulum only); resets come from the device's Philox stream, so results differ "
+                         "CartPole, Pendulum, Acrobot, MountainCar and MountainCarContinuous only); resets come from the device's Philox stream, so results differ "
                          "from a host run with the same --seed")
     first, _ = ap.parse_known_args([a for a in argv if a not in ("-h", "--help")])
     agent_cls = mrl.get_agent_cls(first.agent)

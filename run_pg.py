@@ -40,8 +40,8 @@ def main():
                         help="environments stepped in lockstep with one batched device forward per step "
                              "(0: serial rollouts as the reference); not an agent option")
     parser.add_argument("--device_envs", type=int, default=0,
-                        help="environments per rollout round run on the GPU in one kernel launch (built-in CartPole "
-                             "and Pendulum only; 0: host rollouts); resets and action noise come from the device's "
+                        help="environments per rollout round run on the GPU in one kernel launch (built-in CartPole, "
+                             "Pendulum, Acrobot, MountainCar and MountainCarContinuous only; 0: host rollouts); resets and action noise come from the device's "
                              "Philox stream, so results differ from a host run with the same --seed")
     args, _ = parser.parse_known_args([arg for arg in sys.argv[1:] if arg not in ('-h', '--help')])
     if args.device_envs and args.vec_envs:
