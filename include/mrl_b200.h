@@ -114,7 +114,11 @@ int mrl_zfilter_scan(const void* x, int x_dtype, long long N, int d, double* sta
 
 /* ---------------------------------------------------------------- network (policy or value MLP)
  * dims[0..n_layers] = input dim, hidden sizes..., output dim (agentzoo.py:25-61).  Parameters are the
- * reference's flat vector: per Dense layer [kernel(in,out) C-order, bias], then logstd (core.py:518-557). */
+ * reference's flat vector: per Dense layer [kernel(in,out) C-order, bias], then logstd (core.py:518-557).
+ * Limits: 1..6 layers, every width <= 256, at most 64 outputs, and dims[0] x dims[1] within the tensor-memory
+ * budget of the layer-1 kernels (376 inputs allow a first hidden layer of at most 144 units).  A net whose fused
+ * layers->=2 kernels do not fit in shared memory (e.g. two hidden layers wider than about 88 units) runs those
+ * layers one launch per layer instead; the choice is made here, from the shapes, and no entry point changes. */
 int mrl_net_create(mrl_net** out, int device, int n_layers, const int* dims, int head, int activation);
 int mrl_net_destroy(mrl_net* n);
 long long mrl_net_num_params(const mrl_net* n);

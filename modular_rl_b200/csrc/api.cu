@@ -635,6 +635,8 @@ struct mrl_net {
   long long adam_t = 0;
   DevBuf WC, VC;           // tcgen05 Fisher-vector chain: weight images of theta / of the tangent
   bool tc_fvp = false;
+  bool layers = false;     // layers >= 2 run layer by layer (mlp_layers.cu): the fused mid_* kernels cannot hold the net
+  DevBuf R0, R1;           // its ping-pong buffers (deltas, R-activations)
   DevBuf DG, WBt, WBv, theta, theta_prev, theta_trial, img, imgv, vflat, Z1, cache, part1, partm, loss_part, out32,
       out64, g32, cg_b, cg_x, cg_r, cg_p, p32, x32, fullstep, cgstate, cgscratch, scal, headout, stage;
   unsigned long long params_version = 1, cache_params_version = 0, cache_batch_version = 0;
@@ -668,11 +670,8 @@ extern "C" int mrl_net_create(mrl_net** out, int device, int n_layers, const int
   }
   int dev_smem = 0;
   CK(cudaDeviceGetAttribute(&dev_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, device));
-  const size_t need = mid_backward_smem(n->g, head == MRL_VALUE ? MRL_MODE_GRAD : MRL_MODE_FVP) + 2048;
-  if (need > (size_t)dev_smem) {
-    delete n;
-    return fail("mrl_net_create: network needs %zu B of shared memory per CTA, device offers %d", need, dev_smem);
-  }
+  // a net whose fused reverse-sweep kernel does not fit in shared memory runs layers >= 2 one launch at a time
+  n->layers = mid_backward_smem(n->g, head == MRL_VALUE ? MRL_MODE_GRAD : MRL_MODE_FVP) + 2048 > (size_t)dev_smem;
   const size_t P = n->g.P;
   cudaError_t e = cudaSuccess;
   auto R = [&](DevBuf& b, size_t bytes) { if (e == cudaSuccess) e = b.reserve(bytes); };
@@ -684,7 +683,7 @@ extern "C" int mrl_net_create(mrl_net** out, int device, int n_layers, const int
   R(n->p32, P * 4); R(n->x32, P * 4); R(n->fullstep, P * 8);
   R(n->cgstate, sizeof(CgState)); R(n->scal, 32 * 8); R(n->cgscratch, CG_SCRATCH_DOUBLES * 8);
   {
-    n->tc_fvp = fvp_tc_supported(n->g);
+    n->tc_fvp = !n->layers && fvp_tc_supported(n->g);
     if (n->tc_fvp) {
       R(n->WC, fvp_tc_image_floats(n->g, 0) * 4);
       R(n->VC, fvp_tc_image_floats(n->g, 1) * 4);
@@ -708,7 +707,7 @@ extern "C" int mrl_net_destroy(mrl_net* n) {
   DevBuf* bufs[] = {&n->adam_m, &n->adam_v, &n->sgd_acc, &n->WC, &n->VC, &n->DG, &n->WBt, &n->WBv, &n->theta, &n->theta_prev, &n->theta_trial, &n->img, &n->imgv, &n->vflat,
                     &n->Z1, &n->cache, &n->part1, &n->partm, &n->loss_part, &n->out32, &n->out64, &n->g32,
                     &n->cg_b, &n->cg_x, &n->cg_r, &n->cg_p, &n->p32, &n->x32, &n->fullstep, &n->cgstate, &n->cgscratch, &n->scal,
-                    &n->headout, &n->stage};
+                    &n->headout, &n->stage, &n->R0, &n->R1};
   for (DevBuf* d : bufs) d->release();
   if (n->h_scal) cudaFreeHost(n->h_scal);
   if (n->h_cg) cudaFreeHost(n->h_cg);
@@ -840,6 +839,10 @@ static int reserve_ws(mrl_net* n, const mrl_batch* b, const Plan& pl) {
     }
   }
   CK(n->DG.reserve(l1tc_dg_floats(g, b->n_tiles) * 4));
+  if (n->layers) {
+    CK(n->R0.reserve(layers_ws_floats(g, b->n_tiles) * 4));
+    CK(n->R1.reserve(layers_ws_floats(g, b->n_tiles) * 4));
+  }
   CK(n->part1.reserve((size_t)pl.n_slabs * g.d[0] * g.n1p * 4));
   CK(n->partm.reserve((size_t)pl.n_slabs * g.pmid * 4));
   CK(n->loss_part.reserve((size_t)pl.n_slabs * 4 * 8));
@@ -866,7 +869,13 @@ static int pass_forward(mrl_net* n, mrl_batch* b, bool want_losses, bool want_ca
   a.n_tiles = b->n_tiles;
   a.slab_tiles = pl.slab_tiles;
   a.reverse_kl = reverse_kl;
-  if (chain_fwd_shape(g) != 0) CKP(PK_MIDF, launch_chain_forward(g, a, pl.n_slabs, st), 1);
+  if (n->layers) {
+    // the layer-by-layer path keeps its activations in the cache even when the caller does not want them
+    a.cache = n->cache.as<float>();
+    if (!want_cache) n->cache_batch = nullptr;
+    int nk = 0;
+    CKP(PK_MIDF, launch_layers_forward(g, a, pl.n_slabs, st, &nk), nk);
+  } else if (chain_fwd_shape(g) != 0) CKP(PK_MIDF, launch_chain_forward(g, a, pl.n_slabs, st), 1);
   else CKP(PK_MIDF, launch_mid_forward(g, a, pl.n_slabs, st), 1);
   if (want_losses) {
     CKL(launch_reduce_losses(n->loss_part.as<double>(), pl.n_slabs, 1.0 / (double)b->Nglobal, n->scal.as<double>(), st), 1);
@@ -914,7 +923,11 @@ static int pass_backward(mrl_net* n, mrl_batch* b, int mode, const double* coef_
   a.slab_tiles = pl.slab_tiles;
   a.mode = mode;
   a.reverse_kl = reverse_kl;
-  if (tc) {
+  if (n->layers) {
+    int nk = 0;
+    CKP(mode == MRL_MODE_FVP ? PK_MIDB_FVP : PK_MIDB_GRAD,
+        launch_layers_backward(g, a, n->R0.as<float>(), n->R1.as<float>(), pl.n_slabs, st, &nk), nk);
+  } else if (tc) {
     FvpTcArgs x;
     x.WC = n->WC.as<float>(); x.VC = n->VC.as<float>(); x.vflat = v_dev; x.img = n->img.as<float>();
     x.Zt = n->Z1.as<float>(); x.cache = n->cache.as<float>(); x.DG = n->DG.as<float>(); x.partm = n->partm.as<float>();

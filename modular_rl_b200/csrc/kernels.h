@@ -66,6 +66,15 @@ size_t mid_backward_smem(const NetGeom& g, int mode);
 cudaError_t launch_mid_forward(const NetGeom& g, const MidFwdArgs& a, int n_slabs, cudaStream_t st);
 cudaError_t launch_mid_backward(const NetGeom& g, const MidBwdArgs& a, int n_slabs, cudaStream_t st);
 
+// ---- mlp_layers.cu  (layer-by-layer path for nets whose mid_* kernels do not fit in shared memory, L >= 2)
+// Same contract as launch_mid_*; R0 / R1: ping-pong buffers of layers_ws_floats each (deltas, R-activations).
+// *launches: kernels launched.
+size_t layers_ws_floats(const NetGeom& g, long long n_tiles);
+cudaError_t launch_layers_forward(const NetGeom& g, const MidFwdArgs& a /* cache required */, int n_slabs,
+                                  cudaStream_t st, int* launches);
+cudaError_t launch_layers_backward(const NetGeom& g, const MidBwdArgs& a, float* R0, float* R1, int n_slabs,
+                                   cudaStream_t st, int* launches);
+
 // ---- mlp_chain.cu  (register-resident per-warp chains for the forward and gradient passes)
 #define CH_WARPS 12          // backward chain: 12 warps x 16 timesteps = 3 cache tiles per pass
 #define CH_NE 3             // weight-gradient entries per warp

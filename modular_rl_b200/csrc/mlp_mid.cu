@@ -40,65 +40,6 @@ struct Lane {
 // lo = x - hi (exact in fp32; the tensor core drops its low 13 bits, a 2^-21 relative effect);
 // D += lo.hi + hi.lo + hi.hi keeps FP32-class accuracy (north_star: 1e-5) at 1/3 of the TF32 rate,
 // with ~3x fewer issued instructions than the FFMA formulation (the chain is issue-bound).
-// MT x 2 mma tiles, three passes (lo.hi, hi.lo, hi.hi) so that consecutive MMAs hit different accumulators
-template <int MT>
-__device__ __forceinline__ void mma3_tiles(float (&acc)[MT][2][4], const uint32_t (&ah)[MT][4],
-                                           const uint32_t (&al)[MT][4], const uint32_t (&bh)[2][2],
-                                           const uint32_t (&bl)[2][2]) {
-#pragma unroll
-  for (int mi = 0; mi < MT; ++mi)
-#pragma unroll
-    for (int ni = 0; ni < 2; ++ni) mma_tf32(acc[mi][ni], al[mi], bh[ni]);
-#pragma unroll
-  for (int mi = 0; mi < MT; ++mi)
-#pragma unroll
-    for (int ni = 0; ni < 2; ++ni) mma_tf32(acc[mi][ni], ah[mi], bl[ni]);
-#pragma unroll
-  for (int mi = 0; mi < MT; ++mi)
-#pragma unroll
-    for (int ni = 0; ni < 2; ++ni) mma_tf32(acc[mi][ni], ah[mi], bh[ni]);
-}
-
-// acc[mi][ni] += A^T-tile . B-tile over k in [0,K): A_T[k][r] feature-major activations (ld = MRL_LDT),
-// B[k][c] row-major weights (ld = ldb).  Warp tile (16*MT) rows x 16 cols = MT x 2 mma tiles.
-template <int MT, bool TAIL>
-__device__ __forceinline__ void mma_fwd_step(float (&acc)[MT][2][4], const float* __restrict__ a,
-                                             const float* __restrict__ b0, const float* __restrict__ b1, int ldb4,
-                                             int krem) {
-  // a -> A_T[k0 + t][r0 + g], b0/b1 -> B[k0 + t][c], ldb4 = 4 * ldb ; rows k0+t and k0+t+4
-  const bool va = !TAIL || krem > 0, vb = !TAIL || krem > 4;   // krem = K - (k0 + t)
-  uint32_t bh[2][2], bl[2][2], ah[MT][4], al[MT][4];
-  split_tf32(va ? b0[0] : 0.f, bh[0][0], bl[0][0]);
-  split_tf32(vb ? b0[ldb4] : 0.f, bh[0][1], bl[0][1]);
-  split_tf32(va ? b1[0] : 0.f, bh[1][0], bl[1][0]);
-  split_tf32(vb ? b1[ldb4] : 0.f, bh[1][1], bl[1][1]);
-#pragma unroll
-  for (int mi = 0; mi < MT; ++mi) {
-    split_tf32(va ? a[16 * mi] : 0.f, ah[mi][0], al[mi][0]);
-    split_tf32(va ? a[16 * mi + 8] : 0.f, ah[mi][1], al[mi][1]);
-    split_tf32(vb ? a[4 * MRL_LDT + 16 * mi] : 0.f, ah[mi][2], al[mi][2]);
-    split_tf32(vb ? a[4 * MRL_LDT + 16 * mi + 8] : 0.f, ah[mi][3], al[mi][3]);
-  }
-  mma3_tiles<MT>(acc, ah, al, bh, bl);
-}
-template <int MT>
-__device__ __forceinline__ void mma_fwd_acc(float (&acc)[MT][2][4], const float* __restrict__ A,
-                                            const float* __restrict__ B, int K, int ldb, int r0, int c0,
-                                            int lane) {
-  const int g = lane >> 2, t = lane & 3;
-  const float* a = A + t * MRL_LDT + r0 + g;
-  const float* b0 = B + t * ldb + min(c0 + g, ldb - 1);
-  const float* b1 = B + t * ldb + min(c0 + 8 + g, ldb - 1);
-  const int ldb4 = 4 * ldb, ldb8 = 8 * ldb;
-  int k0 = 0;
-#pragma unroll 2
-  for (; k0 + 8 <= K; k0 += 8) {
-    mma_fwd_step<MT, false>(acc, a, b0, b1, ldb4, 8);
-    a += 8 * MRL_LDT; b0 += ldb8; b1 += ldb8;
-  }
-  if (k0 < K) mma_fwd_step<MT, true>(acc, a, b0, b1, ldb4, K - k0 - t);
-}
-
 // One warp job of  OUT[c][r] = epi(c, r, sum_k A1[k][r] B1[k][c] (+ sum_k A2[k][r] B2[k][c])).
 // job -> (16*MT) rows x 16 cols; epi(c, r, value) is called once per output element.  MT = 1 doubles
 // the number of jobs of a phase that would otherwise leave warps idle.
