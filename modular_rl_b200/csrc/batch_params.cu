@@ -11,7 +11,7 @@
 
 // ------------------------------------------------------------------------------------
 // theta (flat, reference order) -> the shared-memory image and the layer-1 tensor-core operand
-// WB [kg][hi|lo][khalf][ngroup][8][4] (K-major UMMA core-matrix order, hi = rna_tf32(x), lo = rna_tf32(x - hi)).
+// WB (l1_wb_offset: K-major UMMA core-matrix order, hi = rna_tf32(x), lo = rna_tf32(x - hi)).
 __global__ void pack_params_kernel(NetGeom g, const float* __restrict__ theta, float* __restrict__ img,
                                    float* __restrict__ WB, int nu) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -20,7 +20,7 @@ __global__ void pack_params_kernel(NetGeom g, const float* __restrict__ theta, f
     const int k = i / nu, n = i % nu;
     const float x = (k < g.d[0] && n < g.d[1]) ? theta[g.off_flat_W[1] + k * g.d[1] + n] : 0.f;
     const float h = tf32_rna(x);
-    float* base = WB + (size_t)(k >> 3) * (2 * nu * 8) + ((k & 7) >> 2) * (nu * 4) + (n >> 3) * 32 + (n & 7) * 4 + (k & 3);
+    float* base = WB + l1_wb_offset(k >> 3, (k & 7) >> 2, n, nu) + (k & 3);
     base[0] = h;
     base[nu * 8] = tf32_rna(x - h);
     return;

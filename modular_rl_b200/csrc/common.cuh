@@ -48,6 +48,21 @@ struct NetGeom {
   int off_pm_logstd;             // offset of the logstd partial inside a mid partial
 };
 
+// B operands of the layer-1 tcgen05 GEMMs (mlp_l1_tc.cu) in HBM, in the UMMA K-major no-swizzle core-matrix order
+// over N = nu layer-1 units (a multiple of 8) and K (timesteps for DG, input features for WB), in groups of 8 K:
+//   DG  delta_1, raw fp32:            [t/8][khalf][n/8][8 n][4 t]
+//   WB  W1 (or V1) split (hi, lo):    [k/8][hi | lo][khalf][n/8][8 n][4 k]   lo sits nu * 8 floats behind hi
+// A core matrix is 8 rows of n x 4 consecutive K values (16 B): 32 floats.  Core matrices of consecutive 8-row groups
+// are 128 B apart (SBO), the two K halves of a group nu * 16 B apart (LBO); a group of 8 K is one contiguous block of
+// nu * 8 floats (WB: twice that, hi then lo), loaded as a whole by one bulk copy.  The offsets locate element n at
+// K = 8 * group + 4 * khalf; the caller adds K % 4.
+__host__ __device__ __forceinline__ size_t l1_dg_offset(size_t tgroup, int khalf, int n, int nu) {
+  return tgroup * (nu * 8) + khalf * (nu * 4) + (n >> 3) * 32 + (n & 7) * 4;
+}
+__host__ __device__ __forceinline__ size_t l1_wb_offset(size_t kgroup, int khalf, int n, int nu) {
+  return kgroup * (2 * nu * 8) + khalf * (nu * 4) + (n >> 3) * 32 + (n & 7) * 4;
+}
+
 // ----------------------------------------------------------------------------- PTX helpers
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
   return static_cast<uint32_t>(__cvta_generic_to_shared(p));

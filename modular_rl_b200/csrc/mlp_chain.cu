@@ -22,6 +22,7 @@
 // Two barriers per 192 timesteps (the job-list kernel in mlp_mid.cu needs ~10 per 64) and ~2x fewer
 // issued instructions per timestep; see DESIGN.md section 4 for the measured effect.
 #include "common.cuh"
+#include "heads.cuh"
 #include "kernels.h"
 #include "mma_tf32.cuh"
 #include <string.h>
@@ -186,7 +187,7 @@ __device__ __forceinline__ void epi_delta(const float (&acc)[NT][4], const float
 // dL/dz_L of the surrogate / penalised surrogate / squared error at the head (trpo.py:43, ppo.py:47-49,
 // core.py:613-617), un-normalised (1/N is applied by the slab reduce).  ho = cached head output (mean | probs |
 // value) in accumulator order; auxb = this warp's rows of the side inputs.  Also the logstd gradient partials.
-#define CH_LOG1P(x) log1pf(x)
+// The per-element terms are those of heads.cuh.
 template <int NT>
 __device__ __forceinline__ void head_grad(int head, const float (&ho)[NT][4], const float* __restrict__ auxb, int dL,
                                           const float* __restrict__ sig, const float* __restrict__ ivar, float cs,
@@ -213,9 +214,7 @@ __device__ __forceinline__ void head_grad(int head, const float (&ho)[NT][4], co
       for (int i = 0; i < 4; ++i) {
         const int j = 8 * n + 2 * t + (i & 1);
         if (j < dL && ok) {
-          const float sg = sig[j];
-          const float tt = (ac[n][i] - ho[n][i]) / sg, t0 = (ac[n][i] - m0[n][i]) / s0[n][i];
-          const float v = -0.5f * (tt - t0) * (tt + t0) - CH_LOG1P((sg - s0[n][i]) / s0[n][i]);   // logp - oldlogp, term by term
+          const float v = gauss_logratio(ho[n][i], ac[n][i], m0[n][i], s0[n][i], sig[j]);
           if (i < 2) dl0 += v; else dl1 += v;
         }
       }
@@ -229,20 +228,10 @@ __device__ __forceinline__ void head_grad(int head, const float (&ho)[NT][4], co
         const int j = 8 * n + 2 * t + (i & 1);
         const bool valid = i < 2 ? valid0 : valid1;
         if (j < dL && valid) {
-          const float w = i < 2 ? w0 : w1;
-          const float sg = sig[j], iv = ivar[j], mu = ho[n][i], a_ = ac[n][i], m_ = m0[n][i], s_ = s0[n][i];
-          const float t2 = (a_ - mu) * (a_ - mu) * iv;
-          float dkl_dmu, dkl_dls;
-          if (!reverse_kl) {
-            dkl_dmu = (mu - m_) * iv;
-            dkl_dls = ((sg - s_) * (sg + s_) - (m_ - mu) * (m_ - mu)) * iv;   // 1 - (s0^2 + dm^2) / s1^2
-          } else {
-            const float i0 = 1.f / (s_ * s_);
-            dkl_dmu = (mu - m_) * i0;
-            dkl_dls = (sg - s_) * (sg + s_) * i0;                             // -1 + s1^2 / s0^2
-          }
-          d[n][i] = w * (a_ - mu) * iv + ck * dkl_dmu;
-          gls[n][i & 1] += w * (t2 - 1.f) + ck * dkl_dls;
+          float d_ls;
+          gauss_grad(ho[n][i], ac[n][i], m0[n][i], s0[n][i], sig[j], ivar[j], i < 2 ? w0 : w1, ck, reverse_kl, d[n][i],
+                     d_ls);
+          gls[n][i & 1] += d_ls;
         }
       }
   } else if (head == MRL_HEAD_CAT) {
@@ -276,18 +265,14 @@ __device__ __forceinline__ void head_grad(int head, const float (&ho)[NT][4], co
       for (int i = 0; i < 4; ++i) {
         const int j = 8 * n + 2 * t + (i & 1);
         const bool valid = i < 2 ? valid0 : valid1;
-        if (j < dL && valid) {
-          const float p = ho[n][i], q = p0[n][i];
-          const float w = i < 2 ? w0 : w1;
-          const int ai = i < 2 ? ai0 : ai1;
-          const float dk = reverse_kl ? p * (logf(p / q) - (i < 2 ? kl0 : kl1)) : (p - q);
-          d[n][i] = w * ((j == ai ? 1.f : 0.f) - p) + ck * dk;
-        }
+        if (j < dL && valid)
+          d[n][i] = cat_grad(ho[n][i], p0[n][i], i < 2 ? w0 : w1, ck, i < 2 ? kl0 : kl1, j == (i < 2 ? ai0 : ai1),
+                             reverse_kl);
       }
   } else {   // value head: d/dpred of (y - pred)^2
     if (t == 0) {
-      if (valid0) d[0][0] = 2.f * (ho[0][0] - __ldg(auxb));
-      if (valid1) d[0][2] = 2.f * (ho[0][2] - __ldg(auxb + 1));
+      if (valid0) d[0][0] = value_dpred(ho[0][0], __ldg(auxb));
+      if (valid1) d[0][2] = value_dpred(ho[0][2], __ldg(auxb + 1));
     }
   }
 }
@@ -315,8 +300,8 @@ __device__ __forceinline__ void delta_layer(float (&acc)[NI][4], const uint32_t 
   }
 }
 
-// delta_1 for in-blocks nb .. nb+NH-1: bias partial sums + the tcgen05 operand DG as raw fp32
-// [tg = t/8][khalf][ngroup nu/8][8 n][4 timesteps]  (mlp_l1_tc.cu splits it into (hi, lo))
+// delta_1 for in-blocks nb .. nb+NH-1: bias partial sums + the tcgen05 operand DG as raw fp32 (l1_dg_offset;
+// mlp_l1_tc.cu splits it into (hi, lo))
 template <int ACT, int NH, int nb, int N1, int NO>
 __device__ __forceinline__ void delta1_block(const uint32_t (&dhi)[NO][4], const uint32_t (&dlo)[NO][4],
                                              const float* __restrict__ W2, const float* __restrict__ hp,
@@ -349,7 +334,7 @@ __device__ __forceinline__ void delta1_block(const uint32_t (&dhi)[NO][4], const
     if (ok && 8 * (nb + n) < nu) {
       // dg -> the warp's first timestep group.  This thread's timesteps 2g, 2g+1 are adjacent inside a group of 4:
       // one 64-bit store per feature.
-      float* p0 = dg + (size_t)(g >> 2) * (nu * 8) + ((g >> 1) & 1) * (nu * 4) + (nb + n) * 32 + (2 * t) * 4 + 2 * (g & 1);
+      float* p0 = dg + l1_dg_offset(g >> 2, (g >> 1) & 1, 8 * (nb + n) + 2 * t, nu) + 2 * (g & 1);
 #pragma unroll
       for (int b = 0; b < 2; ++b)   // features 2t, 2t+1 of the n-tile
         *reinterpret_cast<float2*>(p0 + b * 4) = make_float2(v[b], v[b + 2]);
@@ -534,15 +519,14 @@ __global__ void __launch_bounds__(CH_THREADS, 1) chain_bwd_kernel(NetGeom g, Mid
         to_frags<N2>(d2, d2h, d2l);
       }
       warp_arrive(&e_full, lane);           // this warp's delta rows are complete; delta_1 below needs nobody else
-      float* dg = a.DG + (size_t)(ct0 * 8 + 2 * warp) * (a.nu * 8);
+      float* dg = a.DG + l1_dg_offset(ct0 * 8 + 2 * warp, 0, 0, a.nu);
       constexpr int NA = (N1 + 1) / 2, NB = N1 - NA;
       delta1_block<ACT, NA, 0, N1, N2>(d2h, d2l, Ws + S::woff(2), cb, g.d[1], ok, gb1s + warp * 8 * N1, dg, a.nu, lane);
       if constexpr (NB > 0)
         delta1_block<ACT, NB, NA, N1, N2>(d2h, d2l, Ws + S::woff(2), cb, g.d[1], ok, gb1s + warp * 8 * N1, dg, a.nu, lane);
       if (ok && a.nu > 8 * N1) {   // the one operand n-group beyond the chain's padded width is zeros
-        float* dgz = dg + 8 * N1 * 4 + lane;
 #pragma unroll
-        for (int k = 0; k < 4; ++k) dgz[(size_t)k * (a.nu * 4)] = 0.f;   // [tg 2][khalf 2] x 32 floats
+        for (int k = 0; k < 4; ++k) dg[l1_dg_offset(k >> 1, k & 1, 8 * N1, a.nu) + lane] = 0.f;   // [tg 2][khalf 2] x 32 floats
       }
     }
     bar_wait(&e_full, tile_no & 1);
@@ -740,7 +724,6 @@ cudaError_t launch_chain_backward(const NetGeom& g, const MidBwdArgs& a, int n_s
 // row-major head output (trpo.py:37-42,60-63; core.py:339-365,402-438,613-617).  Same per-warp register
 // chain as above (16 timesteps per warp, no block barriers inside a slab), 8 warps = 128 timesteps per pass,
 // 2 CTAs per SM.
-#define CH_LOG_2PIE 2.8378770664093453f
 
 __device__ __forceinline__ void st_cfrag(float* __restrict__ p, const float (&v)[4], int f0, int dmax, bool ok) {
   if (ok && f0 < dmax) *reinterpret_cast<float2*>(p + f0 * MRL_LDT) = make_float2(v[0], v[2]);
@@ -793,15 +776,8 @@ __device__ __forceinline__ void head_forward(int head, float (&o)[NT][4], const 
       for (int i = 0; i < 4; ++i) {
         const int j = 8 * n + 2 * t + (i & 1);
         if (j < dL && ok) {
-          const float sg = sig[j], mu = o[n][i];
-          const float tt = (ac[i] - mu) / sg, t0 = (ac[i] - m0[i]) / s0[i];
-          const float lr = log1pf((sg - s0[i]) / s0[i]);            // log(sigma / sigma0)
-          const float dlv = -0.5f * (tt - t0) * (tt + t0) - lr;     // logp - oldlogp, term by term
-          const float dm = m0[i] - mu;
-          // log(s1/s0) + (s0^2 + dm^2) / (2 s1^2) - 1/2 with the s0 ~ s1 cancellation taken analytically
-          const float den = reverse_kl ? s0[i] : sg;
-          const float u = (reverse_kl ? (sg - s0[i]) : (s0[i] - sg)) / den;
-          const float klv = u_minus_log1p(u) + 0.5f * (u * u + (dm / den) * (dm / den));
+          const float dlv = gauss_logratio(o[n][i], ac[i], m0[i], s0[i], sig[j]);
+          const float klv = gauss_kl(o[n][i], m0[i], s0[i], sig[j], reverse_kl);
           if (i < 2) { dl0 += dlv; kl0 += klv; } else { dl1 += dlv; kl1 += klv; }
         }
       }
@@ -853,9 +829,7 @@ __device__ __forceinline__ void head_forward(int head, float (&o)[NT][4], const 
         const int j = 8 * n + 2 * t + (i & 1);
         if (j < dL && ok) {
           const float p = o[n][i];
-          // q log(q/w) = q g(v) - (w - q), v = (w - q)/q : no cancellation between the terms of the sum
-          const float q = reverse_kl ? p : p0[i], w = reverse_kl ? p0[i] : p;
-          const float klv = q * u_minus_log1p((w - q) / q) - (w - q);
+          const float klv = cat_kl(p, p0[i], reverse_kl);
           const float env = -p * logf(p);
           if (i < 2) { kl0 += klv; en0 += env; if (j == ai0) { pa0 = p; qa0 = p0[i]; } }
           else { kl1 += klv; en1 += env; if (j == ai1) { pa1 = p; qa1 = p0[i]; } }
@@ -875,8 +849,8 @@ __device__ __forceinline__ void head_forward(int head, float (&o)[NT][4], const 
     }
   } else {   // value head: squared error against the target row
     if (auxb != nullptr && t == 0) {
-      if (valid0) { const float df = __ldg(auxb) - o[0][0]; s_surr += (double)df * (double)df; }
-      if (valid1) { const float df = __ldg(auxb + 1) - o[0][2]; s_surr += (double)df * (double)df; }
+      if (valid0) s_surr += value_sqerr(__ldg(auxb), o[0][0]);
+      if (valid1) s_surr += value_sqerr(__ldg(auxb + 1), o[0][2]);
     }
   }
 }
@@ -913,7 +887,7 @@ __global__ void __launch_bounds__(FW_THREADS, 2) chain_fwd_kernel(NetGeom g, Mid
   {
     float sls = 0.f;
     for (int j = 0; j < g.d[L] && gauss; ++j) sls += a.img[g.off_pm_logstd + j];
-    ent_row = sls + 0.5f * CH_LOG_2PIE * g.d[L];
+    ent_row = sls + 0.5f * MRL_LOG_2PIE * g.d[L];
   }
   for (int f = tid; f < 8 * NL; f += FW_THREADS) sig[f] = (gauss && f < g.d[L]) ? expf(a.img[g.off_pm_logstd + f]) : 1.f;
   __syncthreads();

@@ -688,7 +688,7 @@ __global__ void __launch_bounds__(FT_THREADS, 1) fvp_tc_kernel(NetGeom g, FtPlan
               }
               if (l == 2) {
                 // ---- final, chunk c: delta_1 = d_1' * act'(h_1) -> DG (K-major tcgen05 B operand of the layer-1 gradient
-                // GEMM as raw fp32: [t/8][khalf][n/8][8 n][4 t]; l1_grad_tc_kernel splits it into (hi, lo)) + bias partial
+                // GEMM as raw fp32, l1_dg_offset; l1_grad_tc_kernel splits it into (hi, lo)) + bias partial
                 // sums.  The two groups take alternate 8-column blocks; a 4 x 4 transpose inside each lane quad turns
                 // (4 features of my timestep) into (my feature at the quad's 4 timesteps) = one 16-byte store.
                 const FtDStage st = P.ds[k];
@@ -704,8 +704,6 @@ __global__ void __launch_bounds__(FT_THREADS, 1) fvp_tc_kernel(NetGeom g, FtPlan
                 mbar_wait_sleep(&dacc_full[k], tcount & 1);
                 tc_fence_after();
                 const uint32_t facc = tlane + st.acc_col;
-                // quad base: timesteps 4 (T / 4) .. + 3 of feature n: + (n / 8) * 32 + (n % 8) * 4
-                float* dgq = a.DG + (size_t)(T >> 3) * (nu * 8) + ((T >> 2) & 1) * (nu * 4);
                 for (; j0 < st.N; j0 += 16) {
                   const int c0 = st.col0 + j0;
                   if (j0 + 16 < st.N) request1(c0 + 16, h1n);
@@ -719,9 +717,9 @@ __global__ void __launch_bounds__(FT_THREADS, 1) fvp_tc_kernel(NetGeom g, FtPlan
                     float tq[4] = {val[4 * hq], val[4 * hq + 1], val[4 * hq + 2], val[4 * hq + 3]};
                     ft_quad_transpose(tq, lane);
                     if (ok) {
-                      const int n = c0 + 4 * hq + (lane & 3);
-                      float* p = dgq + (n >> 3) * 32 + (n & 7) * 4;
-                      *reinterpret_cast<float4*>(p) = make_float4(tq[0], tq[1], tq[2], tq[3]);
+                      const int n = c0 + 4 * hq + (lane & 3);   // timesteps 4 (T / 4) .. + 3 of feature n
+                      *reinterpret_cast<float4*>(a.DG + l1_dg_offset(T >> 3, (T >> 2) & 1, n, nu)) =
+                          make_float4(tq[0], tq[1], tq[2], tq[3]);
                     }
                   }
                   // column sums over the warp's 32 timesteps: 8 -> 4 -> 2 -> 1 values per lane, then the quad
@@ -791,13 +789,13 @@ __global__ void ft_pack_kernel(NetGeom g, FtPackJobs jobs, const float* __restri
                                float* __restrict__ WB1, int nu) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= total) {
-    // the layer-1 operand of the same vector (WB of mlp_l1_tc.cu: [kg][hi|lo][khalf][ngroup][8][4]) in the same launch
+    // the layer-1 operand of the same vector (WB of mlp_l1_tc.cu, l1_wb_offset) in the same launch
     const int j = i - total;
     if (WB1 == nullptr || j >= g.d0p * nu) return;
     const int k = j / nu, n = j % nu;
     const float x = (k < g.d[0] && n < g.d[1]) ? src[g.off_flat_W[1] + k * g.d[1] + n] : 0.f;
     const float h = tf32_rna(x);
-    float* base = WB1 + (size_t)(k >> 3) * (2 * nu * 8) + ((k & 7) >> 2) * (nu * 4) + (n >> 3) * 32 + (n & 7) * 4 + (k & 3);
+    float* base = WB1 + l1_wb_offset(k >> 3, (k & 7) >> 2, n, nu) + (k & 3);
     base[0] = h;
     base[nu * 8] = tf32_rna(x - h);
     return;

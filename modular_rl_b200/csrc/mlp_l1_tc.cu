@@ -8,7 +8,8 @@
 // accumulation in TMEM: per-product error ~2^-21, i.e. FP32-class results at 1/3 of the TF32 rate.
 //
 // Operands are pre-arranged in HBM in the UMMA canonical K-major / no-swizzle core-matrix order
-// (8 rows x 16 bytes per core matrix, SBO = 128 B between row groups, LBO between the two K halves),
+// (8 rows x 16 bytes per core matrix, SBO = 128 B between row groups, LBO between the two K halves; the B
+// operands WB and DG as l1_wb_offset / l1_dg_offset in common.cuh state it),
 // so a pipeline stage is filled by 1-D bulk async copies (UBLKCP) with no tensor map.  The observations
 // - the only operand that does not fit in L2 - are kept in HBM ONCE, as plain fp32 in that order.
 //
@@ -126,7 +127,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) l1_forward_tc_kernel(const floa
     {                  // ---------------- MMA issuer: the whole warp walks the loop, one elected lane issues
       // instruction descriptor (cute/arch/mma_sm100_desc.hpp InstrDescriptor): D=F32, A=B=TF32, K-major both
       const uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(nu >> 3) << 17) | ((TC_M >> 4) << 24);
-      const uint32_t lboB = nu * 4 * 4;   // bytes between the two K halves
+      const uint32_t lboB = nu * 4 * 4;   // bytes between the two K halves (l1_wb_offset)
       const uint32_t desc_hi = (uint32_t)(umma_desc(0, 0, 128) >> 32);
       const uint32_t dB0 = umma_desc_lo(smem_u32(stages) + offB, lboB);
       uint32_t tcount = 0;
@@ -238,8 +239,9 @@ __global__ void __launch_bounds__(TC_THREADS, 1) l1_forward_tc_kernel(const floa
 // part1[slab][f][n] = sum_{t in slab} X[t][f] * delta1[t][n]  on the tensor cores:
 // D[128 features x NU] += A[128 x 8 timesteps] . B[NU x 8 timesteps]^T, K = timesteps.
 //   XG: [tg = t/8][ftile][khalf][fgroup 16][8 features][4 timesteps]  raw fp32 (split by the converter warps)
-//   DG: [tg][khalf][ngroup NU/8][8][4 timesteps]  raw fp32 delta_1 (written by the reverse sweep: fvp_tc_kernel,
-//       chain_bwd_kernel or mid_backward_kernel; split into (hi, lo) in shared memory by the converter warps)
+//   DG: [tg][khalf][ngroup NU/8][8][4 timesteps]  raw fp32 delta_1 (l1_dg_offset; written by the reverse sweep:
+//       fvp_tc_kernel, chain_bwd_kernel, mid_backward_kernel or lw_dg_kernel; split into (hi, lo) in shared memory
+//       by the converter warps)
 // One CTA accumulates a whole slab (<= 1024 timesteps) for all feature tiles in TMEM (ftiles x
 // acc_cols columns), then the epilogue warps store the fp32 partial that reduce_partials_kernel sums
 // in fp64.  Same warp roles and stage ring as the forward kernel.
@@ -305,7 +307,7 @@ __global__ void __launch_bounds__(TC_THREADS, 1) l1_grad_tc_kernel(const float* 
     }
   } else if (warp == 1) {   // MMA issuer: the whole warp walks the loop, one elected lane issues
     // delta_1, the B operand, is K-major: nu x 8 timesteps per stage, hi block then lo block, each
-    // [khalf][ngroup nu/8][8 n][4 t] (LBO = the K halves, SBO = 8-row groups)
+    // [khalf][ngroup nu/8][8 n][4 t] (l1_dg_offset: LBO = the K halves, SBO = 8-row groups)
     const uint32_t idesc = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(nu >> 3) << 17) | ((TC_M >> 4) << 24);
     const uint32_t lboB = nu * 4 * 4;
     const uint32_t desc_hi = (uint32_t)(umma_desc(0, 0, 128) >> 32);

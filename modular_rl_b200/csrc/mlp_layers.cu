@@ -18,14 +18,12 @@
 // deltas and R-activations live in two ping-pong buffers of [n_tiles + 1][max width][LDT].  All sums run in a
 // fixed order (no atomics), so a repeated call is bit-identical.
 //
-// The head code restates the per-row formulas of mid_forward_kernel / mid_backward_kernel (one thread per
-// timestep); it is duplicated rather than shared so that the mid_* kernels compile exactly as before.
+// The heads are the row functions of heads.cuh that mid_forward_kernel / mid_backward_kernel call.
 #include "common.cuh"
+#include "heads.cuh"
 #include "kernels.h"
 #include "mma_tf32.cuh"
 
-#define LW_LOG_2PIE 2.8378770664093453f
-#define LW_MAX_DOUT 64
 #define LW_THREADS 256   // 8 warps: a 64-timestep x 64-column block, one 32 x 16 job per warp
 #define LW_COLS 64       // output columns per GEMM CTA (one weight panel)
 #define LW_LDP 72        // panel row stride in shared memory: conflict-free B-fragment loads
@@ -217,7 +215,7 @@ __global__ void lw_layer1_kernel(const float* __restrict__ Z, const float* __res
   O[tile * ldo + e] = H ? dact_from_h<ACT>(H[tile * ldh + e]) * z : act_fn<ACT>(z);
 }
 
-// delta_1 -> DG (the raw fp32 operand of l1_grad_tc_kernel, same order as mid_backward_kernel writes it)
+// delta_1 -> DG (the raw fp32 operand of l1_grad_tc_kernel, l1_dg_offset)
 __global__ void lw_dg_kernel(const float* __restrict__ D1, long long ldd, int n1, int nu, float* DG, int n_tiles) {
   const long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x;
   if (i >= (long long)n_tiles * 16 * nu) return;
@@ -225,78 +223,29 @@ __global__ void lw_dg_kernel(const float* __restrict__ D1, long long ldd, int n1
   const int rem = (int)(i % (16 * nu)), tq = rem / nu, n = rem % nu;   // timesteps 4*tq .. +3, column n
   float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
   if (n < n1) v = *reinterpret_cast<const float4*>(D1 + tile * ldd + n * MRL_LDT + 4 * tq);
-  float* base = DG + ((size_t)tile * 8 + (tq >> 1)) * (nu * 8) + (tq & 1) * (nu * 4) + (n >> 3) * 32 + (n & 7) * 4;
-  *reinterpret_cast<float4*>(base) = v;
+  *reinterpret_cast<float4*>(DG + l1_dg_offset((size_t)tile * 8 + (tq >> 1), tq & 1, n, nu)) = v;
 }
 
-// ---- heads: one thread per timestep, one CTA per slab
+// ---- heads (heads.cuh): one thread per timestep, one CTA per slab; sigma, log sigma and 1/sigma^2 staged per CTA
 template <int HEAD>
 __global__ void __launch_bounds__(MRL_TILE, 1) lw_head_fwd_kernel(NetGeom g, MidFwdArgs a) {
   __shared__ double red[32];
+  __shared__ float sig[MRL_MAX_DOUT], logsig[MRL_MAX_DOUT];
   const int r = threadIdx.x, L = g.L, dL = g.d[L];
   const int slab = blockIdx.x;
   const int t0 = slab * a.slab_tiles, t1 = min(t0 + a.slab_tiles, a.n_tiles);
+  if (HEAD == MRL_HEAD_GAUSS && r < dL) {
+    const float ls = a.img[g.off_pm_logstd + r];
+    logsig[r] = ls;
+    sig[r] = expf(ls);
+  }
+  __syncthreads();
   double s_surr = 0.0, s_kl = 0.0, s_ent = 0.0;
   for (int tile = t0; tile < t1; ++tile) {
     const bool valid = (long long)tile * MRL_TILE + r < a.N;
     float* headbuf = a.cache + ((size_t)tile * g.act_rows + g.off_act[L]) * MRL_LDT;
     const float* aux = a.aux ? a.aux + (size_t)tile * g.naux * MRL_LDT + r : nullptr;
-    if (HEAD == MRL_HEAD_GAUSS) {
-      if (aux) {
-        const float adv = aux[0];
-        float dl = 0.f, kl = 0.f, sls = 0.f;
-        for (int j = 0; j < dL; ++j) {
-          const float ls = a.img[g.off_pm_logstd + j], sg = expf(ls);
-          const float mu = headbuf[j * MRL_LDT + r];
-          const float ac = aux[(1 + j) * MRL_LDT];
-          const float m0 = aux[(1 + dL + j) * MRL_LDT];
-          const float s0 = aux[(1 + 2 * dL + j) * MRL_LDT];
-          const float t = (ac - mu) / sg, tt0 = (ac - m0) / s0;
-          dl += -0.5f * (t - tt0) * (t + tt0) - log1pf((sg - s0) / s0);
-          const float dm = m0 - mu;
-          const float den = a.reverse_kl ? s0 : sg;
-          const float u = (a.reverse_kl ? (sg - s0) : (s0 - sg)) / den;
-          kl += u_minus_log1p(u) + 0.5f * (u * u + (dm / den) * (dm / den));
-          sls += ls;
-        }
-        if (valid) {
-          s_surr += (double)(expf(dl) * adv);
-          s_kl += (double)kl;
-          s_ent += (double)(sls + 0.5f * LW_LOG_2PIE * dL);
-        }
-      }
-    } else if (HEAD == MRL_HEAD_CAT) {
-      float m = -INFINITY;
-      for (int j = 0; j < dL; ++j) m = fmaxf(m, headbuf[j * MRL_LDT + r]);
-      float s = 0.f;
-      for (int j = 0; j < dL; ++j) {
-        const float e = expf(headbuf[j * MRL_LDT + r] - m);
-        headbuf[j * MRL_LDT + r] = e;
-        s += e;
-      }
-      const float inv = 1.f / s;
-      float kl = 0.f, ent = 0.f, pa = 1.f, p0a = 1.f;
-      const int ai = aux ? (int)aux[1 * MRL_LDT] : 0;
-      for (int j = 0; j < dL; ++j) {
-        const float p = headbuf[j * MRL_LDT + r] * inv;
-        headbuf[j * MRL_LDT + r] = p;
-        if (aux) {
-          const float p0 = aux[(2 + j) * MRL_LDT];
-          const float q = a.reverse_kl ? p : p0, w = a.reverse_kl ? p0 : p;
-          kl += q * u_minus_log1p((w - q) / q) - (w - q);
-          ent -= p * logf(p);
-          if (j == ai) { pa = p; p0a = p0; }
-        }
-      }
-      if (aux && valid) {
-        s_surr += (double)((pa / p0a) * aux[0]);
-        s_kl += (double)kl;
-        s_ent += (double)ent;
-      }
-    } else if (aux && valid) {   // value head: squared error against the target row
-      const float df = aux[0] - headbuf[r];
-      s_surr += (double)df * (double)df;
-    }
+    head_fwd_row<HEAD>(headbuf, aux, r, dL, valid, a.reverse_kl, sig, logsig, s_surr, s_kl, s_ent);
     if (a.head_out && valid)
       for (int j = 0; j < dL; ++j) a.head_out[((size_t)tile * MRL_TILE + r) * dL + j] = headbuf[j * MRL_LDT + r];
   }
@@ -311,92 +260,31 @@ __global__ void __launch_bounds__(MRL_TILE, 1) lw_head_fwd_kernel(NetGeom g, Mid
   }
 }
 
-// delta_L (un-normalised; 1/N is applied by the slab reduce) into E, the logstd partial (gradient mode, DiagGauss)
+// delta_L (Fvp: the metric applied to Rz_L) into E, the logstd partial (gradient mode, DiagGauss)
 template <int HEAD, int MODE>
 __global__ void __launch_bounds__(MRL_TILE, 1) lw_head_bwd_kernel(NetGeom g, MidBwdArgs a, float* E, long long lde) {
-  __shared__ float GL[LW_MAX_DOUT * MRL_TILE];
+  __shared__ float GL[MRL_MAX_DOUT * MRL_TILE];
+  __shared__ float sig[MRL_MAX_DOUT], ivar[MRL_MAX_DOUT];
   const int r = threadIdx.x, L = g.L, dL = g.d[L];
   const int slab = blockIdx.x;
   const int t0 = slab * a.slab_tiles, t1 = min(t0 + a.slab_tiles, a.n_tiles);
   const bool gl_on = MODE == MRL_MODE_GRAD && HEAD == MRL_HEAD_GAUSS;
   if (gl_on)
     for (int j = 0; j < dL; ++j) GL[j * MRL_TILE + r] = 0.f;
+  if (HEAD == MRL_HEAD_GAUSS && r < dL) {
+    const float ls = a.img[g.off_pm_logstd + r];
+    sig[r] = expf(ls);
+    ivar[r] = expf(-2.f * ls);
+  }
+  __syncthreads();
   double c_s = 1.0, c_k = 0.0;
   if (MODE == MRL_MODE_GRAD && a.coef) { c_s = a.coef[0]; c_k = a.coef[1]; }
   const float cs = (float)c_s, ck = (float)c_k;
   for (int tile = t0; tile < t1; ++tile) {
     const bool valid = (long long)tile * MRL_TILE + r < a.N;
     const float* Hh = a.cache + ((size_t)tile * g.act_rows + g.off_act[L]) * MRL_LDT;
-    float* EH = E + (size_t)tile * lde;   // Fvp: holds Rz_L, replaced by the metric applied to it
     const float* aux = a.aux ? a.aux + (size_t)tile * g.naux * MRL_LDT + r : nullptr;
-    if (MODE == MRL_MODE_FVP) {
-      if (HEAD == MRL_HEAD_GAUSS) {          // M = diag(1/sigma^2) on the mean block
-        for (int j = 0; j < dL; ++j)
-          EH[j * MRL_LDT + r] = valid ? EH[j * MRL_LDT + r] * expf(-2.f * a.img[g.off_pm_logstd + j]) : 0.f;
-      } else if (HEAD == MRL_HEAD_CAT) {     // M = diag(p) - p p^T
-        float s = 0.f;
-        for (int j = 0; j < dL; ++j) s += Hh[j * MRL_LDT + r] * EH[j * MRL_LDT + r];
-        for (int j = 0; j < dL; ++j) {
-          const float p = Hh[j * MRL_LDT + r];
-          EH[j * MRL_LDT + r] = valid ? p * (EH[j * MRL_LDT + r] - s) : 0.f;
-        }
-      } else {
-        for (int j = 0; j < dL; ++j)
-          if (!valid) EH[j * MRL_LDT + r] = 0.f;
-      }
-    } else if (!valid) {
-      for (int j = 0; j < dL; ++j) EH[j * MRL_LDT + r] = 0.f;   // padded timesteps contribute nothing
-    } else if (HEAD == MRL_HEAD_GAUSS) {
-      const float adv = aux[0];
-      float dl = 0.f;
-      for (int j = 0; j < dL; ++j) {
-        const float sg = expf(a.img[g.off_pm_logstd + j]);
-        const float mu = Hh[j * MRL_LDT + r];
-        const float ac = aux[(1 + j) * MRL_LDT];
-        const float m0 = aux[(1 + dL + j) * MRL_LDT];
-        const float s0 = aux[(1 + 2 * dL + j) * MRL_LDT];
-        const float t = (ac - mu) / sg, tt0 = (ac - m0) / s0;
-        dl += -0.5f * (t - tt0) * (t + tt0) - log1pf((sg - s0) / s0);
-      }
-      const float w = -expf(dl) * adv * cs;
-      for (int j = 0; j < dL; ++j) {
-        const float ls = a.img[g.off_pm_logstd + j], sg = expf(ls), iv = expf(-2.f * ls);
-        const float mu = Hh[j * MRL_LDT + r];
-        const float ac = aux[(1 + j) * MRL_LDT];
-        const float m0 = aux[(1 + dL + j) * MRL_LDT];
-        const float s0 = aux[(1 + 2 * dL + j) * MRL_LDT];
-        const float t2 = (ac - mu) * (ac - mu) * iv;
-        float dkl_dmu, dkl_dls;
-        if (!a.reverse_kl) {
-          dkl_dmu = (mu - m0) * iv;
-          dkl_dls = ((sg - s0) * (sg + s0) - (m0 - mu) * (m0 - mu)) * iv;   // 1 - (s0^2+dm^2)/s1^2
-        } else {
-          const float i0 = 1.f / (s0 * s0);
-          dkl_dmu = (mu - m0) * i0;
-          dkl_dls = (sg - s0) * (sg + s0) * i0;                              // -1 + s1^2/s0^2
-        }
-        EH[j * MRL_LDT + r] = w * (ac - mu) * iv + ck * dkl_dmu;
-        GL[j * MRL_TILE + r] += w * (t2 - 1.f) + ck * dkl_dls;
-      }
-    } else if (HEAD == MRL_HEAD_CAT) {
-      const float adv = aux[0];
-      const int ai = (int)aux[1 * MRL_LDT];
-      const float pa = Hh[ai * MRL_LDT + r], p0a = aux[(2 + ai) * MRL_LDT];
-      const float w = -(pa / p0a) * adv * cs;
-      float klrow = 0.f;
-      if (a.reverse_kl)
-        for (int j = 0; j < dL; ++j) {
-          const float p = Hh[j * MRL_LDT + r];
-          klrow += p * logf(p / aux[(2 + j) * MRL_LDT]);
-        }
-      for (int j = 0; j < dL; ++j) {
-        const float p = Hh[j * MRL_LDT + r], p0 = aux[(2 + j) * MRL_LDT];
-        const float dk = a.reverse_kl ? p * (logf(p / p0) - klrow) : (p - p0);
-        EH[j * MRL_LDT + r] = w * ((j == ai ? 1.f : 0.f) - p) + ck * dk;
-      }
-    } else {
-      EH[r] = 2.f * (Hh[r] - aux[0]);   // d/dpred of (y - pred)^2
-    }
+    head_bwd_row<HEAD, MODE>(Hh, E + (size_t)tile * lde, GL, aux, r, dL, valid, a.reverse_kl, cs, ck, sig, ivar);
   }
   if (HEAD == MRL_HEAD_GAUSS) {   // logstd partial: the per-timestep columns summed (zero in Fvp mode)
     __syncthreads();

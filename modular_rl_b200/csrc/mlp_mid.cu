@@ -12,12 +12,10 @@
 //   mid_backward_kernel<GRAD> : dL/dz_L from the head, reverse sweep         trpo.py:43, ppo.py:47-49
 //   mid_backward_kernel<FVP>  : R-forward (Pearlmutter), Fisher metric, reverse sweep  trpo.py:45-58
 #include "common.cuh"
+#include "heads.cuh"
 #include "kernels.h"
 #include "mma_tf32.cuh"
 
-#define LOG_2PI 1.8378770664093453f
-#define LOG_2PIE 2.8378770664093453f
-#define MAX_DOUT 64
 #ifndef MRL_BWD_THREADS
 #define MRL_BWD_THREADS 512   // reverse-sweep kernel: 16 warps hide the LDS/MMA latencies of the small tiles
 #endif
@@ -156,7 +154,7 @@ __global__ void __launch_bounds__(MRL_MID_THREADS, 1) mid_forward_kernel(NetGeom
   float* img = smem;
   float* act = img + g.bw_floats;
   __shared__ double red[32];
-  __shared__ float sig[MAX_DOUT], logsig[MAX_DOUT];
+  __shared__ float sig[MRL_MAX_DOUT], logsig[MRL_MAX_DOUT];
   const Lane ln;
   const int tid = threadIdx.x;
   const int L = g.L, dL = g.d[L];
@@ -213,71 +211,8 @@ __global__ void __launch_bounds__(MRL_MID_THREADS, 1) mid_forward_kernel(NetGeom
     }
     // ---- head: one thread per timestep
     if (tid < MRL_TILE) {
-      const int r = tid;
-      const bool valid = r < nvalid;
-      const float* aux = a.aux ? a.aux + (size_t)tile * g.naux * MRL_LDT + r : nullptr;
-      if (HEAD == MRL_HEAD_GAUSS) {
-        if (aux) {
-          const float adv = aux[0];
-          float dl = 0.f, kl = 0.f, sls = 0.f;
-          for (int j = 0; j < dL; ++j) {
-            const float mu = headbuf[j * MRL_LDT + r];
-            const float ac = aux[(1 + j) * MRL_LDT];
-            const float m0 = aux[(1 + dL + j) * MRL_LDT];
-            const float s0 = aux[(1 + 2 * dL + j) * MRL_LDT];
-            const float sg = sig[j];
-            const float t = (ac - mu) / sg, t0 = (ac - m0) / s0;
-            const float lr = log1pf((sg - s0) / s0);         // log(sigma/sigma0)
-            dl += -0.5f * (t - t0) * (t + t0) - lr;           // logp - oldlogp, term by term
-            const float dm = m0 - mu;
-            // log(s1/s0) + (s0^2 + dm^2)/(2 s1^2) - 1/2, with the s0~s1 cancellation taken analytically
-            // = g(u) + u^2/2 + dm^2/(2 s1^2), u = (s0-s1)/s1   (reverse: roles of s0, s1 swapped, ppo.py:40-41)
-            const float den = a.reverse_kl ? s0 : sg;
-            const float u = (a.reverse_kl ? (sg - s0) : (s0 - sg)) / den;
-            kl += u_minus_log1p(u) + 0.5f * (u * u + (dm / den) * (dm / den));
-            sls += logsig[j];
-          }
-          if (valid) {
-            s_surr += (double)(expf(dl) * adv);
-            s_kl += (double)kl;
-            s_ent += (double)(sls + 0.5f * LOG_2PIE * dL);
-          }
-        }
-      } else if (HEAD == MRL_HEAD_CAT) {
-        float m = -INFINITY;
-        for (int j = 0; j < dL; ++j) m = fmaxf(m, headbuf[j * MRL_LDT + r]);
-        float s = 0.f;
-        for (int j = 0; j < dL; ++j) {
-          const float e = expf(headbuf[j * MRL_LDT + r] - m);
-          headbuf[j * MRL_LDT + r] = e;
-          s += e;
-        }
-        const float inv = 1.f / s;
-        float kl = 0.f, ent = 0.f, pa = 1.f, p0a = 1.f;
-        const int ai = aux ? (int)aux[1 * MRL_LDT] : 0;
-        for (int j = 0; j < dL; ++j) {
-          const float p = headbuf[j * MRL_LDT + r] * inv;
-          headbuf[j * MRL_LDT + r] = p;
-          if (aux) {
-            const float p0 = aux[(2 + j) * MRL_LDT];
-            // q log(q/w) = q g(v) - (w - q), v = (w-q)/q : no cancellation between the terms of the sum
-            const float q = a.reverse_kl ? p : p0, w = a.reverse_kl ? p0 : p;
-            kl += q * u_minus_log1p((w - q) / q) - (w - q);
-            ent -= p * logf(p);
-            if (j == ai) { pa = p; p0a = p0; }
-          }
-        }
-        if (aux && valid) {
-          s_surr += (double)((pa / p0a) * aux[0]);
-          s_kl += (double)kl;
-          s_ent += (double)ent;
-        }
-      } else {  // value head: squared error against the target row
-        if (aux && valid) {
-          const float df = aux[0] - headbuf[r];
-          s_surr += (double)df * (double)df;
-        }
-      }
+      const float* aux = a.aux ? a.aux + (size_t)tile * g.naux * MRL_LDT + tid : nullptr;
+      head_fwd_row<HEAD>(headbuf, aux, tid, dL, tid < nvalid, a.reverse_kl, sig, logsig, s_surr, s_kl, s_ent);
     }
     __syncthreads();
     if (a.cache) copy_f4(a.cache + (size_t)tile * g.act_rows * MRL_LDT, act, g.act_rows * MRL_LDT);
@@ -311,7 +246,7 @@ __global__ void __launch_bounds__(MRL_BWD_THREADS, 1) mid_backward_kernel(NetGeo
   const int gl_floats = (MODE == MRL_MODE_GRAD && HEAD == MRL_HEAD_GAUSS) ? g.d[g.L] * MRL_TILE : 0;
   float* H = GL + gl_floats;
   float* E = H + g.act_rows * MRL_LDT;
-  __shared__ float sig[MAX_DOUT], ivar[MAX_DOUT];
+  __shared__ float sig[MRL_MAX_DOUT], ivar[MRL_MAX_DOUT];
   const Lane ln;
   const int tid = threadIdx.x;
   const int L = g.L, dL = g.d[L];
@@ -392,77 +327,8 @@ __global__ void __launch_bounds__(MRL_BWD_THREADS, 1) mid_backward_kernel(NetGeo
     // ---- head: delta_L (un-normalised; 1/N is applied by the slab reduce)
     const bool head_folded = (MODE == MRL_MODE_FVP && HEAD == MRL_HEAD_GAUSS && L > 1);
     if (!head_folded && tid < MRL_TILE) {
-      const int r = tid;
-      const bool valid = r < nvalid;
-      const float* aux = a.aux ? a.aux + (size_t)tile * g.naux * MRL_LDT + r : nullptr;
-      if (MODE == MRL_MODE_FVP) {
-        if (HEAD == MRL_HEAD_GAUSS) {          // M = diag(1/sigma^2) on the mean block
-          for (int j = 0; j < dL; ++j) EH[j * MRL_LDT + r] = valid ? EH[j * MRL_LDT + r] * ivar[j] : 0.f;
-        } else if (HEAD == MRL_HEAD_CAT) {     // M = diag(p) - p p^T
-          float s = 0.f;
-          for (int j = 0; j < dL; ++j) s += Hh[j * MRL_LDT + r] * EH[j * MRL_LDT + r];
-          for (int j = 0; j < dL; ++j) {
-            const float p = Hh[j * MRL_LDT + r];
-            EH[j * MRL_LDT + r] = valid ? p * (EH[j * MRL_LDT + r] - s) : 0.f;
-          }
-        } else {
-          for (int j = 0; j < dL; ++j)
-            if (!valid) EH[j * MRL_LDT + r] = 0.f;
-        }
-      } else if (!valid) {
-        for (int j = 0; j < dL; ++j) EH[j * MRL_LDT + r] = 0.f;   // padded timesteps contribute nothing
-      } else {
-        if (HEAD == MRL_HEAD_GAUSS) {
-          const float adv = aux[0];
-          float dl = 0.f;
-          for (int j = 0; j < dL; ++j) {
-            const float mu = Hh[j * MRL_LDT + r];
-            const float ac = aux[(1 + j) * MRL_LDT];
-            const float m0 = aux[(1 + dL + j) * MRL_LDT];
-            const float s0 = aux[(1 + 2 * dL + j) * MRL_LDT];
-            const float t = (ac - mu) / sig[j], t0 = (ac - m0) / s0;
-            dl += -0.5f * (t - t0) * (t + t0) - log1pf((sig[j] - s0) / s0);
-          }
-          const float w = -expf(dl) * adv * cs;
-          for (int j = 0; j < dL; ++j) {
-            const float mu = Hh[j * MRL_LDT + r];
-            const float ac = aux[(1 + j) * MRL_LDT];
-            const float m0 = aux[(1 + dL + j) * MRL_LDT];
-            const float s0 = aux[(1 + 2 * dL + j) * MRL_LDT];
-            const float iv = ivar[j];
-            const float t2 = (ac - mu) * (ac - mu) * iv;
-            float dkl_dmu, dkl_dls;
-            if (!a.reverse_kl) {
-              dkl_dmu = (mu - m0) * iv;
-              dkl_dls = ((sig[j] - s0) * (sig[j] + s0) - (m0 - mu) * (m0 - mu)) * iv;  // 1 - (s0^2+dm^2)/s1^2
-            } else {
-              const float i0 = 1.f / (s0 * s0);
-              dkl_dmu = (mu - m0) * i0;
-              dkl_dls = (sig[j] - s0) * (sig[j] + s0) * i0;                             // -1 + s1^2/s0^2
-            }
-            EH[j * MRL_LDT + r] = w * (ac - mu) * iv + ck * dkl_dmu;
-            GL[j * MRL_TILE + r] += w * (t2 - 1.f) + ck * dkl_dls;
-          }
-        } else if (HEAD == MRL_HEAD_CAT) {
-          const float adv = aux[0];
-          const int ai = (int)aux[1 * MRL_LDT];
-          const float pa = Hh[ai * MRL_LDT + r], p0a = aux[(2 + ai) * MRL_LDT];
-          const float w = -(pa / p0a) * adv * cs;
-          float klrow = 0.f;
-          if (a.reverse_kl)
-            for (int j = 0; j < dL; ++j) {
-              const float p = Hh[j * MRL_LDT + r];
-              klrow += p * logf(p / aux[(2 + j) * MRL_LDT]);
-            }
-          for (int j = 0; j < dL; ++j) {
-            const float p = Hh[j * MRL_LDT + r], p0 = aux[(2 + j) * MRL_LDT];
-            const float dk = a.reverse_kl ? p * (logf(p / p0) - klrow) : (p - p0);
-            EH[j * MRL_LDT + r] = w * ((j == ai ? 1.f : 0.f) - p) + ck * dk;
-          }
-        } else {
-          EH[r] = 2.f * (Hh[r] - aux[0]);   // d/dpred of (y - pred)^2
-        }
-      }
+      const float* aux = a.aux ? a.aux + (size_t)tile * g.naux * MRL_LDT + tid : nullptr;
+      head_bwd_row<HEAD, MODE>(Hh, EH, GL, aux, tid, dL, tid < nvalid, a.reverse_kl, cs, ck, sig, ivar);
     }
     if (!head_folded) __syncthreads();
     // ---- reverse sweep: layers L..2 (weights in shared memory)
@@ -502,8 +368,7 @@ __global__ void __launch_bounds__(MRL_BWD_THREADS, 1) mid_backward_kernel(NetGeo
           const int tq = i / nu, n = i % nu;       // timesteps 4*tq .. +3 of this tile
           float4 v = make_float4(0.f, 0.f, 0.f, 0.f);
           if (n < n1) v = *reinterpret_cast<const float4*>(D1 + n * MRL_LDT + 4 * tq);
-          float* base = a.DG + ((size_t)tile * 8 + (tq >> 1)) * (nu * 8) + (tq & 1) * (nu * 4) + (n >> 3) * 32 + (n & 7) * 4;
-          *reinterpret_cast<float4*>(base) = v;
+          *reinterpret_cast<float4*>(a.DG + l1_dg_offset((size_t)tile * 8 + (tq >> 1), tq & 1, n, nu)) = v;
         }
       }
     }

@@ -1,10 +1,11 @@
 """The delta_1 hand-off to the layer-1 gradient GEMM, checked on every kernel that writes it.
 
 The reverse sweep stores delta_1 (the layer-1 error) in `DG` as raw fp32 in the UMMA K-major order, and
-l1_grad_tc_kernel splits it into the (hi, lo) TF32 pair in shared memory.  Three kernels write `DG`:
+l1_grad_tc_kernel splits it into the (hi, lo) TF32 pair in shared memory.  Four kernels write `DG`:
 chain_bwd_kernel (gradient of the instantiated chain shapes, e.g. Humanoid), fvp_tc_kernel (Fisher-vector
-product of tanh nets) and mid_backward_kernel (everything else).  Each case below routes the gradient and
-the Fvp to a different pair of them and compares the layer-1 weight and bias blocks with the float64
+product of tanh nets), lw_dg_kernel (nets too wide for the fused kernels, covered by test_gpu_wide_nets.py)
+and mid_backward_kernel (everything else).  Each case below routes the gradient and the Fvp to a different
+pair of the other three and compares the layer-1 weight and bias blocks with the float64
 oracle.  N is not a multiple of 8 or 128, so the last 8-timestep group is partly padding.  The calls are
 interleaved (gradient, Fvp, gradient, Fvp): each writer must overwrite everything the other left in the
 shared buffer, so the repeated calls have to be bit-identical.
