@@ -262,6 +262,40 @@ int mrl_rollout_run_population(mrl_rollout* r, int n_layers, const int* dims, in
 int mrl_rollout_read(mrl_rollout* r, int* lengths, unsigned char* terminated, double* obs, void* act, float* prob,
                      double* reward, double* states);
 
+/* ---------------------------------------------------------------- cross-entropy search on the device (cem.py:10-50)
+ * The diagonal-Gaussian search distribution of the noisy cross-entropy method, resident on the device: the draw of a
+ * generation's candidates and the refit of mean and variance to its elite (cem.py:10-50; here modular_rl_b200/cem.py
+ * _GaussianSearch.draw / refit) run as kernels, so the candidates never cross to the host.  The normals come from
+ * Philox4x32-10 (DESIGN.md 4b "Device search"), not from numpy's generator, so a run differs from the host search.
+ *   mrl_cem_search_create: P parameters (the Dense kernels and biases of a DeterministicAgent, no logstd), M members
+ *     (1..mrl_rollout_max_envs(): one population round), candidate rows of stride ld floats (ld >= P, a multiple of 4:
+ *     16-byte rows, padding columns 0).  Holds mean and var (float64 [P], double-buffered), dev (float64 [P]), the rows
+ *     (float32 [M x ld]) and M scores.  Mean and var start unset: set both before the first draw.
+ *   mrl_cem_search_set_mean / _set_var / _get_mean / _get_var: float64 [P] where `loc` says (MRL_DEVICE: memory of the
+ *     handle's device).  A get to the host synchronises `stream`.  A set discards the last draw (refit needs a new one).
+ *   mrl_cem_search_draw: one launch.  dev[j] = sqrt(var[j] + extra_var * noise_left) with _GaussianSearch.draw's
+ *     rounding; row m = float32(mean + dev * z_m), z_m the normals of member m under the key `seed` (the generation's
+ *     round seed, which run_cem_algorithm also passes to mrl_rollout_run_population).  dev_out (may be NULL) receives
+ *     dev where `loc` says; to the host it synchronises `stream`.
+ *   mrl_cem_search_rows: the device pointer and stride of the rows, valid until mrl_cem_search_destroy; hand them to
+ *     mrl_rollout_run_population with theta_loc = MRL_DEVICE.
+ *   mrl_cem_search_refit: scores[M] float64 where `loc` says, of the rows of the last draw.  The elite is the last
+ *     `keep` members of a stable ascending sort (np.argsort(scores, kind="stable")[-keep:]: ties go to the higher
+ *     index, NaN sorts last); keep == 0 or keep > M selects all M, as numpy's slice does, and keep < 0 is an error.
+ *     The new mean and var (two-pass, ddof 0) are those of the elite rows recomputed in float64 from the draw's
+ *     counters, summed in ascending (score, index) order.  Two launches, no synchronisation. */
+typedef struct mrl_cem_search mrl_cem_search;
+int mrl_cem_search_create(mrl_cem_search** out, int device, long long P, int M, long long ld);
+int mrl_cem_search_destroy(mrl_cem_search* s);
+int mrl_cem_search_set_mean(mrl_cem_search* s, const double* mean, int loc, void* stream);
+int mrl_cem_search_set_var(mrl_cem_search* s, const double* var, int loc, void* stream);
+int mrl_cem_search_get_mean(mrl_cem_search* s, double* mean, int loc, void* stream);
+int mrl_cem_search_get_var(mrl_cem_search* s, double* var, int loc, void* stream);
+int mrl_cem_search_draw(mrl_cem_search* s, unsigned long long seed, double extra_var, double noise_left,
+                        double* dev_out, int loc, void* stream);
+int mrl_cem_search_rows(mrl_cem_search* s, float** rows, long long* ld);
+int mrl_cem_search_refit(mrl_cem_search* s, const double* scores, int loc, int keep, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -101,6 +101,15 @@ _SIGS = {
                                         C.POINTER(ZFilterCfg), _P, _P, C.POINTER(ZFilterCfg), _P, _P,
                                         _P, _I, _I, C.POINTER(_LL), _P]),
     "mrl_rollout_read": (_I, [_P, _P, _P, _P, _P, _P, _P, _P]),
+    "mrl_cem_search_create": (_I, [C.POINTER(_P), _I, _LL, _I, _LL]),
+    "mrl_cem_search_destroy": (_I, [_P]),
+    "mrl_cem_search_set_mean": (_I, [_P, _P, _I, _P]),
+    "mrl_cem_search_set_var": (_I, [_P, _P, _I, _P]),
+    "mrl_cem_search_get_mean": (_I, [_P, _P, _I, _P]),
+    "mrl_cem_search_get_var": (_I, [_P, _P, _I, _P]),
+    "mrl_cem_search_draw": (_I, [_P, C.c_ulonglong, _D, _D, _P, _I, _P]),
+    "mrl_cem_search_rows": (_I, [_P, C.POINTER(_P), C.POINTER(_LL)]),
+    "mrl_cem_search_refit": (_I, [_P, _P, _I, _I, _P]),
 }
 
 

@@ -4,7 +4,8 @@ modular_rl/cem.py API (cem, CEM_OPTIONS, run_cem_algorithm), SURVEY section 8f r
 Every population member is scored by one rollout with its theta loaded into the device-resident net
 (`agent.set_from_flat`), so the per-step `act` is the same device forward the policy-gradient agents use.
 The search arithmetic itself is a few numpy lines on the host, as in the reference.  With DEVICE_ENVS on, a
-generation of a built-in environment is scored by one device rollout round instead (evaluate_population_device)."""
+generation of a built-in environment is scored by one device rollout round instead (evaluate_population_device), and
+with DEVICE_SEARCH on as well the search runs on the device too (_DeviceGaussianSearch)."""
 from __future__ import print_function
 
 import itertools
@@ -67,12 +68,14 @@ def evaluate_population_device(env, agent, ths, timestep_limit, seed):
     round acts with ths[m] (the argmax of the raw outputs / the raw output), its score is the float64 sum of its raw
     rewards in step order, and the agent's filters take the states after the round.  `seed` keys the Philox stream of
     the round's resets, so start states come from the device and not from numpy's generator (which this call never
-    touches).  Raises before any device call for an environment, filter or policy the device cannot run."""
+    touches).  `ths` may be the DeviceRows of a _DeviceGaussianSearch draw, which the round reads in place.  Raises
+    before any device call for an environment, filter or policy the device cannot run."""
     from .core import _advance_filter, _device_filter, _device_rollouts, _filter_arg, check_device_rollouts
-    from .device import DeviceRollouts
+    from .device import DeviceRollouts, DeviceRows
     kind = check_device_rollouts(env, agent)
     pol = agent.policy
-    ths = np.asarray(ths, np.float32)
+    if not isinstance(ths, DeviceRows):
+        ths = np.asarray(ths, np.float32)
     key = (kind, int(ths.shape[0]), int(timestep_limit), pol.net.device)
     if key not in _device_rollouts:
         _device_rollouts[key] = DeviceRollouts(env, ths.shape[0], timestep_limit, device=pol.net.device)
@@ -112,6 +115,49 @@ class _GaussianSearch(object):
         self.generation += 1
 
 
+# Draw and refit each generation on the device (_DeviceGaussianSearch) instead of with numpy.  Needs DEVICE_ENVS: the
+# candidates stay in device memory and only the population round reads them.  A process setting like DEVICE_ENVS:
+# run_cem.py --device_search.
+DEVICE_SEARCH = False
+
+
+class _DeviceGaussianSearch(object):
+    """_GaussianSearch with the distribution on the device (device.DeviceSearch): `draw` fills the device's candidate
+    rows and returns them as DeviceRows, `refit` ranks the M scores and refits mean and variance there.  The normals of
+    generation g come from the device's Philox stream keyed by seed + g, the round seed evaluate_population_device gets
+    for that generation, so numpy's generator is never touched.  `mean` and `dev` are host float64 copies (the info
+    dict's th and std).  The elite rule is np.argsort(scores, kind="stable")[-keep:] (ties to the higher index, NaN
+    last); the host search's default argsort may pick a different member among tied scores."""
+
+    def __init__(self, mean, initial_std, extra_std, std_decay_time, batch_size, seed, device):
+        from .device import DeviceSearch
+        mean = np.asarray(mean, np.float64)
+        self.search = DeviceSearch(mean.size, batch_size, device)
+        self.search.set_mean(mean)
+        self.search.set_var(np.full(mean.size, 1.0) * initial_std)
+        self.mean = mean
+        self.extra_var = np.square(extra_std)
+        self.decay = float(std_decay_time)
+        self.seed = int(seed)
+        self.generation = 0
+
+    def noise_left(self):
+        return max(1.0 - self.generation / self.decay, 0)
+
+    def draw(self, count):
+        if count != self.search.M:
+            raise ValueError("the device search draws %d candidates per generation, not %d" % (self.search.M, count))
+        self.dev = self.search.draw(self.seed + self.generation, self.extra_var, self.noise_left())
+        return self.search.rows
+
+    def refit(self, candidates, scores, keep):
+        if keep < 0:
+            raise ValueError("elite_frac is negative: round(batch_size * elite_frac) = %d elite members" % keep)
+        self.search.refit(np.asarray(scores, np.float64), keep)
+        self.mean = self.search.get_mean()
+        self.generation += 1
+
+
 def _score(f, ths, pool):
     population = getattr(f, "population", None)
     if population is not None:
@@ -119,11 +165,14 @@ def _score(f, ths, pool):
     return np.array([f(th) for th in ths] if pool is None else pool.map(f, ths))
 
 
-def cem(f, th_mean, batch_size, n_iter, elite_frac, initial_std=1.0, extra_std=0.0, std_decay_time=1.0, pool=None):
+def cem(f, th_mean, batch_size, n_iter, elite_frac, initial_std=1.0, extra_std=0.0, std_decay_time=1.0, pool=None,
+        search=None):
     """Generator of one info dict per iteration - the reference's `cem` signature and info keys (cem.py:10-50):
     keep the round(batch_size * elite_frac) best of each generation and refit the search distribution to them.  An
-    objective that has a `population` attribute is scored with one call for the whole generation."""
-    search = _GaussianSearch(th_mean, initial_std, extra_std, std_decay_time)
+    objective that has a `population` attribute is scored with one call for the whole generation.  `search`: the
+    search distribution, already set up from th_mean and the std options (default: the host _GaussianSearch)."""
+    if search is None:
+        search = _GaussianSearch(th_mean, initial_std, extra_std, std_decay_time)
     keep = int(np.round(batch_size * elite_frac))
     for _ in range(n_iter):
         print("extra var", search.noise_left())
@@ -157,7 +206,11 @@ def run_cem_algorithm(env, agent, usercfg=None, callback=None):
     The host paths draw the environments' resets from numpy's global generator; the device path does not touch it,
     so the search's own randn calls are its only numpy draws.  Start states, scores and therefore later generations
     differ from a host run with the same seed (as with run_pg.py --device_envs); equal seeds give identical device
-    runs."""
+    runs.
+
+    DEVICE_SEARCH on (needs DEVICE_ENVS): the candidates are drawn and the distribution refitted on the device
+    (_DeviceGaussianSearch), the draws of generation g keyed by the same round seed as its rollouts.  numpy's
+    generator is not used at all, and the numbers differ from a host search."""
     cfg = update_default_config(CEM_OPTIONS, usercfg)
     if cfg["std_decay_time"] < 0:
         cfg["std_decay_time"] = cfg["n_iter"] / 2
@@ -168,8 +221,15 @@ def run_cem_algorithm(env, agent, usercfg=None, callback=None):
         raise ValueError("parallel=1 (host population path) and DEVICE_ENVS select different scoring paths; choose one")
     if cfg["parallel"]:
         print("parallel=1: population-batched evaluation (one device forward per step for all candidates)")
+    if DEVICE_SEARCH and not DEVICE_ENVS:
+        raise ValueError("DEVICE_SEARCH draws the candidates into device memory that only DEVICE_ENVS rounds read; "
+                         "set both")
+    if DEVICE_SEARCH and cfg["elite_frac"] < 0:
+        raise ValueError("elite_frac = %g is negative" % cfg["elite_frac"])
     if DEVICE_ENVS:
         print("device_envs: one device rollout round per generation")
+    if DEVICE_SEARCH:
+        print("device_search: candidates drawn and refitted on the device")
     timestep_limit = cfg["timestep_limit"]
 
     def objective(th):
@@ -183,8 +243,12 @@ def run_cem_algorithm(env, agent, usercfg=None, callback=None):
         objective.population = lambda ths: evaluate_population_device(env, agent, ths, timestep_limit, next(seeds))
 
     th_mean = agent.get_flat()
+    search = None
+    if DEVICE_SEARCH:
+        search = _DeviceGaussianSearch(th_mean, cfg["initial_std"], cfg["extra_std"], cfg["std_decay_time"],
+                                       cfg["batch_size"], int(cfg.get("seed", 0)), agent.policy.net.device)
     for info in cem(objective, th_mean, cfg["batch_size"], cfg["n_iter"], cfg["elite_frac"],
-                    cfg["initial_std"], cfg["extra_std"], cfg["std_decay_time"]):
+                    cfg["initial_std"], cfg["extra_std"], cfg["std_decay_time"], search=search):
         if callback is not None:
             callback(info)
         ps = np.linspace(0, 100, 5)

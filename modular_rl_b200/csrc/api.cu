@@ -45,10 +45,11 @@ static int fail(const char* fmt, ...) {
   } while (0)
 
 // ---- optional per-kernel-class timing with CUDA events on the launching stream (bench.py's roofline)
-enum { PK_L1F = 0, PK_MIDF, PK_MIDB_GRAD, PK_MIDB_FVP, PK_L1G, PK_REDUCE, PK_CG, PK_GAE, PK_PACK, PK_ROLLOUT, PK_COUNT };
+enum { PK_L1F = 0, PK_MIDF, PK_MIDB_GRAD, PK_MIDB_FVP, PK_L1G, PK_REDUCE, PK_CG, PK_GAE, PK_PACK, PK_ROLLOUT,
+       PK_CEM_SEARCH, PK_COUNT };
 static const char* kPkNames[PK_COUNT] = {"l1_forward", "mid_forward", "mid_backward_grad", "mid_backward_fvp",
                                          "l1_grad",    "reduce",      "cg_vector",         "gae",
-                                         "pack_params", "rollout"};
+                                         "pack_params", "rollout",    "cem_search"};
 struct Prof {
   bool on = false;
   std::vector<cudaEvent_t> pool;
@@ -1527,5 +1528,135 @@ extern "C" int mrl_rollout_read(mrl_rollout* r, int* lengths, unsigned char* ter
   if (states) memcpy(states, r->h_body + lay.state, (size_t)n * r->sd * 8);
   if (prob) memcpy(prob, r->h_body + lay.prob, (size_t)n * r->pd * 4);
   if (act) memcpy(act, r->h_body + lay.act, (size_t)n * ro_act_width(r) * 4);
+  return 0;
+}
+
+// ======================================================================== cross-entropy search (cem_search.cu)
+struct mrl_cem_search {
+  int device = 0, P = 0, M = 0, cur = 0;          // cur: the buffer of each pair that holds the current mean / var
+  long long ld = 0;
+  unsigned long long seed = 0;                    // of the last draw: the refit recomputes its rows
+  bool drawn = false;
+  DevBuf mean[2], var[2], dev, rows, scores, order;
+};
+
+// ptr must be device memory of `device` when loc == MRL_DEVICE
+static int cs_check_loc(const char* who, const char* what, const void* ptr, int loc, int device) {
+  if (loc != MRL_HOST && loc != MRL_DEVICE) return fail("%s: loc = %d (MRL_HOST or MRL_DEVICE)", who, loc);
+  if (loc == MRL_HOST) return 0;
+  cudaPointerAttributes pa;
+  if (cudaPointerGetAttributes(&pa, ptr) != cudaSuccess) {
+    cudaGetLastError();
+    pa.type = cudaMemoryTypeUnregistered;
+  }
+  if ((pa.type != cudaMemoryTypeDevice && pa.type != cudaMemoryTypeManaged) || pa.device != device)
+    return fail("%s: loc = MRL_DEVICE but %s is not device memory of device %d", who, what, device);
+  return 0;
+}
+
+extern "C" int mrl_cem_search_destroy(mrl_cem_search* s) {
+  if (!s) return 0;
+  cudaSetDevice(s->device);
+  DevBuf* bufs[] = {&s->mean[0], &s->mean[1], &s->var[0], &s->var[1], &s->dev, &s->rows, &s->scores, &s->order};
+  for (DevBuf* d : bufs) d->release();
+  delete s;
+  return 0;
+}
+
+extern "C" int mrl_cem_search_create(mrl_cem_search** out, int device, long long P, int M, long long ld) {
+  const char* who = "mrl_cem_search_create";
+  if (!out) return fail("%s: null output", who);
+  if (P < 1 || P > (1LL << 30)) return fail("%s: P = %lld; the search holds 1..%lld parameters", who, P, 1LL << 30);
+  if (M < 1 || M > RO_MAX_ENVS)
+    return fail("%s: M = %d; a generation is one rollout round of 1..%d members", who, M, RO_MAX_ENVS);
+  if (ld < P || ld % 4) return fail("%s: ld = %lld; rows need ld >= P = %lld and a multiple of 4 (16 B)", who, ld, P);
+  CK(cudaSetDevice(device));
+  mrl_cem_search* s = new mrl_cem_search();
+  s->device = device; s->P = (int)P; s->M = M; s->ld = ld;
+  cudaError_t e = cudaSuccess;
+  auto R = [&](DevBuf& b, size_t bytes) { if (e == cudaSuccess) e = b.reserve(bytes); };
+  R(s->mean[0], P * 8); R(s->mean[1], P * 8); R(s->var[0], P * 8); R(s->var[1], P * 8); R(s->dev, P * 8);
+  R(s->rows, (size_t)M * ld * 4); R(s->scores, (size_t)M * 8); R(s->order, (size_t)M * 4);
+  if (e == cudaSuccess) e = cudaMemset(s->rows.p, 0, (size_t)M * ld * 4);     // the padding columns stay 0
+  if (e != cudaSuccess) {
+    mrl_cem_search_destroy(s);
+    return fail("%s: %s", who, cudaGetErrorString(e));
+  }
+  *out = s;
+  return 0;
+}
+
+// which: 0 mean, 1 var; to_lib: caller -> library
+static int cs_copy(mrl_cem_search* s, int which, bool to_lib, void* x, int loc, void* stream, const char* who) {
+  if (!s || !x) return fail("%s: bad arguments", who);
+  RET(cs_check_loc(who, which ? "var" : "mean", x, loc, s->device));
+  CK(cudaSetDevice(s->device));
+  cudaStream_t st = (cudaStream_t)stream;
+  void* lib = (which ? s->var : s->mean)[s->cur].p;
+  const cudaMemcpyKind kind = loc == MRL_HOST ? (to_lib ? cudaMemcpyHostToDevice : cudaMemcpyDeviceToHost)
+                                              : cudaMemcpyDeviceToDevice;
+  CK(cudaMemcpyAsync(to_lib ? lib : x, to_lib ? x : lib, (size_t)s->P * 8, kind, st));
+  if (loc == MRL_HOST) CK(cudaStreamSynchronize(st));
+  if (to_lib) s->drawn = false;                   // the rows of the last draw no longer follow from mean and dev
+  return 0;
+}
+extern "C" int mrl_cem_search_set_mean(mrl_cem_search* s, const double* mean, int loc, void* stream) {
+  return cs_copy(s, 0, true, (void*)mean, loc, stream, "mrl_cem_search_set_mean");
+}
+extern "C" int mrl_cem_search_set_var(mrl_cem_search* s, const double* var, int loc, void* stream) {
+  return cs_copy(s, 1, true, (void*)var, loc, stream, "mrl_cem_search_set_var");
+}
+extern "C" int mrl_cem_search_get_mean(mrl_cem_search* s, double* mean, int loc, void* stream) {
+  return cs_copy(s, 0, false, mean, loc, stream, "mrl_cem_search_get_mean");
+}
+extern "C" int mrl_cem_search_get_var(mrl_cem_search* s, double* var, int loc, void* stream) {
+  return cs_copy(s, 1, false, var, loc, stream, "mrl_cem_search_get_var");
+}
+
+extern "C" int mrl_cem_search_draw(mrl_cem_search* s, unsigned long long seed, double extra_var, double noise_left,
+                                   double* dev_out, int loc, void* stream) {
+  const char* who = "mrl_cem_search_draw";
+  if (!s) return fail("%s: null handle", who);
+  if (dev_out) RET(cs_check_loc(who, "dev_out", dev_out, loc, s->device));
+  CK(cudaSetDevice(s->device));
+  cudaStream_t st = (cudaStream_t)stream;
+  CKP(PK_CEM_SEARCH, launch_cem_draw(s->mean[s->cur].as<double>(), s->var[s->cur].as<double>(), s->dev.as<double>(),
+                                     s->rows.as<float>(), s->P, s->M, s->ld, extra_var, noise_left, seed, st), 1);
+  s->seed = seed;
+  s->drawn = true;
+  if (dev_out) {
+    CK(cudaMemcpyAsync(dev_out, s->dev.p, (size_t)s->P * 8,
+                       loc == MRL_HOST ? cudaMemcpyDeviceToHost : cudaMemcpyDeviceToDevice, st));
+    if (loc == MRL_HOST) CK(cudaStreamSynchronize(st));
+  }
+  return 0;
+}
+
+extern "C" int mrl_cem_search_rows(mrl_cem_search* s, float** rows, long long* ld) {
+  if (!s || !rows || !ld) return fail("mrl_cem_search_rows: bad arguments");
+  *rows = s->rows.as<float>();
+  *ld = s->ld;
+  return 0;
+}
+
+extern "C" int mrl_cem_search_refit(mrl_cem_search* s, const double* scores, int loc, int keep, void* stream) {
+  const char* who = "mrl_cem_search_refit";
+  if (!s || !scores) return fail("%s: bad arguments", who);
+  if (keep < 0) return fail("%s: keep = %d is negative (elite_frac < 0)", who, keep);
+  if (!s->drawn) return fail("%s: no generation has been drawn (mrl_cem_search_draw)", who);
+  RET(cs_check_loc(who, "scores", scores, loc, s->device));
+  CK(cudaSetDevice(s->device));
+  cudaStream_t st = (cudaStream_t)stream;
+  const int n = (keep == 0 || keep > s->M) ? s->M : keep;      // np.argsort(scores)[-keep:]: [-0:] is every member
+  const double* sc = scores;
+  if (loc == MRL_HOST) {
+    CK(cudaMemcpyAsync(s->scores.p, scores, (size_t)s->M * 8, cudaMemcpyHostToDevice, st));
+    sc = s->scores.as<double>();
+  }
+  const int nxt = s->cur ^ 1;
+  CKP(PK_CEM_SEARCH, launch_cem_rank_refit(sc, s->M, n, s->order.as<int>(), s->mean[s->cur].as<double>(),
+                                           s->dev.as<double>(), s->P, s->seed, s->mean[nxt].as<double>(),
+                                           s->var[nxt].as<double>(), st), 2);
+  s->cur = nxt;
   return 0;
 }

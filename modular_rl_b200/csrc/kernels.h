@@ -196,3 +196,14 @@ void rollout_shape(int N, int* n_ctas, int* per_cta, int* threads);
 size_t rollout_smem_bytes(const RolloutArgs& a, int d0, int dout, bool pop);
 cudaError_t launch_rollout(const RolloutArgs& a, int env, int act, bool pop, int n_ctas, int threads, size_t smem,
                            cudaStream_t st);
+
+// ---- cem_search.cu  (device search distribution of the cross-entropy method)
+// rows[m][0..P) = float32(mean + dev * z[m]) for m < M, dev[j] = sqrt(var[j] + extra_var * noise_left); ld % 4 == 0
+cudaError_t launch_cem_draw(const double* mean, const double* var, double* dev, float* rows, int P, int M,
+                            long long ld, double extra_var, double noise_left, unsigned long long seed,
+                            cudaStream_t st);
+// elite = the last `keep` (1..M) of the stable ascending order of scores[M] (device); mean_out / var_out = their
+// float64 mean and variance, rows recomputed from (mean, dev, seed).  order: int32 [M] scratch.  Two launches.
+cudaError_t launch_cem_rank_refit(const double* scores, int M, int keep, int* order, const double* mean,
+                                  const double* dev, int P, unsigned long long seed, double* mean_out, double* var_out,
+                                  cudaStream_t st);

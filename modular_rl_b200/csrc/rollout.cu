@@ -30,29 +30,13 @@
 // the episode lengths) in the same launch, so the host copies only the collected timesteps.
 #include "common.cuh"
 #include "kernels.h"
+#include "philox.cuh"
 #include "../../include/mrl_b200.h"
 
 #include <cooperative_groups.h>
 namespace cgr = cooperative_groups;
 
 #define RO_KMAX 7   // observation features + the reward, scanned together (Acrobot: 6 + 1)
-
-// ---------------------------------------------------------------------------------------------------- Philox4x32-10
-__device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint32_t k0, uint32_t k1) {
-#pragma unroll
-  for (int i = 0; i < 10; ++i) {
-    if (i) { k0 += 0x9E3779B9u; k1 += 0xBB67AE85u; }
-    const uint32_t lo0 = 0xD2511F53u * c.x, hi0 = __umulhi(0xD2511F53u, c.x);
-    const uint32_t lo1 = 0xCD9E8D57u * c.z, hi1 = __umulhi(0xCD9E8D57u, c.z);
-    c = make_uint4(hi1 ^ c.y ^ k0, lo1, hi0 ^ c.w ^ k1, lo0);
-  }
-  return c;
-}
-// 53-bit uniform in [0, 1) from two words: the high word gives the top 32 bits, the high 21 bits of the low word the rest
-__device__ __forceinline__ double u53(uint32_t hi, uint32_t lo) {
-  return (double)(((unsigned long long)hi << 21) | (lo >> 11)) * 0x1p-53;
-}
-enum { RO_PURPOSE_RESET = 0, RO_PURPOSE_ACTION = 1 };
 
 // ---------------------------------------------------------------------------------------------------- Welford
 struct Wf { double n, m, s; };

@@ -407,14 +407,16 @@ class DeviceRollouts:
     def run_population(self, dims: Sequence[int], activation: str, thetas, seed: int, obfilter=None, rewfilter=None,
                        want_rows: bool = False, want_states: bool = False, stream=None) -> dict:
         """One round in which environment m acts deterministically with its own parameters thetas[m] (the
-        cross-entropy method's population).  thetas: [M, ld] float32, numpy (host) or a torch CUDA tensor (read in
-        place); each row holds the Dense kernels and biases of the net `dims` in the reference's flat order (no logstd
+        cross-entropy method's population).  thetas: [M, ld] float32, numpy (host), a torch CUDA tensor or the
+        DeviceRows of a DeviceSearch draw (both read in place); each row holds the Dense kernels and biases of the net `dims` in the reference's flat order (no logstd
         block), ld >= their count, M <= n_envs.  Filters as `run`.  Returns `returns` (float64 [M], the sum of each
         episode's raw rewards), lengths, terminated, the four filter states, and with want_rows the row arrays of `run`
         (prob: the K raw outputs of a Categorical head, [mean, 1] for DiagGauss).  Members act on the argmax of their
         raw outputs (first maximum) or on the raw output itself, which the environment clips."""
         dims = [int(x) for x in dims]
-        if _is_torch_cuda(thetas):
+        if isinstance(thetas, DeviceRows):
+            keep, th_ptr, loc = thetas, thetas.ptr, L.DEVICE
+        elif _is_torch_cuda(thetas):
             import torch
             keep = thetas.to(torch.float32).contiguous()
             th_ptr, loc = C.c_void_p(keep.data_ptr()), L.DEVICE
@@ -455,6 +457,82 @@ class DeviceRollouts:
         out["ob_state"], out["ob_pushed"] = self._state_out(ost, d), self._state_out(opu, d)
         out["rew_state"], out["rew_pushed"] = self._state_out(rst, 1), self._state_out(rpu, 1)
         return out
+
+
+class DeviceRows:
+    """The float32 candidate rows [M, ld] of a DeviceSearch, in the library's device memory (valid while the search
+    lives).  `__cuda_array_interface__` lets torch read them in place: torch.as_tensor(rows, device="cuda")."""
+
+    def __init__(self, owner, ptr: C.c_void_p, shape, device: int):
+        self._owner, self.ptr, self.shape, self.ndim, self.device = owner, ptr, tuple(shape), 2, device
+
+    @property
+    def __cuda_array_interface__(self):
+        return dict(shape=self.shape, typestr="<f4", data=(self.ptr.value, False), version=2, strides=None)
+
+
+class DeviceSearch:
+    """mrl_cem_search_*: the cross-entropy method's diagonal-Gaussian search distribution on the device.  P parameters,
+    M candidates per generation (at most DeviceRollouts.max_envs()); rows padded to a multiple of 4 floats.  Mean and
+    var are float64 [P]; `draw` writes the candidate rows and returns dev (host float64), `refit` takes the M scores
+    (host array or CUDA tensor) and the elite count."""
+
+    def __init__(self, P: int, M: int, device: Optional[int] = None):
+        if device is None:
+            device = parallel.current_device()
+        self.P, self.M, self.device = int(P), int(M), device
+        self.ld = (self.P + 3) // 4 * 4
+        self._h = C.c_void_p()
+        L.check(L.lib().mrl_cem_search_create(C.byref(self._h), device, self.P, self.M, self.ld))
+        p, ld = C.c_void_p(), C.c_longlong()
+        L.check(L.lib().mrl_cem_search_rows(self._h, C.byref(p), C.byref(ld)))
+        self.rows = DeviceRows(self, p, (self.M, int(ld.value)), device)
+
+    def close(self):
+        if getattr(self, "_h", None):
+            L.lib().mrl_cem_search_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def _set(self, fn, x, stream):
+        k, p, dt, loc, shape = _arg(x, (np.dtype(np.float64),))
+        if dt != L.F64 or int(np.prod(shape)) != self.P:
+            raise ValueError("need float64 [%d], got %s %s" % (self.P, tuple(shape), dt))
+        L.check(fn(self._h, p, loc, stream))
+
+    def set_mean(self, mean, stream=None):
+        self._set(L.lib().mrl_cem_search_set_mean, mean, stream)
+
+    def set_var(self, var, stream=None):
+        self._set(L.lib().mrl_cem_search_set_var, var, stream)
+
+    def get_mean(self, stream=None) -> np.ndarray:
+        out = np.empty(self.P)
+        L.check(L.lib().mrl_cem_search_get_mean(self._h, L.ptr(out), L.HOST, stream))
+        return out
+
+    def get_var(self, stream=None) -> np.ndarray:
+        out = np.empty(self.P)
+        L.check(L.lib().mrl_cem_search_get_var(self._h, L.ptr(out), L.HOST, stream))
+        return out
+
+    def draw(self, seed: int, extra_var: float, noise_left: float, stream=None) -> np.ndarray:
+        """Rows of one generation into self.rows; returns dev = sqrt(var + extra_var * noise_left)."""
+        dev = np.empty(self.P)
+        L.check(L.lib().mrl_cem_search_draw(self._h, int(seed) & 0xFFFFFFFFFFFFFFFF, float(extra_var),
+                                            float(noise_left), L.ptr(dev), L.HOST, stream))
+        return dev
+
+    def refit(self, scores, keep: int, stream=None):
+        k, p, dt, loc, shape = _arg(scores, (np.dtype(np.float64),))
+        if dt != L.F64 or tuple(shape) != (self.M,):
+            raise ValueError("scores must be float64 [%d], got %s" % (self.M, tuple(shape)))
+        L.check(L.lib().mrl_cem_search_refit(self._h, p, loc, int(keep), stream))
 
 
 def population_forward(dims: Sequence[int], activation: str, thetas, obs, device: int = 0) -> np.ndarray:

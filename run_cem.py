@@ -2,7 +2,8 @@
 """Cross-entropy-method driver with the reference's run_cem.py command line (GENERAL_OPTIONS, --env, --agent, --plot,
 the agent's own options, CEM_OPTIONS - run_cem.py:13-30).  Candidates are scored through the device-resident
 deterministic policy; with --parallel 1 the whole population is scored in lockstep by one population-batched forward
-per environment step; with --device_envs (the built-in environments) each generation is one device rollout round.
+per environment step; with --device_envs (the built-in environments) each generation is one device rollout round,
+and with --device_search as well the candidates are drawn and the search distribution refitted on the device.
 
   python run_cem.py --env CartPole-v0 --agent modular_rl.agentzoo.DeterministicAgent --n_iter 10 --batch_size 40
 """
@@ -38,11 +39,20 @@ def parse_cli(argv):
                     help="score each generation in one GPU rollout round, one environment per candidate (built-in "
                          "CartPole, Pendulum, Acrobot, MountainCar and MountainCarContinuous only); resets come from the device's Philox stream, so results differ "
                          "from a host run with the same --seed")
+    ap.add_argument("--device_search", action="store_true",
+                    help="with --device_envs: draw each generation's candidates and refit the search distribution on "
+                         "the GPU; the draws come from the device's Philox stream, not numpy's, so results differ "
+                         "from a run without it")
     first, _ = ap.parse_known_args([a for a in argv if a not in ("-h", "--help")])
     agent_cls = mrl.get_agent_cls(first.agent)
     mrl.update_argument_parser(ap, agent_cls.options)
     mrl.update_argument_parser(ap, mrl.CEM_OPTIONS)
     args = ap.parse_args(argv)
+    if args.device_search:
+        if not args.device_envs:
+            ap.error("--device_search needs --device_envs: only a device rollout round reads candidates in device memory")
+        if args.elite_frac < 0:
+            ap.error("--device_search: --elite_frac is %g; it must not be negative" % args.elite_frac)
     if args.device_envs:
         from modular_rl_b200.device import DeviceRollouts
         from modular_rl_b200.envs import device_kind
@@ -105,6 +115,7 @@ def main(argv=None):
         from modular_rl_b200 import cem, core
         core.check_device_rollouts(env, agent)     # an unsupported filter / policy fails before any rollout
         cem.DEVICE_ENVS = True
+        cem.DEVICE_SEARCH = args.device_search
     hdf, diagnostics = mrl.prepare_h5_file(args) if args.use_hdf else (None, None)
     mrl.run_cem_algorithm(env, agent, callback=IterationLog(args, env, agent, results_dir, hdf, diagnostics), usercfg=cfg)
     if hdf is not None:
