@@ -233,7 +233,8 @@ int mrl_population_forward(int device, int n_layers, const int* dims, int activa
  *     returns[n_members] (host, float64) = the sum of each episode's raw rewards in step order.  Filters as
  *     mrl_rollout_run.  want_rows != 0 records the rows for mrl_rollout_read, the prob row then holding the raw
  *     outputs (Categorical: the K logits; DiagGauss: [mean, 1]); want_states (needs want_rows) the raw states.
- *     Synchronises `stream`; *n_timesteps = timesteps collected. */
+ *     Synchronises `stream`; *n_timesteps = timesteps collected.
+ *   User environments (ids >= 64) are accepted by every call above wherever an env is; see below. */
 #define MRL_ENV_CARTPOLE 0
 #define MRL_ENV_PENDULUM 1
 #define MRL_ENV_ACROBOT 2
@@ -261,6 +262,29 @@ int mrl_rollout_run_population(mrl_rollout* r, int n_layers, const int* dims, in
                                long long* n_timesteps, void* stream);
 int mrl_rollout_read(mrl_rollout* r, int* lengths, unsigned char* terminated, double* obs, void* act, float* prob,
                      double* reward, double* states);
+
+/* ---------------------------------------------------------------- user environments in device rollouts
+ * mrl_rollout_env_compile (host code, no device needed): compiles the rollout kernel for an environment given as CUDA
+ *   source and returns its id (>= 64) in *env_out.  The library wraps `source` in
+ *     template <> struct EnvT<id> { static constexpr int D0 = ob_dim, SD = state_dim, DOUT = n_out, PD = ..., HEAD = head;
+ *                                   <source> };
+ *   and `source` defines, in float64:
+ *     __device__ static void reset(double* s, int env, uint32_t k0, uint32_t k1)   the start state of environment env
+ *     __device__ static void obs(const double* s, double* x)                        its observation x[ob_dim]
+ *     __device__ static bool step(double* s, int action, const float* a, double* reward)   -> terminated
+ *   `action` is the Categorical index, `a` the n_out DiagGauss entries (float32).  reset draws its uniforms with
+ *   reset_uniforms(env, block, k0, k1, &u0, &u1): the pair of Philox counter (env, 0, 0, block) in [0, 1).
+ *   RO_PI is pi.  head: MRL_CATEGORICAL with 1 <= n_out <= 16 classes, or MRL_GAUSS with 1 <= n_out <= 8 entries;
+ *   1 <= ob_dim <= 6 (the per-step filter scan carries the observation entries and the reward); 1 <= state_dim <= 16.
+ *   NVRTC (libnvrtc.so.12, opened on first use) compiles the six (activation, population) instances for sm_100a, in
+ *   seconds of host time; the same (source, shapes) returns the same id without compiling again.  A compile error
+ *   fails with NVRTC's log in mrl_last_error(), its line numbers counted in `source`, whose file name is `name`.
+ *   The kernels load at the first mrl_rollout_create of the id.
+ * mrl_rollout_env_log: the compiler's report (ptxas registers and spills of the six instances) of a user environment,
+ *   NUL-terminated and truncated to len bytes. */
+int mrl_rollout_env_compile(const char* name, const char* source, int ob_dim, int state_dim, int head, int n_out,
+                            int* env_out);
+int mrl_rollout_env_log(int env, char* buf, int len);
 
 /* ---------------------------------------------------------------- cross-entropy search on the device (cem.py:10-50)
  * The diagonal-Gaussian search distribution of the noisy cross-entropy method, resident on the device: the draw of a

@@ -16,7 +16,7 @@ F32, F64, I32, I64 = 0, 1, 2, 3
 GAUSS, CATEGORICAL, VALUE = 0, 1, 2
 ACTIVATIONS = {"tanh": 0, "relu": 1, "sigmoid": 2}
 # envs.py device_kind -> MRL_ENV_CARTPOLE, MRL_ENV_PENDULUM, MRL_ENV_ACROBOT, MRL_ENV_MOUNTAIN_CAR,
-# MRL_ENV_MOUNTAIN_CAR_CONTINUOUS
+# MRL_ENV_MOUNTAIN_CAR_CONTINUOUS (user environments, envs.DeviceEnv, get ids >= 64 from mrl_rollout_env_compile)
 DEVICE_ENVS = {"cartpole": 0, "pendulum": 1, "acrobot": 2, "mountaincar": 3, "mountaincar_continuous": 4}
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
@@ -101,6 +101,8 @@ _SIGS = {
                                         C.POINTER(ZFilterCfg), _P, _P, C.POINTER(ZFilterCfg), _P, _P,
                                         _P, _I, _I, C.POINTER(_LL), _P]),
     "mrl_rollout_read": (_I, [_P, _P, _P, _P, _P, _P, _P, _P]),
+    "mrl_rollout_env_compile": (_I, [C.c_char_p, C.c_char_p, _I, _I, _I, _I, C.POINTER(_I)]),
+    "mrl_rollout_env_log": (_I, [_I, C.c_char_p, _I]),
     "mrl_cem_search_create": (_I, [C.POINTER(_P), _I, _LL, _I, _LL]),
     "mrl_cem_search_destroy": (_I, [_P]),
     "mrl_cem_search_set_mean": (_I, [_P, _P, _I, _P]),

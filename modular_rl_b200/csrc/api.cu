@@ -1273,8 +1273,47 @@ struct mrl_rollout {
 };
 static int ro_head_doubles(int d0) { return 9 + 4 * d0; }
 static int ro_act_width(const mrl_rollout* r) { return r->head == MRL_HEAD_CAT ? 1 : r->dout; }
-static const char* ro_env_names = "MRL_ENV_CARTPOLE, MRL_ENV_PENDULUM, MRL_ENV_ACROBOT, MRL_ENV_MOUNTAIN_CAR or "
-                                  "MRL_ENV_MOUNTAIN_CAR_CONTINUOUS";
+static const char* ro_env_names = "MRL_ENV_CARTPOLE, MRL_ENV_PENDULUM, MRL_ENV_ACROBOT, MRL_ENV_MOUNTAIN_CAR, "
+                                  "MRL_ENV_MOUNTAIN_CAR_CONTINUOUS or an id from mrl_rollout_env_compile";
+
+#define RO_USER_MAX_GAUSS 8    // DiagGauss entries of a user environment (per-thread registers of the action draw)
+#define RO_USER_MAX_CLASSES 16
+#define RO_USER_MAX_STATE 16
+extern "C" int mrl_rollout_env_compile(const char* name, const char* source, int ob_dim, int state_dim, int head,
+                                       int n_out, int* env_out) {
+  const char* who = "mrl_rollout_env_compile";
+  if (!name || !source || !env_out) return fail("%s: bad arguments", who);
+  if (head != MRL_HEAD_CAT && head != MRL_HEAD_GAUSS)
+    return fail("%s: head = %d; a user environment acts through a Categorical (%d) or DiagGauss (%d) head", who, head,
+                MRL_HEAD_CAT, MRL_HEAD_GAUSS);
+  if (ob_dim < 1 || ob_dim > RO_KMAX_OBS)
+    return fail("%s: ob_dim = %d; device rollouts take observations of 1..%d entries (the per-step filter scan "
+                "carries the observation entries and the reward)", who, ob_dim, RO_KMAX_OBS);
+  if (state_dim < 1 || state_dim > RO_USER_MAX_STATE)
+    return fail("%s: state_dim = %d; a user environment's state has 1..%d entries", who, state_dim, RO_USER_MAX_STATE);
+  if (head == MRL_HEAD_CAT && (n_out < 1 || n_out > RO_USER_MAX_CLASSES))
+    return fail("%s: n_out = %d; a Categorical head of a user environment has 1..%d classes", who, n_out,
+                RO_USER_MAX_CLASSES);
+  if (head == MRL_HEAD_GAUSS && (n_out < 1 || n_out > RO_USER_MAX_GAUSS))
+    return fail("%s: n_out = %d; a DiagGauss head of a user environment has 1..%d entries", who, n_out,
+                RO_USER_MAX_GAUSS);
+  std::string err;
+  if (rollout_user_compile(name, source, ob_dim, state_dim, head, n_out, env_out, &err)) {
+    g_err = std::string(who) + ": " + err;
+    return 1;
+  }
+  return 0;
+}
+
+extern "C" int mrl_rollout_env_log(int env, char* buf, int len) {
+  const std::string* log = rollout_user_log(env);
+  if (!log) return fail("mrl_rollout_env_log: %d is not the id of a compiled user environment", env);
+  if (!buf || len < 1) return fail("mrl_rollout_env_log: bad arguments");
+  const size_t n = log->size() < (size_t)len - 1 ? log->size() : (size_t)len - 1;
+  memcpy(buf, log->data(), n);
+  buf[n] = '\0';
+  return 0;
+}
 
 extern "C" int mrl_rollout_max_envs(void) { return RO_MAX_ENVS; }
 
@@ -1311,6 +1350,10 @@ extern "C" int mrl_rollout_create(mrl_rollout** out, int device, int env, int n_
     return fail("mrl_rollout_create: n_envs = %d; the rollout kernel runs 1..%d environments per round", n_envs, RO_MAX_ENVS);
   if (timestep_limit < 1) return fail("mrl_rollout_create: timestep_limit must be >= 1");
   CK(cudaSetDevice(device));
+  if (env >= RO_USER_ENV0) {
+    std::string err;
+    if (rollout_user_load(env, &err)) return fail("mrl_rollout_create: %s", err.c_str());
+  }
   mrl_rollout* r = new mrl_rollout();
   r->device = device; r->env = env; r->N = n_envs; r->T = timestep_limit; r->n_round = n_envs;
   r->d0 = d0; r->sd = sd; r->dout = dout; r->pd = pd; r->head = head;
@@ -1419,7 +1462,8 @@ static const char* ro_env_name(const mrl_rollout* r) {
     case MRL_ENV_PENDULUM: return "Pendulum";
     case MRL_ENV_ACROBOT: return "Acrobot";
     case MRL_ENV_MOUNTAIN_CAR: return "MountainCar";
-    default: return "MountainCarContinuous";
+    case MRL_ENV_MOUNTAIN_CAR_CONTINUOUS: return "MountainCarContinuous";
+    default: return rollout_user_name(r->env);
   }
 }
 

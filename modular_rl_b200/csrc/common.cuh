@@ -9,15 +9,13 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include "kernel_defs.cuh"    // MRL_MAX_LAYERS, the head and activation codes, act_fn
 
 #define MRL_TILE 64           // timesteps per tile
 #define MRL_LDT 68            // floats between consecutive features inside a tile
-#define MRL_MAX_LAYERS 6
 #define MRL_MID_THREADS 256
 #define MRL_MAX_SLAB_TILES 16 // <=1024 timesteps accumulate in fp32 before the fp64 reduce
 
-enum { MRL_HEAD_GAUSS = 0, MRL_HEAD_CAT = 1, MRL_HEAD_VALUE = 2 };
-enum { MRL_ACT_TANH = 0, MRL_ACT_RELU = 1, MRL_ACT_SIGMOID = 2 };
 enum { MRL_MODE_GRAD = 0, MRL_MODE_FVP = 1 };
 
 static inline __host__ __device__ int round_up(int x, int m) { return (x + m - 1) / m * m; }
@@ -103,12 +101,6 @@ __device__ __forceinline__ void bulk_g2s(void* dst_smem, const void* src_gmem, u
 }
 
 // ----------------------------------------------------------------------------- math helpers
-template <int ACT>
-__device__ __forceinline__ float act_fn(float z) {
-  if (ACT == MRL_ACT_TANH) return tanhf(z);
-  if (ACT == MRL_ACT_RELU) return fmaxf(z, 0.f);
-  return 1.f / (1.f + expf(-z));
-}
 template <int ACT>
 __device__ __forceinline__ float dact_from_h(float h) {
   if (ACT == MRL_ACT_TANH) return 1.f - h * h;

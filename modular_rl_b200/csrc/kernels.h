@@ -2,6 +2,8 @@
 #pragma once
 #include "common.cuh"
 
+#include <string>
+
 // ---- batch_params.cu
 cudaError_t launch_pack_params(const NetGeom& g, const float* theta, float* img, float* WB, cudaStream_t st);
 cudaError_t launch_reduce_partials(const NetGeom& g, const float* part1, const float* partm, int n_slabs,
@@ -151,51 +153,29 @@ cudaError_t launch_zfilter_scan(const void* x, int x_f64, long long N, int d, do
                                 cudaStream_t st);
 long long zfilter_scratch_doubles(long long N, int d);
 
-// ---- rollout.cu  (device-resident rollouts of the built-in environments, one cluster launch per round)
-#define RO_MAX_CTAS 8          // CTAs of the round's cluster (the portable cluster size)
-#define RO_MAX_THREADS 512     // environments (threads) per CTA
-#define RO_MIN_PER_CTA 32      // fewer environments per CTA than this: use fewer CTAs
-#define RO_MAX_ENVS (RO_MAX_CTAS * RO_MAX_THREADS)
-struct RolloutArgs {
-  int N, T, per_cta;           // environments, timestep limit, environments per CTA
-  int L, d[MRL_MAX_LAYERS + 1], P;
-  int w_floats;                // theta floats staged in shared memory (0: read through L2)
-  int rows_chunk, ldh;         // forward: rows per chunk, activation row stride (floats)
-  const float* theta;          // the policy's flat parameters (reference order), read in place
-  unsigned long long seed;
-  int stochastic;
-  int ob_on, ob_demean, ob_destd, rew_on;
-  double ob_clip;
-  const double* filt_in;       // (n, M[d0], S[d0]) of the observation filter, then (n, M, S) of the reward filter
-  // [T][N] staging rows
-  double* s_obs; double* s_state /* nullptr: not recorded */; float* s_prob; void* s_act; double* s_rew;
-  int* lengths; int* term;
-  double* head;                // total, observation state, its round part, reward state, its round part
-  char* body;                  // compacted path-major rows (rollout_layout)
-  // population rounds (rollout_kernel<ENV, ACT, true>): environment e acts with theta + e * ld_theta
-  long long ld_theta;
-  double* returns;             // [N] the sum of each episode's raw rewards, in step order
-  int want_rows;               // 0: no staging rows, no compaction (lengths, terminated, returns and the header only)
-};
-// Byte offsets of the compacted arrays for n timesteps: f64 sections first, so that every section stays aligned
-struct RolloutLayout { size_t obs, rew, state, prob, act, end; };
-__host__ __device__ inline RolloutLayout rollout_layout(long long n, int d0, int sd, int pd, int ad, int with_states) {
-  RolloutLayout o;
-  size_t p = 0;
-  o.obs = p;   p += (size_t)n * d0 * 8;
-  o.rew = p;   p += (size_t)n * 8;
-  o.state = p; p += with_states ? (size_t)n * sd * 8 : 0;
-  o.prob = p;  p += (size_t)n * pd * 4;
-  o.act = p;   p += (size_t)n * ad * 4;     // int32 (Categorical) or float32 [d] (DiagGauss)
-  o.end = p;
-  return o;
-}
+// ---- rollout.cu  (device-resident rollouts, one cluster launch per round; RolloutArgs: kernel_defs.cuh)
 // observation entries, state entries, policy outputs, prob row width -> head, -1 for an unknown env
 int rollout_env_dims(int env, int* d0, int* sd, int* dout, int* pd);
 void rollout_shape(int N, int* n_ctas, int* per_cta, int* threads);
 size_t rollout_smem_bytes(const RolloutArgs& a, int d0, int dout, bool pop);
+// built-in and user environments; a user environment's kernels must be loaded (rollout_user_load) first
+cudaError_t launch_rollout_kernel(const void* f, const RolloutArgs& a, int n_ctas, int threads, size_t smem,
+                                  cudaStream_t st);
 cudaError_t launch_rollout(const RolloutArgs& a, int env, int act, bool pop, int n_ctas, int threads, size_t smem,
                            cudaStream_t st);
+
+// ---- rollout_user.cu  (user environments: the rollout kernel compiled by NVRTC at run time; host only)
+// Compiles (or finds) the environment of snippet `source` with these shapes -> *env >= RO_USER_ENV0; else *err
+int rollout_user_compile(const char* name, const char* source, int d0, int sd, int head, int dout, int* env,
+                         std::string* err);
+const std::string* rollout_user_log(int env);   // the ptxas lines of its six instances; nullptr for an unknown id
+// rollout_env_dims for ids >= RO_USER_ENV0; -1 for an id that was never compiled
+int rollout_user_dims(int env, int* d0, int* sd, int* dout, int* pd);
+const char* rollout_user_name(int env);   // nullptr for an unknown id
+// Loads the environment's six kernels (once per process)
+int rollout_user_load(int env, std::string* err);
+cudaError_t launch_rollout_user(const RolloutArgs& a, int env, int act, bool pop, int n_ctas, int threads,
+                                size_t smem, cudaStream_t st);
 
 // ---- cem_search.cu  (device search distribution of the cross-entropy method)
 // rows[m][0..P) = float32(mean + dev * z[m]) for m < M, dev[j] = sqrt(var[j] + extra_var * noise_left); ld % 4 == 0

@@ -3,7 +3,12 @@
 // word, high word) and addressed by a counter whose third word is the PURPOSE of the draw, so the streams of
 // different purposes never share a counter.  oracle/rollout.py restates both functions in numpy.
 #pragma once
+#ifdef __CUDACC_RTC__   // NVRTC (rollout_user.cu) has no <stdint.h>
+#include <cuda/std/cstdint>
+using cuda::std::uint32_t;
+#else
 #include <stdint.h>
+#endif
 
 __device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint32_t k0, uint32_t k1) {
 #pragma unroll

@@ -327,12 +327,36 @@ class DeviceNet:
         return sd, fs, dict(shs=sc[0], lm=sc[1], expected_improve_rate=sc[2], cg_rdotr=sc[3])
 
 
-def rollout_env_info(kind: str) -> dict:
+_user_env_ids = {}           # envs.DeviceEnv (bound to its shapes) -> library id
+
+
+def rollout_env_id(kind) -> int:
+    """The library's id of an envs.device_kind: a built-in's MRL_ENV_* code, or for a user environment (a bound
+    envs.DeviceEnv) the id of its kernels, compiled with NVRTC on first use in the process."""
+    if isinstance(kind, str):
+        return L.DEVICE_ENVS[kind]
+    if kind not in _user_env_ids:
+        env = C.c_int()
+        L.check(L.lib().mrl_rollout_env_compile(str(kind.name).encode(), kind.source.encode(), kind.ob_dim,
+                                                kind.state_dim, L.CATEGORICAL if kind.categorical else L.GAUSS,
+                                                kind.n_out, C.byref(env)))
+        _user_env_ids[kind] = env.value
+    return _user_env_ids[kind]
+
+
+def rollout_env_log(kind) -> str:
+    """The compiler's report (ptxas registers and spills of the six kernel instances) of a user environment."""
+    buf = C.create_string_buffer(1 << 16)
+    L.check(L.lib().mrl_rollout_env_log(rollout_env_id(kind), buf, len(buf)))
+    return buf.value.decode(errors="replace")
+
+
+def rollout_env_info(kind) -> dict:
     """mrl_rollout_env_info for an envs.py device kind: ob_dim, state_dim, categorical, n_out (the policy's outputs:
     K classes or the DiagGauss dimension d), act_dim (1 for Categorical, else d) and prob_dim (K, or 2d for
     [mean, std])."""
     ob, st, head, n_out = C.c_int(), C.c_int(), C.c_int(), C.c_int()
-    L.check(L.lib().mrl_rollout_env_info(L.DEVICE_ENVS[kind], C.byref(ob), C.byref(st), C.byref(head), C.byref(n_out)))
+    L.check(L.lib().mrl_rollout_env_info(rollout_env_id(kind), C.byref(ob), C.byref(st), C.byref(head), C.byref(n_out)))
     cat = head.value == L.CATEGORICAL
     return dict(ob_dim=ob.value, state_dim=st.value, categorical=cat, n_out=n_out.value,
                 act_dim=1 if cat else n_out.value, prob_dim=n_out.value if cat else 2 * n_out.value)
@@ -342,7 +366,7 @@ class DeviceRollouts:
     """mrl_rollout_*: rounds of n_envs lockstep rollouts of a built-in environment, each round one kernel launch on
     the device (the policy forward, the action draws, the dynamics and both ZFilters included).  `env`: a built-in
     environment's id ("CartPole-v0", "Pendulum-v0", "Acrobot-v1", "MountainCar-v0", "MountainCarContinuous-v0") or
-    instance."""
+    instance, or a user environment with an envs.DeviceEnv (its id or instance)."""
 
     def __init__(self, env, n_envs: int, timestep_limit: int, device: Optional[int] = None):
         from .envs import device_kind
@@ -350,7 +374,7 @@ class DeviceRollouts:
         if device is None:
             device = parallel.current_device()
         self._h = C.c_void_p()
-        L.check(L.lib().mrl_rollout_create(C.byref(self._h), device, L.DEVICE_ENVS[kind], int(n_envs), int(timestep_limit)))
+        L.check(L.lib().mrl_rollout_create(C.byref(self._h), device, rollout_env_id(kind), int(n_envs), int(timestep_limit)))
         self.kind, self.n_envs, self.timestep_limit, self.device = kind, int(n_envs), int(timestep_limit), device
         info = rollout_env_info(kind)
         self.ob_dim, self.state_dim, self.categorical = info["ob_dim"], info["state_dim"], info["categorical"]

@@ -3,7 +3,13 @@ info) so that BASELINE config 1 (CartPole-v0 TrpoAgent via run_pg.py) and the re
 smoke (run_cem.py on Acrobot, run_pg.py on Pendulum, coverage.sh:6-7) run without gym, which is not installed here.
 Dynamics follow the published classic-control equations (Barto-Sutton-Anderson cart-pole; torque-limited pendulum;
 Sutton-Barto acrobot; Moore's mountain car, discrete and continuous).  Every one of them also runs on the device
-(rollout.cu), which replays the float64 arithmetic of these classes."""
+(rollout.cu), which replays the float64 arithmetic of these classes.
+
+A user environment runs on the device too when its class sets `device_kind = DeviceEnv(source, state_dim)`: the same
+reset / obs / step as a CUDA snippet, which the library compiles into the rollout kernel at run time
+(examples/point_mass.py is the template).  register(id, cls) adds a class to make(), and make("pkg.module:Id")
+imports pkg.module first, as gym's make does."""
+import importlib
 import math
 
 import numpy as np
@@ -256,30 +262,98 @@ class MountainCarContinuousEnv(MountainCarEnv):
         return np.array(self.state), reward, done, {}
 
 
+class DeviceEnv(object):
+    """The device implementation of a user environment: `source` defines, as CUDA in float64,
+        __device__ static void reset(double* s, int env, uint32_t k0, uint32_t k1)
+        __device__ static void obs(const double* s, double* x)
+        __device__ static bool step(double* s, int action, const float* a, double* reward)
+    over a state of `state_dim` entries (include/mrl_b200.h, mrl_rollout_env_compile).  Set it as the class's
+    `device_kind`; the observation, head and action shapes come from the class's spaces (envs.device_kind)."""
+
+    def __init__(self, source, state_dim, name=None, ob_dim=None, categorical=None, n_out=None):
+        self.source, self.state_dim, self.name = str(source), int(state_dim), name
+        self.ob_dim, self.categorical, self.n_out = ob_dim, categorical, n_out
+
+    def _key(self):
+        return (self.source, self.state_dim, self.ob_dim, self.categorical, self.n_out)
+
+    def __eq__(self, other):
+        return isinstance(other, DeviceEnv) and self._key() == other._key()
+
+    def __hash__(self):
+        return hash(self._key())
+
+    def __repr__(self):
+        return "DeviceEnv(%s, ob_dim=%s, %s %s)" % (self.name, self.ob_dim,
+                                                    "Categorical" if self.categorical else "DiagGauss", self.n_out)
+
+    def bind(self, env):
+        """This snippet with the shapes of `env` (an instance): Box observation (k,); Discrete(K) -> Categorical K,
+        Box action (d,) -> DiagGauss d.  Raises ValueError for any other space."""
+        name = getattr(getattr(env, "spec", None), "id", None) or type(env).__name__
+        ob, ac = getattr(env, "observation_space", None), getattr(env, "action_space", None)
+        if not isinstance(ob, Box) or len(ob.shape) != 1:
+            raise ValueError("environment %s: device rollouts need a Box observation space of shape (k,), not %r"
+                             % (name, ob))
+        if isinstance(ac, Discrete):
+            categorical, n_out = True, int(ac.n)
+        elif isinstance(ac, Box) and len(ac.shape) == 1:
+            categorical, n_out = False, int(ac.shape[0])
+        else:
+            raise ValueError("environment %s: device rollouts need a Discrete or a Box action space of shape (d,), "
+                             "not %r" % (name, ac))
+        return DeviceEnv(self.source, self.state_dim, name, int(ob.shape[0]), categorical, n_out)
+
+
 _REGISTRY = {"CartPole-v0": CartPoleEnv, "CartPole": CartPoleEnv, "Pendulum-v0": PendulumEnv,
              "Pendulum": PendulumEnv, "Acrobot-v1": AcrobotEnv, "Acrobot": AcrobotEnv,
              "MountainCar-v0": MountainCarEnv, "MountainCar": MountainCarEnv,
              "MountainCarContinuous-v0": MountainCarContinuousEnv, "MountainCarContinuous": MountainCarContinuousEnv}
 
 
+def register(id_, cls):
+    """Make `cls` (called without arguments) available as make(id_)."""
+    _REGISTRY[str(id_)] = cls
+
+
+def _registered(name):
+    """The class registered as `name`; "pkg.module:Id" imports pkg.module first.  None when unknown."""
+    if ":" in name:
+        module, _, id_ = name.partition(":")
+        try:
+            importlib.import_module(module)
+        except ImportError as e:
+            raise KeyError("environment %r: cannot import module %r (%s)" % (name, module, e))
+        if id_ not in _REGISTRY:
+            raise KeyError("environment %r: module %r registers no environment %r (registered: %s)"
+                           % (name, module, id_, ", ".join(sorted(_REGISTRY))))
+        return _REGISTRY[id_]
+    return _REGISTRY.get(name)
+
+
 def make(name):
-    """gym.envs.make stand-in; falls through to gym when it is installed and the id is unknown."""
-    if name in _REGISTRY:
-        return _REGISTRY[name]()
+    """gym.envs.make stand-in: a registered id, or "pkg.module:Id" (imports pkg.module, which registers Id); falls
+    through to gym when it is installed and the id is unknown."""
+    cls = _registered(name)
+    if cls is not None:
+        return cls()
     try:
         from gym.envs import make as gym_make
     except ImportError:
-        raise KeyError("unknown environment %r (built in: %s; gym is not installed)" % (name, sorted(_REGISTRY)))
+        raise KeyError("unknown environment %r (registered: %s; gym is not installed)" % (name, sorted(_REGISTRY)))
     return gym_make(name)
 
 
 def device_kind(env):
-    """The device implementation of a built-in environment (an instance or an id): 'cartpole', 'pendulum',
-    'acrobot', 'mountaincar' or 'mountaincar_continuous'.  Raises ValueError for any other environment."""
-    cls = _REGISTRY.get(env) if isinstance(env, str) else type(env)
+    """The device implementation of an environment (an instance or an id): 'cartpole', 'pendulum', 'acrobot',
+    'mountaincar' or 'mountaincar_continuous' for the built-ins, the class's DeviceEnv bound to its shapes for a user
+    environment.  Raises ValueError for any other environment."""
+    cls = _registered(env) if isinstance(env, str) else type(env)
     kind = getattr(cls, "device_kind", None)
     if kind is None:
         name = env if isinstance(env, str) else getattr(getattr(env, "spec", None), "id", type(env).__name__)
         raise ValueError("environment %s has no device implementation; device rollouts run the built-in environments "
                          "only: %s" % (name, ", ".join(sorted(_REGISTRY))))
+    if isinstance(kind, DeviceEnv):
+        return kind.bind(cls() if isinstance(env, str) else env)
     return kind

@@ -2,8 +2,9 @@
 """Cross-entropy-method driver with the reference's run_cem.py command line (GENERAL_OPTIONS, --env, --agent, --plot,
 the agent's own options, CEM_OPTIONS - run_cem.py:13-30).  Candidates are scored through the device-resident
 deterministic policy; with --parallel 1 the whole population is scored in lockstep by one population-batched forward
-per environment step; with --device_envs (the built-in environments) each generation is one device rollout round,
-and with --device_search as well the candidates are drawn and the search distribution refitted on the device.
+per environment step; with --device_envs (environments with a device implementation) each generation is one device
+rollout round, and with --device_search as well the candidates are drawn and the search distribution refitted on the
+device.
 
   python run_cem.py --env CartPole-v0 --agent modular_rl.agentzoo.DeterministicAgent --n_iter 10 --batch_size 40
 """
@@ -36,9 +37,9 @@ def parse_cli(argv):
     ap.add_argument("--agent", required=True)
     ap.add_argument("--plot", action="store_true")
     ap.add_argument("--device_envs", action="store_true",
-                    help="score each generation in one GPU rollout round, one environment per candidate (built-in "
-                         "CartPole, Pendulum, Acrobot, MountainCar and MountainCarContinuous only); resets come from the device's Philox stream, so results differ "
-                         "from a host run with the same --seed")
+                    help="score each generation in one GPU rollout round, one environment per candidate (the "
+                         "built-in environments, and user environments whose class has an envs.DeviceEnv); resets "
+                         "come from the device's Philox stream, so results differ from a host run with the same --seed")
     ap.add_argument("--device_search", action="store_true",
                     help="with --device_envs: draw each generation's candidates and refit the search distribution on "
                          "the GPU; the draws come from the device's Philox stream, not numpy's, so results differ "

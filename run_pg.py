@@ -40,9 +40,10 @@ def main():
                         help="environments stepped in lockstep with one batched device forward per step "
                              "(0: serial rollouts as the reference); not an agent option")
     parser.add_argument("--device_envs", type=int, default=0,
-                        help="environments per rollout round run on the GPU in one kernel launch (built-in CartPole, "
-                             "Pendulum, Acrobot, MountainCar and MountainCarContinuous only; 0: host rollouts); resets and action noise come from the device's "
-                             "Philox stream, so results differ from a host run with the same --seed")
+                        help="environments per rollout round run on the GPU in one kernel launch (the built-in "
+                             "environments, and user environments whose class has an envs.DeviceEnv, e.g. --env "
+                             "examples.point_mass:PointMass-v0; 0: host rollouts); resets and action noise come from "
+                             "the device's Philox stream, so results differ from a host run with the same --seed")
     args, _ = parser.parse_known_args([arg for arg in sys.argv[1:] if arg not in ('-h', '--help')])
     if args.device_envs and args.vec_envs:
         parser.error("--device_envs and --vec_envs select different rollout paths; give one")
