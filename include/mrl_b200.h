@@ -185,6 +185,21 @@ int mrl_net_ppo_sgd_step(mrl_net* net, mrl_batch* minibatch, double kl_coeff, do
 int mrl_net_ppo_sgd_read(mrl_net* net, double losses[3], long long* count, void* stream);
 int mrl_net_adam_reset(mrl_net* net, void* stream);
 
+/* ---------------------------------------------------------------- PPO with the clipped surrogate objective
+ * L = -(1/N) sum_t min(r_t A_t, clip(r_t, 1 - clip_eps, 1 + clip_eps) A_t),  r_t = pi(a_t | s_t) / pi_old(a_t | s_t),
+ * pi_old = the prob rows bound with mrl_batch_set_policy_inputs.  A row carries the surrogate's gradient unless
+ * (A > 0 and r > 1 + clip_eps) or (A < 0 and r < 1 - clip_eps); at r = 1 +- clip_eps it does.  clip_eps > 0, +inf
+ * means no clipping; a value net, NULL handles and clip_eps <= 0 or NaN are rejected.
+ * mrl_net_ppo_clip_lossgrad: a full-batch pass: losses = {surr = L, kl = KL[old, new], ent, clipfrac = the fraction of
+ *   rows with r outside [1 - clip_eps, 1 + clip_eps]} (may be NULL); g != NULL: dL/dtheta, float64 [P] (host), summed
+ *   over the ranks of the net's communicator.  Synchronises `stream`.
+ * mrl_net_ppo_clip_sgd_step: one minibatch step: the clipped gradient on the minibatch and the Adam update of
+ *   mrl_net_ppo_sgd_step, on the same moments and step counter (mrl_net_adam_reset restarts them); no host
+ *   synchronisation. */
+int mrl_net_ppo_clip_lossgrad(mrl_net* net, mrl_batch* b, double clip_eps, double* g, double losses[4], void* stream);
+int mrl_net_ppo_clip_sgd_step(mrl_net* net, mrl_batch* minibatch, double clip_eps, double stepsize, double beta1,
+                              double beta2, double epsilon, void* stream);
+
 /* ---------------------------------------------------------------- population forward (cross-entropy method)
  * cem.py:43-44 scores every candidate theta of an iteration by one rollout, one candidate at a time; this entry point
  * evaluates the net of ALL candidates at once: member m has its own flat theta (Dense kernels and biases in the

@@ -83,6 +83,8 @@ _SIGS = {
     "mrl_net_ppo_sgd_step": (_I, [_P, _P, _D, _D, _I, _D, _D, _D, _D, _P]),
     "mrl_net_ppo_sgd_read": (_I, [_P, _P, _P, _P]),
     "mrl_net_adam_reset": (_I, [_P, _P]),
+    "mrl_net_ppo_clip_lossgrad": (_I, [_P, _P, _D, _P, _P, _P]),
+    "mrl_net_ppo_clip_sgd_step": (_I, [_P, _P, _D, _D, _D, _D, _D, _P]),
     "mrl_population_forward": (_I, [_I, _I, C.POINTER(_I), _I, _P, _LL, _P, _I, _P, _I, _P]),
     "mrl_comm_unique_id": (_I, [_P]),
     "mrl_comm_create": (_I, [C.POINTER(_P), _P, _I, _I, _I]),

@@ -6,7 +6,7 @@ from . import parallel
 from .core import (Categorical, DiagGauss, NnVf, PG_OPTIONS, StochPolicyMLP, make_value_net)
 from .filters import ZFilter
 from .misc_utils import IDENTITY, comma_sep_ints, update_default_config
-from .ppo import PpoLbfgsUpdater, PpoSgdUpdater
+from .ppo import PpoClipUpdater, PpoLbfgsUpdater, PpoSgdUpdater
 from .spaces import is_box, is_discrete
 from .trpo import TrpoUpdater
 
@@ -169,4 +169,17 @@ class PpoSgdAgent(AgentWithPolicy):
         policy, self.baseline = make_mlps(ob_space, ac_space, cfg)
         obfilter, rewfilter = make_filters(cfg, ob_space)
         self.updater = PpoSgdUpdater(policy, cfg)
+        AgentWithPolicy.__init__(self, policy, obfilter, rewfilter)
+
+
+class PpoClipAgent(AgentWithPolicy):
+    """PPO with the clipped surrogate objective (ppo.PpoClipUpdater)."""
+    options = MLP_OPTIONS + PG_OPTIONS + PpoClipUpdater.options + FILTER_OPTIONS
+
+    def __init__(self, ob_space, ac_space, usercfg):
+        parallel.reject_data_parallel("PpoClipAgent")
+        cfg = update_default_config(self.options, usercfg)
+        policy, self.baseline = make_mlps(ob_space, ac_space, cfg)
+        obfilter, rewfilter = make_filters(cfg, ob_space)
+        self.updater = PpoClipUpdater(policy, cfg)
         AgentWithPolicy.__init__(self, policy, obfilter, rewfilter)

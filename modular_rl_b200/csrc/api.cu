@@ -850,9 +850,10 @@ static int reserve_ws(mrl_net* n, const mrl_batch* b, const Plan& pl) {
   return 0;
 }
 
-// L1F + mid forward.  losses -> n->scal[0..3] (device, already scaled by 1/N_global and all-reduced)
+// L1F + mid forward.  losses -> n->scal[0..3] (device, already scaled by 1/N_global and all-reduced); clip_eps > 0:
+// scal[0] is the mean clipped objective and scal[3] the fraction of clipped rows
 static int pass_forward(mrl_net* n, mrl_batch* b, bool want_losses, bool want_cache, float* head_out,
-                        cudaStream_t st, int reverse_kl = 0) {
+                        cudaStream_t st, int reverse_kl = 0, float clip_eps = 0.f) {
   const NetGeom& g = n->g;
   const Plan pl = plan_for(b, true);
   RET(reserve_ws(n, b, pl));
@@ -875,9 +876,9 @@ static int pass_forward(mrl_net* n, mrl_batch* b, bool want_losses, bool want_ca
     a.cache = n->cache.as<float>();
     if (!want_cache) n->cache_batch = nullptr;
     int nk = 0;
-    CKP(PK_MIDF, launch_layers_forward(g, a, pl.n_slabs, st, &nk), nk);
-  } else if (chain_fwd_shape(g) != 0) CKP(PK_MIDF, launch_chain_forward(g, a, pl.n_slabs, st), 1);
-  else CKP(PK_MIDF, launch_mid_forward(g, a, pl.n_slabs, st), 1);
+    CKP(PK_MIDF, launch_layers_forward(g, a, pl.n_slabs, st, &nk, clip_eps), nk);
+  } else if (chain_fwd_shape(g) != 0) CKP(PK_MIDF, launch_chain_forward(g, a, pl.n_slabs, st, clip_eps), 1);
+  else CKP(PK_MIDF, launch_mid_forward(g, a, pl.n_slabs, st, clip_eps), 1);
   if (want_losses) {
     CKL(launch_reduce_losses(n->loss_part.as<double>(), pl.n_slabs, 1.0 / (double)b->Nglobal, n->scal.as<double>(), st), 1);
     if (world_of(n) > 1) RET(mrl_comm_allreduce_f64(n->comm, n->scal.as<double>(), 4, st));
@@ -894,8 +895,10 @@ static bool cache_ok(const mrl_net* n, const mrl_batch* b) {
 }
 
 // reverse sweep + layer-1 gradient + slab reduce -> out32 (float[P], device) and out64 (double[P]).
+// MRL_MODE_GRAD_CLIP: the gradient of the PPO clipped objective with clip range clip_eps.
 static int pass_backward(mrl_net* n, mrl_batch* b, int mode, const double* coef_dev, int reverse_kl,
-                         const float* v_dev, double l2c2, float* out32, double* out64, cudaStream_t st) {
+                         const float* v_dev, double l2c2, float* out32, double* out64, cudaStream_t st,
+                         float clip_eps = 0.f) {
   const NetGeom& g = n->g;
   const bool tc = mode == MRL_MODE_FVP && n->tc_fvp;
   const Plan pl = plan_for(b, tc);
@@ -913,7 +916,7 @@ static int pass_backward(mrl_net* n, mrl_batch* b, int mode, const double* coef_
     a.imgv = n->imgv.as<float>();
     a.Zt = n->Z1.as<float>();
   }
-  a.aux = mode == MRL_MODE_GRAD ? aux_of(n, b) : nullptr;
+  a.aux = mode != MRL_MODE_FVP ? aux_of(n, b) : nullptr;
   a.cache = n->cache.as<float>();
   a.coef = coef_dev;
   a.DG = n->DG.as<float>();
@@ -927,15 +930,15 @@ static int pass_backward(mrl_net* n, mrl_batch* b, int mode, const double* coef_
   if (n->layers) {
     int nk = 0;
     CKP(mode == MRL_MODE_FVP ? PK_MIDB_FVP : PK_MIDB_GRAD,
-        launch_layers_backward(g, a, n->R0.as<float>(), n->R1.as<float>(), pl.n_slabs, st, &nk), nk);
+        launch_layers_backward(g, a, n->R0.as<float>(), n->R1.as<float>(), pl.n_slabs, st, &nk, clip_eps), nk);
   } else if (tc) {
     FvpTcArgs x;
     x.WC = n->WC.as<float>(); x.VC = n->VC.as<float>(); x.vflat = v_dev; x.img = n->img.as<float>();
     x.Zt = n->Z1.as<float>(); x.cache = n->cache.as<float>(); x.DG = n->DG.as<float>(); x.partm = n->partm.as<float>();
     x.N = b->N; x.n_tiles = b->n_tiles; x.slab_tiles = pl.slab_tiles; x.n_slabs = pl.n_slabs;
     CKP(PK_MIDB_FVP, launch_fvp_tc(g, x, st), 1);
-  } else if (mode == MRL_MODE_GRAD && chain_bwd_shape(g) != 0) CKP(PK_MIDB_GRAD, launch_chain_backward(g, a, pl.n_slabs, st), 1);
-  else CKP(mode == MRL_MODE_FVP ? PK_MIDB_FVP : PK_MIDB_GRAD, launch_mid_backward(g, a, pl.n_slabs, st), 1);
+  } else if (mode != MRL_MODE_FVP && chain_bwd_shape(g) != 0) CKP(PK_MIDB_GRAD, launch_chain_backward(g, a, pl.n_slabs, st, clip_eps), 1);
+  else CKP(mode == MRL_MODE_FVP ? PK_MIDB_FVP : PK_MIDB_GRAD, launch_mid_backward(g, a, pl.n_slabs, st, clip_eps), 1);
   CKP(PK_L1G, launch_l1_grad_tc(g, b->XG.as<float>(), (b->xdim + 127) / 128, n->DG.as<float>(), n->part1.as<float>(),
                                 pl.slab_tiles, b->n_tiles, pl.n_slabs, st), 1);
   const int world = world_of(n);
@@ -1100,6 +1103,30 @@ extern "C" int mrl_net_vf_lossgrad(mrl_net* n, mrl_batch* b, double l2coeff, dou
 }
 
 // ------------------------------------------------------------------------ PpoSgd minibatch step
+// the Adam moments and step counter of adam_updates (ppo.py:231-258), allocated at the first minibatch step
+static int adam_init(mrl_net* n, cudaStream_t st) {
+  if (n->adam_m.p) return 0;
+  const size_t P = n->g.P;
+  CK(n->adam_m.reserve(P * 4));
+  CK(n->adam_v.reserve(P * 4));
+  CK(n->sgd_acc.reserve(4 * 8));
+  CK(cudaMemsetAsync(n->adam_m.p, 0, P * 4, st));
+  CK(cudaMemsetAsync(n->adam_v.p, 0, P * 4, st));
+  CK(cudaMemsetAsync(n->sgd_acc.p, 0, 4 * 8, st));
+  n->adam_t = 0;
+  return 0;
+}
+// one Adam step on theta with the float64 gradient in out64, then the repack of the parameter images
+static int adam_apply(mrl_net* n, double stepsize, double beta1, double beta2, double epsilon, cudaStream_t st) {
+  n->adam_t += 1;
+  const float f1 = (float)beta1, f2 = (float)beta2;
+  // a_t in float32, operation by operation as the numpy float32 expression of the host version
+  const float a_t = (float)stepsize * sqrtf(1.f - powf(f2, (float)n->adam_t)) / (1.f - powf(f1, (float)n->adam_t));
+  CKL(launch_adam_step((int)n->g.P, n->out64.as<double>(), n->theta.as<float>(), n->adam_m.as<float>(),
+                       n->adam_v.as<float>(), a_t, f1, f2, (float)epsilon, st), 1);
+  return repack(n, st);
+}
+
 // One `train` call of PpoSgdUpdater (ppo.py:162-167,199): penalised-surrogate loss and gradient on the minibatch, then
 // the Adam update of adam_updates (ppo.py:231-258), everything on the device and without a host synchronisation; the
 // losses (evaluated BEFORE the step, as Theano evaluates outputs before applying updates) are added to a running sum.
@@ -1109,16 +1136,7 @@ extern "C" int mrl_net_ppo_sgd_step(mrl_net* n, mrl_batch* b, double kl_coeff, d
   if (n->g.head == MRL_VALUE) return fail("mrl_net_ppo_sgd_step: value net");
   cudaStream_t st = (cudaStream_t)stream;
   CK(cudaSetDevice(n->device));
-  const size_t P = n->g.P;
-  if (!n->adam_m.p) {
-    CK(n->adam_m.reserve(P * 4));
-    CK(n->adam_v.reserve(P * 4));
-    CK(n->sgd_acc.reserve(4 * 8));
-    CK(cudaMemsetAsync(n->adam_m.p, 0, P * 4, st));
-    CK(cudaMemsetAsync(n->adam_v.p, 0, P * 4, st));
-    CK(cudaMemsetAsync(n->sgd_acc.p, 0, 4 * 8, st));
-    n->adam_t = 0;
-  }
+  RET(adam_init(n, st));
   RET(pass_forward(n, b, true, true, nullptr, st, reverse_kl));
   double* scal = n->scal.as<double>();
   negate_first<<<1, 1, 0, st>>>(scal);
@@ -1126,13 +1144,7 @@ extern "C" int mrl_net_ppo_sgd_step(mrl_net* n, mrl_batch* b, double kl_coeff, d
   CKL(launch_ppo_coef(scal, kl_coeff, kl_cutoff, scal + 8, scal + 10, st), 1);
   CKL(launch_accum_losses(scal, n->sgd_acc.as<double>(), st), 1);
   RET(pass_backward(n, b, MRL_MODE_GRAD, scal + 8, reverse_kl, nullptr, 0.0, nullptr, n->out64.as<double>(), st));
-  n->adam_t += 1;
-  const float f1 = (float)beta1, f2 = (float)beta2;
-  // a_t in float32, operation by operation as the numpy float32 expression of the host version
-  const float a_t = (float)stepsize * sqrtf(1.f - powf(f2, (float)n->adam_t)) / (1.f - powf(f1, (float)n->adam_t));
-  CKL(launch_adam_step((int)P, n->out64.as<double>(), n->theta.as<float>(), n->adam_m.as<float>(), n->adam_v.as<float>(), a_t,
-                       f1, f2, (float)epsilon, st), 1);
-  return repack(n, st);
+  return adam_apply(n, stepsize, beta1, beta2, epsilon, st);
 }
 // mean of the minibatch losses accumulated since the last read (surr, kl, ent) and their count; resets the sum
 extern "C" int mrl_net_ppo_sgd_read(mrl_net* n, double losses[3], long long* count, void* stream) {
@@ -1148,6 +1160,46 @@ extern "C" int mrl_net_ppo_sgd_read(mrl_net* n, double losses[3], long long* cou
   CK(cudaMemsetAsync(n->sgd_acc.p, 0, 32, st));
   return 0;
 }
+// ------------------------------------------------------------------------ PPO with the clipped surrogate objective
+// clip_eps must be > 0 also after the rounding to float32 in which the kernels compare; +inf is no clipping
+static int check_clip(const char* fn, const mrl_net* n, const mrl_batch* b, double clip_eps) {
+  if (!((float)clip_eps > 0.f)) return fail("%s: clip_eps must be > 0 (got %g)", fn, clip_eps);
+  if (!n || !b) return fail("%s: null net or batch", fn);
+  if (n->g.head == MRL_VALUE) return fail("%s: value net", fn);
+  return check_pair(n, b, true);
+}
+
+extern "C" int mrl_net_ppo_clip_lossgrad(mrl_net* n, mrl_batch* b, double clip_eps, double* gout, double losses[4],
+                                         void* stream) {
+  RET(check_clip("mrl_net_ppo_clip_lossgrad", n, b, clip_eps));
+  cudaStream_t st = (cudaStream_t)stream;
+  CK(cudaSetDevice(n->device));
+  const float eps = (float)clip_eps;
+  RET(pass_forward(n, b, true, gout != nullptr, nullptr, st, 0, eps));
+  if (gout) RET(pass_backward(n, b, MRL_MODE_GRAD_CLIP, nullptr, 0, nullptr, 0.0, nullptr, n->out64.as<double>(), st, eps));
+  RET(d2h_sync(n->h_scal, n->scal.p, 4 * 8, st));
+  RET(comm_ok(n));
+  if (losses) {
+    losses[0] = -n->h_scal[0]; losses[1] = n->h_scal[1]; losses[2] = n->h_scal[2]; losses[3] = n->h_scal[3];
+  }
+  if (gout) RET(d2h_sync(gout, n->out64.p, (size_t)n->g.P * 8, st));
+  return 0;
+}
+
+// One minibatch step of PPO-clip: forward with the activation cache (no loss sums), the clipped gradient, the Adam
+// step of mrl_net_ppo_sgd_step on the same moments, the repack; no host synchronisation.
+extern "C" int mrl_net_ppo_clip_sgd_step(mrl_net* n, mrl_batch* b, double clip_eps, double stepsize, double beta1,
+                                         double beta2, double epsilon, void* stream) {
+  RET(check_clip("mrl_net_ppo_clip_sgd_step", n, b, clip_eps));
+  cudaStream_t st = (cudaStream_t)stream;
+  CK(cudaSetDevice(n->device));
+  RET(adam_init(n, st));
+  const float eps = (float)clip_eps;
+  RET(pass_forward(n, b, false, true, nullptr, st));
+  RET(pass_backward(n, b, MRL_MODE_GRAD_CLIP, nullptr, 0, nullptr, 0.0, nullptr, n->out64.as<double>(), st, eps));
+  return adam_apply(n, stepsize, beta1, beta2, epsilon, st);
+}
+
 // restart Adam (moments and step counter to zero)
 extern "C" int mrl_net_adam_reset(mrl_net* n, void* stream) {
   if (!n) return fail("mrl_net_adam_reset: null net");

@@ -16,7 +16,7 @@
 #define MRL_MID_THREADS 256
 #define MRL_MAX_SLAB_TILES 16 // <=1024 timesteps accumulate in fp32 before the fp64 reduce
 
-enum { MRL_MODE_GRAD = 0, MRL_MODE_FVP = 1 };
+enum { MRL_MODE_GRAD = 0, MRL_MODE_FVP = 1, MRL_MODE_GRAD_CLIP = 2 };   // GRAD_CLIP: gradient of the PPO clipped objective
 
 static inline __host__ __device__ int round_up(int x, int m) { return (x + m - 1) / m * m; }
 

@@ -54,6 +54,25 @@ __device__ __forceinline__ float cat_grad(float p, float p0, float w, float ck, 
   const float dk = reverse_kl ? p * (logf(p / p0) - klrow) : (p - p0);
   return w * ((hot ? 1.f : 0.f) - p) + ck * dk;
 }
+// PPO clipped surrogate of one row, r = pi / pi_old (the ratio the surrogate forms above): the row's share of the
+// objective min(r A, clip(r, 1 - eps, 1 + eps) A).  eps = +inf: r A.
+__device__ __forceinline__ float clip_objective(float r, float adv, float eps) {
+  return fminf(r * adv, fminf(fmaxf(r, 1.f - eps), 1.f + eps) * adv);
+}
+// the row's gradient is cut off where the clipped branch is the smaller one, outside the inclusive clip range (the
+// derivative torch autograd takes of torch.minimum(r A, torch.clamp(r, 1 - eps, 1 + eps) A); a tie passes it).
+// Ungated rows carry the surrogate's gradient, weight w = -r A, with no KL term.
+__device__ __forceinline__ bool clip_gated(float r, float adv, float eps) {
+  return (adv > 0.f && r > 1.f + eps) || (adv < 0.f && r < 1.f - eps);
+}
+// the row counts towards clipfrac: r outside [1 - eps, 1 + eps]
+__device__ __forceinline__ bool clip_outside(float r, float eps) { return r < 1.f - eps || r > 1.f + eps; }
+// a valid row of the clipped objective: its term added to the surrogate sum, counted in s_clip when outside the range
+__device__ __forceinline__ void clip_row(float r, float adv, float eps, double& s_surr, double& s_clip) {
+  s_surr += (double)clip_objective(r, adv, eps);
+  s_clip += clip_outside(r, eps) ? 1.0 : 0.0;
+}
+
 // value head: squared error against the target y, and its derivative d/dpred
 __device__ __forceinline__ double value_sqerr(float y, float pred) {
   const float df = y - pred;
@@ -66,11 +85,12 @@ __device__ __forceinline__ float value_dpred(float pred, float y) { return 2.f *
 // when there are no losses; valid = r is a timestep of the batch, not padding.  sig, logsig, ivar = sigma, log sigma
 // and 1/sigma^2 per dimension (DiagGauss).
 
-// Forward: the Categorical probabilities rewritten in place of the logits; the row's surr / kl / ent added to the sums
-template <int HEAD>
+// Forward: the Categorical probabilities rewritten in place of the logits; the row's surr / kl / ent added to the sums.
+// CLIP: surr takes the clipped objective of the row (clip range eps) and s_clip counts the rows outside the range.
+template <int HEAD, bool CLIP = false>
 __device__ __forceinline__ void head_fwd_row(float* H, const float* aux, int r, int dL, bool valid, int reverse_kl,
                                              const float* sig, const float* logsig, double& s_surr, double& s_kl,
-                                             double& s_ent) {
+                                             double& s_ent, float eps, double& s_clip) {
   if (HEAD == MRL_HEAD_GAUSS) {
     if (aux) {
       const float adv = aux[0];
@@ -86,7 +106,8 @@ __device__ __forceinline__ void head_fwd_row(float* H, const float* aux, int r, 
         sls += logsig[j];
       }
       if (valid) {
-        s_surr += (double)(expf(dl) * adv);
+        if constexpr (CLIP) clip_row(expf(dl), adv, eps, s_surr, s_clip);
+        else s_surr += (double)(expf(dl) * adv);
         s_kl += (double)kl;
         s_ent += (double)(sls + 0.5f * MRL_LOG_2PIE * dL);
       }
@@ -114,7 +135,8 @@ __device__ __forceinline__ void head_fwd_row(float* H, const float* aux, int r, 
       }
     }
     if (aux && valid) {
-      s_surr += (double)((pa / p0a) * aux[0]);
+      if constexpr (CLIP) clip_row(pa / p0a, aux[0], eps, s_surr, s_clip);
+      else s_surr += (double)((pa / p0a) * aux[0]);
       s_kl += (double)kl;
       s_ent += (double)ent;
     }
@@ -125,11 +147,12 @@ __device__ __forceinline__ void head_fwd_row(float* H, const float* aux, int r, 
 
 // Backward, E holding the head's input rows.  Gradient mode: E = delta_L (un-normalised; 1/N is applied by the slab
 // reduce) and, DiagGauss, the logstd partial added to GL[j * MRL_TILE + r]; cs, ck = the coefficients of the surrogate
-// and the KL.  Fvp mode: E = Rz_L, replaced by the Fisher metric applied to it.  Padded timesteps give zeros.
+// and the KL.  Clipped-gradient mode: the same for the clipped objective (clip range eps), zeros for a gated row.
+// Fvp mode: E = Rz_L, replaced by the Fisher metric applied to it.  Padded timesteps give zeros.
 template <int HEAD, int MODE>
 __device__ __forceinline__ void head_bwd_row(const float* H, float* E, float* GL, const float* aux, int r, int dL,
                                              bool valid, int reverse_kl, float cs, float ck, const float* sig,
-                                             const float* ivar) {
+                                             const float* ivar, float eps = 0.f) {
   if (MODE == MRL_MODE_FVP) {
     if (HEAD == MRL_HEAD_GAUSS) {          // M = diag(1/sigma^2) on the mean block
       for (int j = 0; j < dL; ++j) E[j * MRL_LDT + r] = valid ? E[j * MRL_LDT + r] * ivar[j] : 0.f;
@@ -156,6 +179,15 @@ __device__ __forceinline__ void head_bwd_row(const float* H, float* E, float* GL
       const float s0 = aux[(1 + 2 * dL + j) * MRL_LDT];
       dl += gauss_logratio(mu, ac, m0, s0, sig[j]);
     }
+    if constexpr (MODE == MRL_MODE_GRAD_CLIP) {
+      const float rt = expf(dl);
+      if (clip_gated(rt, adv, eps)) {
+        for (int j = 0; j < dL; ++j) E[j * MRL_LDT + r] = 0.f;
+        return;
+      }
+      cs = 1.f;
+      ck = 0.f;
+    }
     const float w = -expf(dl) * adv * cs;
     for (int j = 0; j < dL; ++j) {
       const float mu = H[j * MRL_LDT + r];
@@ -171,6 +203,15 @@ __device__ __forceinline__ void head_bwd_row(const float* H, float* E, float* GL
     const float adv = aux[0];
     const int ai = (int)aux[1 * MRL_LDT];
     const float pa = H[ai * MRL_LDT + r], p0a = aux[(2 + ai) * MRL_LDT];
+    if constexpr (MODE == MRL_MODE_GRAD_CLIP) {
+      if (clip_gated(pa / p0a, adv, eps)) {
+        for (int j = 0; j < dL; ++j) E[j * MRL_LDT + r] = 0.f;
+        return;
+      }
+      cs = 1.f;
+      ck = 0.f;
+      reverse_kl = 0;
+    }
     const float w = -(pa / p0a) * adv * cs;
     float klrow = 0.f;
     if (reverse_kl)

@@ -63,19 +63,22 @@ struct MidBwdArgs {
   long long N;
   int n_tiles, slab_tiles, mode, reverse_kl;
 };
+// clip_eps (PPO clipped objective; a trailing kernel parameter, so that the argument layout of the other instances
+// stays as it is): forward, > 0: surr is the clipped objective with this clip range and loss slot 3 the count of
+// clipped rows; backward, the clip range of MRL_MODE_GRAD_CLIP.  Policy heads only.
 size_t mid_forward_smem(const NetGeom& g);
 size_t mid_backward_smem(const NetGeom& g, int mode);
-cudaError_t launch_mid_forward(const NetGeom& g, const MidFwdArgs& a, int n_slabs, cudaStream_t st);
-cudaError_t launch_mid_backward(const NetGeom& g, const MidBwdArgs& a, int n_slabs, cudaStream_t st);
+cudaError_t launch_mid_forward(const NetGeom& g, const MidFwdArgs& a, int n_slabs, cudaStream_t st, float clip_eps = 0.f);
+cudaError_t launch_mid_backward(const NetGeom& g, const MidBwdArgs& a, int n_slabs, cudaStream_t st, float clip_eps = 0.f);
 
 // ---- mlp_layers.cu  (layer-by-layer path for nets whose mid_* kernels do not fit in shared memory, L >= 2)
 // Same contract as launch_mid_*; R0 / R1: ping-pong buffers of layers_ws_floats each (deltas, R-activations).
 // *launches: kernels launched.
 size_t layers_ws_floats(const NetGeom& g, long long n_tiles);
 cudaError_t launch_layers_forward(const NetGeom& g, const MidFwdArgs& a /* cache required */, int n_slabs,
-                                  cudaStream_t st, int* launches);
+                                  cudaStream_t st, int* launches, float clip_eps = 0.f);
 cudaError_t launch_layers_backward(const NetGeom& g, const MidBwdArgs& a, float* R0, float* R1, int n_slabs,
-                                   cudaStream_t st, int* launches);
+                                   cudaStream_t st, int* launches, float clip_eps = 0.f);
 
 // ---- mlp_chain.cu  (register-resident per-warp chains for the forward and gradient passes)
 #define CH_WARPS 12          // backward chain: 12 warps x 16 timesteps = 3 cache tiles per pass
@@ -94,9 +97,10 @@ struct ChainEntry {
 };
 struct ChainJobs { ChainEntry e[CH_WARPS][CH_NE]; };
 int chain_bwd_shape(const NetGeom& g);   // 0: not covered by an instantiated chain shape
-cudaError_t launch_chain_backward(const NetGeom& g, const MidBwdArgs& a, int n_slabs, cudaStream_t st);   // gradient mode
+// gradient modes
+cudaError_t launch_chain_backward(const NetGeom& g, const MidBwdArgs& a, int n_slabs, cudaStream_t st, float clip_eps = 0.f);
 int chain_fwd_shape(const NetGeom& g);
-cudaError_t launch_chain_forward(const NetGeom& g, const MidFwdArgs& a, int n_slabs, cudaStream_t st);
+cudaError_t launch_chain_forward(const NetGeom& g, const MidFwdArgs& a, int n_slabs, cudaStream_t st, float clip_eps = 0.f);
 
 // ---- mlp_fvp_tc.cu  (tcgen05 / TMEM Fisher-vector chain of layers >= 2)
 struct FvpTcArgs {

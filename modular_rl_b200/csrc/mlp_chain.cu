@@ -187,17 +187,19 @@ __device__ __forceinline__ void epi_delta(const float (&acc)[NT][4], const float
 // dL/dz_L of the surrogate / penalised surrogate / squared error at the head (trpo.py:43, ppo.py:47-49,
 // core.py:613-617), un-normalised (1/N is applied by the slab reduce).  ho = cached head output (mean | probs |
 // value) in accumulator order; auxb = this warp's rows of the side inputs.  Also the logstd gradient partials.
-// The per-element terms are those of heads.cuh.
-template <int NT>
+// The per-element terms are those of heads.cuh.  CLIP: the PPO clipped objective (clip range eps), no KL term; a
+// gated row gives zeros.
+template <int NT, bool CLIP>
 __device__ __forceinline__ void head_grad(int head, const float (&ho)[NT][4], const float* __restrict__ auxb, int dL,
                                           const float* __restrict__ sig, const float* __restrict__ ivar, float cs,
                                           float ck, int reverse_kl, bool valid0, bool valid1, bool ok,
-                                          float (&gls)[NT][2], float (&d)[NT][4], int lane) {
+                                          float (&gls)[NT][2], float (&d)[NT][4], int lane, float eps) {
   const int t = lane & 3;
 #pragma unroll
   for (int n = 0; n < NT; ++n)
 #pragma unroll
     for (int i = 0; i < 4; ++i) d[n][i] = 0.f;
+  if constexpr (CLIP) { cs = 1.f; ck = 0.f; reverse_kl = 0; }
   if (head == MRL_HEAD_GAUSS) {
     const float adv0 = valid0 ? __ldg(auxb) : 0.f, adv1 = valid1 ? __ldg(auxb + 1) : 0.f;
     float ac[NT][4], m0[NT][4], s0[NT][4];
@@ -221,6 +223,10 @@ __device__ __forceinline__ void head_grad(int head, const float (&ho)[NT][4], co
     dl0 += __shfl_xor_sync(0xffffffffu, dl0, 1); dl0 += __shfl_xor_sync(0xffffffffu, dl0, 2);
     dl1 += __shfl_xor_sync(0xffffffffu, dl1, 1); dl1 += __shfl_xor_sync(0xffffffffu, dl1, 2);
     const float w0 = -expf(dl0) * adv0 * cs, w1 = -expf(dl1) * adv1 * cs;
+    if constexpr (CLIP) {   // a gated row takes no gradient
+      valid0 = valid0 && !clip_gated(expf(dl0), adv0, eps);
+      valid1 = valid1 && !clip_gated(expf(dl1), adv1, eps);
+    }
 #pragma unroll
     for (int n = 0; n < NT; ++n)
 #pragma unroll
@@ -259,6 +265,10 @@ __device__ __forceinline__ void head_grad(int head, const float (&ho)[NT][4], co
       kl0 += __shfl_xor_sync(0xffffffffu, kl0, o); kl1 += __shfl_xor_sync(0xffffffffu, kl1, o);
     }
     const float w0 = valid0 ? -(pa0 / qa0) * adv0 * cs : 0.f, w1 = valid1 ? -(pa1 / qa1) * adv1 * cs : 0.f;
+    if constexpr (CLIP) {
+      valid0 = valid0 && !clip_gated(pa0 / qa0, adv0, eps);
+      valid1 = valid1 && !clip_gated(pa1 / qa1, adv1, eps);
+    }
 #pragma unroll
     for (int n = 0; n < NT; ++n)
 #pragma unroll
@@ -400,8 +410,9 @@ __device__ __forceinline__ void grad_entry(float* __restrict__ Gs, const float* 
     *reinterpret_cast<float4*>(Gs + (q * 32 + lane) * 4) = make_float4(G[q][0], G[q][1], G[q][2], G[q][3]);
 }
 
-template <class S, int ACT>
-__global__ void __launch_bounds__(CH_THREADS, 1) chain_bwd_kernel(NetGeom g, MidBwdArgs a, ChainJobs jobs, int n_slabs) {
+template <class S, int ACT, int MODE>
+__global__ void __launch_bounds__(CH_THREADS, 1) chain_bwd_kernel(NetGeom g, MidBwdArgs a, ChainJobs jobs, int n_slabs,
+                                                                  float clip_eps) {
   constexpr int L = S::L;
   constexpr int N1 = S::nt(1), N2 = S::nt(2), N3 = S::nt(3);
   constexpr int NL = S::nt(L);
@@ -490,7 +501,8 @@ __global__ void __launch_bounds__(CH_THREADS, 1) chain_bwd_kernel(NetGeom g, Mid
       for (int n = 0; n < NL; ++n) ldfrag(ph[n], cb + g.off_act[L] * MRL_LDT, 8 * n + 2 * t, g.d[L], ok);
       float dL[NL][4];   // delta_L (accumulator order)
       const float* auxb = a.aux + (size_t)ctile * g.naux * MRL_LDT + rr;
-      head_grad<NL>(g.head, ph, auxb, g.d[L], sig, ivar, cs, ck, a.reverse_kl, valid0, valid1, ok, gls, dL, lane);
+      head_grad<NL, MODE == MRL_MODE_GRAD_CLIP>(g.head, ph, auxb, g.d[L], sig, ivar, cs, ck, a.reverse_kl, valid0, valid1,
+                                                ok, gls, dL, lane, clip_eps);
       // ---- reverse sweep
       bar_wait(&e_free, (tile_no & 1) ^ 1);   // the previous tile's grad phase has read its delta rows (passes at once for tile 0)
       store_E<NL>(E + (size_t)S::eoff(L) * CH_LDE, dL, warp, lane);
@@ -683,18 +695,23 @@ static bool shape_fits(const NetGeom& g) {
   return build_jobs<S>(g, &jobs);
 }
 
-template <class S>
-static cudaError_t launch_shape(const NetGeom& g, const MidBwdArgs& a, int n_slabs, cudaStream_t st) {
+template <class S, int MODE>
+static cudaError_t launch_shape_mode(const NetGeom& g, const MidBwdArgs& a, int n_slabs, cudaStream_t st, float eps) {
   ChainJobs jobs;
   if (!build_jobs<S>(g, &jobs)) return cudaErrorInvalidConfiguration;
   const size_t sm = S::smem_floats() * 4;
   {
-    cudaError_t e = mrl_func_smem((const void*)chain_bwd_kernel<S, MRL_ACT_TANH>, sm);
+    cudaError_t e = mrl_func_smem((const void*)chain_bwd_kernel<S, MRL_ACT_TANH, MODE>, sm);
     if (e != cudaSuccess) return e;
   }
   const int sms = mrl_sm_count();
-  chain_bwd_kernel<S, MRL_ACT_TANH><<<n_slabs < sms ? n_slabs : sms, CH_THREADS, sm, st>>>(g, a, jobs, n_slabs);
+  chain_bwd_kernel<S, MRL_ACT_TANH, MODE><<<n_slabs < sms ? n_slabs : sms, CH_THREADS, sm, st>>>(g, a, jobs, n_slabs, eps);
   return cudaGetLastError();
+}
+template <class S>
+static cudaError_t launch_shape(const NetGeom& g, const MidBwdArgs& a, int n_slabs, cudaStream_t st, float eps) {
+  if (a.mode == MRL_MODE_GRAD_CLIP) return launch_shape_mode<S, MRL_MODE_GRAD_CLIP>(g, a, n_slabs, st, eps);
+  return launch_shape_mode<S, MRL_MODE_GRAD>(g, a, n_slabs, st, eps);
 }
 
 typedef ChainShape<3, 8, 8, 1, 0> ShapeA;     // 64-64 hidden, <= 8 outputs  (Hopper, Walker2d, CartPole, value nets)
@@ -709,12 +726,12 @@ int chain_bwd_shape(const NetGeom& g) {
   return 0;
 }
 
-cudaError_t launch_chain_backward(const NetGeom& g, const MidBwdArgs& a, int n_slabs, cudaStream_t st) {
-  if (a.mode != MRL_MODE_GRAD) return cudaErrorInvalidValue;   // the chain computes gradients only
+cudaError_t launch_chain_backward(const NetGeom& g, const MidBwdArgs& a, int n_slabs, cudaStream_t st, float clip_eps) {
+  if (a.mode == MRL_MODE_FVP) return cudaErrorInvalidValue;   // the chain computes gradients only
   switch (chain_bwd_shape(g)) {
-    case 1: return launch_shape<ShapeA>(g, a, n_slabs, st);
-    case 2: return launch_shape<ShapeB>(g, a, n_slabs, st);
-    case 3: return launch_shape<ShapeC>(g, a, n_slabs, st);
+    case 1: return launch_shape<ShapeA>(g, a, n_slabs, st, clip_eps);
+    case 2: return launch_shape<ShapeB>(g, a, n_slabs, st, clip_eps);
+    case 3: return launch_shape<ShapeC>(g, a, n_slabs, st, clip_eps);
     default: return cudaErrorInvalidConfiguration;
   }
 }
@@ -752,11 +769,13 @@ __device__ __forceinline__ void fwd_layer(float (&acc)[NO][4], const uint32_t (&
 }
 
 // head of one warp's 16 timesteps: out = acc + b_L -> mean | softmax | value; losses; cache; row-major output
-template <int NT>
+// CLIP: surr takes the clipped objective (clip range eps), s_clip counts the rows outside the clip range
+template <int NT, bool CLIP>
 __device__ __forceinline__ void head_forward(int head, float (&o)[NT][4], const float* __restrict__ bl,
                                              const float* __restrict__ auxb, int dL, const float* __restrict__ sig,
                                              float ent_row, int reverse_kl, bool valid0, bool valid1, bool ok,
-                                             double& s_surr, double& s_kl, double& s_ent, int lane) {
+                                             double& s_surr, double& s_kl, double& s_ent, int lane, float eps,
+                                             double& s_clip) {
   const int t = lane & 3;
 #pragma unroll
   for (int n = 0; n < NT; ++n) {
@@ -788,8 +807,13 @@ __device__ __forceinline__ void head_forward(int head, float (&o)[NT][4], const 
       kl0 += __shfl_xor_sync(0xffffffffu, kl0, q); kl1 += __shfl_xor_sync(0xffffffffu, kl1, q);
     }
     if (t == 0) {
-      if (valid0) { s_surr += (double)(expf(dl0) * __ldg(auxb)); s_kl += (double)kl0; s_ent += (double)ent_row; }
-      if (valid1) { s_surr += (double)(expf(dl1) * __ldg(auxb + 1)); s_kl += (double)kl1; s_ent += (double)ent_row; }
+      if constexpr (CLIP) {
+        if (valid0) { clip_row(expf(dl0), __ldg(auxb), eps, s_surr, s_clip); s_kl += (double)kl0; s_ent += (double)ent_row; }
+        if (valid1) { clip_row(expf(dl1), __ldg(auxb + 1), eps, s_surr, s_clip); s_kl += (double)kl1; s_ent += (double)ent_row; }
+      } else {
+        if (valid0) { s_surr += (double)(expf(dl0) * __ldg(auxb)); s_kl += (double)kl0; s_ent += (double)ent_row; }
+        if (valid1) { s_surr += (double)(expf(dl1) * __ldg(auxb + 1)); s_kl += (double)kl1; s_ent += (double)ent_row; }
+      }
     }
   } else if (head == MRL_HEAD_CAT) {
     float m0_ = -INFINITY, m1_ = -INFINITY;
@@ -844,8 +868,13 @@ __device__ __forceinline__ void head_forward(int head, float (&o)[NT][4], const 
       en0 += __shfl_xor_sync(0xffffffffu, en0, q); en1 += __shfl_xor_sync(0xffffffffu, en1, q);
     }
     if (t == 0) {
-      if (valid0) { s_surr += (double)((pa0 / qa0) * __ldg(auxb)); s_kl += (double)kl0; s_ent += (double)en0; }
-      if (valid1) { s_surr += (double)((pa1 / qa1) * __ldg(auxb + 1)); s_kl += (double)kl1; s_ent += (double)en1; }
+      if constexpr (CLIP) {
+        if (valid0) { clip_row(pa0 / qa0, __ldg(auxb), eps, s_surr, s_clip); s_kl += (double)kl0; s_ent += (double)en0; }
+        if (valid1) { clip_row(pa1 / qa1, __ldg(auxb + 1), eps, s_surr, s_clip); s_kl += (double)kl1; s_ent += (double)en1; }
+      } else {
+        if (valid0) { s_surr += (double)((pa0 / qa0) * __ldg(auxb)); s_kl += (double)kl0; s_ent += (double)en0; }
+        if (valid1) { s_surr += (double)((pa1 / qa1) * __ldg(auxb + 1)); s_kl += (double)kl1; s_ent += (double)en1; }
+      }
     }
   } else {   // value head: squared error against the target row
     if (auxb != nullptr && t == 0) {
@@ -855,8 +884,8 @@ __device__ __forceinline__ void head_forward(int head, float (&o)[NT][4], const 
   }
 }
 
-template <class S, int ACT>
-__global__ void __launch_bounds__(FW_THREADS, 2) chain_fwd_kernel(NetGeom g, MidFwdArgs a, int n_slabs) {
+template <class S, int ACT, bool CLIP>
+__global__ void __launch_bounds__(FW_THREADS, 2) chain_fwd_kernel(NetGeom g, MidFwdArgs a, int n_slabs, float clip_eps) {
   constexpr int L = S::L;
   constexpr int N1 = S::nt(1), N2 = S::nt(2), N3 = S::nt(3);
   constexpr int NL = S::nt(L);
@@ -894,7 +923,7 @@ __global__ void __launch_bounds__(FW_THREADS, 2) chain_fwd_kernel(NetGeom g, Mid
 
   for (int slab = blockIdx.x; slab < n_slabs; slab += gridDim.x) {
     const int t0 = slab * a.slab_tiles, t1 = min(t0 + a.slab_tiles, a.n_tiles);
-    double s_surr = 0.0, s_kl = 0.0, s_ent = 0.0;
+    double s_surr = 0.0, s_kl = 0.0, s_ent = 0.0, s_clip = 0.0;
     for (int ct0 = t0; ct0 < t1; ct0 += 2) {
       const int ctile = ct0 + (warp >> 2);
       const bool ok = ctile < t1;
@@ -957,8 +986,8 @@ __global__ void __launch_bounds__(FW_THREADS, 2) chain_fwd_kernel(NetGeom g, Mid
         zero_acc(o);
         fwd_layer<N3, NL>(o, h3h, h3l, Ws + S::woff(4), lane);
       }
-      head_forward<NL>(g.head, o, bs + S::vboff(L), auxb, g.d[L], sig, ent_row, a.reverse_kl, valid0, valid1, ok,
-                       s_surr, s_kl, s_ent, lane);
+      head_forward<NL, CLIP>(g.head, o, bs + S::vboff(L), auxb, g.d[L], sig, ent_row, a.reverse_kl, valid0, valid1, ok,
+                             s_surr, s_kl, s_ent, lane, clip_eps, s_clip);
       if (cb) {
 #pragma unroll
         for (int n = 0; n < NL; ++n) st_cfrag(cb + g.off_act[L] * MRL_LDT, o[n], 8 * n + 2 * t, g.d[L], ok);
@@ -978,9 +1007,11 @@ __global__ void __launch_bounds__(FW_THREADS, 2) chain_fwd_kernel(NetGeom g, Mid
       double v0 = block_sum(s_surr, red);
       double v1 = block_sum(s_kl, red);
       double v2 = block_sum(s_ent, red);
+      double v3 = 0.0;
+      if constexpr (CLIP) v3 = block_sum(s_clip, red);
       if (tid == 0) {
         double* op = a.loss_part + (size_t)slab * 4;
-        op[0] = v0; op[1] = v1; op[2] = v2; op[3] = 0.0;
+        op[0] = v0; op[1] = v1; op[2] = v2; op[3] = v3;
       }
     }
   }
@@ -993,16 +1024,21 @@ static bool fwd_shape_fits(const NetGeom& g) {
     if ((g.d[l] + 7) / 8 > S::nt(l)) return false;
   return true;
 }
-template <class S>
-static cudaError_t launch_fwd_shape(const NetGeom& g, const MidFwdArgs& a, int n_slabs, cudaStream_t st) {
+template <class S, bool CLIP>
+static cudaError_t launch_fwd_shape_clip(const NetGeom& g, const MidFwdArgs& a, int n_slabs, cudaStream_t st, float eps) {
   const size_t sm = ((size_t)S::wfloats() + S::vbfloats() + 8 * S::nt(S::L)) * 4;
   {
-    cudaError_t e = mrl_func_smem((const void*)chain_fwd_kernel<S, MRL_ACT_TANH>, sm);
+    cudaError_t e = mrl_func_smem((const void*)chain_fwd_kernel<S, MRL_ACT_TANH, CLIP>, sm);
     if (e != cudaSuccess) return e;
   }
   const int sms = mrl_sm_count();
-  chain_fwd_kernel<S, MRL_ACT_TANH><<<n_slabs < 2 * sms ? n_slabs : 2 * sms, FW_THREADS, sm, st>>>(g, a, n_slabs);   // 2 CTAs per SM
+  chain_fwd_kernel<S, MRL_ACT_TANH, CLIP><<<n_slabs < 2 * sms ? n_slabs : 2 * sms, FW_THREADS, sm, st>>>(g, a, n_slabs, eps);   // 2 CTAs per SM
   return cudaGetLastError();
+}
+template <class S>
+static cudaError_t launch_fwd_shape(const NetGeom& g, const MidFwdArgs& a, int n_slabs, cudaStream_t st, float eps) {
+  if (eps > 0.f && g.head != MRL_HEAD_VALUE) return launch_fwd_shape_clip<S, true>(g, a, n_slabs, st, eps);
+  return launch_fwd_shape_clip<S, false>(g, a, n_slabs, st, eps);
 }
 int chain_fwd_shape(const NetGeom& g) {
   if (fwd_shape_fits<ShapeA>(g)) return 1;
@@ -1010,11 +1046,11 @@ int chain_fwd_shape(const NetGeom& g) {
   if (fwd_shape_fits<ShapeC>(g)) return 3;
   return 0;
 }
-cudaError_t launch_chain_forward(const NetGeom& g, const MidFwdArgs& a, int n_slabs, cudaStream_t st) {
+cudaError_t launch_chain_forward(const NetGeom& g, const MidFwdArgs& a, int n_slabs, cudaStream_t st, float clip_eps) {
   switch (chain_fwd_shape(g)) {
-    case 1: return launch_fwd_shape<ShapeA>(g, a, n_slabs, st);
-    case 2: return launch_fwd_shape<ShapeB>(g, a, n_slabs, st);
-    case 3: return launch_fwd_shape<ShapeC>(g, a, n_slabs, st);
+    case 1: return launch_fwd_shape<ShapeA>(g, a, n_slabs, st, clip_eps);
+    case 2: return launch_fwd_shape<ShapeB>(g, a, n_slabs, st, clip_eps);
+    case 3: return launch_fwd_shape<ShapeC>(g, a, n_slabs, st, clip_eps);
     default: return cudaErrorInvalidConfiguration;
   }
 }

@@ -227,8 +227,8 @@ __global__ void lw_dg_kernel(const float* __restrict__ D1, long long ldd, int n1
 }
 
 // ---- heads (heads.cuh): one thread per timestep, one CTA per slab; sigma, log sigma and 1/sigma^2 staged per CTA
-template <int HEAD>
-__global__ void __launch_bounds__(MRL_TILE, 1) lw_head_fwd_kernel(NetGeom g, MidFwdArgs a) {
+template <int HEAD, bool CLIP>
+__global__ void __launch_bounds__(MRL_TILE, 1) lw_head_fwd_kernel(NetGeom g, MidFwdArgs a, float clip_eps) {
   __shared__ double red[32];
   __shared__ float sig[MRL_MAX_DOUT], logsig[MRL_MAX_DOUT];
   const int r = threadIdx.x, L = g.L, dL = g.d[L];
@@ -240,12 +240,14 @@ __global__ void __launch_bounds__(MRL_TILE, 1) lw_head_fwd_kernel(NetGeom g, Mid
     sig[r] = expf(ls);
   }
   __syncthreads();
+  double s_clip = 0.0;   // declared first: the other instances' register assignment stays as it was
   double s_surr = 0.0, s_kl = 0.0, s_ent = 0.0;
   for (int tile = t0; tile < t1; ++tile) {
     const bool valid = (long long)tile * MRL_TILE + r < a.N;
     float* headbuf = a.cache + ((size_t)tile * g.act_rows + g.off_act[L]) * MRL_LDT;
     const float* aux = a.aux ? a.aux + (size_t)tile * g.naux * MRL_LDT + r : nullptr;
-    head_fwd_row<HEAD>(headbuf, aux, r, dL, valid, a.reverse_kl, sig, logsig, s_surr, s_kl, s_ent);
+    head_fwd_row<HEAD, CLIP>(headbuf, aux, r, dL, valid, a.reverse_kl, sig, logsig, s_surr, s_kl, s_ent, clip_eps,
+                             s_clip);
     if (a.head_out && valid)
       for (int j = 0; j < dL; ++j) a.head_out[((size_t)tile * MRL_TILE + r) * dL + j] = headbuf[j * MRL_LDT + r];
   }
@@ -253,22 +255,25 @@ __global__ void __launch_bounds__(MRL_TILE, 1) lw_head_fwd_kernel(NetGeom g, Mid
     const double v0 = block_sum(s_surr, red);
     const double v1 = block_sum(s_kl, red);
     const double v2 = block_sum(s_ent, red);
+    double v3 = 0.0;
+    if constexpr (CLIP) v3 = block_sum(s_clip, red);
     if (r == 0) {
       double* o = a.loss_part + (size_t)slab * 4;
-      o[0] = v0; o[1] = v1; o[2] = v2; o[3] = 0.0;
+      o[0] = v0; o[1] = v1; o[2] = v2; o[3] = v3;
     }
   }
 }
 
 // delta_L (Fvp: the metric applied to Rz_L) into E, the logstd partial (gradient mode, DiagGauss)
 template <int HEAD, int MODE>
-__global__ void __launch_bounds__(MRL_TILE, 1) lw_head_bwd_kernel(NetGeom g, MidBwdArgs a, float* E, long long lde) {
+__global__ void __launch_bounds__(MRL_TILE, 1) lw_head_bwd_kernel(NetGeom g, MidBwdArgs a, float* E, long long lde,
+                                                                float clip_eps) {
   __shared__ float GL[MRL_MAX_DOUT * MRL_TILE];
   __shared__ float sig[MRL_MAX_DOUT], ivar[MRL_MAX_DOUT];
   const int r = threadIdx.x, L = g.L, dL = g.d[L];
   const int slab = blockIdx.x;
   const int t0 = slab * a.slab_tiles, t1 = min(t0 + a.slab_tiles, a.n_tiles);
-  const bool gl_on = MODE == MRL_MODE_GRAD && HEAD == MRL_HEAD_GAUSS;
+  const bool gl_on = MODE != MRL_MODE_FVP && HEAD == MRL_HEAD_GAUSS;
   if (gl_on)
     for (int j = 0; j < dL; ++j) GL[j * MRL_TILE + r] = 0.f;
   if (HEAD == MRL_HEAD_GAUSS && r < dL) {
@@ -278,13 +283,14 @@ __global__ void __launch_bounds__(MRL_TILE, 1) lw_head_bwd_kernel(NetGeom g, Mid
   }
   __syncthreads();
   double c_s = 1.0, c_k = 0.0;
-  if (MODE == MRL_MODE_GRAD && a.coef) { c_s = a.coef[0]; c_k = a.coef[1]; }
+  if (MODE != MRL_MODE_FVP && a.coef) { c_s = a.coef[0]; c_k = a.coef[1]; }
   const float cs = (float)c_s, ck = (float)c_k;
   for (int tile = t0; tile < t1; ++tile) {
     const bool valid = (long long)tile * MRL_TILE + r < a.N;
     const float* Hh = a.cache + ((size_t)tile * g.act_rows + g.off_act[L]) * MRL_LDT;
     const float* aux = a.aux ? a.aux + (size_t)tile * g.naux * MRL_LDT + r : nullptr;
-    head_bwd_row<HEAD, MODE>(Hh, E + (size_t)tile * lde, GL, aux, r, dL, valid, a.reverse_kl, cs, ck, sig, ivar);
+    head_bwd_row<HEAD, MODE>(Hh, E + (size_t)tile * lde, GL, aux, r, dL, valid, a.reverse_kl, cs, ck, sig, ivar,
+                             clip_eps);
   }
   if (HEAD == MRL_HEAD_GAUSS) {   // logstd partial: the per-timestep columns summed (zero in Fvp mode)
     __syncthreads();
@@ -354,7 +360,8 @@ static cudaError_t layer1(const NetGeom& g, const float* Z, const float* b, cons
   } while (0)
 
 template <int HEAD, int ACT>
-static cudaError_t forward_t(const NetGeom& g, const MidFwdArgs& a, int n_slabs, cudaStream_t st, int* launches) {
+static cudaError_t forward_t(const NetGeom& g, const MidFwdArgs& a, int n_slabs, cudaStream_t st, int* launches,
+                             float eps) {
   const long long ldc = (long long)g.act_rows * MRL_LDT;
   LW_TRY(layer1<ACT>(g, a.Zt, a.img + g.off_b[1], nullptr, 0, a.cache, ldc, a.n_tiles, st));
   for (int l = 2; l <= g.L; ++l) {
@@ -366,14 +373,15 @@ static cudaError_t forward_t(const NetGeom& g, const MidFwdArgs& a, int n_slabs,
     p.n_tiles = a.n_tiles;
     LW_TRY(gemm<ACT>(p, st));
   }
-  lw_head_fwd_kernel<HEAD><<<n_slabs, MRL_TILE, 0, st>>>(g, a);
+  if (HEAD != MRL_HEAD_VALUE && eps > 0.f) lw_head_fwd_kernel<HEAD, HEAD != MRL_HEAD_VALUE><<<n_slabs, MRL_TILE, 0, st>>>(g, a, eps);
+  else lw_head_fwd_kernel<HEAD, false><<<n_slabs, MRL_TILE, 0, st>>>(g, a, eps);
   *launches = g.L + 1;
   return cudaGetLastError();
 }
 
 template <int HEAD, int ACT, int MODE>
 static cudaError_t backward_t(const NetGeom& g, const MidBwdArgs& a, float* R0, float* R1, int n_slabs,
-                              cudaStream_t st, int* launches) {
+                              cudaStream_t st, int* launches, float eps) {
   const long long ldc = (long long)g.act_rows * MRL_LDT, ldr = (long long)max_width(g) * MRL_LDT;
   const float* H = a.cache;
   float* cur = R0;
@@ -396,7 +404,7 @@ static cudaError_t backward_t(const NetGeom& g, const MidBwdArgs& a, float* R0, 
       float* s = cur; cur = nxt; nxt = s;
     }
   }
-  lw_head_bwd_kernel<HEAD, MODE><<<n_slabs, MRL_TILE, 0, st>>>(g, a, cur, ldr);
+  lw_head_bwd_kernel<HEAD, MODE><<<n_slabs, MRL_TILE, 0, st>>>(g, a, cur, ldr, eps);
   LW_TRY(cudaGetLastError());
   ++nl;
   for (int l = g.L; l >= 2; --l) {
@@ -436,12 +444,13 @@ static auto backward_fn(const NetGeom& g) {
   }
 }
 
-cudaError_t launch_layers_forward(const NetGeom& g, const MidFwdArgs& a, int n_slabs, cudaStream_t st, int* launches) {
+cudaError_t launch_layers_forward(const NetGeom& g, const MidFwdArgs& a, int n_slabs, cudaStream_t st, int* launches,
+                                  float clip_eps) {
   if (g.L < 2 || a.cache == nullptr) return cudaErrorInvalidValue;
   switch (g.head) {
-    case MRL_HEAD_GAUSS: return forward_fn<MRL_HEAD_GAUSS>(g)(g, a, n_slabs, st, launches);
-    case MRL_HEAD_CAT: return forward_fn<MRL_HEAD_CAT>(g)(g, a, n_slabs, st, launches);
-    default: return forward_fn<MRL_HEAD_VALUE>(g)(g, a, n_slabs, st, launches);
+    case MRL_HEAD_GAUSS: return forward_fn<MRL_HEAD_GAUSS>(g)(g, a, n_slabs, st, launches, clip_eps);
+    case MRL_HEAD_CAT: return forward_fn<MRL_HEAD_CAT>(g)(g, a, n_slabs, st, launches, clip_eps);
+    default: return forward_fn<MRL_HEAD_VALUE>(g)(g, a, n_slabs, st, launches, clip_eps);
   }
 }
 
@@ -449,14 +458,23 @@ template <int MODE>
 static cudaError_t backward_mode(const NetGeom& g, const MidBwdArgs& a, float* R0, float* R1, int n_slabs,
                                  cudaStream_t st, int* launches) {
   switch (g.head) {
-    case MRL_HEAD_GAUSS: return backward_fn<MRL_HEAD_GAUSS, MODE>(g)(g, a, R0, R1, n_slabs, st, launches);
-    case MRL_HEAD_CAT: return backward_fn<MRL_HEAD_CAT, MODE>(g)(g, a, R0, R1, n_slabs, st, launches);
-    default: return backward_fn<MRL_HEAD_VALUE, MODE>(g)(g, a, R0, R1, n_slabs, st, launches);
+    case MRL_HEAD_GAUSS: return backward_fn<MRL_HEAD_GAUSS, MODE>(g)(g, a, R0, R1, n_slabs, st, launches, 0.f);
+    case MRL_HEAD_CAT: return backward_fn<MRL_HEAD_CAT, MODE>(g)(g, a, R0, R1, n_slabs, st, launches, 0.f);
+    default: return backward_fn<MRL_HEAD_VALUE, MODE>(g)(g, a, R0, R1, n_slabs, st, launches, 0.f);
   }
 }
 cudaError_t launch_layers_backward(const NetGeom& g, const MidBwdArgs& a, float* R0, float* R1, int n_slabs,
-                                   cudaStream_t st, int* launches) {
+                                   cudaStream_t st, int* launches, float clip_eps) {
   if (g.L < 2 || a.DG == nullptr) return cudaErrorInvalidValue;
   if (a.mode == MRL_MODE_FVP) return backward_mode<MRL_MODE_FVP>(g, a, R0, R1, n_slabs, st, launches);
+  if (a.mode == MRL_MODE_GRAD_CLIP) {
+    switch (g.head) {   // a value net has no clipped objective
+      case MRL_HEAD_GAUSS:
+        return backward_fn<MRL_HEAD_GAUSS, MRL_MODE_GRAD_CLIP>(g)(g, a, R0, R1, n_slabs, st, launches, clip_eps);
+      case MRL_HEAD_CAT:
+        return backward_fn<MRL_HEAD_CAT, MRL_MODE_GRAD_CLIP>(g)(g, a, R0, R1, n_slabs, st, launches, clip_eps);
+      default: return cudaErrorInvalidValue;
+    }
+  }
   return backward_mode<MRL_MODE_GRAD>(g, a, R0, R1, n_slabs, st, launches);
 }

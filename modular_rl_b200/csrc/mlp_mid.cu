@@ -9,7 +9,9 @@
 //
 //   mid_forward_kernel : h1 = act(Z1+b1), ..., head -> surr/kl/ent (or MSE) sums, activation cache
 //                        trpo.py:37-42,60-63 ; core.py:339-365,402-438 ; core.py:613-617
+//                        <CLIP>: the PPO clipped objective for surr, the clipped-row count in loss slot 3
 //   mid_backward_kernel<GRAD> : dL/dz_L from the head, reverse sweep         trpo.py:43, ppo.py:47-49
+//   mid_backward_kernel<GRAD_CLIP> : the same for the PPO clipped objective
 //   mid_backward_kernel<FVP>  : R-forward (Pearlmutter), Fisher metric, reverse sweep  trpo.py:45-58
 #include "common.cuh"
 #include "heads.cuh"
@@ -148,8 +150,8 @@ __device__ __forceinline__ void copy_f4(float* dst, const float* src, int nfloat
 }
 
 // =====================================================================================
-template <int HEAD, int ACT>
-__global__ void __launch_bounds__(MRL_MID_THREADS, 1) mid_forward_kernel(NetGeom g, MidFwdArgs a) {
+template <int HEAD, int ACT, bool CLIP>
+__global__ void __launch_bounds__(MRL_MID_THREADS, 1) mid_forward_kernel(NetGeom g, MidFwdArgs a, float clip_eps) {
   extern __shared__ __align__(16) float smem[];
   float* img = smem;
   float* act = img + g.bw_floats;
@@ -168,7 +170,7 @@ __global__ void __launch_bounds__(MRL_MID_THREADS, 1) mid_forward_kernel(NetGeom
     logsig[tid] = ls;
     sig[tid] = expf(ls);
   }
-  double s_surr = 0.0, s_kl = 0.0, s_ent = 0.0;
+  double s_surr = 0.0, s_kl = 0.0, s_ent = 0.0, s_clip = 0.0;
   float* headbuf = act + g.off_act[L] * MRL_LDT;
 
   for (int tile = t0; tile < t1; ++tile) {
@@ -212,7 +214,8 @@ __global__ void __launch_bounds__(MRL_MID_THREADS, 1) mid_forward_kernel(NetGeom
     // ---- head: one thread per timestep
     if (tid < MRL_TILE) {
       const float* aux = a.aux ? a.aux + (size_t)tile * g.naux * MRL_LDT + tid : nullptr;
-      head_fwd_row<HEAD>(headbuf, aux, tid, dL, tid < nvalid, a.reverse_kl, sig, logsig, s_surr, s_kl, s_ent);
+      head_fwd_row<HEAD, CLIP>(headbuf, aux, tid, dL, tid < nvalid, a.reverse_kl, sig, logsig, s_surr, s_kl, s_ent,
+                               clip_eps, s_clip);
     }
     __syncthreads();
     if (a.cache) copy_f4(a.cache + (size_t)tile * g.act_rows * MRL_LDT, act, g.act_rows * MRL_LDT);
@@ -228,22 +231,24 @@ __global__ void __launch_bounds__(MRL_MID_THREADS, 1) mid_forward_kernel(NetGeom
     double v0 = block_sum(s_surr, red);
     double v1 = block_sum(s_kl, red);
     double v2 = block_sum(s_ent, red);
+    double v3 = 0.0;
+    if constexpr (CLIP) v3 = block_sum(s_clip, red);
     if (tid == 0) {
       double* o = a.loss_part + (size_t)slab * 4;
-      o[0] = v0; o[1] = v1; o[2] = v2; o[3] = 0.0;
+      o[0] = v0; o[1] = v1; o[2] = v2; o[3] = v3;
     }
   }
 }
 
 // =====================================================================================
 template <int HEAD, int ACT, int MODE>
-__global__ void __launch_bounds__(MRL_BWD_THREADS, 1) mid_backward_kernel(NetGeom g, MidBwdArgs a) {
+__global__ void __launch_bounds__(MRL_BWD_THREADS, 1) mid_backward_kernel(NetGeom g, MidBwdArgs a, float clip_eps) {
   extern __shared__ __align__(16) float smem[];
   float* img = smem;
   float* imgv = img + g.img_floats;
   float* G = imgv + (MODE == MRL_MODE_FVP ? g.bw_floats : 0);
   float* GL = G + g.bw_floats;
-  const int gl_floats = (MODE == MRL_MODE_GRAD && HEAD == MRL_HEAD_GAUSS) ? g.d[g.L] * MRL_TILE : 0;
+  const int gl_floats = (MODE != MRL_MODE_FVP && HEAD == MRL_HEAD_GAUSS) ? g.d[g.L] * MRL_TILE : 0;
   float* H = GL + gl_floats;
   float* E = H + g.act_rows * MRL_LDT;
   __shared__ float sig[MRL_MAX_DOUT], ivar[MRL_MAX_DOUT];
@@ -264,7 +269,7 @@ __global__ void __launch_bounds__(MRL_BWD_THREADS, 1) mid_backward_kernel(NetGeo
     ivar[tid] = expf(-2.f * ls);
   }
   double c_s = 1.0, c_k = 0.0;
-  if (MODE == MRL_MODE_GRAD && a.coef) { c_s = a.coef[0]; c_k = a.coef[1]; }
+  if (MODE != MRL_MODE_FVP && a.coef) { c_s = a.coef[0]; c_k = a.coef[1]; }
   const float cs = (float)c_s, ck = (float)c_k;
   float* Hh = H + g.off_act[L] * MRL_LDT;   // cached head output (mean | probs | value)
   float* EH = E + g.off_act[L] * MRL_LDT;   // Rz_L, then delta_L
@@ -328,7 +333,7 @@ __global__ void __launch_bounds__(MRL_BWD_THREADS, 1) mid_backward_kernel(NetGeo
     const bool head_folded = (MODE == MRL_MODE_FVP && HEAD == MRL_HEAD_GAUSS && L > 1);
     if (!head_folded && tid < MRL_TILE) {
       const float* aux = a.aux ? a.aux + (size_t)tile * g.naux * MRL_LDT + tid : nullptr;
-      head_bwd_row<HEAD, MODE>(Hh, EH, GL, aux, tid, dL, tid < nvalid, a.reverse_kl, cs, ck, sig, ivar);
+      head_bwd_row<HEAD, MODE>(Hh, EH, GL, aux, tid, dL, tid < nvalid, a.reverse_kl, cs, ck, sig, ivar, clip_eps);
     }
     if (!head_folded) __syncthreads();
     // ---- reverse sweep: layers L..2 (weights in shared memory)
@@ -390,26 +395,33 @@ size_t mid_forward_smem(const NetGeom& g) { return ((size_t)g.bw_floats + (size_
 size_t mid_backward_smem(const NetGeom& g, int mode) {
   size_t f = (size_t)g.img_floats + g.bw_floats + 2 * (size_t)g.act_rows * MRL_LDT;
   if (mode == MRL_MODE_FVP) f += g.bw_floats;
-  if (mode == MRL_MODE_GRAD && g.head == MRL_HEAD_GAUSS) f += (size_t)g.d[g.L] * MRL_TILE;
+  if (mode != MRL_MODE_FVP && g.head == MRL_HEAD_GAUSS) f += (size_t)g.d[g.L] * MRL_TILE;
   return f * 4;
 }
 
-template <int HEAD, int ACT>
-static cudaError_t launch_fwd_t(const NetGeom& g, const MidFwdArgs& a, int n_slabs, cudaStream_t st) {
+template <int HEAD, int ACT, bool CLIP>
+static cudaError_t launch_fwd_clip(const NetGeom& g, const MidFwdArgs& a, int n_slabs, cudaStream_t st, float eps) {
   const size_t sm = mid_forward_smem(g);
-  cudaError_t e = cudaFuncSetAttribute(mid_forward_kernel<HEAD, ACT>,
+  cudaError_t e = cudaFuncSetAttribute(mid_forward_kernel<HEAD, ACT, CLIP>,
                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
   if (e != cudaSuccess) return e;
-  mid_forward_kernel<HEAD, ACT><<<n_slabs, MRL_MID_THREADS, sm, st>>>(g, a);
+  mid_forward_kernel<HEAD, ACT, CLIP><<<n_slabs, MRL_MID_THREADS, sm, st>>>(g, a, eps);
   return cudaGetLastError();
 }
+template <int HEAD, int ACT>
+static cudaError_t launch_fwd_t(const NetGeom& g, const MidFwdArgs& a, int n_slabs, cudaStream_t st, float eps) {
+  if constexpr (HEAD != MRL_HEAD_VALUE) {
+    if (eps > 0.f) return launch_fwd_clip<HEAD, ACT, true>(g, a, n_slabs, st, eps);
+  }
+  return launch_fwd_clip<HEAD, ACT, false>(g, a, n_slabs, st, eps);
+}
 template <int HEAD, int ACT, int MODE>
-static cudaError_t launch_bwd_t(const NetGeom& g, const MidBwdArgs& a, int n_slabs, cudaStream_t st) {
+static cudaError_t launch_bwd_t(const NetGeom& g, const MidBwdArgs& a, int n_slabs, cudaStream_t st, float eps) {
   const size_t sm = mid_backward_smem(g, MODE);
   cudaError_t e = cudaFuncSetAttribute(mid_backward_kernel<HEAD, ACT, MODE>,
                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm);
   if (e != cudaSuccess) return e;
-  mid_backward_kernel<HEAD, ACT, MODE><<<n_slabs, MRL_BWD_THREADS, sm, st>>>(g, a);
+  mid_backward_kernel<HEAD, ACT, MODE><<<n_slabs, MRL_BWD_THREADS, sm, st>>>(g, a, eps);
   return cudaGetLastError();
 }
 
@@ -420,24 +432,28 @@ static cudaError_t launch_bwd_t(const NetGeom& g, const MidBwdArgs& a, int n_sla
     default: return FN<HEADV, MRL_ACT_SIGMOID>(__VA_ARGS__);             \
   }
 
-cudaError_t launch_mid_forward(const NetGeom& g, const MidFwdArgs& a, int n_slabs, cudaStream_t st) {
+cudaError_t launch_mid_forward(const NetGeom& g, const MidFwdArgs& a, int n_slabs, cudaStream_t st, float clip_eps) {
   switch (g.head) {
-    case MRL_HEAD_GAUSS: DISPATCH_ACT(launch_fwd_t, MRL_HEAD_GAUSS, g, a, n_slabs, st)
-    case MRL_HEAD_CAT: DISPATCH_ACT(launch_fwd_t, MRL_HEAD_CAT, g, a, n_slabs, st)
-    default: DISPATCH_ACT(launch_fwd_t, MRL_HEAD_VALUE, g, a, n_slabs, st)
+    case MRL_HEAD_GAUSS: DISPATCH_ACT(launch_fwd_t, MRL_HEAD_GAUSS, g, a, n_slabs, st, clip_eps)
+    case MRL_HEAD_CAT: DISPATCH_ACT(launch_fwd_t, MRL_HEAD_CAT, g, a, n_slabs, st, clip_eps)
+    default: DISPATCH_ACT(launch_fwd_t, MRL_HEAD_VALUE, g, a, n_slabs, st, clip_eps)
   }
 }
 
 template <int HEAD, int ACT>
-static cudaError_t launch_bwd_mode(const NetGeom& g, const MidBwdArgs& a, int n_slabs, cudaStream_t st) {
-  if (a.mode == MRL_MODE_FVP) return launch_bwd_t<HEAD, ACT, MRL_MODE_FVP>(g, a, n_slabs, st);
-  return launch_bwd_t<HEAD, ACT, MRL_MODE_GRAD>(g, a, n_slabs, st);
+static cudaError_t launch_bwd_mode(const NetGeom& g, const MidBwdArgs& a, int n_slabs, cudaStream_t st, float eps) {
+  if (a.mode == MRL_MODE_FVP) return launch_bwd_t<HEAD, ACT, MRL_MODE_FVP>(g, a, n_slabs, st, eps);
+  if (a.mode == MRL_MODE_GRAD_CLIP) {
+    if constexpr (HEAD != MRL_HEAD_VALUE) return launch_bwd_t<HEAD, ACT, MRL_MODE_GRAD_CLIP>(g, a, n_slabs, st, eps);
+    return cudaErrorInvalidValue;   // a value net has no clipped objective
+  }
+  return launch_bwd_t<HEAD, ACT, MRL_MODE_GRAD>(g, a, n_slabs, st, eps);
 }
 
-cudaError_t launch_mid_backward(const NetGeom& g, const MidBwdArgs& a, int n_slabs, cudaStream_t st) {
+cudaError_t launch_mid_backward(const NetGeom& g, const MidBwdArgs& a, int n_slabs, cudaStream_t st, float clip_eps) {
   switch (g.head) {
-    case MRL_HEAD_GAUSS: DISPATCH_ACT(launch_bwd_mode, MRL_HEAD_GAUSS, g, a, n_slabs, st)
-    case MRL_HEAD_CAT: DISPATCH_ACT(launch_bwd_mode, MRL_HEAD_CAT, g, a, n_slabs, st)
-    default: DISPATCH_ACT(launch_bwd_mode, MRL_HEAD_VALUE, g, a, n_slabs, st)
+    case MRL_HEAD_GAUSS: DISPATCH_ACT(launch_bwd_mode, MRL_HEAD_GAUSS, g, a, n_slabs, st, clip_eps)
+    case MRL_HEAD_CAT: DISPATCH_ACT(launch_bwd_mode, MRL_HEAD_CAT, g, a, n_slabs, st, clip_eps)
+    default: DISPATCH_ACT(launch_bwd_mode, MRL_HEAD_VALUE, g, a, n_slabs, st, clip_eps)
   }
 }

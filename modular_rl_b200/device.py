@@ -305,6 +305,21 @@ class DeviceNet:
     def adam_reset(self, stream=None):
         L.check(L.lib().mrl_net_adam_reset(self._h, stream))
 
+    def ppo_clip_lossgrad(self, batch: DeviceBatch, clip_eps, want_grad=True, stream=None):
+        """PPO clipped surrogate on the whole batch -> (gradient float64 [P] or None, [surr, kl, ent, clipfrac])."""
+        g = np.empty(self.P, np.float64) if want_grad else None
+        ls = np.zeros(4, np.float64)
+        L.check(L.lib().mrl_net_ppo_clip_lossgrad(self._h, batch._h, float(clip_eps), L.ptr(g), L.ptr(ls), stream))
+        return g, ls
+
+    def ppo_clip_sgd_step(self, minibatch: DeviceBatch, clip_eps, stepsize, beta1=0.9, beta2=0.999, epsilon=1e-8,
+                          stream=None):
+        """One PPO-clip minibatch step on the device: clipped gradient, Adam step (the moments of ppo_sgd_step),
+        no host sync."""
+        self.theta_version += 1
+        L.check(L.lib().mrl_net_ppo_clip_sgd_step(self._h, minibatch._h, float(clip_eps), float(stepsize), float(beta1),
+                                                  float(beta2), float(epsilon), stream))
+
     def vf_lossgrad(self, batch: DeviceBatch, l2coeff=1e-3, want_grad=True, stream=None):
         ls = np.zeros(3, np.float64)
         g = np.empty(self.P, np.float64) if want_grad else None

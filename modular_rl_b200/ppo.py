@@ -9,6 +9,9 @@ coefficient of the KL term is computed from the batch-wide KL without a host rou
 PpoSgdUpdater (ppo.py:115-258, SURVEY 8f rank 2) reuses the same device loss/gradient entry point on
 minibatches of 128 gathered rows; Adam (adam_updates, ppo.py:231-258) runs on the host in float32 like the
 reference's floatX shared variables.
+
+PpoClipUpdater is PPO with the clipped surrogate objective, -(1/N) sum min(r A, clip(r, 1-eps, 1+eps) A): epochs of
+shuffled minibatches, each one device call (mrl_net_ppo_clip_sgd_step) with the float32 Adam of PpoSgdUpdater.
 """
 from collections import OrderedDict
 
@@ -107,6 +110,70 @@ class PpoLbfgsUpdater(EzFlat, EzPickle):
                 info["test_" + name + "_before"] = lossbefore
                 info["test_" + name + "_after"] = lossafter
                 info["test_" + name + "_change"] = lossafter - lossbefore
+        return info
+
+
+class PpoClipUpdater(EzFlat, EzPickle):
+    """PPO with the clipped surrogate objective.  Per call: the old policy is the current one (one forward pass gives
+    its prob rows, as PpoSgdUpdater); the batch is bound once; each epoch draws np.random.permutation(N) from numpy's
+    global generator, uploads it once, and runs one device step per minibatch of `minibatch_size` rows gathered from
+    it (the last, shorter one included).  Adam's moments live on the device and persist across calls (a snapshot
+    restarts them).  The info dict holds surr / kl / ent before and after the update, their change, and clipfrac
+    (the fraction of rows whose ratio is outside [1 - clip_param, 1 + clip_param]) after it."""
+
+    options = [
+        ("clip_param", float, 0.2, "Clip range eps of the ratio pi/pi_old: [1 - eps, 1 + eps]"),
+        ("epochs", int, 10, "Passes over the batch per update"),
+        ("stepsize", float, 3e-4, "Adam step size"),
+        ("minibatch_size", int, 64, "Timesteps per minibatch"),
+    ]
+
+    def __init__(self, stochpol, usercfg):
+        EzPickle.__init__(self, stochpol, usercfg)
+        cfg = update_default_config(self.options, usercfg)
+        print("PPOClipUpdater", cfg)
+        if not cfg["clip_param"] > 0:
+            raise ValueError("clip_param must be > 0, got %r" % (cfg["clip_param"],))
+        if cfg["minibatch_size"] < 1 or cfg["epochs"] < 0:
+            raise ValueError("minibatch_size must be >= 1 and epochs >= 0")
+        self.stochpol = stochpol
+        self.cfg = cfg
+        EzFlat.__init__(self, stochpol.net)
+        self.loss_names = ["surr", "kl", "ent"]
+        self._full = DeviceBatch(stochpol.dims[0], with_time_feature=True)
+        self._mb = DeviceBatch(stochpol.dims[0], with_time_feature=True)
+        stochpol.net.adam_reset()
+
+    def __call__(self, paths):
+        import torch
+        cfg = self.cfg
+        net = self.stochpol.net
+        eps, mb = cfg["clip_param"], cfg["minibatch_size"]
+        ob_no = concat([path["observation"] for path in paths])
+        action_na = concat([path["action"] for path in paths])
+        advantage_n = concat([path["advantage"] for path in paths])
+        ob_no = np.asarray(ob_no).reshape(len(ob_no), -1)
+        N = ob_no.shape[0]
+        head, dout = self.stochpol.probtype.head, self.stochpol.dims[-1]
+
+        self._full.set_obs(ob_no)
+        oldprob_np = self.stochpol.output_from_head(net.forward(self._full))
+        self._full.set_policy_inputs(head, dout, action_na, advantage_n, oldprob_np)
+
+        _, before = net.ppo_clip_lossgrad(self._full, eps, want_grad=False)
+        dev = torch.device("cuda", net.device)
+        for _ in range(cfg["epochs"]):
+            perm = torch.from_numpy(np.random.permutation(N).astype(np.int32)).to(dev)
+            for istart in range(0, N, mb):
+                net.ppo_clip_sgd_step(self._mb.gather_from(self._full, perm[istart:istart + mb]), eps, cfg["stepsize"])
+        _, after = net.ppo_clip_lossgrad(self._full, eps, want_grad=False)
+
+        info = OrderedDict()
+        for (name, lossbefore, lossafter) in zipsame(self.loss_names, before[:3], after[:3]):
+            info[name + "_before"] = lossbefore
+            info[name + "_after"] = lossafter
+            info[name + "_change"] = lossafter - lossbefore
+        info["clipfrac"] = after[3]
         return info
 
 
